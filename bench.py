@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the LiteralKG message-passing + scoring hot path on B200 (contract: see README / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole synthetic graph of BASELINE.json configs[2]
 (N = 1 M entities, E = 20 M triples, R = 64 relations, D = 300, C = 32, L = 3 bi-interaction layers,
@@ -56,7 +56,16 @@ def parse():
                     help="BASELINE.json workload: 3 = 1M / 20M bi-interaction (the metric's config, default); "
                          "5-gcn / 5-graphsage / 5-bi = 10M / 200M aggregator comparison; the per-stage extras "
                          "(scoring = cfg 4, training) ride along with cfg 3")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of what the last timed step computed (entity "
+                         "embeddings and the attention matrix A_in) to DIR/<name>.npy, for comparing two builds; "
+                         "with several ranks, rank 0 writes a sample of its own shard (its head rows), so compare "
+                         "dumps taken with the same number of GPUs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     for k_, v_ in CONFIGS[a.config].items():
         setattr(a, k_, v_)
     return a
@@ -274,6 +283,29 @@ def algorithmic_bytes(n, e, nnz, r, d, c, layers, bi=True):
     return {"attn_update": att, f"aggregate_d{d}": l1, f"aggregate_d{c}": lk}
 
 
+DUMP_EMBEDDING_BYTES = 32 << 20     # sampled embedding rows fill at most 32 MB
+DUMP_ATTENTION_ENTRIES = 1 << 20    # sampled A_in entries: 4 MB of values + 16 MB of (head, tail) ids
+
+
+def dump_outputs(out_dir, emb, a_in, row0):
+    """Writes a seeded sample of one pass's outputs (at most ~52 MB) as float32 / float64 .npy files:
+    embeddings [S, G] float32 (rows of gat_embeddings) with embedding_rows [S] (their entity ids), attention_values [M]
+    float32 (A_in entries, coalesced order) with attention_indices [2, M] (their head and tail ids).  Ids are stored as
+    float64, which holds them exactly.  The sample depends on the output shapes only, so two builds run with the same
+    arguments are compared entry for entry.  Row partitioned, ``emb`` and ``a_in`` hold only this rank's head rows
+    (``row0``: entity id of ``emb``'s first row), so the sample is of the shard and differs from a one-GPU dump."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows, width = emb.shape
+    pick = np.sort(np.random.default_rng(0).choice(rows, min(rows, DUMP_EMBEDDING_BYTES // (4 * width)), replace=False))
+    nnz = a_in._nnz()
+    apick = np.sort(np.random.default_rng(1).choice(nnz, min(nnz, DUMP_ATTENTION_ENTRIES), replace=False))
+    pick, apick = (torch.from_numpy(x).to(emb.device) for x in (pick, apick))
+    arrays = {"embeddings": emb[pick].float(), "embedding_rows": (pick + row0).double(),
+              "attention_values": a_in._values()[apick].float(), "attention_indices": a_in._indices()[:, apick].double()}
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x.cpu().numpy())
+
+
 @torch.no_grad()
 def run_ours(a):
     import torch.distributed as dist
@@ -361,6 +393,8 @@ def run_ours(a):
         host_issue_ms = (time.perf_counter() - t_host) * 1e3 / a.steps     # time to enqueue a pass (no sync inside)
         sync()
     ms = start.elapsed_time(end) / a.steps
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, emb, model.A_in.data, 0 if part is None else part.begin)
     prof = ops.PROFILE
     kern = prof.summary()
     for v_ in kern.values():

@@ -11,7 +11,7 @@ reference's algorithm for the path named in BASELINE.json.  Every function cites
 Pinning: the reference ships no tests or golden vectors (SURVEY.md section 4).  This oracle is pinned
 against the *reference itself*, imported unmodified in the build container by
 ``oracle/make_golden.py``; the resulting vectors live in ``tests/golden/*.npz`` and are checked by
-``tests/test_oracle_golden.py`` (and, when ``/root/reference`` is present, against the live reference
+``tests/test_oracle_golden.py`` (and, when ``LKG_REFERENCE`` names a checkout, against the live reference
 classes in ``tests/test_oracle_vs_reference.py``).
 
 Parameters are passed as a plain ``dict`` whose keys are the reference's ``state_dict`` names

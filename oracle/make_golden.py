@@ -1,8 +1,7 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference).
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from the checkout of the original
+NSLab-CUK/LiteralKG that LKG_REFERENCE names):
 
-Run in the build container only (the GPU box has no /root/reference):
-
-    python oracle/make_golden.py            # writes tests/golden/<case>.npz
+    LKG_REFERENCE=<checkout> python oracle/make_golden.py            # writes tests/golden/<case>.npz
 
 Each file holds the inputs (config, state dict, literal tables, triples) and the reference's own
 outputs for every stage of the hot path: initial Laplacian A_in (dataloader.py:449-495), attention
@@ -25,7 +24,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get("LKG_REFERENCE", "/root/reference")
+REF = os.environ.get("LKG_REFERENCE", "")
 sys.path.insert(0, HERE)
 from literalkg_oracle import OracleConfig  # noqa: E402
 
@@ -288,4 +287,6 @@ def main():
 
 
 if __name__ == "__main__":
+    if not REF:
+        sys.exit("set LKG_REFERENCE to a checkout of the original NSLab-CUK/LiteralKG")
     main()

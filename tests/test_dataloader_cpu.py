@@ -8,7 +8,9 @@ import pytest
 import literalkg_oracle as O
 from literalkg_b200 import dataloader as D
 
-REF_DATA = os.path.join(os.environ.get("LKG_REFERENCE", "/root/reference"), "data", "Test")
+REF = os.environ.get("LKG_REFERENCE", "")         # a checkout of the original NSLab-CUK/LiteralKG, where available
+REF_DATA = os.path.join(REF, "data", "Test")
+NO_REF = "LKG_REFERENCE names no checkout of the original LiteralKG"
 
 
 def _write(tmp_path, name, text):
@@ -48,8 +50,7 @@ def test_numeric_literals_match_the_oracle(tmp_path):
     assert table[2, 0] == 0 and table[2, 1] == np.float32(11.0 / 40.0)     # the later file resets the whole row
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_DATA, "pre_training_train.txt")),
-                    reason="reference checkout not mounted")
+@pytest.mark.skipif(not REF or not os.path.exists(os.path.join(REF_DATA, "pre_training_train.txt")), reason=NO_REF)
 def test_bundled_reference_data_dir():
     path = os.path.join(REF_DATA, "pre_training_train.txt")
     got = D.read_triples(path)
@@ -98,8 +99,7 @@ def test_data_dir_with_text_pickles(tmp_path):
     assert none_num is None and txt_only.shape == (41, 6) and np.allclose(txt_only[40], cc[40])
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(os.environ.get("LKG_REFERENCE", "/root/reference"), "dataloader.py")),
-                    reason="reference checkout not mounted")
+@pytest.mark.skipif(not REF or not os.path.exists(os.path.join(REF, "dataloader.py")), reason=NO_REF)
 @pytest.mark.parametrize("use_num,use_txt", [(True, True), (True, False), (False, True)])
 def test_data_dir_matches_the_reference_loader(tmp_path, use_num, use_txt):
     """The reference's own load_attributes / construct_data / embed_*_literal (dataloader.py:111-152, 369-438) run on a
@@ -107,9 +107,8 @@ def test_data_dir_matches_the_reference_loader(tmp_path, use_num, use_txt):
     import argparse
     import sys
     import torch
-    ref_root = os.environ.get("LKG_REFERENCE", "/root/reference")
-    if ref_root not in sys.path:
-        sys.path.insert(0, ref_root)
+    if REF not in sys.path:
+        sys.path.insert(0, REF)
     import dataloader as ref_dl
     rng = np.random.default_rng(7)
     _make_dir(tmp_path, rng)
