@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define LKG_ABI_VERSION 5
+#define LKG_ABI_VERSION 6
 
 typedef enum {
     LKG_OK = 0,
@@ -446,6 +446,22 @@ int lkg_rank_finalize(const float* emb, int64_t ld_emb, const int64_t* tail_rows
                       int64_t ld_head_emb, const int64_t* head_rows, const int64_t* target_pos, const float* tau,
                       const int32_t* above, const int32_t* band_cnt, const int32_t* band, int32_t band_cap,
                       int64_t n_heads, int64_t n_tails, int32_t dim, int64_t* ranks, void* stream);
+/* ---- filtered rank (link-prediction evaluation): ranks[i] -= #{ f in F(i) that beat the target } --------------------
+ * Query i = (heads[i], rels[i], target at candidate position target_pos[i]).  F(i) = the distinct tails t' of the known
+ * triples (heads[i], rels[i], t') taken from the att order of `known` (rels NULL or rels[i] < 0: of any relation, from
+ * its agg order); the target itself and entities without a candidate position are skipped.  cand_map (nullable) int32
+ * [known->n_entities]: candidate position of an entity, -1 = not a candidate; NULL = the identity.  heads in
+ * [0, known->n_entities).  Applied in place to the raw ranks, on the scores those ranks were counted on:
+ *   lkg_rank_filter         after lkg_rank_finalize: tau = its target scores; emb [*, ld_emb] the matrix holding both the
+ *                           head rows (heads[i]) and the candidate rows (entity f = row f); f is re-scored with the
+ *                           finalize kernel's exact dot product, so a tail is subtracted exactly when finalize counted it;
+ *   lkg_rank_filter_scores  after lkg_topk_rows: scores [n_queries, n_cols] the matrix whose row i was ranked. */
+int lkg_rank_filter(const lkg_graph* known, const int64_t* heads, const int64_t* rels /*nullable*/,
+                    const int32_t* cand_map /*nullable*/, const int64_t* target_pos, int64_t n_queries, const float* emb,
+                    int64_t ld_emb, int32_t dim, const float* tau, int64_t* ranks, void* stream);
+int lkg_rank_filter_scores(const lkg_graph* known, const int64_t* heads, const int64_t* rels /*nullable*/,
+                           const int32_t* cand_map /*nullable*/, const int64_t* target_pos, int64_t n_queries,
+                           const float* scores, int64_t ld_scores, int64_t n_cols, int64_t* ranks, void* stream);
 int lkg_score_topk_workspace_bytes(int64_t n_heads, int32_t cap, int32_t sample_tiles, size_t* bytes /*host out*/);
 /* Per head the k best tails by emb[head] . emb[tail]: larger score first, ties -> lower position in the tail
  * list; values are the exact dot products (fp32 products summed in fp64, rounded once).

@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_PKG, "liblkg.so")
 
 LKG_MAX_SEGMENTS = 4
 LKG_SCALE_FLOATS = 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 SOLO_DEGREE, SEG_DEGREE, MAX_SEGS, SEG_STRIDE = 256, 512, 8, 576
 ACT_NONE, ACT_LEAKY_RELU, ACT_TANH, ACT_ACCUMULATE = 0, 1, 2, 256
 
@@ -95,6 +95,8 @@ SIGNATURES = {
     "lkg_rank_prepare": (C.c_int, [vp, i64, vp, vp, i64, vp, vp, i64, i32, vp, vp, vp, vp, vp, vp]),
     "lkg_score_rank": (C.c_int, [C.POINTER(LkgPlanes), i64, C.POINTER(LkgPlanes), i64, vp, vp, vp, vp, i32, vp]),
     "lkg_rank_finalize": (C.c_int, [vp, i64, vp, vp, i64, vp, vp, vp, vp, vp, vp, i32, i64, i64, i32, vp, vp]),
+    "lkg_rank_filter": (C.c_int, [C.POINTER(LkgGraph), vp, vp, vp, vp, i64, vp, i64, i32, vp, vp, vp]),
+    "lkg_rank_filter_scores": (C.c_int, [C.POINTER(LkgGraph), vp, vp, vp, vp, i64, vp, i64, i64, vp, vp]),
     "lkg_topk_merge": (C.c_int, [vp, vp, i32, i64, i32, vp, vp, vp]),
     "lkg_score_index": (C.c_int, [vp, i64, vp, i64, i32, vp, vp, i64, vp, vp, vp]),
     "lkg_score_topk_workspace_bytes": (C.c_int, [i64, i32, i32, C.POINTER(C.c_size_t)]),

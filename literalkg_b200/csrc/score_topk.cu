@@ -628,6 +628,97 @@ __global__ void __launch_bounds__(256) rank_finalize_kernel(const float* __restr
     }
 }
 
+// ---- filtered rank: subtract the known true tails that beat the target ------------------------------------------
+// Filter run of a query: the tails t' of the known triples (h, r, t') -- a binary search of r in the head's att row,
+// which is sorted by (relation, tail) -- or, without a relation (r < 0), the head's agg row of unique (h, t') pairs.
+// Both runs are sorted by tail; the att run keeps duplicate triples, so callers skip a tail equal to its predecessor.
+__device__ __forceinline__ void filter_run(const lkg_graph& g, int64_t h, int64_t r, const int32_t** tails, int* lo,
+                                           int* hi) {
+    if (r < 0) {
+        *tails = g.col;
+        *lo = g.rowptr[h];
+        *hi = g.rowptr[h + 1];
+        return;
+    }
+    int a = g.att_rowptr[h], b = g.att_rowptr[h + 1];
+    int l = a, u = b;                                  // first index with rel >= r
+    while (l < u) {
+        const int m = (l + u) >> 1;
+        if (g.att_rel[m] < r) l = m + 1; else u = m;
+    }
+    a = l;
+    u = b;                                             // first index with rel > r
+    while (l < u) {
+        const int m = (l + u) >> 1;
+        if (g.att_rel[m] <= r) l = m + 1; else u = m;
+    }
+    *tails = g.att_tail;
+    *lo = a;
+    *hi = l;
+}
+
+// One CTA per query, the run split over the warps like rank_finalize_kernel's band (a hub head can have thousands of
+// known tails).  A filter tail f at candidate position p != t is subtracted when it beats the target under the rule
+// the raw rank was counted with, on the same scores:
+//   kExact  (fused path, after lkg_rank_finalize): s_f = exact_dot8 of the same head row staged the same way, compared
+//           with the same tau by the same float comparison.  finalize counts a column either because the GEMM put it
+//           above tau + E -- and then its exact score is above tau, the band bound being rigorous -- or because its
+//           exact score beats tau; either way the bit-identical re-score here reaches the same verdict;
+//   !kExact (dense path, after lkg_topk_rows): s_f and s_t are read from the score matrix and compared as the
+//           order-preserving keys lkg_topk_rows compares (-0 < +0 there).
+template <bool kExact>
+__global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, const int64_t* __restrict__ heads,
+                                                          const int64_t* __restrict__ rels,
+                                                          const int32_t* __restrict__ cand_map,
+                                                          const int64_t* __restrict__ target_pos,
+                                                          const float* __restrict__ src, int64_t ld, int dim,
+                                                          const float* __restrict__ tau, int64_t* __restrict__ ranks) {
+    __shared__ __align__(16) float s_head[kMaxChunks * kBK];
+    __shared__ int s_sub[8];
+    const int qi = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int grp = lane >> 3, q = lane & 7;
+    const int64_t h = heads[qi];
+    const int64_t tp = target_pos[qi];
+    if (kExact) {
+        const float* hrow = src + h * ld;
+        for (int i = threadIdx.x; i < kMaxChunks * kBK; i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
+        __syncthreads();
+    }
+    const int32_t* run;
+    int lo, hi;
+    filter_run(g, h, rels ? rels[qi] : -1, &run, &lo, &hi);
+    const float* srow = src + (int64_t)qi * ld;                      // dense: this query's row of the score matrix
+    const float t = kExact ? tau[qi] : srow[tp];
+    const int n = hi - lo;
+    int sub = 0;
+    for (int c0 = 4 * warp; c0 < n; c0 += 4 * nwarps) {              // uniform per warp: exact_dot8 shuffles
+        const int c = c0 + grp;
+        bool live = c < n;
+        int f = 0, p = -1;
+        if (live) {
+            f = run[lo + c];
+            p = cand_map ? cand_map[f] : f;
+            live = p >= 0 && p != tp && (c == 0 || run[lo + c - 1] != f);
+        }
+        if (kExact) {
+            const float s = exact_dot8(s_head, src + (int64_t)f * ld, dim, q, live);
+            if (live && q == 0 && (s > t || (s == t && p < tp))) ++sub;
+        } else if (live && q == 0) {
+            const uint32_t ks = enc(srow[p]), kt = enc(t);
+            if (ks > kt || (ks == kt && p < tp)) ++sub;
+        }
+    }
+    sub = (int)warp_sum((float)sub);                 // < 2^24 per warp
+    if (lane == 0) s_sub[warp] = sub;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int64_t tot = 0;
+        for (int w = 0; w < nwarps; ++w) tot += s_sub[w];
+        ranks[qi] -= tot;
+    }
+}
+
 inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
 
 }  // namespace
@@ -693,6 +784,45 @@ extern "C" int lkg_rank_finalize(const float* emb, int64_t ld_emb, const int64_t
                                                                                head_rows, target_pos, tau, above, band_cnt,
                                                                                band, band_cap, (int)n_tails, dim, ranks);
     LKG_LAUNCH_CHECK("rank_finalize_kernel");
+    return LKG_OK;
+}
+
+static int check_filter_args(const lkg_graph* known, const int64_t* heads, const int64_t* target_pos, int64_t n_queries,
+                             int64_t* ranks) {
+    LKG_REQUIRE(known && known->att_rowptr && known->att_tail && known->att_rel && known->rowptr && known->col,
+                "the known plan needs its att and agg arrays");
+    LKG_REQUIRE(heads && target_pos && ranks && n_queries >= 0 && n_queries < (1ll << 31), "bad filter arguments");
+    return LKG_OK;
+}
+
+extern "C" int lkg_rank_filter(const lkg_graph* known, const int64_t* heads, const int64_t* rels,
+                               const int32_t* cand_map, const int64_t* target_pos, int64_t n_queries, const float* emb,
+                               int64_t ld_emb, int32_t dim, const float* tau, int64_t* ranks, void* stream_) {
+    if (int rc = check_filter_args(known, heads, target_pos, n_queries, ranks)) return rc;
+    LKG_REQUIRE(emb && tau, "bad filter arguments");
+    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kMaxChunks * kBK && ld_emb % 4 == 0 && aligned16(emb),
+                "the rank path supports dim %% 4 == 0, dim <= %d, 16-byte aligned rows", kMaxChunks * kBK);
+    if (n_queries == 0) return LKG_OK;
+    rank_filter_kernel<true><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
+                                                                                    target_pos, emb, ld_emb, dim, tau,
+                                                                                    ranks);
+    LKG_LAUNCH_CHECK("rank_filter_kernel<exact>");
+    return LKG_OK;
+}
+
+extern "C" int lkg_rank_filter_scores(const lkg_graph* known, const int64_t* heads, const int64_t* rels,
+                                      const int32_t* cand_map, const int64_t* target_pos, int64_t n_queries,
+                                      const float* scores, int64_t ld_scores, int64_t n_cols, int64_t* ranks,
+                                      void* stream_) {
+    if (int rc = check_filter_args(known, heads, target_pos, n_queries, ranks)) return rc;
+    LKG_REQUIRE(scores && n_cols >= 1 && ld_scores >= n_cols, "bad score matrix");
+    LKG_REQUIRE(cand_map || n_cols == known->n_entities,
+                "without a candidate map the score matrix needs one column per entity of the known plan");
+    if (n_queries == 0) return LKG_OK;
+    rank_filter_kernel<false><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
+                                                                                     target_pos, scores, ld_scores, 0,
+                                                                                     nullptr, ranks);
+    LKG_LAUNCH_CHECK("rank_filter_kernel<scores>");
     return LKG_OK;
 }
 

@@ -1187,6 +1187,129 @@ class LiteralKG(nn.Module):
         scores = ops.score(all_embed, head_ids, tail_ids)
         return ops.topk_rows(scores, k, target_tails)
 
+    def evaluate_ranking(self, heads, tails, relations=None, known=None, candidates=None, ks=(1, 3, 10),
+                         batch_size=2048, all_embed=None):
+        """Filtered link-prediction evaluation (extension: the MR / MRR / Hits@k protocol; the reference only has its
+        threshold metrics).  Query i is (heads[i], relations[i] or any relation, target tails[i]).  Its raw rank is the
+        rank of ``topk``: #{ j in candidates : s_j > s_t, or s_j == s_t and pos(j) < pos(t) }, 0 = best, with
+        s_j = emb[h] . emb[j] (``calc_score``; the relation only selects the filter set) and ``candidates`` a list of
+        entity ids (None = every entity).  The filtered rank subtracts the members of
+            F(i) = { t' : (h, r, t') in known }   with a relation,   { t' : (h, any r, t') in known }   without,
+        that beat the target under the same rule on the same scores; a tail is counted once however often it is known,
+        the target itself and non-candidates never.  ``known``: ``GraphPlan`` of the known true triples (e.g. train +
+        valid + test over the same entity ids), None = raw ranks.  Head prediction (?, r, t): the score is symmetric, so
+        it is this call with heads and tails swapped and ``known`` built from the swapped triples.
+
+        Returns {"mr": mean(rank + 1), "mrr": mean(1 / (rank + 1)), "hits@k": mean(rank < k) for k in ``ks`` (float64,
+        as Python floats), "n": number of queries, "ranks": the filtered ranks, int64 [Q] on the device}.  One embedding
+        pass (or the given ``all_embed``), one tail index for all batches of ``batch_size`` queries, the fused / dense
+        path choice of ``topk``, and ONE host sync, which also carries the argument checks: ids outside
+        [0, n_entities), a target that is not a candidate, duplicate candidates and relation ids outside the plan's
+        range raise ValueError after it (the kernels only ever see clamped ids).
+        Row partitioned (``set_partition``, world > 1) this is a collective: every rank ranks a contiguous slice of the
+        queries on the gathered embeddings, the slices are all-gathered, and every rank returns the same result."""
+        dev = self._param_device()
+        with torch.no_grad():
+            if all_embed is None:
+                all_embed = self.gat_embeddings()
+            all_embed = _lib.f32c(all_embed)
+            n, dim = all_embed.shape
+
+            def ids(x):
+                return torch.as_tensor(x).to(device=dev, dtype=torch.int64).reshape(-1)
+
+            heads, tails = ids(heads), ids(tails)
+            q = heads.numel()
+            rels = None if relations is None else ids(relations)
+            if tails.numel() != q or (rels is not None and rels.numel() != q):
+                raise ValueError("heads, tails and relations must have the same length")
+            if rels is not None and known is None:
+                raise ValueError("relations only select the filter set: pass the known triples as well")
+            if known is not None and known.n_entities != n:
+                raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
+            if candidates is not None and q and len(candidates) == 0:
+                raise ValueError("no candidates")
+
+            def outside(x, hi):
+                return ((x < 0) | (x >= hi)).any()
+
+            bad = {"head or tail ids outside [0, n_entities)": outside(heads, n) | outside(tails, n)}
+            heads, tails = heads.clamp(0, n - 1), tails.clamp(0, n - 1)
+            cmap = cand = None
+            tpos, n_cand = tails, n
+            if candidates is not None:
+                cand = ids(candidates)
+                n_cand = cand.numel()
+                bad["candidate ids outside [0, n_entities)"] = outside(cand, n)
+                cand = cand.clamp(0, n - 1)
+                pos = torch.arange(n_cand, dtype=torch.int32, device=dev)
+                cmap = torch.full((n,), -1, dtype=torch.int32, device=dev)
+                cmap[cand] = pos
+                bad["duplicate candidate ids"] = (cmap[cand] != pos).any()
+                tpos = cmap[tails].long()
+                bad["a target tail is not a candidate"] = (tpos < 0).any()
+                tpos = tpos.clamp_min(0)
+            if rels is not None:
+                bad[f"relation ids outside [0, {known.n_relations})"] = outside(rels, known.n_relations)
+                rels = rels.clamp(0, known.n_relations - 1)
+
+            part = self._part
+            world = 1 if part is None else part.world
+            per = max(1, (q + world - 1) // world)
+            lo = 0 if world == 1 else min(q, part.rank * per)
+            hi = q if world == 1 else min(q, lo + per)
+            sl = slice(lo, hi)
+            ranks = self._rank_queries(all_embed, heads[sl], tpos[sl], None if rels is None else rels[sl], known, cmap,
+                                       cand, n_cand, batch_size)
+            if world > 1:
+                padded = torch.zeros(per, dtype=torch.int64, device=dev)
+                padded[:hi - lo] = ranks
+                ranks = part.all_gather_stack(padded).reshape(-1)[:q]
+
+            r1 = ranks.double() + 1.0
+            ks = [int(k) for k in ks]
+            metrics = [r1.mean(), (1.0 / r1).mean()] + [(ranks < k).double().mean() for k in ks]
+            host = torch.cat([torch.stack(metrics), torch.stack(list(bad.values())).double()]).tolist()
+            for msg, flag in zip(bad, host[len(metrics):]):
+                if flag:
+                    raise ValueError(msg)
+            out = {"mr": host[0], "mrr": host[1]}
+            out.update({f"hits@{k}": v for k, v in zip(ks, host[2:len(metrics)])})
+            out.update(n=q, ranks=ranks)
+            return out
+
+    @staticmethod
+    def _rank_queries(all_embed, heads, tpos, rels, known, cmap, cand, n_cand, batch_size):
+        """Filtered ranks of the queries (heads, target positions, relations or None) against the candidates ``cand``
+        (entity ids or None = every entity; ``cmap`` their position map), ``batch_size`` queries at a time."""
+        m = heads.numel()
+        ranks = torch.empty(m, dtype=torch.int64, device=heads.device)
+        if ops.fused_topk_applicable(n_cand, all_embed.shape[1], 1):
+            index = ops.ScoreIndex(all_embed, cand)
+            tau = torch.empty(m, dtype=torch.float32, device=heads.device)
+            for b0 in range(0, m, batch_size):
+                b = slice(b0, b0 + batch_size)
+                r = ops.score_rank(all_embed, heads[b], tpos[b], index, tau_out=tau[b])
+                if known is not None:
+                    ops.filter_ranks(r, known, heads[b], tpos[b], None if rels is None else rels[b], cmap,
+                                     emb=all_embed, tau=tau[b])
+                ranks[b] = r
+            return ranks
+        # dense path: the raw rank comes from the score matrix, so the filter judges on that matrix too (the second
+        # instance of the filter kernel reads s from it; masking the matrix would cost a write of every filter entry
+        # and make -inf targets ambiguous).  Matrices of at most 2 GB per chunk of queries.
+        rec = ops.scale_from_data(all_embed)
+        cols = torch.arange(n_cand, device=heads.device) if cand is None else cand
+        step = max(1, min(batch_size, (1 << 29) // max(n_cand, 1)))
+        for b0 in range(0, m, step):
+            b = slice(b0, b0 + step)
+            scores = ops.score(all_embed, heads[b], cols, rec=rec)
+            r = ops.topk_rows(scores, 1, tpos[b])[2]
+            if known is not None:
+                ops.filter_ranks(r, known, heads[b], tpos[b], None if rels is None else rels[b], cmap, scores=scores)
+            ranks[b] = r
+        return ranks
+
     def topk_sharded(self, head_ids, k, local_embed, tail_index=None):
         """Row-partitioned all-entity top-k: every rank scores the heads against the entities it owns
         (``local_embed`` = ``gat_embeddings(gather=False)``) and the per-rank survivors are merged.  Returns

@@ -398,10 +398,12 @@ class ScoreIndex:
 
 
 def score_rank(emb: torch.Tensor, heads: Optional[torch.Tensor], target_pos: torch.Tensor, tail_index: ScoreIndex,
-               head_emb: Optional[torch.Tensor] = None, band_cap: int = 8192) -> torch.Tensor:
+               head_emb: Optional[torch.Tensor] = None, band_cap: int = 8192,
+               tau_out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Rank (0 = best) of tail position ``target_pos[i]`` for head i among the tails of ``tail_index`` under "larger
     exact score first, ties -> lower position", without the B x Nt score matrix (lkg_rank_prepare / lkg_score_rank /
-    lkg_rank_finalize).  ``heads`` index ``head_emb`` (default ``emb``), None = every row."""
+    lkg_rank_finalize).  ``heads`` index ``head_emb`` (default ``emb``), None = every row.  ``tau_out`` (optional fp32
+    [B]) receives the exact target scores the ranks were counted against (what ``filter_ranks`` compares with)."""
     ti = tail_index
     hsrc = emb if head_emb is None else head_emb
     assert hsrc.dtype == torch.float32 and hsrc.stride(1) == 1 and hsrc.shape[1] == emb.shape[1]
@@ -414,7 +416,8 @@ def score_rank(emb: torch.Tensor, heads: Optional[torch.Tensor], target_pos: tor
     if nh == 0:
         return ranks
     center, ci, tp = ti.centered()
-    tau = torch.empty(nh, dtype=torch.float32, device=emb.device)
+    tau = torch.empty(nh, dtype=torch.float32, device=emb.device) if tau_out is None else tau_out
+    assert tau.dtype == torch.float32 and tau.is_contiguous() and tau.numel() == nh
     thr = torch.empty((nh, 2), dtype=torch.float32, device=emb.device)
     counters = torch.zeros((2, nh), dtype=torch.int32, device=emb.device)
     band = torch.empty((nh, band_cap), dtype=torch.int32, device=emb.device)
@@ -431,6 +434,38 @@ def score_rank(emb: torch.Tensor, heads: Optional[torch.Tensor], target_pos: tor
                                          _lib.ptr(hrows), tgt.data_ptr(), tau.data_ptr(), counters[0].data_ptr(),
                                          counters[1].data_ptr(), band.data_ptr(), band_cap, nh, ti.m, emb.shape[1],
                                          ranks.data_ptr(), _lib.stream()))
+    return ranks
+
+
+def filter_ranks(ranks: torch.Tensor, known: GraphPlan, heads: torch.Tensor, target_pos: torch.Tensor,
+                 relations: Optional[torch.Tensor] = None, cand_map: Optional[torch.Tensor] = None,
+                 emb: Optional[torch.Tensor] = None, tau: Optional[torch.Tensor] = None,
+                 scores: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Raw ranks -> filtered ranks, in place: subtracts from ``ranks[i]`` the distinct known tails of query i that beat
+    its target on the scores the raw rank was counted on (lkg_rank_filter / lkg_rank_filter_scores).  ``known``: plan of
+    the known triples; ``relations`` (int64 [B] or None): filter by (head, relation), else by head; ``cand_map`` (int32
+    [N] or None = identity): candidate position of every entity, -1 = not a candidate.  The scores are either
+    ``emb`` + ``tau`` (after ``score_rank`` on ``emb``: the same exact re-score and target scores) or ``scores`` (the
+    [B, Nc] matrix ``topk_rows`` ranked)."""
+    assert ranks.dtype == torch.int64 and ranks.is_contiguous()
+    dev = ranks.device
+    heads, tgt = _ids(heads, dev), _ids(target_pos, dev)
+    rels = None if relations is None else _ids(relations, dev)
+    assert heads.numel() == tgt.numel() == ranks.numel() and (rels is None or rels.numel() == ranks.numel())
+    assert cand_map is None or (cand_map.dtype == torch.int32 and cand_map.is_contiguous())
+    assert (scores is None) != (emb is None or tau is None), "give emb + tau (fused path) or scores (dense path)"
+    with _dev_guard(ranks, "filter_ranks"):
+        if scores is None:
+            _rowmajor(emb)
+            _lib.check(_lib.load().lkg_rank_filter(known.byref(), heads.data_ptr(), _lib.ptr(rels), _lib.ptr(cand_map),
+                                                   tgt.data_ptr(), ranks.numel(), emb.data_ptr(), emb.stride(0),
+                                                   emb.shape[1], tau.data_ptr(), ranks.data_ptr(), _lib.stream()))
+        else:
+            _rowmajor(scores)
+            _lib.check(_lib.load().lkg_rank_filter_scores(known.byref(), heads.data_ptr(), _lib.ptr(rels),
+                                                          _lib.ptr(cand_map), tgt.data_ptr(), ranks.numel(),
+                                                          scores.data_ptr(), scores.stride(0), scores.shape[1],
+                                                          ranks.data_ptr(), _lib.stream()))
     return ranks
 
 
