@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define LKG_ABI_VERSION 6
+#define LKG_ABI_VERSION 7
 
 typedef enum {
     LKG_OK = 0,
@@ -246,7 +246,22 @@ int lkg_gate_fwd(const lkg_planes* x, int64_t m, const lkg_planes* w_pair, const
  *     o2 = (ego * side) @ P2 + r2[row]             (bi-interaction only, P2 non-NULL)
  *     emb = leaky(o1) (+ leaky(o2));  x = LayerNorm(emb) * mask;  xn = x / max(|x|_2, 1e-12)
  * Pa, Pb, P2: [d_in, d_out] row-major.  r1/r2: per-row terms with leading dimension ld_r
- * (ld_r == 0 broadcasts one [d_out] vector, i.e. a plain bias). */
+ * (ld_r == 0 broadcasts one [d_out] vector, i.e. a plain bias).
+ * Envelope: d_in % 4 == 0, d_in <= 512, d_out <= 64, and the chosen kernel's shared memory within 227 KB.  The
+ * two-matrix modes (Pa != Pb, or P2) keep both [d_in, d_out] tiles in shared memory: at d_in >= 404 they need
+ * d_out <= 60.  The pre-projected z mode runs on the wide-row stream kernel only, which exists for
+ * ceil(d_in / 128) in {1, 2, 3, 4} with d_out <= 32 and for ceil(d_in / 128) == 3 with d_out <= 64, within the same
+ * shared-memory limit (e.g. not at d_in = 256 with d_out > 32, nor at d_in = 300 with d_out >= 56).  lkg_aggregate_supported tells
+ * which shapes run. */
+typedef enum {
+    LKG_AGG_MODE_ONE_TERM = 0,   /* P2 NULL, Pa NULL or Pa == Pb */
+    LKG_AGG_MODE_TWO_TERMS = 1,  /* P2 NULL, Pa != Pb */
+    LKG_AGG_MODE_BI = 2,         /* P2 given, z NULL */
+    LKG_AGG_MODE_BI_Z = 3        /* P2 and z given */
+} lkg_agg_mode;
+/* *ok = 1 iff lkg_aggregate_fwd runs (d_in, d_out) in `mode` with 16-byte aligned operands and a plan that has a row
+ * schedule (every plan of lkg_plan_build), 0 if it refuses the shape.  Host call, no device needed. */
+int lkg_aggregate_supported(int32_t d_in, int32_t d_out, int32_t mode, int32_t* ok /*host out*/);
 int lkg_aggregate_workspace_bytes(size_t* bytes /*host out*/);
 int lkg_aggregate_fwd(const lkg_graph* g, const float* a_values, const float* ego, int64_t ld_ego,
                       int32_t d_in, int32_t d_out, const float* pa, const float* pb, const float* p2,

@@ -13,9 +13,10 @@ LIB_PATH = os.path.join(_PKG, "liblkg.so")
 
 LKG_MAX_SEGMENTS = 4
 LKG_SCALE_FLOATS = 8
-ABI_VERSION = 6
+ABI_VERSION = 7
 SOLO_DEGREE, SEG_DEGREE, MAX_SEGS, SEG_STRIDE = 256, 512, 8, 576
 ACT_NONE, ACT_LEAKY_RELU, ACT_TANH, ACT_ACCUMULATE = 0, 1, 2, 256
+AGG_ONE_TERM, AGG_TWO_TERMS, AGG_BI, AGG_BI_Z = 0, 1, 2, 3     # lkg_agg_mode
 
 i32, i64, f32p, vp = C.c_int32, C.c_int64, C.c_void_p, C.c_void_p
 
@@ -63,6 +64,7 @@ SIGNATURES = {
                                        vp, i64, i64, vp, vp]),
     "lkg_gate_fwd": (C.c_int, [C.POINTER(LkgPlanes), i64, C.POINTER(LkgPlanes), vp, i32, vp, i64, vp, i64, vp, i64,
                                i64, vp, vp, i64, vp]),
+    "lkg_aggregate_supported": (C.c_int, [i32, i32, i32, C.POINTER(i32)]),
     "lkg_aggregate_workspace_bytes": (C.c_int, [C.POINTER(C.c_size_t)]),
     "lkg_aggregate_fwd": (C.c_int, [C.POINTER(LkgGraph), vp, vp, i64, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp,
                                     vp, vp, i64, vp, i64, vp, i64, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, vp]),

@@ -20,6 +20,8 @@ namespace {
 constexpr int kRows = 2;  // head rows per warp per step (P is read from shared memory once per kRows rows)
 
 enum Mode { kOneTerm = 0, kTwoTerms = 1, kBi = 2, kBiZ = 3 /* bi-interaction with a pre-projected sum term */ };
+static_assert(kOneTerm == LKG_AGG_MODE_ONE_TERM && kTwoTerms == LKG_AGG_MODE_TWO_TERMS && kBi == LKG_AGG_MODE_BI &&
+                  kBiZ == LKG_AGG_MODE_BI_Z, "lkg_agg_mode mirrors the kernel modes");
 
 struct AggParams {
     lkg_graph g;
@@ -1011,14 +1013,8 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
 }
 
 template <int S, int NC, int MODE>
-int launch_stream(const AggParams& p, cudaStream_t stream) {
+int launch_stream(const AggParams& p, size_t smem, cudaStream_t stream) {
     auto kern = aggregate_stream_kernel<S, NC, MODE>;
-    constexpr int NT = (MODE == kOneTerm || MODE == kBiZ) ? 1 : 2;
-    const size_t z_bytes = MODE == kBiZ ? (size_t)p.d_out * 4 : 0;
-    const size_t smem = (size_t)NT * p.nvec * 32 * NC * 16 +
-                        (size_t)kStreamWarps * (stream_ring(MODE) * (p.nvec * 16 + z_bytes) + (size_t)NT * p.nvec * 16) +
-                        kStreamWarps * stream_ring(MODE) * 8;
-    if (smem > 227 * 1024) return 1;                             // does not fit: the caller falls back
     LKG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<sm_count(), kStreamWarps * 32, smem, stream>>>(p);
     LKG_LAUNCH_CHECK("aggregate_stream_kernel");
@@ -1026,12 +1022,12 @@ int launch_stream(const AggParams& p, cudaStream_t stream) {
 }
 
 template <int S, int NC>
-int dispatch_stream(int mode, const AggParams& p, cudaStream_t stream) {
+int dispatch_stream(int mode, const AggParams& p, size_t smem, cudaStream_t stream) {
     switch (mode) {
-        case kOneTerm: return launch_stream<S, NC, kOneTerm>(p, stream);
-        case kTwoTerms: return launch_stream<S, NC, kTwoTerms>(p, stream);
-        case kBiZ: return launch_stream<S, NC, kBiZ>(p, stream);
-        default: return launch_stream<S, NC, kBi>(p, stream);
+        case kOneTerm: return launch_stream<S, NC, kOneTerm>(p, smem, stream);
+        case kTwoTerms: return launch_stream<S, NC, kTwoTerms>(p, smem, stream);
+        case kBiZ: return launch_stream<S, NC, kBiZ>(p, smem, stream);
+        default: return launch_stream<S, NC, kBi>(p, smem, stream);
     }
 }
 
@@ -1055,6 +1051,46 @@ int dispatch_mode(int mode, const AggParams& p, int threads, size_t smem, cudaSt
         case kTwoTerms: return launch<S, NC, kTwoTerms>(p, threads, smem, stream);
         default: return launch<S, NC, kBi>(p, threads, smem, stream);
     }
+}
+
+// ---- which kernel runs a shape ---------------------------------------------------------------------------------
+// One host function decides: lkg_aggregate_fwd launches what it returns and lkg_aggregate_supported answers from it,
+// so a caller can ask before it builds operands for a mode (the model picks layer 1's pre-projected z path this way).
+constexpr size_t kMaxSmem = 227 * 1024;
+enum Route { kRouteNone = 0, kRouteNarrow, kRouteStream, kRouteGeneric };
+struct AggRoute {
+    Route route;
+    size_t smem;   // stream / generic kernel: dynamic shared memory
+    int warps;     // generic kernel: warps per CTA
+};
+
+// narrow_ok: d_in in {16, 32, 64}, d_out % 4 == 0 and every operand the narrow kernel moves as float4 is aligned;
+// stream_ok: d_in >= 128 and the plan has a 16-byte aligned row schedule
+AggRoute agg_route(int mode, int d_in, int d_out, bool narrow_ok, bool stream_ok) {
+    const int nvec = d_in / 4;
+    if (mode != kBiZ && narrow_ok) return {kRouteNarrow, 0, 0};
+    if (stream_ok) {
+        const int slots_w = (nvec + 31) / 32, nc_w = (d_out + 31) / 32;
+        // one 128-wide slot: only the z mode (layer 1 of a bi-interaction model at embed_dim 128); the other modes
+        // keep the generic kernel there
+        const bool instance = (slots_w == 1 && nc_w == 1 && mode == kBiZ) || (slots_w == 2 && nc_w == 1) ||
+                              (slots_w == 3 && nc_w == 1) || (slots_w == 3 && nc_w == 2) || (slots_w == 4 && nc_w == 1);
+        const int nt = (mode == kOneTerm || mode == kBiZ) ? 1 : 2;
+        const size_t z_bytes = mode == kBiZ ? (size_t)d_out * 4 : 0;
+        const size_t smem = (size_t)nt * nvec * 32 * nc_w * 16 +
+                            (size_t)kStreamWarps * (stream_ring(mode) * (nvec * 16 + z_bytes) + (size_t)nt * nvec * 16) +
+                            kStreamWarps * stream_ring(mode) * 8;
+        if (instance && smem <= kMaxSmem) return {kRouteStream, smem, 0};
+    }
+    if (mode == kBiZ) return {kRouteNone, 0, 0};           // only the stream kernel gathers z
+    const int nt = mode == kOneTerm ? 1 : 2;
+    const size_t p_bytes = (size_t)nt * d_in * ((d_out + 3) / 4 * 4) * sizeof(float);
+    const size_t stage_per_warp = (size_t)kRows * nt * d_in * sizeof(float);
+    int warps = 16;
+    while (warps > 4 && p_bytes + warps * stage_per_warp > 200 * 1024) warps /= 2;
+    const size_t smem = p_bytes + warps * stage_per_warp;
+    if (smem > kMaxSmem) return {kRouteNone, smem, warps};
+    return {kRouteGeneric, smem, warps};
 }
 
 }  // namespace
@@ -1152,52 +1188,60 @@ extern "C" int lkg_aggregate_fwd(const lkg_graph* g, const float* a_values, cons
     // lane c reads sp[d * ps + c]: any stride is conflict free for 32 consecutive channels; pad to a
     // multiple of 4 floats to keep rows 16-byte aligned
     p.p_stride = (d_out + 3) / 4 * 4;
-    LKG_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(int), stream));
-
     // narrow rows: LPR lanes per row (needs 16-byte aligned rows everywhere the kernel moves float4 / 8-byte halves)
-    if ((d_in == 16 || d_in == 32 || d_in == 64) && d_out % 4 == 0) {
-        const bool al = aligned16(x_out) && ld_x % 4 == 0 && (!xn_out || (aligned16(xn_out) && ld_xn % 4 == 0)) &&
-                        (!r1 || (aligned16(r1) && ld_r % 4 == 0)) && (!r2 || (aligned16(r2) && ld_r % 4 == 0)) &&
-                        aligned16(ln_weight) && aligned16(ln_bias) && (!drop_mask || aligned16(drop_mask)) &&
-                        (!xn_planes || ((reinterpret_cast<uintptr_t>(xn_planes) & 7u) == 0 && ld_planes % 4 == 0 &&
-                                        plane_stride % 4 == 0));
+    const bool narrow_ok =
+        (d_in == 16 || d_in == 32 || d_in == 64) && d_out % 4 == 0 && aligned16(x_out) && ld_x % 4 == 0 &&
+        (!xn_out || (aligned16(xn_out) && ld_xn % 4 == 0)) && (!r1 || (aligned16(r1) && ld_r % 4 == 0)) &&
+        (!r2 || (aligned16(r2) && ld_r % 4 == 0)) && aligned16(ln_weight) && aligned16(ln_bias) &&
+        (!drop_mask || aligned16(drop_mask)) &&
+        (!xn_planes || ((reinterpret_cast<uintptr_t>(xn_planes) & 7u) == 0 && ld_planes % 4 == 0 && plane_stride % 4 == 0));
+    // wide rows with a schedule: the shared-memory ring kernel
+    const bool stream_ok = d_in >= 128 && g->row_sched && aligned16(g->row_sched);
+    const AggRoute rt = agg_route(mode, d_in, d_out, narrow_ok, stream_ok);
+    if (rt.route == kRouteNone) {                            // refused before anything is enqueued
+        if (z) LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate with a pre-projected sum term: d_in %d d_out %d not supported",
+                        d_in, d_out);
+        LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate shapes d_in %d d_out %d need %zu bytes of shared memory (%zu fit)",
+                 d_in, d_out, rt.smem, kMaxSmem);
+    }
+    LKG_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(int), stream));
+    if (rt.route == kRouteNarrow) {
         const int chunks = d_out / 4;
-        if (al) {
 #define LKG_NARROW_CASE(LL, CC) \
     if (d_in == 4 * LL && (chunks + LL - 1) / LL == CC) return dispatch_narrow<LL, CC>(mode, p, stream);
-            LKG_NARROW_CASE(4, 1) LKG_NARROW_CASE(4, 2) LKG_NARROW_CASE(4, 3) LKG_NARROW_CASE(4, 4)
-            LKG_NARROW_CASE(8, 1) LKG_NARROW_CASE(8, 2)
-            LKG_NARROW_CASE(16, 1)
+        LKG_NARROW_CASE(4, 1) LKG_NARROW_CASE(4, 2) LKG_NARROW_CASE(4, 3) LKG_NARROW_CASE(4, 4)
+        LKG_NARROW_CASE(8, 1) LKG_NARROW_CASE(8, 2)
+        LKG_NARROW_CASE(16, 1)
 #undef LKG_NARROW_CASE
-        }
     }
-
-    // wide rows with a schedule: the shared-memory ring kernel (returns 1 when the shapes do not fit its smem)
-    if (d_in >= 128 && g->row_sched && aligned16(g->row_sched)) {
+    if (rt.route == kRouteStream) {
         const int slots_w = (p.nvec + 31) / 32, nc_w = (d_out + 31) / 32;
-        int rc = 1;
-        if (slots_w == 2 && nc_w == 1) rc = dispatch_stream<2, 1>(mode, p, stream);
-        if (slots_w == 3 && nc_w == 1) rc = dispatch_stream<3, 1>(mode, p, stream);
-        if (slots_w == 3 && nc_w == 2) rc = dispatch_stream<3, 2>(mode, p, stream);
-        if (slots_w == 4 && nc_w == 1) rc = dispatch_stream<4, 1>(mode, p, stream);
-        if (rc <= 0) return rc;
+        if (slots_w == 1 && nc_w == 1) return launch_stream<1, 1, kBiZ>(p, rt.smem, stream);
+        if (slots_w == 2 && nc_w == 1) return dispatch_stream<2, 1>(mode, p, rt.smem, stream);
+        if (slots_w == 3 && nc_w == 1) return dispatch_stream<3, 1>(mode, p, rt.smem, stream);
+        if (slots_w == 3 && nc_w == 2) return dispatch_stream<3, 2>(mode, p, rt.smem, stream);
+        if (slots_w == 4 && nc_w == 1) return dispatch_stream<4, 1>(mode, p, rt.smem, stream);
     }
-    if (z) LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate with a pre-projected sum term: d_in %d d_out %d not supported", d_in, d_out);
-
-    const int nt = mode == kOneTerm ? 1 : 2;
-    const size_t p_bytes = (size_t)nt * d_in * p.p_stride * sizeof(float);
-    const size_t stage_per_warp = (size_t)kRows * nt * d_in * sizeof(float);
-    int warps = 16;
-    while (warps > 4 && p_bytes + warps * stage_per_warp > 200 * 1024) warps /= 2;
-    const size_t smem = p_bytes + warps * stage_per_warp;
-    if (smem > 227 * 1024) LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate shapes need %zu bytes of shared memory", smem);
-    const int threads = warps * 32;
-    const int slots = (p.nvec + 31) / 32;
-    const int nc = (d_out + 31) / 32;
+    if (rt.route == kRouteGeneric) {
+        const int threads = rt.warps * 32;
+        const int slots = (p.nvec + 31) / 32;
+        const int nc = (d_out + 31) / 32;
 #define LKG_AGG_CASE(SS, CC) \
-    if (slots == SS && nc == CC) return dispatch_mode<SS, CC>(mode, p, threads, smem, stream);
-    LKG_AGG_CASE(1, 1) LKG_AGG_CASE(2, 1) LKG_AGG_CASE(3, 1) LKG_AGG_CASE(4, 1)
-    LKG_AGG_CASE(1, 2) LKG_AGG_CASE(2, 2) LKG_AGG_CASE(3, 2) LKG_AGG_CASE(4, 2)
+    if (slots == SS && nc == CC) return dispatch_mode<SS, CC>(mode, p, threads, rt.smem, stream);
+        LKG_AGG_CASE(1, 1) LKG_AGG_CASE(2, 1) LKG_AGG_CASE(3, 1) LKG_AGG_CASE(4, 1)
+        LKG_AGG_CASE(1, 2) LKG_AGG_CASE(2, 2) LKG_AGG_CASE(3, 2) LKG_AGG_CASE(4, 2)
 #undef LKG_AGG_CASE
-    LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate: no kernel for d_in %d d_out %d", d_in, d_out);
+    }
+    LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate: no kernel instance for d_in %d d_out %d", d_in, d_out);
+}
+
+extern "C" int lkg_aggregate_supported(int32_t d_in, int32_t d_out, int32_t mode, int32_t* ok) {
+    LKG_REQUIRE(ok != nullptr, "ok is null");
+    LKG_REQUIRE(mode >= LKG_AGG_MODE_ONE_TERM && mode <= LKG_AGG_MODE_BI_Z, "unknown aggregate mode %d", mode);
+    *ok = 0;
+    if (d_in <= 0 || d_in % 4 != 0 || d_in > 512 || d_out <= 0 || d_out > 64) return LKG_OK;
+    if (mode == LKG_AGG_MODE_BI_Z && (d_in < 128 || d_out % 4 != 0)) return LKG_OK;
+    const bool narrow_ok = (d_in == 16 || d_in == 32 || d_in == 64) && d_out % 4 == 0;
+    *ok = agg_route(mode, d_in, d_out, narrow_ok, d_in >= 128).route != kRouteNone;
+    return LKG_OK;
 }

@@ -556,10 +556,11 @@ int make_map(CUtensorMap* map, const void* base, int64_t rows, int k, int64_t ld
     return LKG_OK;
 }
 
-int pick_bn(int n) {
+int pick_bn(int n, int min_tiles = 1) {
     // smallest number of N tiles, then the smallest tile (multiple of 16) that covers n.  (Measured in round 1: taking
     // more, narrower N tiles to fit a third cta_group::1 stage re-reads A and gains nothing: gate 2.69 -> 2.83 ms.)
-    const int tiles = (n + kMaxBN - 1) / kMaxBN;
+    int tiles = (n + kMaxBN - 1) / kMaxBN;
+    if (tiles < min_tiles) tiles = min_tiles;
     const int b = ((n + tiles - 1) / tiles + 15) / 16 * 16;
     return b < 16 ? 16 : b;
 }
@@ -638,6 +639,10 @@ int launch_tc(TcParams& p, const lkg_planes* a, int64_t m, const lkg_planes* b, 
     const int64_t pair_tiles = ((m + 2 * kBM - 1) / (2 * kBM)) * ((n + p.bn - 1) / p.bn);
     int cg = (p.bn % 16 == 0 && pair_tiles >= sm_count() / 2) ? 2 : 1;
     if (forced_cg() == 1 || (forced_cg() == 2 && p.bn % 16 == 0)) cg = forced_cg();
+    // one CTA staging a whole 256-column B tile next to the gate's three epilogue groups has room for one pipeline
+    // stage only (2 * dim = 256 or 512 at embed_dim 128 / 256): narrower N tiles until two stages fit
+    constexpr int G = EPI == kEpiGate ? 3 : 2;
+    for (int t = 2; stages_for(p.bn / cg, G) < 2 && t <= (n + 15) / 16; ++t) p.bn = pick_bn(n, t);
     return cg == 2 ? launch_tc_cg<EPI, 2>(p, a, m, b, n, stream) : launch_tc_cg<EPI, 1>(p, a, m, b, n, stream);
 }
 

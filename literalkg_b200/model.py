@@ -423,6 +423,7 @@ class LiteralKG(nn.Module):
             self.A_in.data = A_in
         self.A_in.requires_grad = False
         self.milestone_score = args.milestone_score
+        self._check_layer_shapes()
 
         # device-side plan state (not part of the state dict)
         self._agg_plan: Optional[GraphPlan] = None        # CSR of the current A_in
@@ -595,7 +596,6 @@ class LiteralKG(nn.Module):
     def _stack_q(self, folds):
         """The h0 @ Q GEMM of all layers as ONE stacked weight: rows = [layer 0: q1 + pa | q2 | layer 1: q1 | q2 ...
         | z columns = layer 0's pb].  Returns (wq [cols, embed_dim], cq [cols], offsets, zcol)."""
-        d = self.embed_dim
         qs, cs, off, offsets = [], [], 0, []
         for k, f in enumerate(folds):
             q1 = f["q1"] + f["pa"] if k == 0 else f["q1"]      # layer 0: ego == h0, fold ego @ Pa into h0 @ Q
@@ -606,10 +606,40 @@ class LiteralKG(nn.Module):
         # layer 0 again: z = h0 @ Pb, the neighbour sum term projected BEFORE the aggregation
         # ((A h0) Pb == A (h0 Pb)): 32 more GEMM columns replace a 300 x 32 combine per row, and for
         # gcn / graphsage the 1 200-byte neighbour gather of layer 1 altogether
-        zcol = off if d >= 128 and folds[0]["pb"].shape[1] % 4 == 0 else -1
+        zcol = off if self._layer1_z_path() else -1
         if zcol >= 0:
             qs.append(folds[0]["pb"]); cs.append(torch.zeros_like(folds[0]["c1"])); off += folds[0]["pb"].shape[1]
         return torch.cat(qs, dim=1).t().contiguous(), torch.cat(cs), offsets, zcol
+
+    def _layer1_z_path(self) -> bool:
+        """Layer 1 of a residual model with wide h0 gathers the pre-projected sum term z = h0 @ Pb.  gcn / graphsage
+        then run on the d_out-wide z table (any width); bi-interaction needs the library's z mode at (embed_dim,
+        conv_dim), which only the wide-row stream kernel has -- elsewhere layer 1 combines side @ Pb itself."""
+        if not self.use_residual or self.n_layers == 0:
+            return False
+        d, c = self.embed_dim, self.aggregator_layers[0].out_dim
+        if d < 128 or c % 4 != 0:
+            return False
+        return self.aggregation_type != 'bi-interaction' or ops.aggregate_supported(d, c, _lib.AGG_BI_Z)
+
+    def _check_layer_shapes(self) -> None:
+        """Refuses, at construction, widths the aggregation kernels do not run (instead of at the first forward)."""
+        z1 = self._layer1_z_path()
+        for k, layer in enumerate(self.aggregator_layers):
+            if k == 0 and z1:
+                continue                                  # supported by definition of the z path
+            folded_ego = k == 0 and self.use_residual     # layer 1's ego @ Pa rides in the h0 @ Q GEMM
+            if self.aggregation_type == 'bi-interaction':
+                mode = _lib.AGG_BI
+            elif self.aggregation_type == 'graphsage' and not folded_ego:
+                mode = _lib.AGG_TWO_TERMS
+            else:
+                mode = _lib.AGG_ONE_TERM
+            if not ops.aggregate_supported(layer.in_dim, layer.out_dim, mode):
+                raise ValueError(
+                    f"aggregator layer {k + 1} ({self.aggregation_type}, {layer.in_dim} -> {layer.out_dim}) is outside the "
+                    "aggregation kernels: they need in_dim % 4 == 0, in_dim <= 512 and out_dim <= 64, and out_dim <= 60 "
+                    "from in_dim 404 on where two combine matrices share the 227 KB of shared memory (include/lkg.h)")
 
     def _exchange_table(self, part, name: str, d: int, training: bool):
         """Symmetric-memory exchange table for the rows of one activation (``parallel.PeerTable``), or None: NCCL
@@ -646,10 +676,8 @@ class LiteralKG(nn.Module):
         """Inference pass of the bi-interaction model with the pre-projected sum term: the gate output h0 and
         z = h0 @ Pb live side by side in ONE table [rows, d + C] -- layer 1 fetches a neighbour's (h0 | z) row with one
         bulk copy, and the row partition exchanges one table instead of two."""
-        d = self.embed_dim
-        return (keep is None and pre is None and self.scale_gat_dim is not None and self.n_layers > 0
-                and self.use_residual and self.aggregation_type == 'bi-interaction' and d >= 128 and d % 4 == 0
-                and self.aggregator_layers[0].out_dim % 4 == 0)
+        return (keep is None and pre is None and self.scale_gat_dim is not None
+                and self.aggregation_type == 'bi-interaction' and self._layer1_z_path())
 
     def _residual_gemm(self, h0_planes, folds, z_out=None):
         """h0 @ Q for all layers (+ layer 1's ego @ Pa and the z columns) as one GEMM -> (h0q, offsets, zoff).
@@ -682,9 +710,7 @@ class LiteralKG(nn.Module):
         cat = None if combined else torch.empty((n_own, total), dtype=torch.float32, device=dev)
         gather_h0 = False
         if part is not None and self.n_layers > 0:
-            c0 = self.aggregator_layers[0].out_dim
-            z_path = self.use_residual and d >= 128 and c0 % 4 == 0      # see _stack_q
-            gather_h0 = not z_path or self.aggregation_type == 'bi-interaction'
+            gather_h0 = not self._layer1_z_path() or self.aggregation_type == 'bi-interaction'
         peer = None
         if combined:
             if part is None:

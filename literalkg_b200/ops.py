@@ -247,6 +247,13 @@ def gate(segments: Sequence, w_pair: torch.Tensor, bias_pair: torch.Tensor, x_en
     return out
 
 
+def aggregate_supported(d_in: int, d_out: int, mode: int) -> bool:
+    """True iff ``aggregate`` runs (d_in, d_out) in ``mode`` (_lib.AGG_*) with aligned operands (host call)."""
+    ok = C.c_int32(0)
+    _lib.check(_lib.load().lkg_aggregate_supported(int(d_in), int(d_out), int(mode), C.byref(ok)))
+    return bool(ok.value)
+
+
 def aggregate(plan: GraphPlan, a_values: torch.Tensor, ego: torch.Tensor, d_out: int,
               pa: Optional[torch.Tensor], pb: torch.Tensor, p2: Optional[torch.Tensor],
               r1: Optional[torch.Tensor], r2: Optional[torch.Tensor],

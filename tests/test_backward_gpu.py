@@ -339,9 +339,23 @@ def test_golden_gradients(g, mode):
     ("bi-interaction", False, 2, 1, REL), ("graphsage", False, 2, 1, REL), ("gcn", False, 1, 1, REL),
     ("bi-interaction", True, 3, 20, 1e-2)])
 def test_oracle_gradients(agg, res, layers, ent_scale, tol, monkeypatch):
+    _oracle_gradients(O.OracleConfig(n_conv_layers=layers, aggregation_type=agg, use_residual=res, mess_dropout=0.0),
+                      ent_scale, tol, monkeypatch)
+
+
+# widths off the default: (300, 64) bi-interaction + residual does not fit the pre-projected z kernel, so layer 1
+# combines side @ Pb itself (generic kernel) and its backward runs without the z columns
+@pytest.mark.parametrize("agg,res,d,c", [("bi-interaction", True, 300, 64), ("bi-interaction", True, 128, 32),
+                                         ("graphsage", True, 256, 16)])
+def test_oracle_gradients_other_widths(agg, res, d, c, monkeypatch):
+    cfg = O.OracleConfig(n_conv_layers=2, aggregation_type=agg, use_residual=res, mess_dropout=0.0, embed_dim=d,
+                         relation_dim=d, conv_dim=c)
+    _oracle_gradients(cfg, 1, REL, monkeypatch)
+
+
+def _oracle_gradients(cfg, ent_scale, tol, monkeypatch):
     import literalkg_b200 as L
     n, n_rel, e = 4000, 6, 40000
-    cfg = O.OracleConfig(n_conv_layers=layers, aggregation_type=agg, use_residual=res, mess_dropout=0.0)
     kg = L.synthetic.make_kg(n, e, n_rel, seed=11, max_out_degree=300)
     num, txt = L.synthetic.make_literals(n, seed=11)
     p = O.init_params(cfg, n, n_rel, seed=11)

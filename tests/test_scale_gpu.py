@@ -91,6 +91,32 @@ def test_default_dims_vs_oracle(agg, res):
     assert torch.equal(pos.cpu()[clear], tp[:, :10][clear])
 
 
+# widths other than the default reach other aggregation kernels: bi-interaction + residual takes layer 1's pre-projected
+# z path only where that kernel runs (at 128 / 32 the one-slot stream instance; not at 128 / 48, 256 / 48 or 300 / 64:
+# there the generic kernel combines side @ Pb), gcn / graphsage run layer 1 on the z table at d_out = 64 / 16
+@pytest.mark.parametrize("agg,res,d,c", [("bi-interaction", True, 128, 32), ("bi-interaction", True, 128, 48),
+                                         ("bi-interaction", True, 256, 48),
+                                         ("bi-interaction", True, 300, 64), ("gcn", True, 300, 64),
+                                         ("graphsage", True, 256, 16), ("bi-interaction", False, 300, 64)])
+def test_other_dims_vs_oracle(agg, res, d, c):
+    cfg = O.OracleConfig(aggregation_type=agg, use_residual=res, n_conv_layers=2, mess_dropout=0.0, embed_dim=d,
+                         relation_dim=d, conv_dim=c)
+    n, e, n_rel = 4000, 40000, 8
+    kg, num, txt, p, kt, m = build(cfg, n, e, n_rel)
+    h, t, r = (torch.from_numpy(x) for x in (kg.h, kg.t, kg.r))
+    m(kt.h_list, kt.t_list, kt.r_list, kt.relations, device="cuda", mode="update_att")
+    out = m.gat_embeddings()
+    p64 = O.cast_params(p, torch.float64)
+    oi64, ov64 = O.update_attention(p64["entity_embed.weight"], p64["relation_embed.weight"], h, t, r, kt.relations, n)
+    assert np.array_equal(m.A_in.data.indices().cpu().numpy(), oi64.numpy())
+    assert rel_err(m.A_in.data.values(), ov64) < REL
+    ref64 = O.gat_embeddings(p64, cfg, oi64, ov64, num.double(), txt.double())
+    big = ref64.abs() > 0.1 * ref64.abs().max()
+    el = ((out.cpu().double() - ref64).abs()[big] / ref64.abs()[big]).max().item()
+    print(f"{agg} residual={res} D={d} C={c}: CUDA vs fp64 {rel_err(out, ref64):.2e} (element-wise {el:.2e})")
+    assert rel_err(out, ref64) < REL and el < 5 * REL
+
+
 @pytest.mark.parametrize("agg", ["bi-interaction", "gcn"])
 def test_heavy_rows_vs_oracle(agg):
     """Head rows with thousands of neighbours (longer than every per-warp staging limit: shared-memory logit slots,
