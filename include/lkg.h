@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define LKG_ABI_VERSION 7
+#define LKG_ABI_VERSION 8
 
 typedef enum {
     LKG_OK = 0,
@@ -477,6 +477,39 @@ int lkg_rank_filter(const lkg_graph* known, const int64_t* heads, const int64_t*
 int lkg_rank_filter_scores(const lkg_graph* known, const int64_t* heads, const int64_t* rels /*nullable*/,
                            const int32_t* cand_map /*nullable*/, const int64_t* target_pos, int64_t n_queries,
                            const float* scores, int64_t ld_scores, int64_t n_cols, int64_t* ranks, void* stream);
+/* ---- distance rank: the triple score s(h, r, t) = -|q - p_t|^2 of TransR / TransE (link-prediction evaluation) -------
+ * q = the query rows (emb[h] M_r + e_r for (h, r, ?); emb[t] M_r - e_r for (?, r, t)), p_j = the candidates' projected
+ * rows (emb[j] M_r; TransE: M_r = I), both fp32 [*, dim] with dim % 4 == 0, dim <= 508, 16-byte aligned rows.
+ * d_j = |q - p_j|^2 EXACTLY (differences and squares in fp64, summed in fp64, rounded once to fp32); rank_i =
+ * #{ j : d_j < d_t or (d_j == d_t and j < t_i) } with t_i = target_pos[i] (a row of the candidate table).  With
+ * c = the candidates' mean row, d_j = |q - c|^2 - 2 ((q - c) . (p_j - c) - |p_j - c|^2 / 2): the counting GEMM of
+ * lkg_score_rank, unchanged, on augmented operands of width K = dim + 4.  Calls on one stream:
+ *   lkg_l2_rank_rows     out [m, ld_out >= dim + 4] = the augmented rows of src[rows ? rows[r] : r] - center:
+ *                        LKG_L2_CANDIDATE: [p - c, -|p - c|^2 / (2 alpha), 0..] and stats (float[2]) = {max |p - c|,
+ *                        max row norm}, rounded up (two passes: the first finds max |p - c|, which fixes the power of
+ *                        two alpha); LKG_L2_QUERY: [q - c, alpha, 0..] with alpha read from the candidates' stats;
+ *   (lkg_split_planes of both, each with its own scale record)
+ *   lkg_rank_prepare_l2  tau = d_t (exact), thr = the band around the target's GEMM value, a rigorous bound of the GEMM's
+ *                        error at K (rec_query / rec_cand: the planes' scale records) and of the fp32 roundings of
+ *                        q - c, p - c and the norm column;
+ *   lkg_score_rank       the query planes against the candidate planes;
+ *   lkg_rank_finalize_l2 the band columns (every column on overflow) re-scored exactly;
+ *   lkg_rank_filter_l2   as lkg_rank_filter; f is re-scored with the same exact distance against its row of the
+ *                        candidate table, cand_map[f] (NULL: row f), and the same tau. */
+enum lkg_l2_mode { LKG_L2_QUERY = 0, LKG_L2_CANDIDATE = 1 };
+int lkg_l2_rank_rows(const float* src, int64_t ld, const int64_t* rows /*nullable*/, int64_t m, int32_t dim,
+                     const float* center, int32_t mode, float* stats, float* out, int64_t ld_out, void* stream);
+int lkg_rank_prepare_l2(const float* cand, int64_t ld_cand, const float* query, int64_t ld_query, const float* query_aug,
+                        int64_t ld_aug, const int64_t* target_pos, int64_t n_queries, int32_t dim, const float* stats,
+                        const float* rec_query, const float* rec_cand, float* tau, float* thr, void* stream);
+int lkg_rank_finalize_l2(const float* cand, int64_t ld_cand, const float* query, int64_t ld_query,
+                         const int64_t* target_pos, const float* tau, const int32_t* above, const int32_t* band_cnt,
+                         const int32_t* band, int32_t band_cap, int64_t n_queries, int64_t n_cand, int32_t dim,
+                         int64_t* ranks, void* stream);
+int lkg_rank_filter_l2(const lkg_graph* known, const int64_t* anchors, const int64_t* rels /*nullable*/,
+                       const int32_t* cand_map /*nullable*/, const int64_t* target_pos, int64_t n_queries,
+                       const float* cand, int64_t ld_cand, const float* query, int64_t ld_query, int32_t dim,
+                       const float* tau, int64_t* ranks, void* stream);
 int lkg_score_topk_workspace_bytes(int64_t n_heads, int32_t cap, int32_t sample_tiles, size_t* bytes /*host out*/);
 /* Per head the k best tails by emb[head] . emb[tail]: larger score first, ties -> lower position in the tail
  * list; values are the exact dot products (fp32 products summed in fp64, rounded once).

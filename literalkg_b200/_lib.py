@@ -13,10 +13,11 @@ LIB_PATH = os.path.join(_PKG, "liblkg.so")
 
 LKG_MAX_SEGMENTS = 4
 LKG_SCALE_FLOATS = 8
-ABI_VERSION = 7
+ABI_VERSION = 8
 SOLO_DEGREE, SEG_DEGREE, MAX_SEGS, SEG_STRIDE = 256, 512, 8, 576
 ACT_NONE, ACT_LEAKY_RELU, ACT_TANH, ACT_ACCUMULATE = 0, 1, 2, 256
 AGG_ONE_TERM, AGG_TWO_TERMS, AGG_BI, AGG_BI_Z = 0, 1, 2, 3     # lkg_agg_mode
+L2_QUERY, L2_CANDIDATE = 0, 1                                  # lkg_l2_mode
 
 i32, i64, f32p, vp = C.c_int32, C.c_int64, C.c_void_p, C.c_void_p
 
@@ -99,6 +100,10 @@ SIGNATURES = {
     "lkg_rank_finalize": (C.c_int, [vp, i64, vp, vp, i64, vp, vp, vp, vp, vp, vp, i32, i64, i64, i32, vp, vp]),
     "lkg_rank_filter": (C.c_int, [C.POINTER(LkgGraph), vp, vp, vp, vp, i64, vp, i64, i32, vp, vp, vp]),
     "lkg_rank_filter_scores": (C.c_int, [C.POINTER(LkgGraph), vp, vp, vp, vp, i64, vp, i64, i64, vp, vp]),
+    "lkg_l2_rank_rows": (C.c_int, [vp, i64, vp, i64, i32, vp, i32, vp, vp, i64, vp]),
+    "lkg_rank_prepare_l2": (C.c_int, [vp, i64, vp, i64, vp, i64, vp, i64, i32, vp, vp, vp, vp, vp, vp]),
+    "lkg_rank_finalize_l2": (C.c_int, [vp, i64, vp, i64, vp, vp, vp, vp, vp, i32, i64, i64, i32, vp, vp]),
+    "lkg_rank_filter_l2": (C.c_int, [C.POINTER(LkgGraph), vp, vp, vp, vp, i64, vp, i64, vp, i64, i32, vp, vp, vp]),
     "lkg_topk_merge": (C.c_int, [vp, vp, i32, i64, i32, vp, vp, vp]),
     "lkg_score_index": (C.c_int, [vp, i64, vp, i64, i32, vp, vp, i64, vp, vp, vp]),
     "lkg_score_topk_workspace_bytes": (C.c_int, [i64, i32, i32, C.POINTER(C.c_size_t)]),

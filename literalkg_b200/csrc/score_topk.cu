@@ -367,6 +367,13 @@ __device__ __forceinline__ float dec(uint32_t u) {
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
+// Score kinds of the rank kernels: the dot product emb[h] . emb[j], or the negated squared distance -|q - p_j|^2 of the
+// relation-aware triple score (TransR / TransE), and the dense instance of the filter that reads a score matrix.
+constexpr int kDot = 0, kL2 = 1, kScores = 2;
+constexpr int kL2MaxDim = 508;           // distance rows: dim % 4 == 0, the augmented width dim + 4 <= 512
+constexpr int kL2Vec = (kL2MaxDim + 4) / 32;    // float4 per lane in exact_l2 (8 lanes per row)
+template <int Kind> constexpr int row_floats() { return Kind == kL2 ? kL2MaxDim + 4 : kMaxChunks * kBK; }
+
 // Exact score of one (head, tail): fp32 products are exact in fp64, summed in fp64, one rounding to fp32 at the end.
 // Eight lanes share a tail row (lane q of the group takes float4 q, q + 8, ...), so a warp scores four candidates
 // at once with all its row loads in flight together; the head row is read from shared memory.
@@ -395,6 +402,49 @@ __device__ __forceinline__ float exact_dot8(const float* __restrict__ s_head, co
     acc += __shfl_xor_sync(kFull, acc, 2);
     acc += __shfl_xor_sync(kFull, acc, 1);
     return (float)acc;
+}
+
+// Exact squared distance |a - b|^2 of two fp32 rows: each difference is exact in fp64, squared and summed in fp64
+// (one fma per element), one rounding to fp32.  The lane layout of exact_dot8 over widths up to 512.  `a` (the query
+// row) may live in shared or global memory: prepare reads it from global, finalize and the filter from shared memory,
+// and the three see the same values in the same order, so they return the same bits.
+__device__ __forceinline__ float exact_l2(const float* a, const float* __restrict__ b, int dim, int q, bool live) {
+    double acc = 0.0;
+    const int nv = dim >> 2;                                   // dim % 4 == 0 is checked on the host side
+    float4 t[kL2Vec];
+#pragma unroll
+    for (int i = 0; i < kL2Vec; ++i) {
+        const int v = q + 8 * i;
+        t[i] = (live && v < nv) ? __ldg(reinterpret_cast<const float4*>(b) + v) : make_float4(0, 0, 0, 0);
+    }
+#pragma unroll
+    for (int i = 0; i < kL2Vec; ++i) {
+        const int v = q + 8 * i;
+        if (v < nv) {
+            const float4 h = *reinterpret_cast<const float4*>(a + 4 * v);
+            double d = (double)h.x - (double)t[i].x;
+            acc = fma(d, d, acc);
+            d = (double)h.y - (double)t[i].y;
+            acc = fma(d, d, acc);
+            d = (double)h.z - (double)t[i].z;
+            acc = fma(d, d, acc);
+            d = (double)h.w - (double)t[i].w;
+            acc = fma(d, d, acc);
+        }
+    }
+    acc += __shfl_xor_sync(kFull, acc, 4);
+    acc += __shfl_xor_sync(kFull, acc, 2);
+    acc += __shfl_xor_sync(kFull, acc, 1);
+    return (float)acc;
+}
+
+// The exact score the rank kernels compare: s = emb[h] . emb[j], or s = -d for the distance (negation is exact, and
+// "s_j > s_t" is "d_j < d_t", so one comparison and one tie rule serve both kinds).
+template <int Kind>
+__device__ __forceinline__ float exact_score(const float* s_head, const float* __restrict__ row, int dim, int q,
+                                             bool live) {
+    if constexpr (Kind == kL2) return -exact_l2(s_head, row, dim, q, live);
+    else return exact_dot8(s_head, row, dim, q, live);
 }
 
 __device__ void bitonic_desc(unsigned long long* keys, int n_pow2) {
@@ -536,6 +586,73 @@ __global__ void __launch_bounds__(kFinalThreads) score_finalize_kernel(FinalPara
 //   3. lkg_rank_finalize  the listed columns re-scored exactly and compared with tau under the tie rule.
 constexpr float kRankErr = 1.0e-5f;
 
+// The same bound as a function of the GEMM's K (the engine runs whole 64-wide chunks: 3 MMAs per 16 columns of them),
+// relative to |a| |b| of the two operand rows: per MMA 2^-23 of the running magnitude, 3 * 2^-22 for the hi/lo
+// representation of both operands and the dropped lo * lo product, times 1.5.  DESIGN.md §6 has the derivation.
+__host__ __device__ constexpr double rank_err(int k) {
+    return 1.5 * (3.0 * ((k + kBK - 1) / kBK) * (kBK / 16) * 0x1p-23 + 3.0 * 0x1p-22);
+}
+static_assert(rank_err(kMaxChunks * kBK) <= kRankErr, "kRankErr must cover the dot rank GEMM at K = 256");
+
+// ---- distance rank (the triple score, TransR / TransE) -----------------------------------------------------------
+// d_j = |q - p_j|^2 is turned into the counting GEMM's form by centring on c (the candidates' mean row) and one
+// augmented column: with u = q - c, w_j = p_j - c and nu_j = -|w_j|^2 / 2,
+//     d_j = |u|^2 - 2 (u . w_j + nu_j),
+// so "closer" is "larger u~ . v~_j" with u~ = [u, alpha, 0..] and v~_j = [w_j, nu_j / alpha, 0..].  alpha is a power of
+// two near max_j |w_j| (exact division): it keeps |u~| and |v~_j| of the order of the rows' own norms, so the GEMM's
+// error band scales like the distances do whatever the embeddings' magnitude.
+// stats (float[2] per candidate table): {W = max_j |w_j|, V = max_j |v~_j|}, both rounded up.
+__device__ __forceinline__ float l2_alpha(float w) {
+    if (!(w > 0.f && w < 3.0e38f)) return 1.f;
+    int ex;
+    frexpf(w, &ex);                                     // w in [2^(ex-1), 2^ex)
+    ex = ex - 1 > 60 ? 60 : (ex - 1 < -60 ? -60 : ex - 1);
+    return ldexpf(1.f, ex);
+}
+
+// One warp per row.  pass 0: the norms of the centred rows only (stats[0] = W); pass 1: candidates [w, nu / alpha, 0..]
+// and stats[1] = V; pass 2: queries [u, alpha, 0..].  The row norm is accumulated in fp64 from the ROUNDED fp32 x - c
+// (the values the GEMM and the bound see) and rounded once.
+__global__ void l2_rank_rows_kernel(const float* __restrict__ src, int64_t ld, const int64_t* __restrict__ rows,
+                                    int64_t m, int dim, const float* __restrict__ center, int pass,
+                                    float* __restrict__ stats, float* __restrict__ out, int64_t ld_out) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int nv = dim >> 2;
+    const float alpha = pass == 0 ? 1.f : l2_alpha(__ldg(stats));
+    float wmax = 0.f;
+    for (int64_t r = warp; r < m; r += nwarps) {
+        const float4* x4 = reinterpret_cast<const float4*>(src + (rows ? rows[r] : r) * ld);
+        float4* o4 = reinterpret_cast<float4*>(out + r * ld_out);
+        double nn = 0.0;
+        for (int v = lane; v < nv; v += 32) {
+            const float4 x = __ldg(x4 + v), c = __ldg(reinterpret_cast<const float4*>(center) + v);
+            const float4 u = make_float4(x.x - c.x, x.y - c.y, x.z - c.z, x.w - c.w);
+            nn = fma((double)u.x, (double)u.x, nn);
+            nn = fma((double)u.y, (double)u.y, nn);
+            nn = fma((double)u.z, (double)u.z, nn);
+            nn = fma((double)u.w, (double)u.w, nn);
+            if (pass != 0) o4[v] = u;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) nn += __shfl_xor_sync(kFull, nn, o);
+        if (pass == 0) {
+            wmax = fmaxf(wmax, __double2float_ru(__dsqrt_ru(nn)));
+        } else if (lane == 0) {
+            float aug = alpha;
+            if (pass == 1) {
+                aug = (float)(-0.5 * nn) / alpha;
+                wmax = fmaxf(wmax, __double2float_ru(__dsqrt_ru(nn + (double)aug * aug)));
+            }
+            o4[nv] = make_float4(aug, 0.f, 0.f, 0.f);
+        }
+    }
+    wmax = warp_max(wmax);
+    if (pass != 2 && lane == 0 && wmax > 0.f)
+        atomicMax(reinterpret_cast<uint32_t*>(stats + (pass == 0 ? 0 : 1)), __float_as_uint(wmax));
+}
+
 // center (nullable, [dim]): the GEMM's tails are t_j - center (a common shift moves every score of a head by the same
 // h . center, so the ranking is unchanged while the error bound shrinks from |h| max|t| to |h| max|t - center| -- the
 // embeddings of a trained or freshly initialised model are tightly clustered around their mean, and a band relative
@@ -551,12 +668,64 @@ __global__ void shift_rows_kernel(const float* __restrict__ src, int64_t ld, con
     }
 }
 
+// What the distance instance of rank_prepare_kernel reads besides the dot instance's arguments (which it reads as:
+// emb = the candidates' projected rows p_j, head_emb = the query rows q, tail_max_norm = the stats of the candidate
+// operand, rec = the scale record of its planes).
+struct L2Prep {
+    const float* aug;        // [n_heads, ld_aug] the query operand u~ = [q - c, alpha, 0..]
+    int64_t ld_aug;
+    const float* rec_q;      // scale record of its planes
+};
+
+template <int Kind>
 __global__ void rank_prepare_kernel(const float* __restrict__ emb, int64_t ld, const int64_t* __restrict__ tail_rows,
                                     const float* __restrict__ head_emb, int64_t ld_h,
                                     const int64_t* __restrict__ head_rows, const int64_t* __restrict__ target_pos,
                                     int n_heads, int dim, const float* __restrict__ tail_max_norm,
                                     const float* __restrict__ rec, const float* __restrict__ center,
-                                    float* __restrict__ tau, float* __restrict__ thr) {
+                                    float* __restrict__ tau, float* __restrict__ thr, const L2Prep l2) {
+    if constexpr (Kind == kL2) {
+        // 8 lanes per query (the exact_l2 layout), 4 queries per warp.  tau = d_t by exact_l2 on the same rows, in the
+        // same order, as finalize and the filter re-score.  With D_j the exact distance on the fp32 rows q, p_j, the
+        // GEMM value g_j and S~_j = u . w_j + nu_j on the rounded fp32 operands (DESIGN.md §6):
+        //   |g_j - S~_j| <= E = rank_err(K) |u~| V + 2^-24 sqrt(K) (V / s_q + |u~| / s_c)  (the second term: fp16
+        //                       subnormals of the lo planes, 1 / s the record's inverse scales),
+        //   |D_j - (|u|^2 - 2 S~_j)| <= R = 2^-21 (|u| + W)^2  (rounding of q - c, p_j - c and nu_j),
+        // so g_j > sigma + M implies D_j < d_t (1 - 2^-22), hence d_j = fl(D_j) < d_t, and g_j < sigma - M implies
+        // d_j > d_t, with sigma = (|u|^2 - d_t) / 2 and M = E + R / 2 + 2^-21 d_t + the fp64 rounding of sigma.
+        const int gq = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3);
+        const int q = threadIdx.x & 7;
+        const bool live = gq < n_heads;
+        const int head = live ? gq : 0;
+        const int64_t tp = target_pos[head];
+        const float t = exact_l2(head_emb + (int64_t)head * ld_h, emb + tp * ld, dim, q, live);
+        const float* arow = l2.aug + (int64_t)head * l2.ld_aug;
+        double uu = 0.0;
+        for (int v = q; v < (dim >> 2); v += 8) {
+            const float4 u = __ldg(reinterpret_cast<const float4*>(arow) + v);
+            uu = fma((double)u.x, (double)u.x, uu);
+            uu = fma((double)u.y, (double)u.y, uu);
+            uu = fma((double)u.z, (double)u.z, uu);
+            uu = fma((double)u.w, (double)u.w, uu);
+        }
+        uu += __shfl_xor_sync(kFull, uu, 4);
+        uu += __shfl_xor_sync(kFull, uu, 2);
+        uu += __shfl_xor_sync(kFull, uu, 1);
+        if (live && q == 0) {
+            const int k = dim + 4;
+            const double w = tail_max_norm[0], vmax = tail_max_norm[1], alpha = arow[dim];
+            const double nu = __dsqrt_ru(uu) * (1.0 + 0x1p-40), nua = __dsqrt_ru(uu + alpha * alpha) * (1.0 + 0x1p-40);
+            const double e = rank_err(k) * nua * vmax + 0x1p-24 * sqrt((double)k) * 1.001 *
+                                                            (vmax * __ldg(l2.rec_q + 2) + nua * __ldg(rec + 2));
+            const double r = 0x1p-21 * (nu + w) * (nu + w);
+            const double sigma = 0.5 * (uu - (double)t);
+            const double mrg = e + 0.5 * r + 0x1p-21 * (double)t + (uu + fabs(sigma)) * 0x1p-40 + 1e-30;
+            tau[head] = t;
+            thr[2 * head] = __double2float_rd(sigma - mrg);
+            thr[2 * head + 1] = __double2float_ru(sigma + mrg);
+        }
+        return;
+    }
     const int lane = threadIdx.x & 31;
     const int head = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     if (head >= n_heads) return;
@@ -588,6 +757,9 @@ __global__ void rank_prepare_kernel(const float* __restrict__ emb, int64_t ld, c
     }
 }
 
+// Kind == kL2: emb = the candidates' projected rows p_j (tail_rows NULL), head_emb = the query rows q, tau = d_t; the
+// comparison runs on s = -d against -tau, so the tie rule and the counting are the dot instance's.
+template <int Kind>
 __global__ void __launch_bounds__(256) rank_finalize_kernel(const float* __restrict__ emb, int64_t ld,
                                                             const int64_t* __restrict__ tail_rows,
                                                             const float* __restrict__ head_emb, int64_t ld_h,
@@ -596,15 +768,15 @@ __global__ void __launch_bounds__(256) rank_finalize_kernel(const float* __restr
                                                             const float* __restrict__ tau, const int* __restrict__ above,
                                                             const int* __restrict__ band_cnt, const int* __restrict__ band,
                                                             int cap, int n_tails, int dim, int64_t* __restrict__ ranks) {
-    __shared__ __align__(16) float s_head[kMaxChunks * kBK];
+    __shared__ __align__(16) float s_head[row_floats<Kind>()];
     __shared__ int s_better[8];
     const int head = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int grp = lane >> 3, q = lane & 7;
     const float* hrow = head_emb + (head_rows ? head_rows[head] : head) * ld_h;
-    for (int i = threadIdx.x; i < kMaxChunks * kBK; i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
+    for (int i = threadIdx.x; i < row_floats<Kind>(); i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
     __syncthreads();
-    const float t = tau[head];
+    const float t = Kind == kL2 ? -tau[head] : tau[head];
     const int64_t tp = target_pos[head];
     const int n_band = band_cnt[head];
     const bool overflow = n_band > cap;            // the band held more columns than the list: exact scan of every tail
@@ -615,7 +787,7 @@ __global__ void __launch_bounds__(256) rank_finalize_kernel(const float* __restr
         const bool live = c < n;
         const int col = live ? (overflow ? c : band[(int64_t)head * cap + c]) : 0;
         const float* trow = emb + (tail_rows ? tail_rows[col] : col) * ld;
-        const float s = exact_dot8(s_head, trow, dim, q, live);
+        const float s = exact_score<Kind>(s_head, trow, dim, q, live);
         if (live && q == 0 && (s > t || (s == t && col < tp))) ++better;
     }
     better = (int)warp_sum((float)better);          // < 2^24 per warp
@@ -664,16 +836,20 @@ __device__ __forceinline__ void filter_run(const lkg_graph& g, int64_t h, int64_
 //           with the same tau by the same float comparison.  finalize counts a column either because the GEMM put it
 //           above tau + E -- and then its exact score is above tau, the band bound being rigorous -- or because its
 //           exact score beats tau; either way the bit-identical re-score here reaches the same verdict;
-//   !kExact (dense path, after lkg_topk_rows): s_f and s_t are read from the score matrix and compared as the
+//   kL2     (distance path, after lkg_rank_finalize_l2): the same argument with s = -exact_l2 of the query row (row qi
+//           of qrows, staged like finalize stages it) and f's row in the candidate table (src row p), against -tau;
+//   kScores (dense path, after lkg_topk_rows): s_f and s_t are read from the score matrix and compared as the
 //           order-preserving keys lkg_topk_rows compares (-0 < +0 there).
-template <bool kExact>
+template <int Kind>
 __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, const int64_t* __restrict__ heads,
                                                           const int64_t* __restrict__ rels,
                                                           const int32_t* __restrict__ cand_map,
                                                           const int64_t* __restrict__ target_pos,
                                                           const float* __restrict__ src, int64_t ld, int dim,
-                                                          const float* __restrict__ tau, int64_t* __restrict__ ranks) {
-    __shared__ __align__(16) float s_head[kMaxChunks * kBK];
+                                                          const float* __restrict__ tau, int64_t* __restrict__ ranks,
+                                                          const float* __restrict__ qrows, int64_t ld_q) {
+    constexpr bool kExact = Kind != kScores;
+    __shared__ __align__(16) float s_head[row_floats<Kind>()];
     __shared__ int s_sub[8];
     const int qi = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
@@ -681,15 +857,15 @@ __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, con
     const int64_t h = heads[qi];
     const int64_t tp = target_pos[qi];
     if (kExact) {
-        const float* hrow = src + h * ld;
-        for (int i = threadIdx.x; i < kMaxChunks * kBK; i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
+        const float* hrow = Kind == kL2 ? qrows + (int64_t)qi * ld_q : src + h * ld;
+        for (int i = threadIdx.x; i < row_floats<Kind>(); i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
         __syncthreads();
     }
     const int32_t* run;
     int lo, hi;
     filter_run(g, h, rels ? rels[qi] : -1, &run, &lo, &hi);
     const float* srow = src + (int64_t)qi * ld;                      // dense: this query's row of the score matrix
-    const float t = kExact ? tau[qi] : srow[tp];
+    const float t = Kind == kL2 ? -tau[qi] : (kExact ? tau[qi] : srow[tp]);
     const int n = hi - lo;
     int sub = 0;
     for (int c0 = 4 * warp; c0 < n; c0 += 4 * nwarps) {              // uniform per warp: exact_dot8 shuffles
@@ -702,7 +878,7 @@ __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, con
             live = p >= 0 && p != tp && (c == 0 || run[lo + c - 1] != f);
         }
         if (kExact) {
-            const float s = exact_dot8(s_head, src + (int64_t)f * ld, dim, q, live);
+            const float s = exact_score<Kind>(s_head, src + (int64_t)(Kind == kL2 ? p : f) * ld, dim, q, live);
             if (live && q == 0 && (s > t || (s == t && p < tp))) ++sub;
         } else if (live && q == 0) {
             const uint32_t ks = enc(srow[p]), kt = enc(t);
@@ -762,10 +938,11 @@ extern "C" int lkg_rank_prepare(const float* emb, int64_t ld_emb, const int64_t*
                 "bad rank arguments");
     if (n_heads == 0) return LKG_OK;
     const int64_t blocks = (n_heads * 32 + 255) / 256;
-    rank_prepare_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(emb, ld_emb, tail_rows, head_emb, ld_head_emb,
-                                                                             head_rows, target_pos, (int)n_heads, dim,
-                                                                             tail_max_norm, rec, center, tau, thr);
-    LKG_LAUNCH_CHECK("rank_prepare_kernel");
+    rank_prepare_kernel<kDot><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(emb, ld_emb, tail_rows, head_emb,
+                                                                                   ld_head_emb, head_rows, target_pos,
+                                                                                   (int)n_heads, dim, tail_max_norm, rec,
+                                                                                   center, tau, thr, L2Prep{});
+    LKG_LAUNCH_CHECK("rank_prepare_kernel<dot>");
     return LKG_OK;
 }
 
@@ -780,10 +957,10 @@ extern "C" int lkg_rank_finalize(const float* emb, int64_t ld_emb, const int64_t
                     aligned16(emb) && aligned16(head_emb) && n_tails < (1ll << 31),
                 "the rank path supports dim %% 4 == 0, dim <= %d, 16-byte aligned rows", kMaxChunks * kBK);
     if (n_heads == 0) return LKG_OK;
-    rank_finalize_kernel<<<(unsigned)n_heads, 256, 0, (cudaStream_t)stream_>>>(emb, ld_emb, tail_rows, head_emb, ld_head_emb,
+    rank_finalize_kernel<kDot><<<(unsigned)n_heads, 256, 0, (cudaStream_t)stream_>>>(emb, ld_emb, tail_rows, head_emb, ld_head_emb,
                                                                                head_rows, target_pos, tau, above, band_cnt,
                                                                                band, band_cap, (int)n_tails, dim, ranks);
-    LKG_LAUNCH_CHECK("rank_finalize_kernel");
+    LKG_LAUNCH_CHECK("rank_finalize_kernel<dot>");
     return LKG_OK;
 }
 
@@ -803,9 +980,9 @@ extern "C" int lkg_rank_filter(const lkg_graph* known, const int64_t* heads, con
     LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kMaxChunks * kBK && ld_emb % 4 == 0 && aligned16(emb),
                 "the rank path supports dim %% 4 == 0, dim <= %d, 16-byte aligned rows", kMaxChunks * kBK);
     if (n_queries == 0) return LKG_OK;
-    rank_filter_kernel<true><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
+    rank_filter_kernel<kDot><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
                                                                                     target_pos, emb, ld_emb, dim, tau,
-                                                                                    ranks);
+                                                                                    ranks, nullptr, 0);
     LKG_LAUNCH_CHECK("rank_filter_kernel<exact>");
     return LKG_OK;
 }
@@ -819,10 +996,94 @@ extern "C" int lkg_rank_filter_scores(const lkg_graph* known, const int64_t* hea
     LKG_REQUIRE(cand_map || n_cols == known->n_entities,
                 "without a candidate map the score matrix needs one column per entity of the known plan");
     if (n_queries == 0) return LKG_OK;
-    rank_filter_kernel<false><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
+    rank_filter_kernel<kScores><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
                                                                                      target_pos, scores, ld_scores, 0,
-                                                                                     nullptr, ranks);
+                                                                                     nullptr, ranks, nullptr, 0);
     LKG_LAUNCH_CHECK("rank_filter_kernel<scores>");
+    return LKG_OK;
+}
+
+// ---- distance rank (triple score) --------------------------------------------------------------------------------
+static int check_l2_rows(const char* what, const float* p, int64_t ld, int32_t dim) {
+    LKG_REQUIRE(p, "%s is null", what);
+    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kL2MaxDim,
+                "the distance rank path supports dim %% 4 == 0, 4 <= dim <= %d (augmented width dim + 4 <= 512), got %d",
+                kL2MaxDim, dim);
+    LKG_REQUIRE(ld >= dim && ld % 4 == 0 && aligned16(p), "%s rows must be 16-byte aligned (ld %% 4 == 0, ld >= dim)",
+                what);
+    return LKG_OK;
+}
+
+extern "C" int lkg_l2_rank_rows(const float* src, int64_t ld, const int64_t* rows, int64_t m, int32_t dim,
+                                const float* center, int32_t mode, float* stats, float* out, int64_t ld_out,
+                                void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (int rc = check_l2_rows("src", src, ld, dim)) return rc;
+    LKG_REQUIRE(center && aligned16(center), "center must be a 16-byte aligned [dim] vector");
+    LKG_REQUIRE(stats && out && m >= 0, "bad operand arguments (stats, out, m)");
+    LKG_REQUIRE(ld_out >= dim + 4 && ld_out % 4 == 0 && aligned16(out),
+                "out rows need dim + 4 columns and 16-byte alignment (ld_out %% 4 == 0)");
+    LKG_REQUIRE(mode == LKG_L2_QUERY || mode == LKG_L2_CANDIDATE, "mode must be LKG_L2_QUERY or LKG_L2_CANDIDATE");
+    if (mode == LKG_L2_CANDIDATE) LKG_CUDA(cudaMemsetAsync(stats, 0, 2 * sizeof(float), stream));
+    if (m == 0) return LKG_OK;
+    const int64_t blocks = (m * 32 + 255) / 256, cap = (int64_t)sm_count() * 16;
+    const unsigned grid = (unsigned)(blocks > cap ? cap : blocks);
+    for (int pass = mode == LKG_L2_CANDIDATE ? 0 : 2; pass < (mode == LKG_L2_CANDIDATE ? 2 : 3); ++pass) {
+        l2_rank_rows_kernel<<<grid, 256, 0, stream>>>(src, ld, rows, m, dim, center, pass, stats, out, ld_out);
+        LKG_LAUNCH_CHECK("l2_rank_rows_kernel");
+    }
+    return LKG_OK;
+}
+
+extern "C" int lkg_rank_prepare_l2(const float* cand, int64_t ld_cand, const float* query, int64_t ld_query,
+                                   const float* query_aug, int64_t ld_aug, const int64_t* target_pos, int64_t n_queries,
+                                   int32_t dim, const float* stats, const float* rec_query, const float* rec_cand,
+                                   float* tau, float* thr, void* stream_) {
+    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(query_aug && ld_aug >= dim + 4 && ld_aug % 4 == 0 && aligned16(query_aug),
+                "query_aug rows need dim + 4 columns and 16-byte alignment");
+    LKG_REQUIRE(target_pos && stats && rec_query && rec_cand && tau && thr && n_queries >= 0 && n_queries < (1ll << 31),
+                "bad rank arguments");
+    if (n_queries == 0) return LKG_OK;
+    const L2Prep l2{query_aug, ld_aug, rec_query};
+    rank_prepare_kernel<kL2><<<(unsigned)((n_queries * 8 + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(
+        cand, ld_cand, nullptr, query, ld_query, nullptr, target_pos, (int)n_queries, dim, stats, rec_cand, nullptr, tau,
+        thr, l2);
+    LKG_LAUNCH_CHECK("rank_prepare_kernel<l2>");
+    return LKG_OK;
+}
+
+extern "C" int lkg_rank_finalize_l2(const float* cand, int64_t ld_cand, const float* query, int64_t ld_query,
+                                    const int64_t* target_pos, const float* tau, const int32_t* above,
+                                    const int32_t* band_cnt, const int32_t* band, int32_t band_cap, int64_t n_queries,
+                                    int64_t n_cand, int32_t dim, int64_t* ranks, void* stream_) {
+    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(target_pos && tau && above && band_cnt && band && ranks && band_cap > 0 && n_queries >= 0 &&
+                    n_queries < (1ll << 31) && n_cand >= 0 && n_cand < (1ll << 31),
+                "bad rank arguments");
+    if (n_queries == 0) return LKG_OK;
+    rank_finalize_kernel<kL2><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(
+        cand, ld_cand, nullptr, query, ld_query, nullptr, target_pos, tau, above, band_cnt, band, band_cap, (int)n_cand,
+        dim, ranks);
+    LKG_LAUNCH_CHECK("rank_finalize_kernel<l2>");
+    return LKG_OK;
+}
+
+extern "C" int lkg_rank_filter_l2(const lkg_graph* known, const int64_t* anchors, const int64_t* rels,
+                                  const int32_t* cand_map, const int64_t* target_pos, int64_t n_queries,
+                                  const float* cand, int64_t ld_cand, const float* query, int64_t ld_query, int32_t dim,
+                                  const float* tau, int64_t* ranks, void* stream_) {
+    if (int rc = check_filter_args(known, anchors, target_pos, n_queries, ranks)) return rc;
+    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(tau, "bad filter arguments");
+    if (n_queries == 0) return LKG_OK;
+    rank_filter_kernel<kL2><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, anchors, rels, cand_map,
+                                                                                   target_pos, cand, ld_cand, dim, tau,
+                                                                                   ranks, query, ld_query);
+    LKG_LAUNCH_CHECK("rank_filter_kernel<l2>");
     return LKG_OK;
 }
 

@@ -208,6 +208,15 @@ class GraphPlan:
             self._transposed = tuple(x[:self.nnz] for x in (t_tail, t_head, t_perm))
         return self._transposed
 
+    def reversed(self) -> "GraphPlan":
+        """Plan of the swapped triples (t, h, r): the known set of head prediction (?, r, t), whose filter run is the
+        heads h' of (h', r, t).  Built from this plan's own att arrays (its kept triples) on first use, cached."""
+        if getattr(self, "_reversed", None) is None:
+            counts = (self.att_rowptr[1:] - self.att_rowptr[:-1]).long()
+            heads = torch.repeat_interleave(torch.arange(self.n_entities, device=self.device), counts)
+            self._reversed = GraphPlan(self.att_tail, heads, self.att_rel, self.n_entities, self.n_relations)
+        return self._reversed
+
     def runs(self):
         """The (head, relation) RUNS of the att order (triples sorted by (h, r, t)): what the relation-projected
         attention projects once each.  -> dict(run_ptr int32 [n_runs + 1], run_head int64 [n_runs], run_rel int64

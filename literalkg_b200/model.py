@@ -1214,7 +1214,7 @@ class LiteralKG(nn.Module):
         return ops.topk_rows(scores, k, target_tails)
 
     def evaluate_ranking(self, heads, tails, relations=None, known=None, candidates=None, ks=(1, 3, 10),
-                         batch_size=2048, all_embed=None):
+                         batch_size=2048, all_embed=None, score="dot", predict="tail"):
         """Filtered link-prediction evaluation (extension: the MR / MRR / Hits@k protocol; the reference only has its
         threshold metrics).  Query i is (heads[i], relations[i] or any relation, target tails[i]).  Its raw rank is the
         rank of ``topk``: #{ j in candidates : s_j > s_t, or s_j == s_t and pos(j) < pos(t) }, 0 = best, with
@@ -1233,7 +1233,32 @@ class LiteralKG(nn.Module):
         [0, n_entities), a target that is not a candidate, duplicate candidates and relation ids outside the plan's
         range raise ValueError after it (the kernels only ever see clamped ids).
         Row partitioned (``set_partition``, world > 1) this is a collective: every rank ranks a contiguous slice of the
-        queries on the gathered embeddings, the slices are all-gathered, and every rank returns the same result."""
+        queries on the gathered embeddings, the slices are all-gathered, and every rank returns the same result.
+
+        ``predict="head"``: query i is (?, relations[i], tails[i]) with target heads[i]; the candidates are ranked as
+        heads and the filter set is { h' : (h', r, t) in known } (``known.reversed()``).  Ranks stay in input order.
+        ``score="triple"``: rank by the model's own triple score s(h, r, t) = -d(h, r, t) instead of the dot product,
+        d = |emb[h] M_r + e_r - emb[t] M_r|^2 (TransR, the distance ``calc_triplet_loss`` trains; ``model_bce``: TransE,
+        M_r = I), e_r = relation_embed.weight[r]; for head prediction the query row is emb[t] M_r - e_r.  The projected
+        rows are the fp32 results of the projection GEMM; d is exact on them (differences and squares in fp64, one
+        rounding to fp32) and the ranks are bit exact w.r.t. that rule.  ``relations`` are required (ids of the model's
+        relations); the scoring width (``relation_dim``) must be <= 508.  The queries are ranked relation by relation
+        (one host read-back of the per-relation counts, which also carries the argument checks, before the first
+        launch)."""
+        if score not in ("dot", "triple"):
+            raise ValueError('score must be "dot" or "triple"')
+        if predict not in ("tail", "head"):
+            raise ValueError('predict must be "tail" or "head"')
+        triple = score == "triple"
+        if triple:
+            if relations is None:
+                raise ValueError("the triple score needs the relation of every query")
+            d_s = self.relation_embed.weight.shape[1]
+            if d_s > ops.L2_RANK_MAX_DIM:
+                raise ValueError(f"the triple score supports widths up to {ops.L2_RANK_MAX_DIM} (relation_dim {d_s})")
+        if predict == "head":
+            heads, tails = tails, heads
+            known = None if known is None else known.reversed()
         dev = self._param_device()
         with torch.no_grad():
             if all_embed is None:
@@ -1249,8 +1274,11 @@ class LiteralKG(nn.Module):
             rels = None if relations is None else ids(relations)
             if tails.numel() != q or (rels is not None and rels.numel() != q):
                 raise ValueError("heads, tails and relations must have the same length")
-            if rels is not None and known is None:
+            if rels is not None and known is None and not triple:
                 raise ValueError("relations only select the filter set: pass the known triples as well")
+            if triple and self._triple_projection() is None and dim != self.relation_embed.weight.shape[1]:
+                raise ValueError(f"the TransE score adds relation embeddings ({self.relation_embed.weight.shape[1]} wide) "
+                                 f"to rows of the embeddings ({dim} wide)")
             if known is not None and known.n_entities != n:
                 raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
             if candidates is not None and q and len(candidates) == 0:
@@ -1275,7 +1303,10 @@ class LiteralKG(nn.Module):
                 tpos = cmap[tails].long()
                 bad["a target tail is not a candidate"] = (tpos < 0).any()
                 tpos = tpos.clamp_min(0)
-            if rels is not None:
+            if triple:               # the relation selects M_r and e_r, not only a filter run
+                bad[f"relation ids outside [0, {self.n_relations}) of the model"] = outside(rels, self.n_relations)
+                rels = rels.clamp(0, self.n_relations - 1)
+            if rels is not None and known is not None:
                 bad[f"relation ids outside [0, {known.n_relations})"] = outside(rels, known.n_relations)
                 rels = rels.clamp(0, known.n_relations - 1)
 
@@ -1285,8 +1316,17 @@ class LiteralKG(nn.Module):
             lo = 0 if world == 1 else min(q, part.rank * per)
             hi = q if world == 1 else min(q, lo + per)
             sl = slice(lo, hi)
-            ranks = self._rank_queries(all_embed, heads[sl], tpos[sl], None if rels is None else rels[sl], known, cmap,
-                                       cand, n_cand, batch_size)
+            if triple:
+                counts = torch.bincount(rels[sl], minlength=self.n_relations)
+                host = torch.cat([torch.stack(list(bad.values())).long(), counts]).tolist()
+                for msg, flag in zip(bad, host):
+                    if flag:
+                        raise ValueError(msg)
+                ranks = self._rank_triple(all_embed, heads[sl], tpos[sl], rels[sl], host[len(bad):], known, cmap, cand,
+                                          n_cand, batch_size, 1.0 if predict == "tail" else -1.0)
+            else:
+                ranks = self._rank_queries(all_embed, heads[sl], tpos[sl], None if rels is None else rels[sl], known,
+                                           cmap, cand, n_cand, batch_size)
             if world > 1:
                 padded = torch.zeros(per, dtype=torch.int64, device=dev)
                 padded[:hi - lo] = ranks
@@ -1334,6 +1374,57 @@ class LiteralKG(nn.Module):
             if known is not None:
                 ops.filter_ranks(r, known, heads[b], tpos[b], None if rels is None else rels[b], cmap, scores=scores)
             ranks[b] = r
+        return ranks
+
+    def _triple_projection(self):
+        """M_r of the triple score: TransR's ``gat_trans_M`` [R, embed width, relation_dim]; None = TransE (identity)."""
+        return self.gat_trans_M
+
+    def _rank_triple(self, all_embed, anchors, tpos, rels, counts, known, cmap, cand, n_cand, batch_size, sign):
+        """Filtered ranks under the triple score: the queries (anchor rows, target positions, relations; ``counts``
+        = host list of queries per relation) are taken relation by relation in stable order.  Per relation the
+        candidate rows are projected once (P_r = emb[cand] M_r, the projection GEMM) and indexed (``ops.L2Index``,
+        buffers reused), then each batch of queries is projected (emb[anchor] M_r + sign * e_r), ranked and filtered."""
+        dev = anchors.device
+        ranks = torch.empty(anchors.numel(), dtype=torch.int64, device=dev)
+        proj = self._triple_projection()
+        rel_w = _lib.f32c(self.relation_embed.weight.detach())
+        d_s = rel_w.shape[1]
+        d4 = (d_s + 3) // 4 * 4                  # zero columns up to a multiple of 4 add nothing to a distance
+        order = torch.sort(rels, stable=True).indices
+        qbuf = torch.zeros((max(1, min(batch_size, anchors.numel())), d4), dtype=torch.float32, device=dev)
+        if proj is None:                         # TransE: the candidate rows are the embeddings, for every relation
+            if cand is None and d4 == d_s:
+                table = all_embed
+            else:
+                table = torch.zeros((max(n_cand, 1), d4), dtype=torch.float32, device=dev)[:n_cand]
+                table[:, :d_s] = all_embed if cand is None else all_embed[cand]
+            index, cand_planes = ops.L2Index(table), None
+        else:
+            table = torch.zeros((max(n_cand, 1), d4), dtype=torch.float32, device=dev)[:n_cand]
+            index, cand_planes = None, ops.split_planes(all_embed, cand)
+        off = 0
+        for r, c in enumerate(counts):
+            if c == 0:
+                continue
+            sel, off = order[off:off + c], off + c
+            if proj is not None:
+                w_r = proj[r].detach().t()
+                ops.linear([cand_planes], w_r, None, out=table[:, :d_s])
+                index = ops.L2Index(table) if index is None else index.refill()
+            bias = rel_w[r] * sign
+            for b0 in range(0, c, batch_size):
+                qs = sel[b0:b0 + batch_size]
+                q = qbuf[:qs.numel()]
+                if proj is None:
+                    q[:, :d_s] = all_embed[anchors[qs]] + bias
+                else:
+                    ops.linear([ops.split_planes(all_embed, anchors[qs])], w_r, bias, out=q[:, :d_s])
+                tau = torch.empty(qs.numel(), dtype=torch.float32, device=dev)
+                rk = ops.score_rank_l2(index, q, tpos[qs], tau_out=tau)
+                if known is not None:
+                    ops.filter_ranks_l2(rk, known, anchors[qs], tpos[qs], rels[qs], cmap, index, q, tau)
+                ranks[qs] = rk
         return ranks
 
     def topk_sharded(self, head_ids, k, local_embed, tail_index=None):

@@ -362,6 +362,18 @@ FUSED_TOPK_MAX_DIM = 256
 FUSED_TOPK_CAP = 4096             # candidate slots per head (a head that overflows is re-scanned exactly)
 
 
+def mean_row(emb: torch.Tensor, rows: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Mean of the rows ``emb[rows]`` (None: every row), fp32 [dim]: the centre of the rank GEMMs' candidates."""
+    if rows is None:
+        center = colsum(emb)
+    else:                                        # a gathered candidate list: its own column sums
+        center = torch.zeros(emb.shape[1], dtype=torch.float32, device=emb.device)
+        for c0 in range(0, rows.numel(), 1 << 20):
+            colsum(emb[rows[c0:c0 + (1 << 20)]], out=center)
+    m = emb.shape[0] if rows is None else rows.numel()
+    return (center / float(max(m, 1))).contiguous()
+
+
 class ScoreIndex:
     """Scaled fp16 hi plane + norms of a set of rows of an embedding matrix (lkg_score_index).  The index of the
     candidate tails only depends on the embedding matrix: build it once and reuse it for every head batch."""
@@ -387,13 +399,7 @@ class ScoreIndex:
         A common shift of the tails changes no head's ranking, and the error band of the GEMM is relative to
         max|t - center| instead of max|t| (model embeddings are tightly clustered).  Built on first use."""
         if getattr(self, "_centered", None) is None:
-            if self.rows is None:
-                center = colsum(self.emb)
-            else:                                        # a gathered tail list: its own column sums
-                center = torch.zeros(self.dim, dtype=torch.float32, device=self.emb.device)
-                for c0 in range(0, self.m, 1 << 20):
-                    colsum(self.emb[self.rows[c0:c0 + (1 << 20)]], out=center)
-            center = (center / float(max(self.m, 1))).contiguous()
+            center = mean_row(self.emb, self.rows)
             shifted = torch.empty((max(self.m, 1), self.dim), dtype=torch.float32, device=self.emb.device)[:self.m]
             with _dev_guard(self.emb, "shift_rows"):
                 _lib.check(_lib.load().lkg_shift_rows(self.emb.data_ptr(), self.emb.stride(0), _lib.ptr(self.rows), self.m,
@@ -473,6 +479,111 @@ def filter_ranks(ranks: torch.Tensor, known: GraphPlan, heads: torch.Tensor, tar
                                                           _lib.ptr(cand_map), tgt.data_ptr(), ranks.numel(),
                                                           scores.data_ptr(), scores.stride(0), scores.shape[1],
                                                           ranks.data_ptr(), _lib.stream()))
+    return ranks
+
+
+# ---- distance rank: the triple score -|q - p_j|^2 (TransR / TransE) ------------------------------------------------
+L2_RANK_MAX_DIM = 508              # the augmented GEMM width dim + 4 must stay <= 512
+
+
+def l2_rank_rows(src: torch.Tensor, center: torch.Tensor, mode: int, stats: torch.Tensor,
+                 out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Augmented operand of the distance rank GEMM (lkg_l2_rank_rows): ``mode`` _lib.L2_CANDIDATE writes
+    [p - c, -|p - c|^2 / (2 alpha), 0, 0, 0] per row and fills ``stats`` (fp32 [2]); _lib.L2_QUERY writes
+    [q - c, alpha, 0, 0, 0] with alpha taken from the candidates' ``stats``.  -> fp32 [m, dim + 4]."""
+    _rowmajor(src)
+    m, dim = src.shape
+    if out is None:
+        out = torch.empty((max(m, 1), dim + 4), dtype=torch.float32, device=src.device)[:m]
+    with _dev_guard(src, "l2_rank_rows", 2 if mode == _lib.L2_CANDIDATE else 1):
+        _lib.check(_lib.load().lkg_l2_rank_rows(src.data_ptr(), src.stride(0), None, m, dim, center.data_ptr(), int(mode),
+                                                stats.data_ptr(), out.data_ptr(), out.stride(0), _lib.stream()))
+    return out
+
+
+class L2Index:
+    """Candidate side of the distance rank: the candidates' rows p_j (fp32 [Nc, dim], dim % 4 == 0, e.g. the projected
+    rows emb[cand] M_r zero padded to a multiple of 4 -- zero columns add nothing to a distance), their mean c (as
+    ``ScoreIndex.centered`` takes it), and the hi/lo planes of the augmented rows [p_j - c, -|p_j - c|^2 / (2 alpha)].
+    ``refill()`` rebuilds it in place after ``cand`` was overwritten (the next relation's projection): one relation's
+    tables are alive at a time."""
+
+    def __init__(self, cand: torch.Tensor):
+        _rowmajor(cand)
+        self.cand, (self.m, self.dim) = cand, cand.shape
+        if self.dim % 4 or self.dim > L2_RANK_MAX_DIM:
+            raise ValueError(f"the distance rank path needs a width that is a multiple of 4 and <= {L2_RANK_MAX_DIM}")
+        dev = cand.device
+        self.stats = torch.zeros(2, dtype=torch.float32, device=dev)
+        self.aug = torch.empty((max(self.m, 1), self.dim + 4), dtype=torch.float32, device=dev)[:self.m]
+        self.planes = _lib.Planes(self.m, self.dim + 4, dev)
+        self.refill()
+
+    def refill(self) -> "L2Index":
+        self.center = mean_row(self.cand)
+        l2_rank_rows(self.cand, self.center, _lib.L2_CANDIDATE, self.stats, out=self.aug)
+        split_planes(self.aug, None, out=self.planes)
+        return self
+
+
+def score_rank_l2(index: L2Index, query: torch.Tensor, target_pos: torch.Tensor, band_cap: int = 8192,
+                  tau_out: Optional[torch.Tensor] = None, stats: Optional[dict] = None) -> torch.Tensor:
+    """Rank (0 = best) of candidate ``target_pos[i]`` for query row ``query[i]`` (fp32 [B, index.dim]) under "smaller
+    exact distance first, ties -> lower position", d_j = |q_i - p_j|^2 in fp64 rounded once to fp32, without the B x Nc
+    matrix (lkg_l2_rank_rows / lkg_rank_prepare_l2 / lkg_score_rank / lkg_rank_finalize_l2).  ``tau_out`` (fp32 [B])
+    receives the exact target distances (what ``filter_ranks_l2`` compares with); ``stats`` (a dict) receives
+    "band": int32 [B] columns inside each query's error band (above ``band_cap``: the query was re-scanned exactly)."""
+    _rowmajor(query)
+    nq, dev = query.shape[0], query.device
+    assert query.shape[1] == index.dim
+    tgt = target_pos.to(device=dev, dtype=torch.int64).contiguous()
+    assert tgt.numel() == nq
+    ranks = torch.empty(nq, dtype=torch.int64, device=dev)
+    if nq == 0:
+        return ranks
+    aug = l2_rank_rows(query, index.center, _lib.L2_QUERY, index.stats)
+    qp = split_planes(aug)                               # own scale record: the two operands' factors multiply
+    tau = torch.empty(nq, dtype=torch.float32, device=dev) if tau_out is None else tau_out
+    assert tau.dtype == torch.float32 and tau.is_contiguous() and tau.numel() == nq
+    thr = torch.empty((nq, 2), dtype=torch.float32, device=dev)
+    counters = torch.zeros((2, nq), dtype=torch.int32, device=dev)
+    band = torch.empty((nq, band_cap), dtype=torch.int32, device=dev)
+    a, b = _lib.planes_operand([qp]), _lib.planes_operand([index.planes])
+    with _dev_guard(query, "score_rank_l2", 3):
+        lib = _lib.load()
+        _lib.check(lib.lkg_rank_prepare_l2(index.cand.data_ptr(), index.cand.stride(0), query.data_ptr(), query.stride(0),
+                                           aug.data_ptr(), aug.stride(0), tgt.data_ptr(), nq, index.dim,
+                                           index.stats.data_ptr(), qp.rec.data_ptr(), index.planes.rec.data_ptr(),
+                                           tau.data_ptr(), thr.data_ptr(), _lib.stream()))
+        _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), index.m, thr.data_ptr(), counters[0].data_ptr(),
+                                      counters[1].data_ptr(), band.data_ptr(), band_cap, _lib.stream()))
+        _lib.check(lib.lkg_rank_finalize_l2(index.cand.data_ptr(), index.cand.stride(0), query.data_ptr(),
+                                            query.stride(0), tgt.data_ptr(), tau.data_ptr(), counters[0].data_ptr(),
+                                            counters[1].data_ptr(), band.data_ptr(), band_cap, nq, index.m, index.dim,
+                                            ranks.data_ptr(), _lib.stream()))
+    if stats is not None:
+        stats["band"] = counters[1]
+    return ranks
+
+
+def filter_ranks_l2(ranks: torch.Tensor, known: GraphPlan, anchors: torch.Tensor, target_pos: torch.Tensor,
+                    relations: Optional[torch.Tensor], cand_map: Optional[torch.Tensor], index: L2Index,
+                    query: torch.Tensor, tau: torch.Tensor) -> torch.Tensor:
+    """``filter_ranks`` after ``score_rank_l2`` (lkg_rank_filter_l2): query i's filter set is the run of
+    (anchors[i], relations[i]) in ``known``; a member f is re-scored with the same exact distance between ``query[i]``
+    and its candidate row ``index.cand[cand_map[f]]`` and compared with the same ``tau``."""
+    assert ranks.dtype == torch.int64 and ranks.is_contiguous()
+    dev = ranks.device
+    anchors, tgt = _ids(anchors, dev), _ids(target_pos, dev)
+    rels = None if relations is None else _ids(relations, dev)
+    assert anchors.numel() == tgt.numel() == ranks.numel() and (rels is None or rels.numel() == ranks.numel())
+    assert cand_map is None or (cand_map.dtype == torch.int32 and cand_map.is_contiguous())
+    _rowmajor(query)
+    with _dev_guard(ranks, "filter_ranks_l2"):
+        _lib.check(_lib.load().lkg_rank_filter_l2(known.byref(), anchors.data_ptr(), _lib.ptr(rels), _lib.ptr(cand_map),
+                                                  tgt.data_ptr(), ranks.numel(), index.cand.data_ptr(),
+                                                  index.cand.stride(0), query.data_ptr(), query.stride(0), index.dim,
+                                                  tau.data_ptr(), ranks.data_ptr(), _lib.stream()))
     return ranks
 
 
