@@ -510,6 +510,33 @@ int lkg_rank_filter_l2(const lkg_graph* known, const int64_t* anchors, const int
                        const int32_t* cand_map /*nullable*/, const int64_t* target_pos, int64_t n_queries,
                        const float* cand, int64_t ld_cand, const float* query, int64_t ld_query, int32_t dim,
                        const float* tau, int64_t* ranks, void* stream);
+/* ---- relation-aware top-k under the triple score: the k best candidates of (h, r, ?) / (?, r, t) ----------------------
+ * Rows and d_j as for the distance rank above.  Per query i the k candidates j not excluded with the smallest d_j, ties
+ * -> lower position: dist [n_queries, k] fp32 ascending, pos [n_queries, k] int64 candidate positions (rows of the
+ * candidate table), padded with +inf / -1 when fewer than k remain.  Excluded (known NULL: nothing): the candidates
+ * whose entity id (cand_ids[j], NULL: j) is in the run of (anchors[i], rels[i]) of `known` (rels NULL: of any
+ * relation); duplicate triples count once.  Calls on one stream, after lkg_l2_rank_rows / lkg_split_planes of the
+ * query operand as for the rank:
+ *   lkg_topk_threshold_l2  theta_i = the exact k-th smallest distance among the n_sample (1 <= n_sample <= n_cand)
+ *                          strided positions floor(s n_cand / n_sample) that are not excluded (+inf if fewer than k);
+ *                          thr [n_queries][2] = {sigma - M, +inf}, sigma = (|u|^2 - theta) / 2 and M the band margin of
+ *                          lkg_rank_prepare_l2 with d_t = theta (-inf when theta is +inf); theta (nullable) [n_queries];
+ *   lkg_score_rank         the query planes against the candidate planes with thr: every column with a GEMM value
+ *                          >= sigma - M is listed in band (band_cnt / above zeroed first; above stays 0).  A column not
+ *                          listed is farther than theta, so every member of the top-k is listed;
+ *   lkg_topk_finalize_l2   the listed columns re-scored exactly, excluded ones dropped, sorted, first k written; a query
+ *                          whose list overflowed (band_cnt > cap) is re-scanned exactly over every candidate.
+ *                          1 <= k <= 1024, 2k <= cap <= 16384; shared memory next_pow2(cap) * 8 bytes per CTA. */
+int lkg_topk_threshold_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query, int64_t ld_query,
+                          const float* query_aug, int64_t ld_aug, int64_t n_queries, int32_t dim, const float* stats,
+                          const float* rec_query, const float* rec_cand, int32_t k, int32_t n_sample,
+                          const lkg_graph* known /*nullable*/, const int64_t* anchors, const int64_t* rels /*nullable*/,
+                          const int64_t* cand_ids /*nullable*/, float* thr, float* theta /*nullable*/, void* stream);
+int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query, int64_t ld_query,
+                         int64_t n_queries, int32_t dim, const int32_t* band_cnt, const int32_t* band, int32_t cap,
+                         int32_t k, const lkg_graph* known /*nullable*/, const int64_t* anchors,
+                         const int64_t* rels /*nullable*/, const int64_t* cand_ids /*nullable*/, float* dist,
+                         int64_t* pos, void* stream);
 int lkg_score_topk_workspace_bytes(int64_t n_heads, int32_t cap, int32_t sample_tiles, size_t* bytes /*host out*/);
 /* Per head the k best tails by emb[head] . emb[tail]: larger score first, ties -> lower position in the tail
  * list; values are the exact dot products (fp32 products summed in fp64, rounded once).

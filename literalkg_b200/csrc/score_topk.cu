@@ -668,6 +668,22 @@ __global__ void shift_rows_kernel(const float* __restrict__ src, int64_t ld, con
     }
 }
 
+// M of the distance band: with the GEMM value g_j of a candidate, g_j > sigma + M implies d_j < t and g_j < sigma - M
+// implies d_j > t, for a target distance t and sigma = (|u|^2 - t) / 2 (derivation in rank_prepare_kernel and DESIGN.md
+// §6 "Bound").  uu = |u|^2 and alpha: the query operand u~ = [u, alpha]; stats: the candidate operand's {W, V}; inv_q,
+// inv_c: the inverse scales (record slot 2) of the query's and the candidates' planes.  The rank prepare kernel and the
+// top-k threshold kernel both take their band from here.
+__device__ __forceinline__ double l2_band_margin(double uu, double alpha, double t, int dim, const float* stats,
+                                                 float inv_q, float inv_c) {
+    const int k = dim + 4;
+    const double w = stats[0], vmax = stats[1];
+    const double nu = __dsqrt_ru(uu) * (1.0 + 0x1p-40), nua = __dsqrt_ru(uu + alpha * alpha) * (1.0 + 0x1p-40);
+    const double e = rank_err(k) * nua * vmax + 0x1p-24 * sqrt((double)k) * 1.001 * (vmax * inv_q + nua * inv_c);
+    const double r = 0x1p-21 * (nu + w) * (nu + w);
+    const double sigma = 0.5 * (uu - t);
+    return e + 0.5 * r + 0x1p-21 * t + (uu + fabs(sigma)) * 0x1p-40 + 1e-30;
+}
+
 // What the distance instance of rank_prepare_kernel reads besides the dot instance's arguments (which it reads as:
 // emb = the candidates' projected rows p_j, head_emb = the query rows q, tail_max_norm = the stats of the candidate
 // operand, rec = the scale record of its planes).
@@ -712,14 +728,8 @@ __global__ void rank_prepare_kernel(const float* __restrict__ emb, int64_t ld, c
         uu += __shfl_xor_sync(kFull, uu, 2);
         uu += __shfl_xor_sync(kFull, uu, 1);
         if (live && q == 0) {
-            const int k = dim + 4;
-            const double w = tail_max_norm[0], vmax = tail_max_norm[1], alpha = arow[dim];
-            const double nu = __dsqrt_ru(uu) * (1.0 + 0x1p-40), nua = __dsqrt_ru(uu + alpha * alpha) * (1.0 + 0x1p-40);
-            const double e = rank_err(k) * nua * vmax + 0x1p-24 * sqrt((double)k) * 1.001 *
-                                                            (vmax * __ldg(l2.rec_q + 2) + nua * __ldg(rec + 2));
-            const double r = 0x1p-21 * (nu + w) * (nu + w);
             const double sigma = 0.5 * (uu - (double)t);
-            const double mrg = e + 0.5 * r + 0x1p-21 * (double)t + (uu + fabs(sigma)) * 0x1p-40 + 1e-30;
+            const double mrg = l2_band_margin(uu, arow[dim], t, dim, tail_max_norm, __ldg(l2.rec_q + 2), __ldg(rec + 2));
             tau[head] = t;
             thr[2 * head] = __double2float_rd(sigma - mrg);
             thr[2 * head + 1] = __double2float_ru(sigma + mrg);
@@ -892,6 +902,204 @@ __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, con
         int64_t tot = 0;
         for (int w = 0; w < nwarps; ++w) tot += s_sub[w];
         ranks[qi] -= tot;
+    }
+}
+
+// ---- relation-aware top-k under the distance (triple score) -------------------------------------------------------
+// Per query (q_i, excluded set X_i) the k candidates j not in X_i with the smallest d_j = exact_l2(q_i, p_j), ties ->
+// lower position.  The counting GEMM serves as a candidate filter (DESIGN.md §6):
+//   1. lkg_topk_threshold_l2  theta_i = the exact k-th smallest distance among S strided samples not in X_i (so at
+//                             least k admissible candidates lie within theta_i: the true k-th best is <= theta_i), and
+//                             thr_i = {sigma - M, +inf} with sigma = (|u|^2 - theta_i) / 2 and M = l2_band_margin;
+//   2. lkg_score_rank         lists every column with g_j >= sigma - M (above stays 0): g_j < sigma - M implies
+//                             d_j > theta_i, so every top-k member is listed;
+//   3. lkg_topk_finalize_l2   the listed columns re-scored with exact_l2, X_i dropped, sorted, first k written; a query
+//                             whose list overflowed is re-scanned exactly.
+constexpr int kTopkThreads = 256;
+constexpr int kThetaChunk = 1024;        // samples scored per round of the threshold kernel
+constexpr int kThetaBuf = 2048;          // kept distances: after a round <= k + kThetaChunk <= 2048 (k <= 1024)
+constexpr int kTopkMaxK = 1024;
+constexpr int kTopkMaxCap = 16384;
+
+// The excluded set of a query: the entities of the (anchors[i], rels[i]) run of a known plan (g.att_rowptr NULL: none;
+// rels NULL: of any relation), looked up by the entity id of a candidate position (cand_ids NULL: position = id).
+struct TopkExclude {
+    lkg_graph g;
+    const int64_t* anchors;
+    const int64_t* rels;
+    const int64_t* cand_ids;
+};
+
+struct KnownRun {
+    const int32_t* ent;      // sorted by entity id; duplicate triples repeat an id, which a lower bound passes over
+    int lo, hi;
+    __device__ bool has(int64_t e) const {
+        int l = lo, u = hi;
+        while (l < u) {
+            const int m = (l + u) >> 1;
+            if (ent[m] < e) l = m + 1; else u = m;
+        }
+        return l < hi && ent[l] == e;
+    }
+};
+
+__device__ __forceinline__ KnownRun known_run(const TopkExclude& x, int qi) {
+    KnownRun run{nullptr, 0, 0};
+    if (x.g.att_rowptr) filter_run(x.g, x.anchors[qi], x.rels ? x.rels[qi] : -1, &run.ent, &run.lo, &run.hi);
+    return run;
+}
+
+__device__ __forceinline__ bool is_excluded(const KnownRun& run, const TopkExclude& x, int p) {
+    return run.hi > run.lo && run.has(x.cand_ids ? x.cand_ids[p] : (int64_t)p);
+}
+
+// One CTA per query.  Samples i = 0 .. n_sample - 1 at positions floor(i n_cand / n_sample), kThetaChunk per round;
+// a sample enters the buffer only when it is closer than the current k-th smallest (theta so far), and the buffer is
+// sorted and cut to k when the next round might not fit.  Exact selection: theta is a real admissible distance.
+__global__ void __launch_bounds__(kTopkThreads) topk_threshold_l2_kernel(
+    const float* __restrict__ cand, int64_t ld, int n_cand, const float* __restrict__ query, int64_t ld_q,
+    const float* __restrict__ aug, int64_t ld_aug, int dim, int k, int n_sample, const float* __restrict__ stats,
+    const float* __restrict__ rec_q, const float* __restrict__ rec_c, const TopkExclude x, float* __restrict__ thr,
+    float* __restrict__ theta) {
+    __shared__ __align__(16) float s_q[row_floats<kL2>()];
+    __shared__ unsigned long long keys[kThetaBuf];       // ~enc(d) << 32: a descending sort puts the closest first
+    __shared__ int s_cnt;
+    __shared__ float s_theta;
+    __shared__ double s_uu;
+    const int qi = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int grp = lane >> 3, q = lane & 7;
+    const float* qrow = query + (int64_t)qi * ld_q;
+    for (int i = threadIdx.x; i < row_floats<kL2>(); i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
+    const float* arow = aug + (int64_t)qi * ld_aug;
+    if (warp == 0) {                                     // |u|^2 of the query operand, in fp64
+        double uu = 0.0;
+        for (int v = lane; v < (dim >> 2); v += 32) {
+            const float4 u = __ldg(reinterpret_cast<const float4*>(arow) + v);
+            uu = fma((double)u.x, (double)u.x, uu);
+            uu = fma((double)u.y, (double)u.y, uu);
+            uu = fma((double)u.z, (double)u.z, uu);
+            uu = fma((double)u.w, (double)u.w, uu);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) uu += __shfl_xor_sync(kFull, uu, o);
+        if (lane == 0) {
+            s_uu = uu;
+            s_cnt = 0;
+            s_theta = INFINITY;
+        }
+    }
+    const KnownRun run = known_run(x, qi);
+    __syncthreads();
+    for (int base = 0; base < n_sample; base += kThetaChunk) {
+        const int chunk = min(kThetaChunk, n_sample - base);
+        const float bound = s_theta;
+        for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {   // uniform per warp: exact_l2 shuffles
+            const int c = c0 + grp;
+            const bool live = c < chunk;
+            const int p = live ? (int)((int64_t)(base + c) * n_cand / n_sample) : 0;
+            const float d = exact_l2(s_q, cand + (int64_t)p * ld, dim, q, live);
+            if (live && q == 0 && d < bound && !is_excluded(run, x, p))
+                keys[atomicAdd(&s_cnt, 1)] = (unsigned long long)(~enc(d)) << 32;
+        }
+        __syncthreads();
+        const int cnt = s_cnt;
+        __syncthreads();                                 // every thread has read cnt before the next round adds to it
+        if (cnt > kThetaBuf - kThetaChunk || base + kThetaChunk >= n_sample) {
+            int p2 = 1;
+            while (p2 < cnt) p2 <<= 1;
+            for (int i = cnt + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
+            __syncthreads();
+            bitonic_desc(keys, p2);
+            if (threadIdx.x == 0) {
+                if (cnt >= k) s_theta = dec(~(uint32_t)(keys[k - 1] >> 32));
+                s_cnt = min(cnt, k);
+            }
+            __syncthreads();
+        }
+    }
+    if (threadIdx.x == 0) {
+        const float th = s_theta;
+        float lo = -INFINITY;                            // fewer than k admissible samples: every column is listed
+        if (th < INFINITY) {
+            const double uu = s_uu, sigma = 0.5 * (uu - (double)th);
+            lo = __double2float_rd(sigma - l2_band_margin(uu, arow[dim], th, dim, stats, __ldg(rec_q + 2),
+                                                          __ldg(rec_c + 2)));
+        }
+        thr[2 * qi] = lo;
+        thr[2 * qi + 1] = INFINITY;
+        if (theta) theta[qi] = th;
+    }
+}
+
+// One CTA per query.  keys [next_pow2(cap)]: (enc(-d) << 32) | ~position, so a descending sort gives "smaller distance
+// first, ties -> lower position"; an excluded or missing entry is key 0, which sorts last and is never written out.
+__global__ void __launch_bounds__(kTopkThreads) topk_finalize_l2_kernel(
+    const float* __restrict__ cand, int64_t ld, int n_cand, const float* __restrict__ query, int64_t ld_q, int dim,
+    const int* __restrict__ band_cnt, const int* __restrict__ band, int cap, int k, const TopkExclude x,
+    float* __restrict__ dist, int64_t* __restrict__ pos) {
+    extern __shared__ unsigned long long keys[];
+    __shared__ __align__(16) float s_q[row_floats<kL2>()];
+    __shared__ int s_kept;
+    const int qi = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int grp = lane >> 3, q = lane & 7;
+    const float* qrow = query + (int64_t)qi * ld_q;
+    for (int i = threadIdx.x; i < row_floats<kL2>(); i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
+    if (threadIdx.x == 0) s_kept = 0;
+    const KnownRun run = known_run(x, qi);
+    __syncthreads();
+    auto key_of = [&](float d, int p) -> unsigned long long {
+        return is_excluded(run, x, p) ? 0ull : ((unsigned long long)enc(-d) << 32) | (uint32_t)(~(uint32_t)p);
+    };
+    const int n_band = band_cnt[qi];
+    int n;
+    if (n_band <= cap) {
+        n = n_band;
+        const int* list = band + (int64_t)qi * cap;
+        for (int c0 = 4 * warp; c0 < n; c0 += 4 * nwarps) {
+            const int c = c0 + grp;
+            const bool live = c < n;
+            const int p = live ? list[c] : 0;
+            const float d = exact_l2(s_q, cand + (int64_t)p * ld, dim, q, live);
+            if (live && q == 0) keys[c] = key_of(d, p);
+        }
+        __syncthreads();
+        int p2 = 1;
+        while (p2 < n) p2 <<= 1;
+        for (int i = n + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
+        __syncthreads();
+        bitonic_desc(keys, p2);
+    } else {
+        // Overflow (more than cap columns listed, e.g. a weak theta or a plateau of equal distances): exact scan of
+        // every candidate keeping the best cap / 2 keys, as score_finalize_kernel does (cap / 2 >= k is checked).
+        const int half = cap / 2;
+        for (int base = 0; base < n_cand; base += half) {
+            const int chunk = min(half, n_cand - base);
+            const int kept = s_kept;
+            for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {
+                const int c = c0 + grp;
+                const bool live = c < chunk;
+                const int p = live ? base + c : 0;
+                const float d = exact_l2(s_q, cand + (int64_t)p * ld, dim, q, live);
+                if (live && q == 0) keys[kept + c] = key_of(d, p);
+            }
+            __syncthreads();
+            const int tot = kept + chunk;
+            int p2 = 1;
+            while (p2 < tot) p2 <<= 1;
+            for (int i = tot + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
+            __syncthreads();
+            bitonic_desc(keys, p2);
+            if (threadIdx.x == 0) s_kept = min(tot, half);
+            __syncthreads();
+        }
+        n = s_kept;
+    }
+    for (int i = threadIdx.x; i < k; i += blockDim.x) {
+        const unsigned long long key = i < n ? keys[i] : 0ull;
+        dist[(int64_t)qi * k + i] = key ? -dec((uint32_t)(key >> 32)) : INFINITY;
+        pos[(int64_t)qi * k + i] = key ? (int64_t)(~(uint32_t)(key & 0xffffffffu)) : -1;
     }
 }
 
@@ -1194,5 +1402,70 @@ extern "C" int lkg_score_topk(const uint16_t* heads_hi, int64_t ld_heads_hi, con
         score_finalize_kernel<<<(unsigned)nh, kFinalThreads, fsmem, stream>>>(f);
         LKG_LAUNCH_CHECK("score_finalize_kernel");
     }
+    return LKG_OK;
+}
+
+// ---- relation-aware top-k under the distance ----------------------------------------------------------------------
+static int topk_exclude(const lkg_graph* known, const int64_t* anchors, const int64_t* rels, const int64_t* cand_ids,
+                        TopkExclude* x) {
+    *x = TopkExclude{};
+    if (!known) return LKG_OK;
+    LKG_REQUIRE(known->att_rowptr && known->att_tail && known->att_rel && known->rowptr && known->col,
+                "the known plan needs its att and agg arrays");
+    LKG_REQUIRE(anchors, "the anchors are required with a known plan");
+    x->g = *known;
+    x->anchors = anchors;
+    x->rels = rels;
+    x->cand_ids = cand_ids;
+    return LKG_OK;
+}
+
+extern "C" int lkg_topk_threshold_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
+                                     int64_t ld_query, const float* query_aug, int64_t ld_aug, int64_t n_queries,
+                                     int32_t dim, const float* stats, const float* rec_query, const float* rec_cand,
+                                     int32_t k, int32_t n_sample, const lkg_graph* known, const int64_t* anchors,
+                                     const int64_t* rels, const int64_t* cand_ids, float* thr, float* theta,
+                                     void* stream_) {
+    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(query_aug && ld_aug >= dim + 4 && ld_aug % 4 == 0 && aligned16(query_aug),
+                "query_aug rows need dim + 4 columns and 16-byte alignment");
+    LKG_REQUIRE(stats && rec_query && rec_cand && thr, "bad top-k arguments (stats, rec_query, rec_cand, thr)");
+    LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
+                "bad top-k shape (n_queries, n_cand)");
+    LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
+    LKG_REQUIRE(n_sample >= 1 && n_sample <= n_cand, "n_sample must be in [1, n_cand], got %d", n_sample);
+    TopkExclude x;
+    if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
+    if (n_queries == 0) return LKG_OK;
+    topk_threshold_l2_kernel<<<(unsigned)n_queries, kTopkThreads, 0, (cudaStream_t)stream_>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, query_aug, ld_aug, dim, k, n_sample, stats, rec_query, rec_cand, x,
+        thr, theta);
+    LKG_LAUNCH_CHECK("topk_threshold_l2_kernel");
+    return LKG_OK;
+}
+
+extern "C" int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
+                                    int64_t ld_query, int64_t n_queries, int32_t dim, const int32_t* band_cnt,
+                                    const int32_t* band, int32_t cap, int32_t k, const lkg_graph* known,
+                                    const int64_t* anchors, const int64_t* rels, const int64_t* cand_ids, float* dist,
+                                    int64_t* pos, void* stream_) {
+    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(band_cnt && band && dist && pos, "bad top-k arguments (band_cnt, band, dist, pos)");
+    LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
+                "bad top-k shape (n_queries, n_cand)");
+    LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
+    LKG_REQUIRE(cap >= 2 * k && cap <= kTopkMaxCap, "cap must be in [2k, %d], got %d (k = %d)", kTopkMaxCap, cap, k);
+    TopkExclude x;
+    if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
+    if (n_queries == 0) return LKG_OK;
+    int p2 = 1;
+    while (p2 < cap) p2 <<= 1;
+    const int smem = p2 * (int)sizeof(unsigned long long);
+    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_l2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    topk_finalize_l2_kernel<<<(unsigned)n_queries, kTopkThreads, smem, (cudaStream_t)stream_>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, dist, pos);
+    LKG_LAUNCH_CHECK("topk_finalize_l2_kernel");
     return LKG_OK;
 }

@@ -1344,6 +1344,105 @@ class LiteralKG(nn.Module):
             out.update(n=q, ranks=ranks)
             return out
 
+    def topk_triple(self, anchors, relations, k, known=None, candidates=None, predict="tail", batch_size=2048,
+                    all_embed=None):
+        """Knowledge-graph completion under the model's own triple score: per query the k most likely tails of
+        (anchors[i], relations[i], ?) (``predict="tail"``) or heads of (?, relations[i], anchors[i]) (``"head"``),
+        leaving out the triples already known.  The distance is the one of ``evaluate_ranking(score="triple")``:
+        d_j = |q - emb[j] M_r|^2 with q = emb[a] M_r + e_r for tails and emb[a] M_r - e_r for heads (``model_bce``:
+        TransE, M_r = I), exact on the fp32 projected rows (fp64 differences and squares, one rounding).  Excluded:
+        { t' : (a, r, t') in known } for tails, { h' : (h', r, a) in known } for heads (``known.reversed()``); the anchor
+        itself only if it is known.  ``candidates``: entity ids (None = every entity).
+
+        Returns (dist fp32 [Q, k], ids int64 [Q, k] entity ids): per query the k non-excluded candidates ordered by
+        (d ascending, candidate position ascending), padded with +inf / -1 when fewer than k remain.  With the same
+        queries, ``batch_size`` and ``known``, ``evaluate_ranking(score="triple")`` gives entity ids[i, j] the filtered
+        rank j (the raw rank j with ``known=None``): both calls project the queries in the same batches.  1 <= k <= 1024,
+        relations are required, widths up to 508; the argument checks ride on one host read-back before the first
+        launch.  Row partitioned (``set_partition``, world > 1) this is a collective: every rank completes a contiguous
+        slice of the queries and every rank returns the whole result."""
+        if predict not in ("tail", "head"):
+            raise ValueError('predict must be "tail" or "head"')
+        if relations is None:
+            raise ValueError("the triple score needs the relation of every query")
+        if isinstance(k, bool) or int(k) != k or not 1 <= k <= ops.TOPK_L2_MAX_K:
+            raise ValueError(f"k must be an integer in [1, {ops.TOPK_L2_MAX_K}], got {k}")
+        k = int(k)
+        d_s = self.relation_embed.weight.shape[1]
+        if d_s > ops.L2_RANK_MAX_DIM:
+            raise ValueError(f"the triple score supports widths up to {ops.L2_RANK_MAX_DIM} (relation_dim {d_s})")
+        if predict == "head" and known is not None:
+            known = known.reversed()
+        dev = self._param_device()
+        with torch.no_grad():
+            if all_embed is None:
+                all_embed = self.gat_embeddings()
+            all_embed = _lib.f32c(all_embed)
+            n, dim = all_embed.shape
+
+            def ids(x):
+                return torch.as_tensor(x).to(device=dev, dtype=torch.int64).reshape(-1)
+
+            anchors, rels = ids(anchors), ids(relations)
+            q = anchors.numel()
+            if rels.numel() != q:
+                raise ValueError("anchors and relations must have the same length")
+            if self._triple_projection() is None and dim != d_s:
+                raise ValueError(f"the TransE score adds relation embeddings ({d_s} wide) to rows of the embeddings "
+                                 f"({dim} wide)")
+            if known is not None and known.n_entities != n:
+                raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
+            if candidates is not None and len(candidates) == 0:
+                raise ValueError("no candidates")
+
+            def outside(x, hi):
+                return ((x < 0) | (x >= hi)).any()
+
+            bad = {"anchor ids outside [0, n_entities)": outside(anchors, n)}
+            anchors = anchors.clamp(0, n - 1)
+            cand, n_cand = None, n
+            if candidates is not None:
+                cand = ids(candidates)
+                n_cand = cand.numel()
+                bad["candidate ids outside [0, n_entities)"] = outside(cand, n)
+                cand = cand.clamp(0, n - 1)
+                pos = torch.arange(n_cand, dtype=torch.int32, device=dev)
+                cmap = torch.full((n,), -1, dtype=torch.int32, device=dev)
+                cmap[cand] = pos
+                bad["duplicate candidate ids"] = (cmap[cand] != pos).any()
+            bad[f"relation ids outside [0, {self.n_relations}) of the model"] = outside(rels, self.n_relations)
+            rels = rels.clamp(0, self.n_relations - 1)
+            if known is not None:
+                bad[f"relation ids outside [0, {known.n_relations})"] = outside(rels, known.n_relations)
+                rels = rels.clamp(0, known.n_relations - 1)
+
+            part = self._part
+            world = 1 if part is None else part.world
+            per = max(1, (q + world - 1) // world)
+            lo = 0 if world == 1 else min(q, part.rank * per)
+            hi = q if world == 1 else min(q, lo + per)
+            sl = slice(lo, hi)
+            counts = torch.bincount(rels[sl], minlength=self.n_relations)
+            host = torch.cat([torch.stack(list(bad.values())).long(), counts]).tolist()
+            for msg, flag in zip(bad, host):
+                if flag:
+                    raise ValueError(msg)
+            mine, a_sl, r_sl = hi - lo, anchors[sl], rels[sl]
+            dist = torch.empty((mine, k), dtype=torch.float32, device=dev)
+            pos = torch.empty((mine, k), dtype=torch.int64, device=dev)
+            for qs, index, qrows in self._triple_batches(all_embed, a_sl, r_sl, host[len(bad):], cand, n_cand,
+                                                         batch_size, 1.0 if predict == "tail" else -1.0):
+                exclude = None if known is None else (known, a_sl[qs], r_sl[qs], cand)
+                dist[qs], pos[qs] = ops.score_topk_l2(index, qrows, k, exclude=exclude)
+            ent = pos if cand is None else torch.where(pos >= 0, cand[pos.clamp_min(0)], pos)
+            if world > 1:
+                pd = torch.full((per, k), float("inf"), dtype=torch.float32, device=dev)
+                pi = torch.full((per, k), -1, dtype=torch.int64, device=dev)
+                pd[:mine], pi[:mine] = dist, ent
+                dist = part.all_gather_stack(pd).reshape(-1, k)[:q]
+                ent = part.all_gather_stack(pi).reshape(-1, k)[:q]
+            return dist, ent
+
     @staticmethod
     def _rank_queries(all_embed, heads, tpos, rels, known, cmap, cand, n_cand, batch_size):
         """Filtered ranks of the queries (heads, target positions, relations or None) against the candidates ``cand``
@@ -1381,12 +1480,26 @@ class LiteralKG(nn.Module):
         return self.gat_trans_M
 
     def _rank_triple(self, all_embed, anchors, tpos, rels, counts, known, cmap, cand, n_cand, batch_size, sign):
-        """Filtered ranks under the triple score: the queries (anchor rows, target positions, relations; ``counts``
-        = host list of queries per relation) are taken relation by relation in stable order.  Per relation the
-        candidate rows are projected once (P_r = emb[cand] M_r, the projection GEMM) and indexed (``ops.L2Index``,
-        buffers reused), then each batch of queries is projected (emb[anchor] M_r + sign * e_r), ranked and filtered."""
+        """Filtered ranks under the triple score, batch by batch of ``_triple_batches``: each batch is ranked and
+        filtered on its projected query rows."""
+        ranks = torch.empty(anchors.numel(), dtype=torch.int64, device=anchors.device)
+        for qs, index, q in self._triple_batches(all_embed, anchors, rels, counts, cand, n_cand, batch_size, sign):
+            tau = torch.empty(qs.numel(), dtype=torch.float32, device=anchors.device)
+            rk = ops.score_rank_l2(index, q, tpos[qs], tau_out=tau)
+            if known is not None:
+                ops.filter_ranks_l2(rk, known, anchors[qs], tpos[qs], rels[qs], cmap, index, q, tau)
+            ranks[qs] = rk
+        return ranks
+
+    def _triple_batches(self, all_embed, anchors, rels, counts, cand, n_cand, batch_size, sign):
+        """The per-relation loop of the triple score, shared by ``evaluate_ranking`` and ``topk_triple`` so that both
+        see bit-identical rows: the queries (anchor rows, relations; ``counts`` = host list of queries per relation)
+        are taken relation by relation in stable order.  Per relation the candidate rows are projected once
+        (P_r = emb[cand] M_r, the projection GEMM) and indexed (``ops.L2Index``, buffers reused), then each batch of
+        ``batch_size`` queries is projected (emb[anchor] M_r + sign * e_r; the projection's scale record comes from the
+        batch, so the batching is part of the rows).  Yields (query indices, index, query rows [len, d4]); the index
+        and the rows are valid until the next step."""
         dev = anchors.device
-        ranks = torch.empty(anchors.numel(), dtype=torch.int64, device=dev)
         proj = self._triple_projection()
         rel_w = _lib.f32c(self.relation_embed.weight.detach())
         d_s = rel_w.shape[1]
@@ -1420,12 +1533,7 @@ class LiteralKG(nn.Module):
                     q[:, :d_s] = all_embed[anchors[qs]] + bias
                 else:
                     ops.linear([ops.split_planes(all_embed, anchors[qs])], w_r, bias, out=q[:, :d_s])
-                tau = torch.empty(qs.numel(), dtype=torch.float32, device=dev)
-                rk = ops.score_rank_l2(index, q, tpos[qs], tau_out=tau)
-                if known is not None:
-                    ops.filter_ranks_l2(rk, known, anchors[qs], tpos[qs], rels[qs], cmap, index, q, tau)
-                ranks[qs] = rk
-        return ranks
+                yield qs, index, q
 
     def topk_sharded(self, head_ids, k, local_embed, tail_index=None):
         """Row-partitioned all-entity top-k: every rank scores the heads against the entities it owns

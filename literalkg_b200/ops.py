@@ -587,6 +587,71 @@ def filter_ranks_l2(ranks: torch.Tensor, known: GraphPlan, anchors: torch.Tensor
     return ranks
 
 
+TOPK_L2_CAP = 8192                 # listed columns per query (a query that overflows is re-scanned exactly)
+TOPK_L2_MAX_K = 1024
+
+
+def topk_l2_samples(n_cand: int, k: int) -> int:
+    """Default sample count S of the top-k threshold: about k n_cand / S ~ 4096 columns fall within the sampled k-th
+    distance, plus the GEMM's error band.  Sampling costs S exact distances per query and finalize about as many
+    listed re-scores plus their sort.  Chosen from a sweep at 1 M candidates on a B200 (DESIGN.md §6): half this S
+    already lets lists overflow the default cap of 8192."""
+    return min(n_cand, max(4096, -(-k * n_cand // 4096)))
+
+
+def score_topk_l2(index: L2Index, query: torch.Tensor, k: int, exclude=None, cap: int = TOPK_L2_CAP,
+                  n_sample: Optional[int] = None, stats: Optional[dict] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Per query row ``query[i]`` (fp32 [B, index.dim]) the k candidates of ``index`` with the smallest exact distance
+    d_j = |q_i - p_j|^2 (fp64, rounded once to fp32), ties -> lower position, without the B x Nc matrix
+    (lkg_l2_rank_rows / lkg_topk_threshold_l2 / lkg_score_rank / lkg_topk_finalize_l2).  -> (dist fp32 [B, k]
+    ascending, pos int64 [B, k] candidate positions), padded with +inf / -1 when fewer than k candidates remain.
+    ``exclude`` = (known plan, anchors [B], relations [B] or None, candidate entity ids [Nc] or None = identity): query
+    i leaves out the candidates whose entity is in the (anchors[i], relations[i]) run of the plan.  ``cap``: listed
+    columns per query (2k <= cap <= 16384); ``n_sample``: samples of the threshold (default ``topk_l2_samples``);
+    ``stats`` (a dict) receives "listed" (int32 [B], above ``cap``: re-scanned exactly) and "theta" (fp32 [B])."""
+    _rowmajor(query)
+    nq, dev = query.shape[0], query.device
+    assert query.shape[1] == index.dim
+    dist = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    pos = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    if nq == 0:
+        return dist, pos
+    if n_sample is None:
+        n_sample = topk_l2_samples(index.m, k)
+    known = anchors = rels = cids = None
+    if exclude is not None:
+        known, anchors, rels, cids = exclude
+        anchors = _ids(anchors, dev)
+        rels = None if rels is None else _ids(rels, dev)
+        cids = None if cids is None else _ids(cids, dev)
+        assert anchors.numel() == nq and (rels is None or rels.numel() == nq)
+        assert cids is None or cids.numel() == index.m
+    kb = None if known is None else known.byref()
+    aug = l2_rank_rows(query, index.center, _lib.L2_QUERY, index.stats)
+    qp = split_planes(aug)                               # own scale record: the two operands' factors multiply
+    thr = torch.empty((nq, 2), dtype=torch.float32, device=dev)
+    theta = torch.empty(nq, dtype=torch.float32, device=dev)
+    counters = torch.zeros((2, nq), dtype=torch.int32, device=dev)
+    band = torch.empty((nq, max(cap, 1)), dtype=torch.int32, device=dev)
+    a, b = _lib.planes_operand([qp]), _lib.planes_operand([index.planes])
+    with _dev_guard(query, "score_topk_l2", 3):
+        lib = _lib.load()
+        _lib.check(lib.lkg_topk_threshold_l2(index.cand.data_ptr(), index.cand.stride(0), index.m, query.data_ptr(),
+                                             query.stride(0), aug.data_ptr(), aug.stride(0), nq, index.dim,
+                                             index.stats.data_ptr(), qp.rec.data_ptr(), index.planes.rec.data_ptr(),
+                                             int(k), int(n_sample), kb, _lib.ptr(anchors), _lib.ptr(rels),
+                                             _lib.ptr(cids), thr.data_ptr(), theta.data_ptr(), _lib.stream()))
+        _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), index.m, thr.data_ptr(), counters[0].data_ptr(),
+                                      counters[1].data_ptr(), band.data_ptr(), cap, _lib.stream()))
+        _lib.check(lib.lkg_topk_finalize_l2(index.cand.data_ptr(), index.cand.stride(0), index.m, query.data_ptr(),
+                                            query.stride(0), nq, index.dim, counters[1].data_ptr(), band.data_ptr(), cap,
+                                            int(k), kb, _lib.ptr(anchors), _lib.ptr(rels), _lib.ptr(cids),
+                                            dist.data_ptr(), pos.data_ptr(), _lib.stream()))
+    if stats is not None:
+        stats["listed"], stats["theta"] = counters[1], theta
+    return dist, pos
+
+
 def fused_topk_applicable(n_tails: int, dim: int, k: int) -> bool:
     """The fused path needs enough 128-tail tiles to bound the k-th best score from tile maxima."""
     return (dim <= FUSED_TOPK_MAX_DIM and dim % 4 == 0 and n_tails >= max(FUSED_TOPK_MIN_TAILS, 512 * k)
