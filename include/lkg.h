@@ -537,6 +537,38 @@ int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t n_cand, con
                          int32_t k, const lkg_graph* known /*nullable*/, const int64_t* anchors,
                          const int64_t* rels /*nullable*/, const int64_t* cand_ids /*nullable*/, float* dist,
                          int64_t* pos, void* stream);
+/* ---- filtered top-k under the dot score: the k best new links of an anchor ----------------------------------------
+ * s_j = emb[a] . emb[j], the exact dot product of lkg_score_topk (fp32 products summed in fp64, rounded once), on rows
+ * of width dim (dim % 4 == 0, 4 <= dim <= 512, 16-byte aligned).  Query i's row is query[query_rows[i]] (query_rows
+ * NULL: row i), candidate position p's row is cand[cand_rows[p]] (cand_rows NULL: row p).  Per query the k candidates
+ * not excluded with the largest s_j, ties -> lower position: score [n_queries, k] fp32 descending, pos [n_queries, k]
+ * int64 candidate positions, padded with -inf / -1 when fewer than k remain.  Excluded: as for the distance top-k
+ * above (the run of (anchors[i], rels[i]) of `known`, rels NULL: of any relation; by entity id cand_ids[p], NULL: p).
+ * Calls on one stream, with the candidate operand of ScoreIndex.centered (the rows w_p = fl(t_p - center) as hi/lo
+ * planes, their max norm cand_max_norm as lkg_score_index records it) and lkg_split_planes of the query rows:
+ *   lkg_topk_threshold_dot  theta_i = the exact k-th largest score among the n_sample (1 <= n_sample <= n_cand)
+ *                           strided positions floor(s n_cand / n_sample) that are not excluded (-inf if fewer than k);
+ *                           thr [n_queries][2] = {theta - h . center - M, +inf} rounded down, M the band margin of the
+ *                           3-product GEMM at K = dim (-inf when theta is -inf); theta (nullable) [n_queries];
+ *   lkg_score_rank          the query planes against the centred candidate planes with thr: every column whose GEMM
+ *                           value reaches thr is listed in band (band_cnt / above zeroed first; above stays 0).  A
+ *                           column not listed scores below theta, so every member of the top-k is listed;
+ *   lkg_topk_finalize_dot   the listed columns re-scored exactly on the uncentred rows, excluded ones dropped, sorted,
+ *                           first k written; a query whose list overflowed (band_cnt > cap) is re-scanned exactly.
+ *                           1 <= k <= 1024, 2k <= cap <= 16384; shared memory next_pow2(cap) * 8 bytes per CTA. */
+int lkg_topk_threshold_dot(const float* cand, int64_t ld_cand, const int64_t* cand_rows /*nullable*/, int64_t n_cand,
+                           const float* query, int64_t ld_query, const int64_t* query_rows /*nullable*/,
+                           int64_t n_queries, int32_t dim, const float* center, const float* cand_max_norm,
+                           const float* rec_query, const float* rec_cand, int32_t k, int32_t n_sample,
+                           const lkg_graph* known /*nullable*/, const int64_t* anchors,
+                           const int64_t* rels /*nullable*/, const int64_t* cand_ids /*nullable*/, float* thr,
+                           float* theta /*nullable*/, void* stream);
+int lkg_topk_finalize_dot(const float* cand, int64_t ld_cand, const int64_t* cand_rows /*nullable*/, int64_t n_cand,
+                          const float* query, int64_t ld_query, const int64_t* query_rows /*nullable*/,
+                          int64_t n_queries, int32_t dim, const int32_t* band_cnt, const int32_t* band, int32_t cap,
+                          int32_t k, const lkg_graph* known /*nullable*/, const int64_t* anchors,
+                          const int64_t* rels /*nullable*/, const int64_t* cand_ids /*nullable*/, float* score,
+                          int64_t* pos, void* stream);
 int lkg_score_topk_workspace_bytes(int64_t n_heads, int32_t cap, int32_t sample_tiles, size_t* bytes /*host out*/);
 /* Per head the k best tails by emb[head] . emb[tail]: larger score first, ties -> lower position in the tail
  * list; values are the exact dot products (fp32 products summed in fp64, rounded once).

@@ -108,6 +108,10 @@ SIGNATURES = {
                                         C.POINTER(LkgGraph), vp, vp, vp, vp, vp, vp]),
     "lkg_topk_finalize_l2": (C.c_int, [vp, i64, i64, vp, i64, i64, i32, vp, vp, i32, i32, C.POINTER(LkgGraph), vp, vp,
                                        vp, vp, vp, vp]),
+    "lkg_topk_threshold_dot": (C.c_int, [vp, i64, vp, i64, vp, i64, vp, i64, i32, vp, vp, vp, vp, i32, i32,
+                                         C.POINTER(LkgGraph), vp, vp, vp, vp, vp, vp]),
+    "lkg_topk_finalize_dot": (C.c_int, [vp, i64, vp, i64, vp, i64, vp, i64, i32, vp, vp, i32, i32, C.POINTER(LkgGraph),
+                                        vp, vp, vp, vp, vp, vp]),
     "lkg_topk_merge": (C.c_int, [vp, vp, i32, i64, i32, vp, vp, vp]),
     "lkg_score_index": (C.c_int, [vp, i64, vp, i64, i32, vp, vp, i64, vp, vp, vp]),
     "lkg_score_topk_workspace_bytes": (C.c_int, [i64, i32, i32, C.POINTER(C.c_size_t)]),

@@ -376,19 +376,22 @@ template <int Kind> constexpr int row_floats() { return Kind == kL2 ? kL2MaxDim 
 
 // Exact score of one (head, tail): fp32 products are exact in fp64, summed in fp64, one rounding to fp32 at the end.
 // Eight lanes share a tail row (lane q of the group takes float4 q, q + 8, ...), so a warp scores four candidates
-// at once with all its row loads in flight together; the head row is read from shared memory.
+// at once with all its row loads in flight together; the head row is read from shared memory.  NV float4 per lane:
+// 8 covers widths up to 256 (the rank, top-k and filter kernels), 16 up to 512 (the filtered dot top-k).  Float4
+// v >= dim / 4 is skipped, so for dim <= 256 both instances load the same values and sum them in the same order.
+template <int NV = 8>
 __device__ __forceinline__ float exact_dot8(const float* __restrict__ s_head, const float* __restrict__ trow, int dim,
                                             int q, bool live) {
     double acc = 0.0;
     const int nv = dim >> 2;                                   // dim % 4 == 0 is checked on the host side
-    float4 t[8];
+    float4 t[NV];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < NV; ++i) {
         const int v = q + 8 * i;
         t[i] = (live && v < nv) ? __ldg(reinterpret_cast<const float4*>(trow) + v) : make_float4(0, 0, 0, 0);
     }
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < NV; ++i) {
         const int v = q + 8 * i;
         if (v < nv) {
             const float4 h = *reinterpret_cast<const float4*>(s_head + 4 * v);
@@ -905,21 +908,53 @@ __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, con
     }
 }
 
-// ---- relation-aware top-k under the distance (triple score) -------------------------------------------------------
-// Per query (q_i, excluded set X_i) the k candidates j not in X_i with the smallest d_j = exact_l2(q_i, p_j), ties ->
-// lower position.  The counting GEMM serves as a candidate filter (DESIGN.md §6):
-//   1. lkg_topk_threshold_l2  theta_i = the exact k-th smallest distance among S strided samples not in X_i (so at
-//                             least k admissible candidates lie within theta_i: the true k-th best is <= theta_i), and
-//                             thr_i = {sigma - M, +inf} with sigma = (|u|^2 - theta_i) / 2 and M = l2_band_margin;
-//   2. lkg_score_rank         lists every column with g_j >= sigma - M (above stays 0): g_j < sigma - M implies
-//                             d_j > theta_i, so every top-k member is listed;
-//   3. lkg_topk_finalize_l2   the listed columns re-scored with exact_l2, X_i dropped, sorted, first k written; a query
-//                             whose list overflowed is re-scanned exactly.
+// ---- filtered top-k: the triple score (distance) and the dot score ------------------------------------------------
+// Per query (q_i, excluded set X_i) the k candidates j not in X_i with the best exact score, ties -> lower position:
+// kL2 the smallest d_j = exact_l2(q_i, p_j), kDot the largest s_j = exact_dot8<16>(h_i, t_j).  The counting GEMM
+// serves as a candidate filter (DESIGN.md §6):
+//   1. lkg_topk_threshold_*  theta_i = the exact k-th best score among S strided samples not in X_i (so at least k
+//                            admissible candidates score at least as well: the true k-th best is no worse than
+//                            theta_i), and thr_i = {lo, +inf}: kL2 lo = sigma - M with sigma = (|u|^2 - theta_i) / 2
+//                            and M = l2_band_margin, kDot lo = theta_i - h . c - M with M = dot_band_margin;
+//   2. lkg_score_rank        lists every column with g_j >= lo (above stays 0): g_j < lo implies that j scores worse
+//                            than theta_i, so every top-k member is listed;
+//   3. lkg_topk_finalize_*   the listed columns re-scored exactly, X_i dropped, sorted, first k written; a query
+//                            whose list overflowed is re-scanned exactly.
 constexpr int kTopkThreads = 256;
 constexpr int kThetaChunk = 1024;        // samples scored per round of the threshold kernel
 constexpr int kThetaBuf = 2048;          // kept distances: after a round <= k + kThetaChunk <= 2048 (k <= 1024)
 constexpr int kTopkMaxK = 1024;
 constexpr int kTopkMaxCap = 16384;
+constexpr int kTopkRow = 512;            // staged query row: the distance's augmented width, the dot score's dim
+constexpr int kDotTopkVec = kTopkRow / 32;      // float4 per lane of exact_dot8 in the dot instances
+static_assert(row_floats<kL2>() == kTopkRow, "the distance instances stage their rows as before");
+
+// M of the dot band: with the GEMM value g_j = h . w_j (w_j = fl(t_j - c), the centred candidate operand) of a
+// candidate, g_j < theta - hc - M implies s_j = fl(h . t_j) < theta (derivation in DESIGN.md §6, "Filtered top-k
+// under the dot score").  hh = |h|^2, hc = h . c and hca = sum |h_k c_k|, all three summed in fp64; max_w = max_j |w_j|
+// as lkg_score_index records it (scaled units, fp32 sums); inv_q, inv_c: the inverse scales (record slot 2) of the
+// query's and the candidates' planes.  W = max_w inv_c (1 + 2^-15) bounds max_j |w_j| in real units (the recorded norm
+// is off by less than 2^-19 relative: <= 64 fp32 additions of positive squares, a square root, the factor 1.000001).
+// Terms: the 3-product GEMM's error E at K = dim; the rounding of the centred rows, |h . (w_j - (t_j - c))| <=
+// 2^-24 |h| W; the fp64 sum of h . c over <= 512 products, <= 2^-43 hca; half an ulp of theta, <= 2^-24 |theta|
+// (2^-149 for a subnormal); and the fp64 roundings of theta - hc - M.
+__device__ __forceinline__ double dot_band_margin(double hh, double hc, double hca, double theta, int dim, float max_w,
+                                                  float inv_q, float inv_c) {
+    const double w = (double)max_w * inv_c * (1.0 + 0x1p-15);
+    const double nh = __dsqrt_ru(hh) * (1.0 + 0x1p-40);
+    const double e = rank_err(dim) * nh * w + 0x1p-24 * sqrt((double)dim) * 1.001 * (w * inv_q + nh * inv_c);
+    const double r = 0x1p-24 * nh * w * (1.0 + 0x1p-20);
+    return e + r + 0x1p-43 * hca + 0x1p-24 * fabs(theta) + 0x1p-149 + (fabs(theta) + fabs(hc)) * 0x1p-40 + 1e-30;
+}
+
+// What the dot instances of the top-k kernels read besides the distance instances' arguments (which they read as:
+// cand = the embedding rows of the candidates, query = the embedding rows of the anchors, stats = max_j |w_j| of the
+// centred candidate operand in its planes' scaled units, aug unused).
+struct TopkDot {
+    const int64_t* cand_rows;    // nullable: candidate position p -> row of cand
+    const int64_t* query_rows;   // nullable: query i -> row of query
+    const float* center;         // [dim] c, the centre the candidate operand was shifted by
+};
 
 // The excluded set of a query: the entities of the (anchors[i], rels[i]) run of a known plan (g.att_rowptr NULL: none;
 // rels NULL: of any relation), looked up by the entity id of a candidate position (cand_ids NULL: position = id).
@@ -953,40 +988,93 @@ __device__ __forceinline__ bool is_excluded(const KnownRun& run, const TopkExclu
     return run.hi > run.lo && run.has(x.cand_ids ? x.cand_ids[p] : (int64_t)p);
 }
 
+// The candidate row of position p and the exact score of the top-k kernels: kL2 the distance d (smaller is better),
+// kDot the dot product s (larger is better) on the uncentred rows.
+template <int Kind>
+__device__ __forceinline__ const float* topk_cand_row(const float* cand, int64_t ld, const TopkDot& dot, int p) {
+    if constexpr (Kind == kDot) return cand + (dot.cand_rows ? dot.cand_rows[p] : (int64_t)p) * ld;
+    else return cand + (int64_t)p * ld;
+}
+
+template <int Kind>
+__device__ __forceinline__ float topk_score(const float* s_q, const float* __restrict__ row, int dim, int q, bool live) {
+    if constexpr (Kind == kDot) return exact_dot8<kDotTopkVec>(s_q, row, dim, q, live);
+    else return exact_l2(s_q, row, dim, q, live);
+}
+
+// Order-preserving 32-bit code of a score, larger = better: enc(s) for the dot product, ~enc(d) = enc(-d) for the
+// distance (d >= 0).
+template <int Kind>
+__device__ __forceinline__ uint32_t topk_code(float s) {
+    if constexpr (Kind == kDot) return enc(s);
+    else return ~enc(s);
+}
+template <int Kind>
+__device__ __forceinline__ float topk_decode(uint32_t code) {
+    if constexpr (Kind == kDot) return dec(code);
+    else return dec(~code);
+}
+
 // One CTA per query.  Samples i = 0 .. n_sample - 1 at positions floor(i n_cand / n_sample), kThetaChunk per round;
-// a sample enters the buffer only when it is closer than the current k-th smallest (theta so far), and the buffer is
-// sorted and cut to k when the next round might not fit.  Exact selection: theta is a real admissible distance.
-__global__ void __launch_bounds__(kTopkThreads) topk_threshold_l2_kernel(
+// a sample enters the buffer only when it scores better than the current k-th best (theta so far), and the buffer is
+// sorted and cut to k when the next round might not fit.  Exact selection: theta is a real admissible score.
+template <int Kind>
+__global__ void __launch_bounds__(kTopkThreads) topk_threshold_kernel(
     const float* __restrict__ cand, int64_t ld, int n_cand, const float* __restrict__ query, int64_t ld_q,
     const float* __restrict__ aug, int64_t ld_aug, int dim, int k, int n_sample, const float* __restrict__ stats,
     const float* __restrict__ rec_q, const float* __restrict__ rec_c, const TopkExclude x, float* __restrict__ thr,
-    float* __restrict__ theta) {
-    __shared__ __align__(16) float s_q[row_floats<kL2>()];
-    __shared__ unsigned long long keys[kThetaBuf];       // ~enc(d) << 32: a descending sort puts the closest first
+    float* __restrict__ theta, const TopkDot dot) {
+    constexpr float kWorst = Kind == kDot ? -INFINITY : INFINITY;
+    __shared__ __align__(16) float s_q[kTopkRow];
+    __shared__ unsigned long long keys[kThetaBuf];       // topk_code << 32: a descending sort puts the best first
     __shared__ int s_cnt;
     __shared__ float s_theta;
-    __shared__ double s_uu;
+    __shared__ double s_uu, s_hc, s_hca;
     const int qi = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int grp = lane >> 3, q = lane & 7;
-    const float* qrow = query + (int64_t)qi * ld_q;
-    for (int i = threadIdx.x; i < row_floats<kL2>(); i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
+    const float* qrow = query + (Kind == kDot && dot.query_rows ? dot.query_rows[qi] : (int64_t)qi) * ld_q;
+    for (int i = threadIdx.x; i < kTopkRow; i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
     const float* arow = aug + (int64_t)qi * ld_aug;
-    if (warp == 0) {                                     // |u|^2 of the query operand, in fp64
-        double uu = 0.0;
+    if (warp == 0) {
+        // kL2: |u|^2 of the query operand; kDot: |h|^2, h . c and sum |h_k c_k| of the anchor row; in fp64
+        double uu = 0.0, hc = 0.0, hca = 0.0;
         for (int v = lane; v < (dim >> 2); v += 32) {
-            const float4 u = __ldg(reinterpret_cast<const float4*>(arow) + v);
-            uu = fma((double)u.x, (double)u.x, uu);
-            uu = fma((double)u.y, (double)u.y, uu);
-            uu = fma((double)u.z, (double)u.z, uu);
-            uu = fma((double)u.w, (double)u.w, uu);
+            if constexpr (Kind == kDot) {
+                const float4 h = __ldg(reinterpret_cast<const float4*>(qrow) + v);
+                const float4 c = __ldg(reinterpret_cast<const float4*>(dot.center) + v);
+                uu = fma((double)h.x, (double)h.x, uu);
+                uu = fma((double)h.y, (double)h.y, uu);
+                uu = fma((double)h.z, (double)h.z, uu);
+                uu = fma((double)h.w, (double)h.w, uu);
+                hc = fma((double)h.x, (double)c.x, hc);
+                hc = fma((double)h.y, (double)c.y, hc);
+                hc = fma((double)h.z, (double)c.z, hc);
+                hc = fma((double)h.w, (double)c.w, hc);
+                hca += fabs((double)h.x * c.x) + fabs((double)h.y * c.y) + fabs((double)h.z * c.z) +
+                       fabs((double)h.w * c.w);
+            } else {
+                const float4 u = __ldg(reinterpret_cast<const float4*>(arow) + v);
+                uu = fma((double)u.x, (double)u.x, uu);
+                uu = fma((double)u.y, (double)u.y, uu);
+                uu = fma((double)u.z, (double)u.z, uu);
+                uu = fma((double)u.w, (double)u.w, uu);
+            }
         }
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) uu += __shfl_xor_sync(kFull, uu, o);
+        for (int o = 16; o > 0; o >>= 1) {
+            uu += __shfl_xor_sync(kFull, uu, o);
+            if constexpr (Kind == kDot) {
+                hc += __shfl_xor_sync(kFull, hc, o);
+                hca += __shfl_xor_sync(kFull, hca, o);
+            }
+        }
         if (lane == 0) {
             s_uu = uu;
+            s_hc = hc;
+            s_hca = hca;
             s_cnt = 0;
-            s_theta = INFINITY;
+            s_theta = kWorst;
         }
     }
     const KnownRun run = known_run(x, qi);
@@ -994,13 +1082,14 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_l2_kernel(
     for (int base = 0; base < n_sample; base += kThetaChunk) {
         const int chunk = min(kThetaChunk, n_sample - base);
         const float bound = s_theta;
-        for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {   // uniform per warp: exact_l2 shuffles
+        for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {   // uniform per warp: the exact scores shuffle
             const int c = c0 + grp;
             const bool live = c < chunk;
             const int p = live ? (int)((int64_t)(base + c) * n_cand / n_sample) : 0;
-            const float d = exact_l2(s_q, cand + (int64_t)p * ld, dim, q, live);
-            if (live && q == 0 && d < bound && !is_excluded(run, x, p))
-                keys[atomicAdd(&s_cnt, 1)] = (unsigned long long)(~enc(d)) << 32;
+            const float s = topk_score<Kind>(s_q, topk_cand_row<Kind>(cand, ld, dot, p), dim, q, live);
+            const bool better = Kind == kDot ? s > bound : s < bound;
+            if (live && q == 0 && better && !is_excluded(run, x, p))
+                keys[atomicAdd(&s_cnt, 1)] = (unsigned long long)topk_code<Kind>(s) << 32;
         }
         __syncthreads();
         const int cnt = s_cnt;
@@ -1012,7 +1101,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_l2_kernel(
             __syncthreads();
             bitonic_desc(keys, p2);
             if (threadIdx.x == 0) {
-                if (cnt >= k) s_theta = dec(~(uint32_t)(keys[k - 1] >> 32));
+                if (cnt >= k) s_theta = topk_decode<Kind>((uint32_t)(keys[k - 1] >> 32));
                 s_cnt = min(cnt, k);
             }
             __syncthreads();
@@ -1021,10 +1110,16 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_l2_kernel(
     if (threadIdx.x == 0) {
         const float th = s_theta;
         float lo = -INFINITY;                            // fewer than k admissible samples: every column is listed
-        if (th < INFINITY) {
-            const double uu = s_uu, sigma = 0.5 * (uu - (double)th);
-            lo = __double2float_rd(sigma - l2_band_margin(uu, arow[dim], th, dim, stats, __ldg(rec_q + 2),
-                                                          __ldg(rec_c + 2)));
+        if (Kind == kDot ? th > -INFINITY : th < INFINITY) {
+            if constexpr (Kind == kDot) {
+                const double hc = s_hc;
+                lo = __double2float_rd(((double)th - hc) - dot_band_margin(s_uu, hc, s_hca, th, dim, __ldg(stats),
+                                                                           __ldg(rec_q + 2), __ldg(rec_c + 2)));
+            } else {
+                const double uu = s_uu, sigma = 0.5 * (uu - (double)th);
+                lo = __double2float_rd(sigma - l2_band_margin(uu, arow[dim], th, dim, stats, __ldg(rec_q + 2),
+                                                              __ldg(rec_c + 2)));
+            }
         }
         thr[2 * qi] = lo;
         thr[2 * qi + 1] = INFINITY;
@@ -1032,25 +1127,28 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_l2_kernel(
     }
 }
 
-// One CTA per query.  keys [next_pow2(cap)]: (enc(-d) << 32) | ~position, so a descending sort gives "smaller distance
-// first, ties -> lower position"; an excluded or missing entry is key 0, which sorts last and is never written out.
-__global__ void __launch_bounds__(kTopkThreads) topk_finalize_l2_kernel(
+// One CTA per query.  keys [next_pow2(cap)]: (enc(s) << 32) | ~position with s the dot product or -d, so a descending
+// sort gives "better score first, ties -> lower position"; an excluded or missing entry is key 0, which sorts last and
+// is never written out.
+template <int Kind>
+__global__ void __launch_bounds__(kTopkThreads) topk_finalize_kernel(
     const float* __restrict__ cand, int64_t ld, int n_cand, const float* __restrict__ query, int64_t ld_q, int dim,
     const int* __restrict__ band_cnt, const int* __restrict__ band, int cap, int k, const TopkExclude x,
-    float* __restrict__ dist, int64_t* __restrict__ pos) {
+    float* __restrict__ dist, int64_t* __restrict__ pos, const TopkDot dot) {
     extern __shared__ unsigned long long keys[];
-    __shared__ __align__(16) float s_q[row_floats<kL2>()];
+    __shared__ __align__(16) float s_q[kTopkRow];
     __shared__ int s_kept;
     const int qi = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int grp = lane >> 3, q = lane & 7;
-    const float* qrow = query + (int64_t)qi * ld_q;
-    for (int i = threadIdx.x; i < row_floats<kL2>(); i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
+    const float* qrow = query + (Kind == kDot && dot.query_rows ? dot.query_rows[qi] : (int64_t)qi) * ld_q;
+    for (int i = threadIdx.x; i < kTopkRow; i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
     if (threadIdx.x == 0) s_kept = 0;
     const KnownRun run = known_run(x, qi);
     __syncthreads();
-    auto key_of = [&](float d, int p) -> unsigned long long {
-        return is_excluded(run, x, p) ? 0ull : ((unsigned long long)enc(-d) << 32) | (uint32_t)(~(uint32_t)p);
+    auto key_of = [&](float s, int p) -> unsigned long long {
+        const uint32_t code = enc(Kind == kDot ? s : -s);
+        return is_excluded(run, x, p) ? 0ull : ((unsigned long long)code << 32) | (uint32_t)(~(uint32_t)p);
     };
     const int n_band = band_cnt[qi];
     int n;
@@ -1061,8 +1159,8 @@ __global__ void __launch_bounds__(kTopkThreads) topk_finalize_l2_kernel(
             const int c = c0 + grp;
             const bool live = c < n;
             const int p = live ? list[c] : 0;
-            const float d = exact_l2(s_q, cand + (int64_t)p * ld, dim, q, live);
-            if (live && q == 0) keys[c] = key_of(d, p);
+            const float s = topk_score<Kind>(s_q, topk_cand_row<Kind>(cand, ld, dot, p), dim, q, live);
+            if (live && q == 0) keys[c] = key_of(s, p);
         }
         __syncthreads();
         int p2 = 1;
@@ -1071,7 +1169,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_finalize_l2_kernel(
         __syncthreads();
         bitonic_desc(keys, p2);
     } else {
-        // Overflow (more than cap columns listed, e.g. a weak theta or a plateau of equal distances): exact scan of
+        // Overflow (more than cap columns listed, e.g. a weak theta or a plateau of equal scores): exact scan of
         // every candidate keeping the best cap / 2 keys, as score_finalize_kernel does (cap / 2 >= k is checked).
         const int half = cap / 2;
         for (int base = 0; base < n_cand; base += half) {
@@ -1081,8 +1179,8 @@ __global__ void __launch_bounds__(kTopkThreads) topk_finalize_l2_kernel(
                 const int c = c0 + grp;
                 const bool live = c < chunk;
                 const int p = live ? base + c : 0;
-                const float d = exact_l2(s_q, cand + (int64_t)p * ld, dim, q, live);
-                if (live && q == 0) keys[kept + c] = key_of(d, p);
+                const float s = topk_score<Kind>(s_q, topk_cand_row<Kind>(cand, ld, dot, p), dim, q, live);
+                if (live && q == 0) keys[kept + c] = key_of(s, p);
             }
             __syncthreads();
             const int tot = kept + chunk;
@@ -1098,7 +1196,8 @@ __global__ void __launch_bounds__(kTopkThreads) topk_finalize_l2_kernel(
     }
     for (int i = threadIdx.x; i < k; i += blockDim.x) {
         const unsigned long long key = i < n ? keys[i] : 0ull;
-        dist[(int64_t)qi * k + i] = key ? -dec((uint32_t)(key >> 32)) : INFINITY;
+        if constexpr (Kind == kDot) dist[(int64_t)qi * k + i] = key ? dec((uint32_t)(key >> 32)) : -INFINITY;
+        else dist[(int64_t)qi * k + i] = key ? -dec((uint32_t)(key >> 32)) : INFINITY;
         pos[(int64_t)qi * k + i] = key ? (int64_t)(~(uint32_t)(key & 0xffffffffu)) : -1;
     }
 }
@@ -1438,10 +1537,10 @@ extern "C" int lkg_topk_threshold_l2(const float* cand, int64_t ld_cand, int64_t
     TopkExclude x;
     if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
     if (n_queries == 0) return LKG_OK;
-    topk_threshold_l2_kernel<<<(unsigned)n_queries, kTopkThreads, 0, (cudaStream_t)stream_>>>(
+    topk_threshold_kernel<kL2><<<(unsigned)n_queries, kTopkThreads, 0, (cudaStream_t)stream_>>>(
         cand, ld_cand, (int)n_cand, query, ld_query, query_aug, ld_aug, dim, k, n_sample, stats, rec_query, rec_cand, x,
-        thr, theta);
-    LKG_LAUNCH_CHECK("topk_threshold_l2_kernel");
+        thr, theta, TopkDot{});
+    LKG_LAUNCH_CHECK("topk_threshold_kernel<l2>");
     return LKG_OK;
 }
 
@@ -1463,9 +1562,71 @@ extern "C" int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t 
     int p2 = 1;
     while (p2 < cap) p2 <<= 1;
     const int smem = p2 * (int)sizeof(unsigned long long);
-    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_l2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    topk_finalize_l2_kernel<<<(unsigned)n_queries, kTopkThreads, smem, (cudaStream_t)stream_>>>(
-        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, dist, pos);
-    LKG_LAUNCH_CHECK("topk_finalize_l2_kernel");
+    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_kernel<kL2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    topk_finalize_kernel<kL2><<<(unsigned)n_queries, kTopkThreads, smem, (cudaStream_t)stream_>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, dist, pos, TopkDot{});
+    LKG_LAUNCH_CHECK("topk_finalize_kernel<l2>");
+    return LKG_OK;
+}
+
+// ---- filtered top-k under the dot score -----------------------------------------------------------------------------
+static int check_dot_rows(const char* what, const float* p, int64_t ld, int32_t dim) {
+    LKG_REQUIRE(p, "%s is null", what);
+    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kTopkRow,
+                "the dot top-k path supports dim %% 4 == 0, 4 <= dim <= %d, got %d", kTopkRow, dim);
+    LKG_REQUIRE(ld >= dim && ld % 4 == 0 && aligned16(p), "%s rows must be 16-byte aligned (ld %% 4 == 0, ld >= dim)",
+                what);
+    return LKG_OK;
+}
+
+extern "C" int lkg_topk_threshold_dot(const float* cand, int64_t ld_cand, const int64_t* cand_rows, int64_t n_cand,
+                                      const float* query, int64_t ld_query, const int64_t* query_rows,
+                                      int64_t n_queries, int32_t dim, const float* center, const float* cand_max_norm,
+                                      const float* rec_query, const float* rec_cand, int32_t k, int32_t n_sample,
+                                      const lkg_graph* known, const int64_t* anchors, const int64_t* rels,
+                                      const int64_t* cand_ids, float* thr, float* theta, void* stream_) {
+    if (int rc = check_dot_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_dot_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(center && aligned16(center), "center must be a 16-byte aligned [dim] vector");
+    LKG_REQUIRE(cand_max_norm && rec_query && rec_cand && thr,
+                "bad top-k arguments (cand_max_norm, rec_query, rec_cand, thr)");
+    LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
+                "bad top-k shape (n_queries, n_cand)");
+    LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
+    LKG_REQUIRE(n_sample >= 1 && n_sample <= n_cand, "n_sample must be in [1, n_cand], got %d", n_sample);
+    TopkExclude x;
+    if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
+    if (n_queries == 0) return LKG_OK;
+    topk_threshold_kernel<kDot><<<(unsigned)n_queries, kTopkThreads, 0, (cudaStream_t)stream_>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, nullptr, 0, dim, k, n_sample, cand_max_norm, rec_query, rec_cand,
+        x, thr, theta, TopkDot{cand_rows, query_rows, center});
+    LKG_LAUNCH_CHECK("topk_threshold_kernel<dot>");
+    return LKG_OK;
+}
+
+extern "C" int lkg_topk_finalize_dot(const float* cand, int64_t ld_cand, const int64_t* cand_rows, int64_t n_cand,
+                                     const float* query, int64_t ld_query, const int64_t* query_rows,
+                                     int64_t n_queries, int32_t dim, const int32_t* band_cnt, const int32_t* band,
+                                     int32_t cap, int32_t k, const lkg_graph* known, const int64_t* anchors,
+                                     const int64_t* rels, const int64_t* cand_ids, float* score, int64_t* pos,
+                                     void* stream_) {
+    if (int rc = check_dot_rows("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_dot_rows("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(band_cnt && band && score && pos, "bad top-k arguments (band_cnt, band, score, pos)");
+    LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
+                "bad top-k shape (n_queries, n_cand)");
+    LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
+    LKG_REQUIRE(cap >= 2 * k && cap <= kTopkMaxCap, "cap must be in [2k, %d], got %d (k = %d)", kTopkMaxCap, cap, k);
+    TopkExclude x;
+    if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
+    if (n_queries == 0) return LKG_OK;
+    int p2 = 1;
+    while (p2 < cap) p2 <<= 1;
+    const int smem = p2 * (int)sizeof(unsigned long long);
+    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_kernel<kDot>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    topk_finalize_kernel<kDot><<<(unsigned)n_queries, kTopkThreads, smem, (cudaStream_t)stream_>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, score, pos,
+        TopkDot{cand_rows, query_rows, nullptr});
+    LKG_LAUNCH_CHECK("topk_finalize_kernel<dot>");
     return LKG_OK;
 }

@@ -48,6 +48,39 @@ def _identity(n: int, device) -> torch.Tensor:
     return _EYE[key]
 
 
+def _query_ids(x, dev) -> torch.Tensor:
+    """Ids of a query call (any sequence or tensor) as a flat int64 tensor on ``dev``."""
+    return torch.as_tensor(x).to(device=dev, dtype=torch.int64).reshape(-1)
+
+
+def _outside(x: torch.Tensor, hi: int) -> torch.Tensor:
+    """Device flag: some id of ``x`` lies outside [0, hi)."""
+    return ((x < 0) | (x >= hi)).any()
+
+
+def _candidate_ids(candidates, n: int, dev, bad: dict):
+    """The candidate list of a query call: -> (cand int64 clamped to [0, n), n_cand, cmap int32 [n] = candidate position
+    of every entity or -1), or (None, n, None) for every entity.  Adds the device flags "candidate ids outside
+    [0, n_entities)" and "duplicate candidate ids" to ``bad``; they are raised after the call's one host read-back."""
+    if candidates is None:
+        return None, n, None
+    cand = _query_ids(candidates, dev)
+    n_cand = cand.numel()
+    bad["candidate ids outside [0, n_entities)"] = _outside(cand, n)
+    cand = cand.clamp(0, n - 1)
+    pos = torch.arange(n_cand, dtype=torch.int32, device=dev)
+    cmap = torch.full((n,), -1, dtype=torch.int32, device=dev)
+    cmap[cand] = pos
+    bad["duplicate candidate ids"] = (cmap[cand] != pos).any()
+    return cand, n_cand, cmap
+
+
+def _raise_flags(bad: dict, host: list) -> None:
+    for msg, flag in zip(bad, host):
+        if flag:
+            raise ValueError(msg)
+
+
 def _L2_loss_mean(x):
     return torch.mean(torch.sum(torch.pow(x, 2), dim=1, keepdim=False) / 2.)
 
@@ -1266,12 +1299,9 @@ class LiteralKG(nn.Module):
             all_embed = _lib.f32c(all_embed)
             n, dim = all_embed.shape
 
-            def ids(x):
-                return torch.as_tensor(x).to(device=dev, dtype=torch.int64).reshape(-1)
-
-            heads, tails = ids(heads), ids(tails)
+            heads, tails = _query_ids(heads, dev), _query_ids(tails, dev)
             q = heads.numel()
-            rels = None if relations is None else ids(relations)
+            rels = None if relations is None else _query_ids(relations, dev)
             if tails.numel() != q or (rels is not None and rels.numel() != q):
                 raise ValueError("heads, tails and relations must have the same length")
             if rels is not None and known is None and not triple:
@@ -1284,44 +1314,27 @@ class LiteralKG(nn.Module):
             if candidates is not None and q and len(candidates) == 0:
                 raise ValueError("no candidates")
 
-            def outside(x, hi):
-                return ((x < 0) | (x >= hi)).any()
-
-            bad = {"head or tail ids outside [0, n_entities)": outside(heads, n) | outside(tails, n)}
+            bad = {"head or tail ids outside [0, n_entities)": _outside(heads, n) | _outside(tails, n)}
             heads, tails = heads.clamp(0, n - 1), tails.clamp(0, n - 1)
-            cmap = cand = None
-            tpos, n_cand = tails, n
+            cand, n_cand, cmap = _candidate_ids(candidates, n, dev, bad)
+            tpos = tails
             if candidates is not None:
-                cand = ids(candidates)
-                n_cand = cand.numel()
-                bad["candidate ids outside [0, n_entities)"] = outside(cand, n)
-                cand = cand.clamp(0, n - 1)
-                pos = torch.arange(n_cand, dtype=torch.int32, device=dev)
-                cmap = torch.full((n,), -1, dtype=torch.int32, device=dev)
-                cmap[cand] = pos
-                bad["duplicate candidate ids"] = (cmap[cand] != pos).any()
                 tpos = cmap[tails].long()
                 bad["a target tail is not a candidate"] = (tpos < 0).any()
                 tpos = tpos.clamp_min(0)
             if triple:               # the relation selects M_r and e_r, not only a filter run
-                bad[f"relation ids outside [0, {self.n_relations}) of the model"] = outside(rels, self.n_relations)
+                bad[f"relation ids outside [0, {self.n_relations}) of the model"] = _outside(rels, self.n_relations)
                 rels = rels.clamp(0, self.n_relations - 1)
             if rels is not None and known is not None:
-                bad[f"relation ids outside [0, {known.n_relations})"] = outside(rels, known.n_relations)
+                bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
                 rels = rels.clamp(0, known.n_relations - 1)
 
-            part = self._part
-            world = 1 if part is None else part.world
-            per = max(1, (q + world - 1) // world)
-            lo = 0 if world == 1 else min(q, part.rank * per)
-            hi = q if world == 1 else min(q, lo + per)
+            part, world, per, lo, hi = self._query_slice(q)
             sl = slice(lo, hi)
             if triple:
                 counts = torch.bincount(rels[sl], minlength=self.n_relations)
                 host = torch.cat([torch.stack(list(bad.values())).long(), counts]).tolist()
-                for msg, flag in zip(bad, host):
-                    if flag:
-                        raise ValueError(msg)
+                _raise_flags(bad, host)
                 ranks = self._rank_triple(all_embed, heads[sl], tpos[sl], rels[sl], host[len(bad):], known, cmap, cand,
                                           n_cand, batch_size, 1.0 if predict == "tail" else -1.0)
             else:
@@ -1336,9 +1349,7 @@ class LiteralKG(nn.Module):
             ks = [int(k) for k in ks]
             metrics = [r1.mean(), (1.0 / r1).mean()] + [(ranks < k).double().mean() for k in ks]
             host = torch.cat([torch.stack(metrics), torch.stack(list(bad.values())).double()]).tolist()
-            for msg, flag in zip(bad, host[len(metrics):]):
-                if flag:
-                    raise ValueError(msg)
+            _raise_flags(bad, host[len(metrics):])
             out = {"mr": host[0], "mrr": host[1]}
             out.update({f"hits@{k}": v for k, v in zip(ks, host[2:len(metrics)])})
             out.update(n=q, ranks=ranks)
@@ -1380,10 +1391,7 @@ class LiteralKG(nn.Module):
             all_embed = _lib.f32c(all_embed)
             n, dim = all_embed.shape
 
-            def ids(x):
-                return torch.as_tensor(x).to(device=dev, dtype=torch.int64).reshape(-1)
-
-            anchors, rels = ids(anchors), ids(relations)
+            anchors, rels = _query_ids(anchors, dev), _query_ids(relations, dev)
             q = anchors.numel()
             if rels.numel() != q:
                 raise ValueError("anchors and relations must have the same length")
@@ -1395,38 +1403,20 @@ class LiteralKG(nn.Module):
             if candidates is not None and len(candidates) == 0:
                 raise ValueError("no candidates")
 
-            def outside(x, hi):
-                return ((x < 0) | (x >= hi)).any()
-
-            bad = {"anchor ids outside [0, n_entities)": outside(anchors, n)}
+            bad = {"anchor ids outside [0, n_entities)": _outside(anchors, n)}
             anchors = anchors.clamp(0, n - 1)
-            cand, n_cand = None, n
-            if candidates is not None:
-                cand = ids(candidates)
-                n_cand = cand.numel()
-                bad["candidate ids outside [0, n_entities)"] = outside(cand, n)
-                cand = cand.clamp(0, n - 1)
-                pos = torch.arange(n_cand, dtype=torch.int32, device=dev)
-                cmap = torch.full((n,), -1, dtype=torch.int32, device=dev)
-                cmap[cand] = pos
-                bad["duplicate candidate ids"] = (cmap[cand] != pos).any()
-            bad[f"relation ids outside [0, {self.n_relations}) of the model"] = outside(rels, self.n_relations)
+            cand, n_cand, _ = _candidate_ids(candidates, n, dev, bad)
+            bad[f"relation ids outside [0, {self.n_relations}) of the model"] = _outside(rels, self.n_relations)
             rels = rels.clamp(0, self.n_relations - 1)
             if known is not None:
-                bad[f"relation ids outside [0, {known.n_relations})"] = outside(rels, known.n_relations)
+                bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
                 rels = rels.clamp(0, known.n_relations - 1)
 
-            part = self._part
-            world = 1 if part is None else part.world
-            per = max(1, (q + world - 1) // world)
-            lo = 0 if world == 1 else min(q, part.rank * per)
-            hi = q if world == 1 else min(q, lo + per)
+            part, world, per, lo, hi = self._query_slice(q)
             sl = slice(lo, hi)
             counts = torch.bincount(rels[sl], minlength=self.n_relations)
             host = torch.cat([torch.stack(list(bad.values())).long(), counts]).tolist()
-            for msg, flag in zip(bad, host):
-                if flag:
-                    raise ValueError(msg)
+            _raise_flags(bad, host)
             mine, a_sl, r_sl = hi - lo, anchors[sl], rels[sl]
             dist = torch.empty((mine, k), dtype=torch.float32, device=dev)
             pos = torch.empty((mine, k), dtype=torch.int64, device=dev)
@@ -1434,14 +1424,107 @@ class LiteralKG(nn.Module):
                                                          batch_size, 1.0 if predict == "tail" else -1.0):
                 exclude = None if known is None else (known, a_sl[qs], r_sl[qs], cand)
                 dist[qs], pos[qs] = ops.score_topk_l2(index, qrows, k, exclude=exclude)
-            ent = pos if cand is None else torch.where(pos >= 0, cand[pos.clamp_min(0)], pos)
-            if world > 1:
-                pd = torch.full((per, k), float("inf"), dtype=torch.float32, device=dev)
-                pi = torch.full((per, k), -1, dtype=torch.int64, device=dev)
-                pd[:mine], pi[:mine] = dist, ent
-                dist = part.all_gather_stack(pd).reshape(-1, k)[:q]
-                ent = part.all_gather_stack(pi).reshape(-1, k)[:q]
-            return dist, ent
+            return self._gather_topk(dist, pos, cand, q, per, float("inf"))
+
+    def topk_links(self, anchors, k, relations=None, known=None, candidates=None, predict="tail", batch_size=2048,
+                   all_embed=None):
+        """Link prediction under the fine-tuned dot score s(a, j) = emb[a] . emb[j] (``calc_score``): per anchor the k
+        most likely new tails (``predict="tail"``) or heads (``"head"``; the score is symmetric, so only the excluded
+        set changes), leaving out the links already known.  s_j is the exact dot product ``score_topk`` returns and
+        the fused ``evaluate_ranking(score="dot")`` compares (fp32 products summed in fp64, rounded once).  Excluded:
+        { t' : (a, relations[i], t') in known } with relations, { t' : (a, any r, t') in known } without -- the filter
+        set of ``evaluate_ranking``; for heads the same sets of ``known.reversed()``.  Duplicate triples count once,
+        non-candidates are ignored, the anchor itself is excluded only if it is known.  ``candidates``: entity ids
+        (None = every entity).
+
+        Returns (scores fp32 [Q, k], ids int64 [Q, k] entity ids): per query the k non-excluded candidates ordered by
+        (s descending, candidate position ascending), padded with -inf / -1 when fewer than k remain.  With the same
+        ``known`` and ``relations``, ``evaluate_ranking`` gives entity ids[i, j] the filtered rank j wherever it takes
+        its fused path.  1 <= k <= 1024; embedding widths up to 512 (a width that is not a multiple of 4 is zero padded
+        once per call).  One embedding pass (or the given ``all_embed``), one candidate index for all batches of
+        ``batch_size`` queries, no B x N score matrix at any width; the argument checks ride on one host read-back
+        before the first launch.  Row partitioned (``set_partition``, world > 1) this is a collective: every rank
+        completes a contiguous slice of the queries and every rank returns the whole result."""
+        if predict not in ("tail", "head"):
+            raise ValueError('predict must be "tail" or "head"')
+        if isinstance(k, bool) or int(k) != k or not 1 <= k <= ops.TOPK_L2_MAX_K:
+            raise ValueError(f"k must be an integer in [1, {ops.TOPK_L2_MAX_K}], got {k}")
+        k = int(k)
+        if relations is not None and known is None:
+            raise ValueError("relations only select the excluded set: pass the known triples as well")
+
+        def check_width(emb):
+            if emb.shape[1] > ops.TOPK_DOT_MAX_DIM:
+                raise ValueError(f"the dot top-k supports widths up to {ops.TOPK_DOT_MAX_DIM} (got {emb.shape[1]})")
+
+        if all_embed is not None:
+            check_width(all_embed)
+        if predict == "head" and known is not None:
+            known = known.reversed()
+        dev = self._param_device()
+        with torch.no_grad():
+            if all_embed is None:
+                all_embed = self.gat_embeddings()
+                check_width(all_embed)
+            all_embed = _lib.f32c(all_embed)
+            n, dim = all_embed.shape
+            anchors = _query_ids(anchors, dev)
+            q = anchors.numel()
+            rels = None if relations is None else _query_ids(relations, dev)
+            if rels is not None and rels.numel() != q:
+                raise ValueError("anchors and relations must have the same length")
+            if known is not None and known.n_entities != n:
+                raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
+            if candidates is not None and len(candidates) == 0:
+                raise ValueError("no candidates")
+
+            bad = {"anchor ids outside [0, n_entities)": _outside(anchors, n)}
+            anchors = anchors.clamp(0, n - 1)
+            cand, n_cand, _ = _candidate_ids(candidates, n, dev, bad)
+            if rels is not None:
+                bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
+                rels = rels.clamp(0, known.n_relations - 1)
+            part, world, per, lo, hi = self._query_slice(q)
+            _raise_flags(bad, torch.stack(list(bad.values())).tolist())
+
+            if dim % 4:                          # zero columns add nothing to a dot product
+                padded = torch.zeros((n, (dim + 3) // 4 * 4), dtype=torch.float32, device=dev)
+                padded[:, :dim] = all_embed
+                all_embed = padded
+            index = ops.ScoreIndex(all_embed, cand)
+            mine, a_sl = hi - lo, anchors[lo:hi]
+            r_sl = None if rels is None else rels[lo:hi]
+            vals = torch.empty((mine, k), dtype=torch.float32, device=dev)
+            pos = torch.empty((mine, k), dtype=torch.int64, device=dev)
+            for b0 in range(0, mine, batch_size):
+                b = slice(b0, b0 + batch_size)
+                exclude = None if known is None else (known, a_sl[b], None if r_sl is None else r_sl[b], cand)
+                vals[b], pos[b] = ops.score_topk_dot(all_embed, a_sl[b], k, index, exclude=exclude)
+            return self._gather_topk(vals, pos, cand, q, per, float("-inf"))
+
+    def _query_slice(self, q: int):
+        """The queries a rank answers in a row-partitioned collective: -> (part, world, per, lo, hi), a contiguous
+        slice [lo, hi) of ``per`` = ceil(q / world) queries (world 1: all of them)."""
+        part = self._part
+        world = 1 if part is None else part.world
+        per = max(1, (q + world - 1) // world)
+        lo = 0 if world == 1 else min(q, part.rank * per)
+        hi = q if world == 1 else min(q, lo + per)
+        return part, world, per, lo, hi
+
+    def _gather_topk(self, vals, pos, cand, q, per, pad):
+        """Candidate positions -> entity ids (-1 pads stay), then, row partitioned, the [per, k] slices of every rank
+        all-gathered (padded with ``pad`` / -1) into the whole [q, k] result."""
+        ent = pos if cand is None else torch.where(pos >= 0, cand[pos.clamp_min(0)], pos)
+        part = self._part
+        if part is not None and part.world > 1:
+            k, mine = vals.shape[1], vals.shape[0]
+            pv = torch.full((per, k), pad, dtype=torch.float32, device=vals.device)
+            pi = torch.full((per, k), -1, dtype=torch.int64, device=vals.device)
+            pv[:mine], pi[:mine] = vals, ent
+            vals = part.all_gather_stack(pv).reshape(-1, k)[:q]
+            ent = part.all_gather_stack(pi).reshape(-1, k)[:q]
+        return vals, ent
 
     @staticmethod
     def _rank_queries(all_embed, heads, tpos, rels, known, cmap, cand, n_cand, batch_size):

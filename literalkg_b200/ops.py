@@ -652,6 +652,67 @@ def score_topk_l2(index: L2Index, query: torch.Tensor, k: int, exclude=None, cap
     return dist, pos
 
 
+TOPK_DOT_MAX_DIM = 512
+
+
+def score_topk_dot(emb: torch.Tensor, anchors: torch.Tensor, k: int, index: ScoreIndex, exclude=None,
+                   cap: int = TOPK_L2_CAP, n_sample: Optional[int] = None,
+                   stats: Optional[dict] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Per anchor row ``emb[anchors[i]]`` the k candidates of ``index`` (rows of ``index.emb``) with the largest exact
+    dot product s_j = emb[a] . t_j (fp32 products summed in fp64, rounded once: the value ``score_topk`` returns), ties
+    -> lower position, without the B x Nc matrix (lkg_topk_threshold_dot / lkg_score_rank / lkg_topk_finalize_dot on
+    the centred candidate operand of ``index.centered()``).  Widths dim % 4 == 0 up to 512.  -> (scores fp32 [B, k]
+    descending, pos int64 [B, k] candidate positions), padded with -inf / -1 when fewer than k candidates remain.
+    ``exclude``, ``cap``, ``n_sample`` and ``stats`` as for ``score_topk_l2`` (the default sample count is
+    ``topk_l2_samples``: a sweep under the dot score at 1 M candidates kept it, DESIGN.md §6)."""
+    _rowmajor(emb)
+    dev, dim = emb.device, emb.shape[1]
+    assert index.dim == dim and index.emb.stride(1) == 1
+    anchors = _ids(anchors, dev)
+    nq = anchors.numel()
+    vals = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    pos = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    if nq == 0:
+        return vals, pos
+    if n_sample is None:
+        n_sample = topk_l2_samples(index.m, k)
+    known = ex_anchors = rels = cids = None
+    if exclude is not None:
+        known, ex_anchors, rels, cids = exclude
+        ex_anchors = _ids(ex_anchors, dev)
+        rels = None if rels is None else _ids(rels, dev)
+        cids = None if cids is None else _ids(cids, dev)
+        assert ex_anchors.numel() == nq and (rels is None or rels.numel() == nq)
+        assert cids is None or cids.numel() == index.m
+    kb = None if known is None else known.byref()
+    center, ci, cp = index.centered()
+    qp = split_planes(emb, anchors)                      # own scale record: the two operands' factors multiply
+    thr = torch.empty((nq, 2), dtype=torch.float32, device=dev)
+    theta = torch.empty(nq, dtype=torch.float32, device=dev)
+    counters = torch.zeros((2, nq), dtype=torch.int32, device=dev)
+    band = torch.empty((nq, max(cap, 1)), dtype=torch.int32, device=dev)
+    a, b = _lib.planes_operand([qp]), _lib.planes_operand([cp])
+    src = index.emb
+    with _dev_guard(emb, "score_topk_dot", 3):
+        lib = _lib.load()
+        _lib.check(lib.lkg_topk_threshold_dot(src.data_ptr(), src.stride(0), _lib.ptr(index.rows), index.m,
+                                              emb.data_ptr(), emb.stride(0), anchors.data_ptr(), nq, dim,
+                                              center.data_ptr(), ci.max_norm.data_ptr(), qp.rec.data_ptr(),
+                                              ci.rec.data_ptr(), int(k), int(n_sample), kb, _lib.ptr(ex_anchors),
+                                              _lib.ptr(rels), _lib.ptr(cids), thr.data_ptr(), theta.data_ptr(),
+                                              _lib.stream()))
+        _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), index.m, thr.data_ptr(), counters[0].data_ptr(),
+                                      counters[1].data_ptr(), band.data_ptr(), cap, _lib.stream()))
+        _lib.check(lib.lkg_topk_finalize_dot(src.data_ptr(), src.stride(0), _lib.ptr(index.rows), index.m,
+                                             emb.data_ptr(), emb.stride(0), anchors.data_ptr(), nq, dim,
+                                             counters[1].data_ptr(), band.data_ptr(), cap, int(k), kb,
+                                             _lib.ptr(ex_anchors), _lib.ptr(rels), _lib.ptr(cids), vals.data_ptr(),
+                                             pos.data_ptr(), _lib.stream()))
+    if stats is not None:
+        stats["listed"], stats["theta"] = counters[1], theta
+    return vals, pos
+
+
 def fused_topk_applicable(n_tails: int, dim: int, k: int) -> bool:
     """The fused path needs enough 128-tail tiles to bound the k-th best score from tile maxima."""
     return (dim <= FUSED_TOPK_MAX_DIM and dim % 4 == 0 and n_tails >= max(FUSED_TOPK_MIN_TAILS, 512 * k)

@@ -27,7 +27,7 @@ import torch
 
 from eval_ranking import device_info, embeddings
 
-KERNELS = {"threshold": "topk_threshold_l2_kernel", "gemm": "tc_gemm_kernel", "finalize": "topk_finalize_l2_kernel"}
+KERNELS = {"threshold": "topk_threshold_kernel<1>", "gemm": "tc_gemm_kernel", "finalize": "topk_finalize_kernel<1>"}
 
 
 def one_relation(index, queries, k, n_sample, cap, exclude_of):
