@@ -323,42 +323,9 @@ __global__ void score_threshold_kernel(const float* __restrict__ theta, int64_t 
     thr[i] = th == -INFINITY ? -INFINITY : th * s2 - err - fabsf(th * s2) * 1e-6f;
 }
 
-// thr = (k-th largest tile maximum of the sampled tiles) - 2E.  The tile maxima are k distinct tails whose
-// APPROXIMATE scores reach m_k, so their exact scores reach m_k - E, so the exact k-th best is >= m_k - E and every
-// member of the true top-k has an approximate score >= m_k - 2E.  One CTA per head, bitonic sort in shared memory.
-__global__ void __launch_bounds__(256) score_sample_threshold_kernel(const float* __restrict__ tilemax, int n_st, int k,
-                                                                     const float* __restrict__ head_norms,
-                                                                     const float* __restrict__ tail_max_norm, int dim,
-                                                                     float* __restrict__ thr) {
-    extern __shared__ float sv[];
-    const int head = blockIdx.x;
-    int p2 = 1;
-    while (p2 < n_st) p2 <<= 1;
-    for (int i = threadIdx.x; i < p2; i += blockDim.x) sv[i] = i < n_st ? tilemax[(int64_t)head * n_st + i] : -INFINITY;
-    __syncthreads();
-    for (int size = 2; size <= p2; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            for (int i = threadIdx.x; i < p2; i += blockDim.x) {
-                const int j = i ^ stride;
-                if (j > i) {
-                    const bool desc = (i & size) == 0;
-                    const float a = sv[i], b = sv[j];
-                    if ((a < b) == desc) {
-                        sv[i] = b;
-                        sv[j] = a;
-                    }
-                }
-            }
-            __syncthreads();
-        }
-    }
-    if (threadIdx.x == 0) {
-        const float mk = k <= n_st ? sv[k - 1] : -INFINITY;
-        thr[head] = mk == -INFINITY ? -INFINITY : mk - 2.f * score_err(head_norms[head], *tail_max_norm, dim) - fabsf(mk) * 1e-6f;
-    }
-}
-
-// ---- finalize ----------------------------------------------------------------------------------------------------
+// ---- keys and their sort -----------------------------------------------------------------------------------------
+// enc: order-preserving 32-bit code of a float (-0 < +0); the selection kernels sort 64-bit keys (enc(s) << 32) | ~p,
+// so a descending sort gives "larger score first, ties -> lower position", and key 0 sorts last.
 __device__ __forceinline__ uint32_t enc(float f) {
     const uint32_t u = __float_as_uint(f);
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -367,93 +334,16 @@ __device__ __forceinline__ float dec(uint32_t u) {
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
-// Score kinds of the rank kernels: the dot product emb[h] . emb[j], or the negated squared distance -|q - p_j|^2 of the
-// relation-aware triple score (TransR / TransE), and the dense instance of the filter that reads a score matrix.
-constexpr int kDot = 0, kL2 = 1, kScores = 2;
-constexpr int kL2MaxDim = 508;           // distance rows: dim % 4 == 0, the augmented width dim + 4 <= 512
-constexpr int kL2Vec = (kL2MaxDim + 4) / 32;    // float4 per lane in exact_l2 (8 lanes per row)
-template <int Kind> constexpr int row_floats() { return Kind == kL2 ? kL2MaxDim + 4 : kMaxChunks * kBK; }
-
-// Exact score of one (head, tail): fp32 products are exact in fp64, summed in fp64, one rounding to fp32 at the end.
-// Eight lanes share a tail row (lane q of the group takes float4 q, q + 8, ...), so a warp scores four candidates
-// at once with all its row loads in flight together; the head row is read from shared memory.  NV float4 per lane:
-// 8 covers widths up to 256 (the rank, top-k and filter kernels), 16 up to 512 (the filtered dot top-k).  Float4
-// v >= dim / 4 is skipped, so for dim <= 256 both instances load the same values and sum them in the same order.
-template <int NV = 8>
-__device__ __forceinline__ float exact_dot8(const float* __restrict__ s_head, const float* __restrict__ trow, int dim,
-                                            int q, bool live) {
-    double acc = 0.0;
-    const int nv = dim >> 2;                                   // dim % 4 == 0 is checked on the host side
-    float4 t[NV];
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        const int v = q + 8 * i;
-        t[i] = (live && v < nv) ? __ldg(reinterpret_cast<const float4*>(trow) + v) : make_float4(0, 0, 0, 0);
-    }
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        const int v = q + 8 * i;
-        if (v < nv) {
-            const float4 h = *reinterpret_cast<const float4*>(s_head + 4 * v);
-            acc = fma((double)h.x, (double)t[i].x, acc);
-            acc = fma((double)h.y, (double)t[i].y, acc);
-            acc = fma((double)h.z, (double)t[i].z, acc);
-            acc = fma((double)h.w, (double)t[i].w, acc);
-        }
-    }
-    acc += __shfl_xor_sync(kFull, acc, 4);
-    acc += __shfl_xor_sync(kFull, acc, 2);
-    acc += __shfl_xor_sync(kFull, acc, 1);
-    return (float)acc;
-}
-
-// Exact squared distance |a - b|^2 of two fp32 rows: each difference is exact in fp64, squared and summed in fp64
-// (one fma per element), one rounding to fp32.  The lane layout of exact_dot8 over widths up to 512.  `a` (the query
-// row) may live in shared or global memory: prepare reads it from global, finalize and the filter from shared memory,
-// and the three see the same values in the same order, so they return the same bits.
-__device__ __forceinline__ float exact_l2(const float* a, const float* __restrict__ b, int dim, int q, bool live) {
-    double acc = 0.0;
-    const int nv = dim >> 2;                                   // dim % 4 == 0 is checked on the host side
-    float4 t[kL2Vec];
-#pragma unroll
-    for (int i = 0; i < kL2Vec; ++i) {
-        const int v = q + 8 * i;
-        t[i] = (live && v < nv) ? __ldg(reinterpret_cast<const float4*>(b) + v) : make_float4(0, 0, 0, 0);
-    }
-#pragma unroll
-    for (int i = 0; i < kL2Vec; ++i) {
-        const int v = q + 8 * i;
-        if (v < nv) {
-            const float4 h = *reinterpret_cast<const float4*>(a + 4 * v);
-            double d = (double)h.x - (double)t[i].x;
-            acc = fma(d, d, acc);
-            d = (double)h.y - (double)t[i].y;
-            acc = fma(d, d, acc);
-            d = (double)h.z - (double)t[i].z;
-            acc = fma(d, d, acc);
-            d = (double)h.w - (double)t[i].w;
-            acc = fma(d, d, acc);
-        }
-    }
-    acc += __shfl_xor_sync(kFull, acc, 4);
-    acc += __shfl_xor_sync(kFull, acc, 2);
-    acc += __shfl_xor_sync(kFull, acc, 1);
-    return (float)acc;
-}
-
-// The exact score the rank kernels compare: s = emb[h] . emb[j], or s = -d for the distance (negation is exact, and
-// "s_j > s_t" is "d_j < d_t", so one comparison and one tie rule serve both kinds).
-template <int Kind>
-__device__ __forceinline__ float exact_score(const float* s_head, const float* __restrict__ row, int dim, int q,
-                                             bool live) {
-    if constexpr (Kind == kL2) return -exact_l2(s_head, row, dim, q, live);
-    else return exact_dot8(s_head, row, dim, q, live);
-}
-
-__device__ void bitonic_desc(unsigned long long* keys, int n_pow2) {
-    for (int size = 2; size <= n_pow2; size <<= 1) {
+// Sorts keys[0, n) descending in place (shared memory, the whole block): 0 keys pad the list to the next power of two
+// (keys must have room for them), then a bitonic network.
+__device__ void sort_keys_desc(unsigned long long* keys, int n) {
+    int p2 = 1;
+    while (p2 < n) p2 <<= 1;
+    for (int i = n + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
+    __syncthreads();
+    for (int size = 2; size <= p2; size <<= 1) {
         for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            for (int i = threadIdx.x; i < n_pow2; i += blockDim.x) {
+            for (int i = threadIdx.x; i < p2; i += blockDim.x) {
                 const int j = i ^ stride;
                 if (j > i) {
                     const bool desc = (i & size) == 0;
@@ -467,6 +357,190 @@ __device__ void bitonic_desc(unsigned long long* keys, int n_pow2) {
             __syncthreads();
         }
     }
+}
+
+// thr = (k-th largest tile maximum of the sampled tiles) - 2E.  The tile maxima are k distinct tails whose
+// APPROXIMATE scores reach m_k, so their exact scores reach m_k - E, so the exact k-th best is >= m_k - E and every
+// member of the true top-k has an approximate score >= m_k - 2E.  One CTA per head, the maxima sorted as enc() keys.
+__global__ void __launch_bounds__(256) score_sample_threshold_kernel(const float* __restrict__ tilemax, int n_st, int k,
+                                                                     const float* __restrict__ head_norms,
+                                                                     const float* __restrict__ tail_max_norm, int dim,
+                                                                     float* __restrict__ thr) {
+    extern __shared__ unsigned long long sv[];
+    const int head = blockIdx.x;
+    for (int i = threadIdx.x; i < n_st; i += blockDim.x) sv[i] = enc(tilemax[(int64_t)head * n_st + i]);
+    sort_keys_desc(sv, n_st);
+    if (threadIdx.x == 0) {
+        const float mk = k <= n_st ? dec((uint32_t)sv[k - 1]) : -INFINITY;
+        thr[head] = mk == -INFINITY ? -INFINITY : mk - 2.f * score_err(head_norms[head], *tail_max_norm, dim) - fabsf(mk) * 1e-6f;
+    }
+}
+
+// Score kinds: the dot product emb[h] . emb[j], or the negated squared distance -|q - p_j|^2 of the relation-aware
+// triple score (TransR / TransE), and the dense instance of the filter that reads a score matrix.
+constexpr int kDot = 0, kL2 = 1, kScores = 2;
+constexpr int kL2MaxDim = 508;           // distance rows: dim % 4 == 0, the augmented width dim + 4 <= 512
+// Query row staged by the rank kernels (zero padded): the distance's augmented width, the dot score's GEMM K.
+template <int Kind> constexpr int row_floats() { return Kind == kL2 ? kL2MaxDim + 4 : kMaxChunks * kBK; }
+
+// Exact score of one (query, candidate) pair, larger = better: s = a . b (kDot) or s = -|a - b|^2 (kL2).  Products
+// and differences of fp32 values are exact in fp64; they are summed in fp64 with one fma per element and rounded once
+// to fp32 (the distance is then negated, which is exact, so "s_j > s_t" is "d_j < d_t" and one comparison and one tie
+// rule serve both kinds).  Eight lanes share a candidate row (lane q of the group takes float4 q, q + 8, ...), so a
+// warp scores four candidates at once with all its row loads in flight together.  NV float4 per lane: 8 covers widths
+// up to 256, 16 up to 512; float4 v >= dim / 4 is skipped, so for dim <= 256 both instances load the same values and
+// sum them in the same order.  `a` (the query row) may live in shared or global memory: every caller of a kind sees
+// the same values in the same order, so rank prepare, finalize and the filter, or the top-k threshold and finalize,
+// return the same bits for the same pair.
+template <int Kind, int NV>
+__device__ __forceinline__ float exact_score(const float* a, const float* __restrict__ b, int dim, int q, bool live) {
+    double acc = 0.0;
+    const int nv = dim >> 2;                                   // dim % 4 == 0 is checked on the host side
+    float4 t[NV];
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+        const int v = q + 8 * i;
+        t[i] = (live && v < nv) ? __ldg(reinterpret_cast<const float4*>(b) + v) : make_float4(0, 0, 0, 0);
+    }
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+        const int v = q + 8 * i;
+        if (v < nv) {
+            const float4 h = *reinterpret_cast<const float4*>(a + 4 * v);
+            if constexpr (Kind == kL2) {
+                double d = (double)h.x - (double)t[i].x;
+                acc = fma(d, d, acc);
+                d = (double)h.y - (double)t[i].y;
+                acc = fma(d, d, acc);
+                d = (double)h.z - (double)t[i].z;
+                acc = fma(d, d, acc);
+                d = (double)h.w - (double)t[i].w;
+                acc = fma(d, d, acc);
+            } else {
+                acc = fma((double)h.x, (double)t[i].x, acc);
+                acc = fma((double)h.y, (double)t[i].y, acc);
+                acc = fma((double)h.z, (double)t[i].z, acc);
+                acc = fma((double)h.w, (double)t[i].w, acc);
+            }
+        }
+    }
+    acc += __shfl_xor_sync(kFull, acc, 4);
+    acc += __shfl_xor_sync(kFull, acc, 2);
+    acc += __shfl_xor_sync(kFull, acc, 1);
+    return Kind == kL2 ? -(float)acc : (float)acc;
+}
+
+// The rank kernels' instance: the float4 count of their staged row.
+template <int Kind>
+__device__ __forceinline__ float rank_score(const float* a, const float* __restrict__ b, int dim, int q, bool live) {
+    return exact_score<Kind, row_floats<Kind>() / 32>(a, b, dim, q, live);
+}
+
+// fp64 sums over the float4s v = lane, lane + L, ... of a row, reduced over L lanes: |a|^2 and, with a centre c
+// (nullable), a . c and sum |a_k c_k|.  The band margins take the norms of the query operand from here.
+struct RowSums {
+    double aa, ac, aca;
+};
+template <int L>
+__device__ __forceinline__ RowSums row_sums(const float* __restrict__ a, const float* __restrict__ c, int dim,
+                                            int lane) {
+    RowSums r{0.0, 0.0, 0.0};
+    for (int v = lane; v < (dim >> 2); v += L) {
+        const float4 x = __ldg(reinterpret_cast<const float4*>(a) + v);
+        r.aa = fma((double)x.x, (double)x.x, r.aa);
+        r.aa = fma((double)x.y, (double)x.y, r.aa);
+        r.aa = fma((double)x.z, (double)x.z, r.aa);
+        r.aa = fma((double)x.w, (double)x.w, r.aa);
+        if (c) {
+            const float4 y = __ldg(reinterpret_cast<const float4*>(c) + v);
+            r.ac = fma((double)x.x, (double)y.x, r.ac);
+            r.ac = fma((double)x.y, (double)y.y, r.ac);
+            r.ac = fma((double)x.z, (double)y.z, r.ac);
+            r.ac = fma((double)x.w, (double)y.w, r.ac);
+            r.aca += fabs((double)x.x * y.x) + fabs((double)x.y * y.y) + fabs((double)x.z * y.z) +
+                     fabs((double)x.w * y.w);
+        }
+    }
+#pragma unroll
+    for (int o = L / 2; o > 0; o >>= 1) {
+        r.aa += __shfl_xor_sync(kFull, r.aa, o);
+        if (c) {
+            r.ac += __shfl_xor_sync(kFull, r.ac, o);
+            r.aca += __shfl_xor_sync(kFull, r.aca, o);
+        }
+    }
+    return r;
+}
+
+// Stages a query row in shared memory, zero padded to N floats (the exact scorer reads whole float4s of it).
+template <int N>
+__device__ __forceinline__ void stage_row(float* s_row, const float* __restrict__ row, int dim) {
+    for (int i = threadIdx.x; i < N; i += blockDim.x) s_row[i] = i < dim ? __ldg(row + i) : 0.f;
+}
+
+// Exact scan of positions [0, n) keeping the best `half` keys (keys holds 2 half): each chunk of `half` positions is
+// keyed after the kept keys, sorted with them and cut back to `half`.  score(p, q, live) is the exact score of
+// position p (all 8 lanes of a group call it: the scorer shuffles), key(s, p) its key.  -> the number of kept keys.
+template <class Score, class Key>
+__device__ int scan_best(unsigned long long* keys, int n, int half, Score score, Key key) {
+    __shared__ int s_kept;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int grp = lane >> 3, q = lane & 7;
+    if (threadIdx.x == 0) s_kept = 0;
+    __syncthreads();
+    for (int base = 0; base < n; base += half) {
+        const int chunk = min(half, n - base);
+        const int kept = s_kept;
+        for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {
+            const int c = c0 + grp;
+            const bool live = c < chunk;
+            const int p = live ? base + c : 0;
+            const float s = score(p, q, live);
+            if (live && q == 0) keys[kept + c] = key(s, p);
+        }
+        __syncthreads();
+        sort_keys_desc(keys, kept + chunk);
+        if (threadIdx.x == 0) s_kept = min(kept + chunk, half);
+        __syncthreads();
+    }
+    return s_kept;
+}
+
+// Writes the first k of n sorted keys as (score, position), padded with -1 and the worst score; kL2 writes d = -s.
+template <int Kind>
+__device__ __forceinline__ void write_first_k(const unsigned long long* keys, int n, int k, float* val, int64_t* pos) {
+    for (int i = threadIdx.x; i < k; i += blockDim.x) {
+        const unsigned long long key = i < n ? keys[i] : 0ull;
+        const float s = dec((uint32_t)(key >> 32));
+        val[i] = key ? (Kind == kL2 ? -s : s) : (Kind == kL2 ? INFINITY : -INFINITY);
+        pos[i] = key ? (int64_t)(~(uint32_t)(key & 0xffffffffu)) : -1;
+    }
+}
+
+// Block-wide count of the columns c in [0, n) that beat the target (score t, position tp) under the tie rule of the
+// ranks: s > t, or s == t and p < tp -- compared as enc() keys for kScores (-0 < +0 there).  Four columns per warp, 8
+// lanes each: score(c, q, &p) is called by all lanes of column c's group (c >= n included: the exact scorer shuffles)
+// and sets p, the column's candidate position, or p < 0 when the column does not count.  -> the total, in thread 0.
+template <int Kind, class Score>
+__device__ int64_t count_beating(int n, float t, int64_t tp, Score score) {
+    __shared__ int s_cnt[32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int grp = lane >> 3, q = lane & 7;
+    int cnt = 0;
+    for (int c0 = 4 * warp; c0 < n; c0 += 4 * nwarps) {
+        int p = -1;
+        const float s = score(c0 + grp, q, p);
+        const bool beats = Kind == kScores ? enc(s) > enc(t) || (enc(s) == enc(t) && p < tp)
+                                           : s > t || (s == t && p < tp);
+        if (p >= 0 && q == 0 && beats) ++cnt;
+    }
+    cnt = (int)warp_sum((float)cnt);                 // < 2^24 per warp
+    if (lane == 0) s_cnt[warp] = cnt;
+    __syncthreads();
+    int64_t tot = 0;
+    if (threadIdx.x == 0)
+        for (int w = 0; w < nwarps; ++w) tot += s_cnt[w];
+    return tot;
 }
 
 struct FinalParams {
@@ -489,15 +563,12 @@ struct FinalParams {
 // lower column".
 __global__ void __launch_bounds__(kFinalThreads) score_finalize_kernel(FinalParams p) {
     extern __shared__ unsigned long long keys[];
-    __shared__ int s_kept;
     const int head = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = kFinalThreads / 32;
     const int grp = lane >> 3, q = lane & 7;                    // 4 candidates per warp, 8 lanes each
-    const int kk = min(p.k, p.n_tails);
     __shared__ __align__(16) float s_head[kMaxChunks * kBK];
-    const float* hrow = p.head_emb + (p.head_rows ? p.head_rows[head] : p.head_row_base + head) * p.ld_head_emb;
-    for (int i = threadIdx.x; i < kMaxChunks * kBK; i += blockDim.x) s_head[i] = i < p.dim ? __ldg(hrow + i) : 0.f;
-    if (threadIdx.x == 0) s_kept = 0;
+    stage_row<kMaxChunks * kBK>(s_head, p.head_emb + (p.head_rows ? p.head_rows[head] : p.head_row_base + head) *
+                                                         p.ld_head_emb, p.dim);
     // gather the head's sublists (one per CTA stream of the filter kernel) into one column list
     int* cols = reinterpret_cast<int*>(keys + p.cap);
     __shared__ int s_off[161], s_n, s_over;
@@ -517,10 +588,12 @@ __global__ void __launch_bounds__(kFinalThreads) score_finalize_kernel(FinalPara
         s_over = over;
     }
     __syncthreads();
-    const bool overflow = s_over != 0;
-    int n = 0;
-    auto tail_row = [&](int col) { return p.emb + (p.tail_rows ? p.tail_rows[col] : col) * p.ld_emb; };
-    if (!overflow) {
+    auto score = [&](int col, int q, bool live) {
+        return exact_score<kDot, 8>(s_head, p.emb + (p.tail_rows ? p.tail_rows[col] : col) * p.ld_emb, p.dim, q, live);
+    };
+    auto key = [](float s, int col) { return ((unsigned long long)enc(s) << 32) | (uint32_t)(~(uint32_t)col); };
+    int n;
+    if (s_over == 0) {
         n = s_n;
         for (int sidx = warp; sidx < p.n_streams; sidx += nwarps) {
             const int o = s_off[sidx], c = s_off[sidx + 1] - o;
@@ -532,49 +605,16 @@ __global__ void __launch_bounds__(kFinalThreads) score_finalize_kernel(FinalPara
             const int c = c0 + grp;
             const bool live = c < n;
             const int col = live ? cols[c] : 0;
-            const float s = exact_dot8(s_head, tail_row(col), p.dim, q, live);
-            if (live && q == 0) keys[c] = ((unsigned long long)enc(s) << 32) | (uint32_t)(~(uint32_t)col);
+            const float s = score(col, q, live);
+            if (live && q == 0) keys[c] = key(s, col);
         }
+        sort_keys_desc(keys, n);
     } else {
         // Overflow fallback (the candidate band held more than `cap` tails, e.g. a plateau of near-identical
-        // scores): exact scan of every tail, keeping the best `cap / 2` keys seen so far: when the buffer fills up
-        // it is sorted and its lower half dropped (cap / 2 >= k is checked on the host side).
-        const int half = p.cap / 2;
-        for (int base = 0; base < p.n_tails; base += half) {
-            const int chunk = min(half, p.n_tails - base);
-            const int kept = s_kept;
-            for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {
-                const int c = c0 + grp;
-                const bool live = c < chunk;
-                const int col = live ? base + c : 0;
-                const float s = exact_dot8(s_head, tail_row(col), p.dim, q, live);
-                if (live && q == 0) keys[kept + c] = ((unsigned long long)enc(s) << 32) | (uint32_t)(~(uint32_t)col);
-            }
-            __syncthreads();
-            const int tot = kept + chunk;
-            int p2 = 1;
-            while (p2 < tot) p2 <<= 1;
-            for (int i = tot + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
-            __syncthreads();
-            bitonic_desc(keys, p2);
-            if (threadIdx.x == 0) s_kept = min(tot, half);
-            __syncthreads();
-        }
-        n = s_kept;
+        // scores): exact scan of every tail (cap / 2 >= k is checked on the host side).
+        n = scan_best(keys, p.n_tails, p.cap / 2, score, key);
     }
-    __syncthreads();
-    if (!overflow) {
-        int p2 = 1;
-        while (p2 < n) p2 <<= 1;
-        for (int i = n + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
-        __syncthreads();
-        bitonic_desc(keys, p2);
-    }
-    for (int i = threadIdx.x; i < p.k; i += blockDim.x) {
-        const bool ok = i < kk && i < n;
-        p.top_val[(int64_t)head * p.k + i] = ok ? dec((uint32_t)(keys[i] >> 32)) : -INFINITY;
-        p.top_col[(int64_t)head * p.k + i] = ok ? (int64_t)(~(uint32_t)(keys[i] & 0xffffffffu)) : -1;
-    }
+    write_first_k<kDot>(keys, n, p.k, p.top_val + (int64_t)head * p.k, p.top_col + (int64_t)head * p.k);
 }
 
 // ---- rank of a given tail per head (north star (d): "top-k and rank epilogue") -----------------------------------
@@ -703,33 +743,26 @@ __global__ void rank_prepare_kernel(const float* __restrict__ emb, int64_t ld, c
                                     int n_heads, int dim, const float* __restrict__ tail_max_norm,
                                     const float* __restrict__ rec, const float* __restrict__ center,
                                     float* __restrict__ tau, float* __restrict__ thr, const L2Prep l2) {
+    // 8 lanes per query (the exact scorer's layout), 4 queries per warp.  The target's score s_t comes from the scorer
+    // finalize and the filter re-score with, on the same rows in the same order, so the target never beats itself.
+    const int gq = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3);
+    const int q = threadIdx.x & 7;
+    const bool live = gq < n_heads;
+    const int head = live ? gq : 0;
+    const float* hrow = head_emb + (head_rows ? head_rows[head] : head) * ld_h;
+    const int64_t tp = target_pos[head];
+    const float s = rank_score<Kind>(hrow, emb + (tail_rows ? tail_rows[tp] : tp) * ld, dim, q, live);
     if constexpr (Kind == kL2) {
-        // 8 lanes per query (the exact_l2 layout), 4 queries per warp.  tau = d_t by exact_l2 on the same rows, in the
-        // same order, as finalize and the filter re-score.  With D_j the exact distance on the fp32 rows q, p_j, the
-        // GEMM value g_j and S~_j = u . w_j + nu_j on the rounded fp32 operands (DESIGN.md §6):
+        // tau = d_t = -s.  With D_j the exact distance on the fp32 rows q, p_j, the GEMM value g_j and
+        // S~_j = u . w_j + nu_j on the rounded fp32 operands (DESIGN.md §6):
         //   |g_j - S~_j| <= E = rank_err(K) |u~| V + 2^-24 sqrt(K) (V / s_q + |u~| / s_c)  (the second term: fp16
         //                       subnormals of the lo planes, 1 / s the record's inverse scales),
         //   |D_j - (|u|^2 - 2 S~_j)| <= R = 2^-21 (|u| + W)^2  (rounding of q - c, p_j - c and nu_j),
         // so g_j > sigma + M implies D_j < d_t (1 - 2^-22), hence d_j = fl(D_j) < d_t, and g_j < sigma - M implies
         // d_j > d_t, with sigma = (|u|^2 - d_t) / 2 and M = E + R / 2 + 2^-21 d_t + the fp64 rounding of sigma.
-        const int gq = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3);
-        const int q = threadIdx.x & 7;
-        const bool live = gq < n_heads;
-        const int head = live ? gq : 0;
-        const int64_t tp = target_pos[head];
-        const float t = exact_l2(head_emb + (int64_t)head * ld_h, emb + tp * ld, dim, q, live);
+        const float t = -s;
         const float* arow = l2.aug + (int64_t)head * l2.ld_aug;
-        double uu = 0.0;
-        for (int v = q; v < (dim >> 2); v += 8) {
-            const float4 u = __ldg(reinterpret_cast<const float4*>(arow) + v);
-            uu = fma((double)u.x, (double)u.x, uu);
-            uu = fma((double)u.y, (double)u.y, uu);
-            uu = fma((double)u.z, (double)u.z, uu);
-            uu = fma((double)u.w, (double)u.w, uu);
-        }
-        uu += __shfl_xor_sync(kFull, uu, 4);
-        uu += __shfl_xor_sync(kFull, uu, 2);
-        uu += __shfl_xor_sync(kFull, uu, 1);
+        const double uu = row_sums<8>(arow, nullptr, dim, q).aa;
         if (live && q == 0) {
             const double sigma = 0.5 * (uu - (double)t);
             const double mrg = l2_band_margin(uu, arow[dim], t, dim, tail_max_norm, __ldg(l2.rec_q + 2), __ldg(rec + 2));
@@ -737,36 +770,17 @@ __global__ void rank_prepare_kernel(const float* __restrict__ emb, int64_t ld, c
             thr[2 * head] = __double2float_rd(sigma - mrg);
             thr[2 * head + 1] = __double2float_ru(sigma + mrg);
         }
-        return;
-    }
-    const int lane = threadIdx.x & 31;
-    const int head = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-    if (head >= n_heads) return;
-    const float* hrow = head_emb + (head_rows ? head_rows[head] : head) * ld_h;
-    const int64_t tp = target_pos[head];
-    const float* trow = emb + (tail_rows ? tail_rows[tp] : tp) * ld;
-    double acc = 0.0, nh = 0.0, hc = 0.0;
-    for (int c = lane; c < dim; c += 32) {
-        const float a = __ldg(hrow + c), b = __ldg(trow + c);
-        acc = fma((double)a, (double)b, acc);
-        nh = fma((double)a, (double)a, nh);
-        if (center) hc = fma((double)a, (double)__ldg(center + c), hc);
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        acc += __shfl_xor_sync(kFull, acc, o);
-        nh += __shfl_xor_sync(kFull, nh, o);
-        hc += __shfl_xor_sync(kFull, hc, o);
-    }
-    if (lane == 0) {
-        const float t = (float)acc;                          // exact target score, rounded once (what finalize compares)
-        const float ts = (float)(acc - hc);                  // the same in the GEMM's (shifted) frame
-        // bound of the GEMM's error (norms of the tails: scaled units) + the rounding of the two fp32 numbers above
-        const float e = kRankErr * (float)sqrt(nh) * (*tail_max_norm) * rec[2] * 1.0001f +
-                        (fabsf(t) + fabsf(ts) + (float)fabs(hc)) * 2e-7f + 1e-30f;
-        tau[head] = t;
-        thr[2 * head] = ts - e;
-        thr[2 * head + 1] = ts + e;
+    } else {
+        const RowSums h = row_sums<8>(hrow, center, dim, q);         // |h|^2 and h . c
+        if (live && q == 0) {
+            const float ts = (float)((double)s - h.ac);              // the target score in the GEMM's (shifted) frame
+            // bound of the GEMM's error (norms of the tails: scaled units) + the roundings of s_t and ts
+            const float e = kRankErr * (float)sqrt(h.aa) * (*tail_max_norm) * rec[2] * 1.0001f +
+                            (fabsf(s) + fabsf(ts) + (float)fabs(h.ac)) * 2e-7f + 1e-30f;
+            tau[head] = s;
+            thr[2 * head] = ts - e;
+            thr[2 * head + 1] = ts + e;
+        }
     }
 }
 
@@ -782,35 +796,21 @@ __global__ void __launch_bounds__(256) rank_finalize_kernel(const float* __restr
                                                             const int* __restrict__ band_cnt, const int* __restrict__ band,
                                                             int cap, int n_tails, int dim, int64_t* __restrict__ ranks) {
     __shared__ __align__(16) float s_head[row_floats<Kind>()];
-    __shared__ int s_better[8];
     const int head = blockIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    const int grp = lane >> 3, q = lane & 7;
-    const float* hrow = head_emb + (head_rows ? head_rows[head] : head) * ld_h;
-    for (int i = threadIdx.x; i < row_floats<Kind>(); i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
+    stage_row<row_floats<Kind>()>(s_head, head_emb + (head_rows ? head_rows[head] : head) * ld_h, dim);
     __syncthreads();
     const float t = Kind == kL2 ? -tau[head] : tau[head];
-    const int64_t tp = target_pos[head];
     const int n_band = band_cnt[head];
     const bool overflow = n_band > cap;            // the band held more columns than the list: exact scan of every tail
     const int n = overflow ? n_tails : n_band;
-    int better = 0;
-    for (int c0 = 4 * warp; c0 < n; c0 += 4 * nwarps) {
-        const int c = c0 + grp;
+    const int64_t better = count_beating<Kind>(n, t, target_pos[head], [&](int c, int q, int& p) {
         const bool live = c < n;
         const int col = live ? (overflow ? c : band[(int64_t)head * cap + c]) : 0;
-        const float* trow = emb + (tail_rows ? tail_rows[col] : col) * ld;
-        const float s = exact_score<Kind>(s_head, trow, dim, q, live);
-        if (live && q == 0 && (s > t || (s == t && col < tp))) ++better;
-    }
-    better = (int)warp_sum((float)better);          // < 2^24 per warp
-    if (lane == 0) s_better[warp] = better;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int64_t tot = overflow ? 0 : above[head];
-        for (int w = 0; w < nwarps; ++w) tot += s_better[w];
-        ranks[head] = tot;
-    }
+        const float s = rank_score<Kind>(s_head, emb + (tail_rows ? tail_rows[col] : col) * ld, dim, q, live);
+        p = live ? col : -1;
+        return s;
+    });
+    if (threadIdx.x == 0) ranks[head] = better + (overflow ? 0 : above[head]);
 }
 
 // ---- filtered rank: subtract the known true tails that beat the target ------------------------------------------
@@ -845,11 +845,11 @@ __device__ __forceinline__ void filter_run(const lkg_graph& g, int64_t h, int64_
 // One CTA per query, the run split over the warps like rank_finalize_kernel's band (a hub head can have thousands of
 // known tails).  A filter tail f at candidate position p != t is subtracted when it beats the target under the rule
 // the raw rank was counted with, on the same scores:
-//   kExact  (fused path, after lkg_rank_finalize): s_f = exact_dot8 of the same head row staged the same way, compared
+//   kExact  (fused path, after lkg_rank_finalize): s_f = rank_score of the same head row staged the same way, compared
 //           with the same tau by the same float comparison.  finalize counts a column either because the GEMM put it
 //           above tau + E -- and then its exact score is above tau, the band bound being rigorous -- or because its
 //           exact score beats tau; either way the bit-identical re-score here reaches the same verdict;
-//   kL2     (distance path, after lkg_rank_finalize_l2): the same argument with s = -exact_l2 of the query row (row qi
+//   kL2     (distance path, after lkg_rank_finalize_l2): the same argument with s = rank_score = -d of the query row (row qi
 //           of qrows, staged like finalize stages it) and f's row in the candidate table (src row p), against -tau;
 //   kScores (dense path, after lkg_topk_rows): s_f and s_t are read from the score matrix and compared as the
 //           order-preserving keys lkg_topk_rows compares (-0 < +0 there).
@@ -863,15 +863,11 @@ __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, con
                                                           const float* __restrict__ qrows, int64_t ld_q) {
     constexpr bool kExact = Kind != kScores;
     __shared__ __align__(16) float s_head[row_floats<Kind>()];
-    __shared__ int s_sub[8];
     const int qi = blockIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    const int grp = lane >> 3, q = lane & 7;
     const int64_t h = heads[qi];
     const int64_t tp = target_pos[qi];
     if (kExact) {
-        const float* hrow = Kind == kL2 ? qrows + (int64_t)qi * ld_q : src + h * ld;
-        for (int i = threadIdx.x; i < row_floats<Kind>(); i += blockDim.x) s_head[i] = i < dim ? __ldg(hrow + i) : 0.f;
+        stage_row<row_floats<Kind>()>(s_head, Kind == kL2 ? qrows + (int64_t)qi * ld_q : src + h * ld, dim);
         __syncthreads();
     }
     const int32_t* run;
@@ -880,38 +876,27 @@ __global__ void __launch_bounds__(256) rank_filter_kernel(const lkg_graph g, con
     const float* srow = src + (int64_t)qi * ld;                      // dense: this query's row of the score matrix
     const float t = Kind == kL2 ? -tau[qi] : (kExact ? tau[qi] : srow[tp]);
     const int n = hi - lo;
-    int sub = 0;
-    for (int c0 = 4 * warp; c0 < n; c0 += 4 * nwarps) {              // uniform per warp: exact_dot8 shuffles
-        const int c = c0 + grp;
+    const int64_t sub = count_beating<Kind>(n, t, tp, [&](int c, int q, int& p) {
         bool live = c < n;
-        int f = 0, p = -1;
+        int f = 0;
         if (live) {
             f = run[lo + c];
             p = cand_map ? cand_map[f] : f;
             live = p >= 0 && p != tp && (c == 0 || run[lo + c - 1] != f);
         }
-        if (kExact) {
-            const float s = exact_score<Kind>(s_head, src + (int64_t)(Kind == kL2 ? p : f) * ld, dim, q, live);
-            if (live && q == 0 && (s > t || (s == t && p < tp))) ++sub;
-        } else if (live && q == 0) {
-            const uint32_t ks = enc(srow[p]), kt = enc(t);
-            if (ks > kt || (ks == kt && p < tp)) ++sub;
-        }
-    }
-    sub = (int)warp_sum((float)sub);                 // < 2^24 per warp
-    if (lane == 0) s_sub[warp] = sub;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int64_t tot = 0;
-        for (int w = 0; w < nwarps; ++w) tot += s_sub[w];
-        ranks[qi] -= tot;
-    }
+        float s = 0.f;
+        if constexpr (kExact) s = rank_score<Kind>(s_head, src + (int64_t)(Kind == kL2 ? p : f) * ld, dim, q, live);
+        else if (live) s = srow[p];
+        if (!live) p = -1;
+        return s;
+    });
+    if (threadIdx.x == 0) ranks[qi] -= sub;
 }
 
 // ---- filtered top-k: the triple score (distance) and the dot score ------------------------------------------------
 // Per query (q_i, excluded set X_i) the k candidates j not in X_i with the best exact score, ties -> lower position:
-// kL2 the smallest d_j = exact_l2(q_i, p_j), kDot the largest s_j = exact_dot8<16>(h_i, t_j).  The counting GEMM
-// serves as a candidate filter (DESIGN.md §6):
+// kL2 the smallest d_j = |q_i - p_j|^2, kDot the largest s_j = h_i . t_j, both by exact_score<Kind, 16>.  The counting
+// GEMM serves as a candidate filter (DESIGN.md §6):
 //   1. lkg_topk_threshold_*  theta_i = the exact k-th best score among S strided samples not in X_i (so at least k
 //                            admissible candidates score at least as well: the true k-th best is no worse than
 //                            theta_i), and thr_i = {lo, +inf}: kL2 lo = sigma - M with sigma = (|u|^2 - theta_i) / 2
@@ -926,7 +911,6 @@ constexpr int kThetaBuf = 2048;          // kept distances: after a round <= k +
 constexpr int kTopkMaxK = 1024;
 constexpr int kTopkMaxCap = 16384;
 constexpr int kTopkRow = 512;            // staged query row: the distance's augmented width, the dot score's dim
-constexpr int kDotTopkVec = kTopkRow / 32;      // float4 per lane of exact_dot8 in the dot instances
 static_assert(row_floats<kL2>() == kTopkRow, "the distance instances stage their rows as before");
 
 // M of the dot band: with the GEMM value g_j = h . w_j (w_j = fl(t_j - c), the centred candidate operand) of a
@@ -988,31 +972,18 @@ __device__ __forceinline__ bool is_excluded(const KnownRun& run, const TopkExclu
     return run.hi > run.lo && run.has(x.cand_ids ? x.cand_ids[p] : (int64_t)p);
 }
 
-// The candidate row of position p and the exact score of the top-k kernels: kL2 the distance d (smaller is better),
-// kDot the dot product s (larger is better) on the uncentred rows.
+// The exact score of candidate position p under the top-k kernels' instance of the scorer: s = h . t_p on the
+// uncentred rows, or s = -d_p (larger is better for both).
 template <int Kind>
-__device__ __forceinline__ const float* topk_cand_row(const float* cand, int64_t ld, const TopkDot& dot, int p) {
-    if constexpr (Kind == kDot) return cand + (dot.cand_rows ? dot.cand_rows[p] : (int64_t)p) * ld;
-    else return cand + (int64_t)p * ld;
+__device__ __forceinline__ float topk_score(const float* s_q, const float* cand, int64_t ld, const TopkDot& dot, int p,
+                                            int dim, int q, bool live) {
+    const int64_t row = Kind == kDot && dot.cand_rows ? dot.cand_rows[p] : (int64_t)p;
+    return exact_score<Kind, kTopkRow / 32>(s_q, cand + row * ld, dim, q, live);
 }
 
 template <int Kind>
-__device__ __forceinline__ float topk_score(const float* s_q, const float* __restrict__ row, int dim, int q, bool live) {
-    if constexpr (Kind == kDot) return exact_dot8<kDotTopkVec>(s_q, row, dim, q, live);
-    else return exact_l2(s_q, row, dim, q, live);
-}
-
-// Order-preserving 32-bit code of a score, larger = better: enc(s) for the dot product, ~enc(d) = enc(-d) for the
-// distance (d >= 0).
-template <int Kind>
-__device__ __forceinline__ uint32_t topk_code(float s) {
-    if constexpr (Kind == kDot) return enc(s);
-    else return ~enc(s);
-}
-template <int Kind>
-__device__ __forceinline__ float topk_decode(uint32_t code) {
-    if constexpr (Kind == kDot) return dec(code);
-    else return dec(~code);
+__device__ __forceinline__ const float* topk_query_row(const float* query, int64_t ld_q, const TopkDot& dot, int qi) {
+    return query + (Kind == kDot && dot.query_rows ? dot.query_rows[qi] : (int64_t)qi) * ld_q;
 }
 
 // One CTA per query.  Samples i = 0 .. n_sample - 1 at positions floor(i n_cand / n_sample), kThetaChunk per round;
@@ -1024,57 +995,24 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_kernel(
     const float* __restrict__ aug, int64_t ld_aug, int dim, int k, int n_sample, const float* __restrict__ stats,
     const float* __restrict__ rec_q, const float* __restrict__ rec_c, const TopkExclude x, float* __restrict__ thr,
     float* __restrict__ theta, const TopkDot dot) {
-    constexpr float kWorst = Kind == kDot ? -INFINITY : INFINITY;
     __shared__ __align__(16) float s_q[kTopkRow];
-    __shared__ unsigned long long keys[kThetaBuf];       // topk_code << 32: a descending sort puts the best first
+    __shared__ unsigned long long keys[kThetaBuf];       // enc(s) << 32: a descending sort puts the best first
     __shared__ int s_cnt;
-    __shared__ float s_theta;
-    __shared__ double s_uu, s_hc, s_hca;
+    __shared__ float s_theta;                            // the k-th best score s so far (kL2: s = -d)
+    __shared__ RowSums s_rs;
     const int qi = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int grp = lane >> 3, q = lane & 7;
-    const float* qrow = query + (Kind == kDot && dot.query_rows ? dot.query_rows[qi] : (int64_t)qi) * ld_q;
-    for (int i = threadIdx.x; i < kTopkRow; i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
+    const float* qrow = topk_query_row<Kind>(query, ld_q, dot, qi);
+    stage_row<kTopkRow>(s_q, qrow, dim);
     const float* arow = aug + (int64_t)qi * ld_aug;
     if (warp == 0) {
-        // kL2: |u|^2 of the query operand; kDot: |h|^2, h . c and sum |h_k c_k| of the anchor row; in fp64
-        double uu = 0.0, hc = 0.0, hca = 0.0;
-        for (int v = lane; v < (dim >> 2); v += 32) {
-            if constexpr (Kind == kDot) {
-                const float4 h = __ldg(reinterpret_cast<const float4*>(qrow) + v);
-                const float4 c = __ldg(reinterpret_cast<const float4*>(dot.center) + v);
-                uu = fma((double)h.x, (double)h.x, uu);
-                uu = fma((double)h.y, (double)h.y, uu);
-                uu = fma((double)h.z, (double)h.z, uu);
-                uu = fma((double)h.w, (double)h.w, uu);
-                hc = fma((double)h.x, (double)c.x, hc);
-                hc = fma((double)h.y, (double)c.y, hc);
-                hc = fma((double)h.z, (double)c.z, hc);
-                hc = fma((double)h.w, (double)c.w, hc);
-                hca += fabs((double)h.x * c.x) + fabs((double)h.y * c.y) + fabs((double)h.z * c.z) +
-                       fabs((double)h.w * c.w);
-            } else {
-                const float4 u = __ldg(reinterpret_cast<const float4*>(arow) + v);
-                uu = fma((double)u.x, (double)u.x, uu);
-                uu = fma((double)u.y, (double)u.y, uu);
-                uu = fma((double)u.z, (double)u.z, uu);
-                uu = fma((double)u.w, (double)u.w, uu);
-            }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            uu += __shfl_xor_sync(kFull, uu, o);
-            if constexpr (Kind == kDot) {
-                hc += __shfl_xor_sync(kFull, hc, o);
-                hca += __shfl_xor_sync(kFull, hca, o);
-            }
-        }
+        // kL2: |u|^2 of the query operand; kDot: |h|^2, h . c and sum |h_k c_k| of the anchor row
+        const RowSums rs = Kind == kDot ? row_sums<32>(qrow, dot.center, dim, lane) : row_sums<32>(arow, nullptr, dim, lane);
         if (lane == 0) {
-            s_uu = uu;
-            s_hc = hc;
-            s_hca = hca;
+            s_rs = rs;
             s_cnt = 0;
-            s_theta = kWorst;
+            s_theta = -INFINITY;
         }
     }
     const KnownRun run = known_run(x, qi);
@@ -1086,37 +1024,32 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_kernel(
             const int c = c0 + grp;
             const bool live = c < chunk;
             const int p = live ? (int)((int64_t)(base + c) * n_cand / n_sample) : 0;
-            const float s = topk_score<Kind>(s_q, topk_cand_row<Kind>(cand, ld, dot, p), dim, q, live);
-            const bool better = Kind == kDot ? s > bound : s < bound;
-            if (live && q == 0 && better && !is_excluded(run, x, p))
-                keys[atomicAdd(&s_cnt, 1)] = (unsigned long long)topk_code<Kind>(s) << 32;
+            const float s = topk_score<Kind>(s_q, cand, ld, dot, p, dim, q, live);
+            if (live && q == 0 && s > bound && !is_excluded(run, x, p))
+                keys[atomicAdd(&s_cnt, 1)] = (unsigned long long)enc(s) << 32;
         }
         __syncthreads();
         const int cnt = s_cnt;
         __syncthreads();                                 // every thread has read cnt before the next round adds to it
         if (cnt > kThetaBuf - kThetaChunk || base + kThetaChunk >= n_sample) {
-            int p2 = 1;
-            while (p2 < cnt) p2 <<= 1;
-            for (int i = cnt + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
-            __syncthreads();
-            bitonic_desc(keys, p2);
+            sort_keys_desc(keys, cnt);
             if (threadIdx.x == 0) {
-                if (cnt >= k) s_theta = topk_decode<Kind>((uint32_t)(keys[k - 1] >> 32));
+                if (cnt >= k) s_theta = dec((uint32_t)(keys[k - 1] >> 32));
                 s_cnt = min(cnt, k);
             }
             __syncthreads();
         }
     }
     if (threadIdx.x == 0) {
-        const float th = s_theta;
+        const float th = Kind == kL2 ? -s_theta : s_theta;          // theta: the k-th best s, or d for kL2
         float lo = -INFINITY;                            // fewer than k admissible samples: every column is listed
-        if (Kind == kDot ? th > -INFINITY : th < INFINITY) {
+        if (s_theta > -INFINITY) {
             if constexpr (Kind == kDot) {
-                const double hc = s_hc;
-                lo = __double2float_rd(((double)th - hc) - dot_band_margin(s_uu, hc, s_hca, th, dim, __ldg(stats),
+                const double hc = s_rs.ac;
+                lo = __double2float_rd(((double)th - hc) - dot_band_margin(s_rs.aa, hc, s_rs.aca, th, dim, __ldg(stats),
                                                                            __ldg(rec_q + 2), __ldg(rec_c + 2)));
             } else {
-                const double uu = s_uu, sigma = 0.5 * (uu - (double)th);
+                const double uu = s_rs.aa, sigma = 0.5 * (uu - (double)th);
                 lo = __double2float_rd(sigma - l2_band_margin(uu, arow[dim], th, dim, stats, __ldg(rec_q + 2),
                                                               __ldg(rec_c + 2)));
             }
@@ -1127,9 +1060,8 @@ __global__ void __launch_bounds__(kTopkThreads) topk_threshold_kernel(
     }
 }
 
-// One CTA per query.  keys [next_pow2(cap)]: (enc(s) << 32) | ~position with s the dot product or -d, so a descending
-// sort gives "better score first, ties -> lower position"; an excluded or missing entry is key 0, which sorts last and
-// is never written out.
+// One CTA per query.  keys [next_pow2(cap)]: (enc(s) << 32) | ~position; an excluded or missing entry is key 0, which
+// sorts last and is never written out.
 template <int Kind>
 __global__ void __launch_bounds__(kTopkThreads) topk_finalize_kernel(
     const float* __restrict__ cand, int64_t ld, int n_cand, const float* __restrict__ query, int64_t ld_q, int dim,
@@ -1137,18 +1069,15 @@ __global__ void __launch_bounds__(kTopkThreads) topk_finalize_kernel(
     float* __restrict__ dist, int64_t* __restrict__ pos, const TopkDot dot) {
     extern __shared__ unsigned long long keys[];
     __shared__ __align__(16) float s_q[kTopkRow];
-    __shared__ int s_kept;
     const int qi = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int grp = lane >> 3, q = lane & 7;
-    const float* qrow = query + (Kind == kDot && dot.query_rows ? dot.query_rows[qi] : (int64_t)qi) * ld_q;
-    for (int i = threadIdx.x; i < kTopkRow; i += blockDim.x) s_q[i] = i < dim ? __ldg(qrow + i) : 0.f;
-    if (threadIdx.x == 0) s_kept = 0;
+    stage_row<kTopkRow>(s_q, topk_query_row<Kind>(query, ld_q, dot, qi), dim);
     const KnownRun run = known_run(x, qi);
     __syncthreads();
-    auto key_of = [&](float s, int p) -> unsigned long long {
-        const uint32_t code = enc(Kind == kDot ? s : -s);
-        return is_excluded(run, x, p) ? 0ull : ((unsigned long long)code << 32) | (uint32_t)(~(uint32_t)p);
+    auto score = [&](int p, int q, bool live) { return topk_score<Kind>(s_q, cand, ld, dot, p, dim, q, live); };
+    auto key = [&](float s, int p) -> unsigned long long {
+        return is_excluded(run, x, p) ? 0ull : ((unsigned long long)enc(s) << 32) | (uint32_t)(~(uint32_t)p);
     };
     const int n_band = band_cnt[qi];
     int n;
@@ -1159,47 +1088,16 @@ __global__ void __launch_bounds__(kTopkThreads) topk_finalize_kernel(
             const int c = c0 + grp;
             const bool live = c < n;
             const int p = live ? list[c] : 0;
-            const float s = topk_score<Kind>(s_q, topk_cand_row<Kind>(cand, ld, dot, p), dim, q, live);
-            if (live && q == 0) keys[c] = key_of(s, p);
+            const float s = score(p, q, live);
+            if (live && q == 0) keys[c] = key(s, p);
         }
-        __syncthreads();
-        int p2 = 1;
-        while (p2 < n) p2 <<= 1;
-        for (int i = n + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
-        __syncthreads();
-        bitonic_desc(keys, p2);
+        sort_keys_desc(keys, n);
     } else {
         // Overflow (more than cap columns listed, e.g. a weak theta or a plateau of equal scores): exact scan of
-        // every candidate keeping the best cap / 2 keys, as score_finalize_kernel does (cap / 2 >= k is checked).
-        const int half = cap / 2;
-        for (int base = 0; base < n_cand; base += half) {
-            const int chunk = min(half, n_cand - base);
-            const int kept = s_kept;
-            for (int c0 = 4 * warp; c0 < chunk; c0 += 4 * nwarps) {
-                const int c = c0 + grp;
-                const bool live = c < chunk;
-                const int p = live ? base + c : 0;
-                const float s = topk_score<Kind>(s_q, topk_cand_row<Kind>(cand, ld, dot, p), dim, q, live);
-                if (live && q == 0) keys[kept + c] = key_of(s, p);
-            }
-            __syncthreads();
-            const int tot = kept + chunk;
-            int p2 = 1;
-            while (p2 < tot) p2 <<= 1;
-            for (int i = tot + threadIdx.x; i < p2; i += blockDim.x) keys[i] = 0ull;
-            __syncthreads();
-            bitonic_desc(keys, p2);
-            if (threadIdx.x == 0) s_kept = min(tot, half);
-            __syncthreads();
-        }
-        n = s_kept;
+        // every candidate, as score_finalize_kernel does (cap / 2 >= k is checked).
+        n = scan_best(keys, n_cand, cap / 2, score, key);
     }
-    for (int i = threadIdx.x; i < k; i += blockDim.x) {
-        const unsigned long long key = i < n ? keys[i] : 0ull;
-        if constexpr (Kind == kDot) dist[(int64_t)qi * k + i] = key ? dec((uint32_t)(key >> 32)) : -INFINITY;
-        else dist[(int64_t)qi * k + i] = key ? -dec((uint32_t)(key >> 32)) : INFINITY;
-        pos[(int64_t)qi * k + i] = key ? (int64_t)(~(uint32_t)(key & 0xffffffffu)) : -1;
-    }
+    write_first_k<Kind>(keys, n, k, dist + (int64_t)qi * k, pos + (int64_t)qi * k);
 }
 
 inline size_t align_up(size_t x, size_t a = 256) { return (x + a - 1) / a * a; }
@@ -1237,14 +1135,24 @@ extern "C" int lkg_shift_rows(const float* src, int64_t ld, const int64_t* rows,
     return LKG_OK;
 }
 
+// The rows the dot rank kernels score with exact_score<kDot, 8>: float4 loads of widths up to the GEMM's K.
+static int check_rank_rows(const float* emb, int64_t ld_emb, const float* head_emb, int64_t ld_head_emb, int32_t dim) {
+    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kMaxChunks * kBK && ld_emb % 4 == 0 && ld_head_emb % 4 == 0 &&
+                    aligned16(emb) && aligned16(head_emb),
+                "the rank path supports dim %% 4 == 0, dim <= %d, 16-byte aligned rows", kMaxChunks * kBK);
+    return LKG_OK;
+}
+
 extern "C" int lkg_rank_prepare(const float* emb, int64_t ld_emb, const int64_t* tail_rows, const float* head_emb,
                                 int64_t ld_head_emb, const int64_t* head_rows, const int64_t* target_pos, int64_t n_heads,
                                 int32_t dim, const float* tail_max_norm, const float* rec, const float* center,
                                 float* tau, float* thr, void* stream_) {
-    LKG_REQUIRE(emb && head_emb && target_pos && tail_max_norm && rec && tau && thr && n_heads >= 0 && dim > 0,
+    LKG_REQUIRE(emb && head_emb && target_pos && tail_max_norm && rec && tau && thr && n_heads >= 0 &&
+                    n_heads < (1ll << 31) && dim > 0,
                 "bad rank arguments");
+    if (int rc = check_rank_rows(emb, ld_emb, head_emb, ld_head_emb, dim)) return rc;
     if (n_heads == 0) return LKG_OK;
-    const int64_t blocks = (n_heads * 32 + 255) / 256;
+    const int64_t blocks = (n_heads * 8 + 255) / 256;
     rank_prepare_kernel<kDot><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(emb, ld_emb, tail_rows, head_emb,
                                                                                    ld_head_emb, head_rows, target_pos,
                                                                                    (int)n_heads, dim, tail_max_norm, rec,
@@ -1258,11 +1166,10 @@ extern "C" int lkg_rank_finalize(const float* emb, int64_t ld_emb, const int64_t
                                  const float* tau, const int32_t* above, const int32_t* band_cnt, const int32_t* band,
                                  int32_t band_cap, int64_t n_heads, int64_t n_tails, int32_t dim, int64_t* ranks,
                                  void* stream_) {
-    LKG_REQUIRE(emb && head_emb && target_pos && tau && above && band_cnt && band && ranks && band_cap > 0,
+    LKG_REQUIRE(emb && head_emb && target_pos && tau && above && band_cnt && band && ranks && band_cap > 0 &&
+                    n_tails < (1ll << 31),
                 "bad rank arguments");
-    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kMaxChunks * kBK && ld_emb % 4 == 0 && ld_head_emb % 4 == 0 &&
-                    aligned16(emb) && aligned16(head_emb) && n_tails < (1ll << 31),
-                "the rank path supports dim %% 4 == 0, dim <= %d, 16-byte aligned rows", kMaxChunks * kBK);
+    if (int rc = check_rank_rows(emb, ld_emb, head_emb, ld_head_emb, dim)) return rc;
     if (n_heads == 0) return LKG_OK;
     rank_finalize_kernel<kDot><<<(unsigned)n_heads, 256, 0, (cudaStream_t)stream_>>>(emb, ld_emb, tail_rows, head_emb, ld_head_emb,
                                                                                head_rows, target_pos, tau, above, band_cnt,
@@ -1284,8 +1191,7 @@ extern "C" int lkg_rank_filter(const lkg_graph* known, const int64_t* heads, con
                                int64_t ld_emb, int32_t dim, const float* tau, int64_t* ranks, void* stream_) {
     if (int rc = check_filter_args(known, heads, target_pos, n_queries, ranks)) return rc;
     LKG_REQUIRE(emb && tau, "bad filter arguments");
-    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kMaxChunks * kBK && ld_emb % 4 == 0 && aligned16(emb),
-                "the rank path supports dim %% 4 == 0, dim <= %d, 16-byte aligned rows", kMaxChunks * kBK);
+    if (int rc = check_rank_rows(emb, ld_emb, emb, ld_emb, dim)) return rc;
     if (n_queries == 0) return LKG_OK;
     rank_filter_kernel<kDot><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, heads, rels, cand_map,
                                                                                     target_pos, emb, ld_emb, dim, tau,
@@ -1311,11 +1217,15 @@ extern "C" int lkg_rank_filter_scores(const lkg_graph* known, const int64_t* hea
 }
 
 // ---- distance rank (triple score) --------------------------------------------------------------------------------
-static int check_l2_rows(const char* what, const float* p, int64_t ld, int32_t dim) {
+// The rows of the distance paths (kL2: dim <= 508, the augmented width dim + 4 <= 512) and of the dot top-k (kDot:
+// dim <= 512): float4 loads by the exact scorer.
+template <int Kind>
+static int check_rows(const char* what, const float* p, int64_t ld, int32_t dim) {
+    constexpr int max_dim = Kind == kL2 ? kL2MaxDim : kTopkRow;
     LKG_REQUIRE(p, "%s is null", what);
-    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kL2MaxDim,
-                "the distance rank path supports dim %% 4 == 0, 4 <= dim <= %d (augmented width dim + 4 <= 512), got %d",
-                kL2MaxDim, dim);
+    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= max_dim, "the %s path supports dim %% 4 == 0, 4 <= dim <= %d%s, got %d",
+                Kind == kL2 ? "distance rank" : "dot top-k", max_dim,
+                Kind == kL2 ? " (augmented width dim + 4 <= 512)" : "", dim);
     LKG_REQUIRE(ld >= dim && ld % 4 == 0 && aligned16(p), "%s rows must be 16-byte aligned (ld %% 4 == 0, ld >= dim)",
                 what);
     return LKG_OK;
@@ -1325,7 +1235,7 @@ extern "C" int lkg_l2_rank_rows(const float* src, int64_t ld, const int64_t* row
                                 const float* center, int32_t mode, float* stats, float* out, int64_t ld_out,
                                 void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (int rc = check_l2_rows("src", src, ld, dim)) return rc;
+    if (int rc = check_rows<kL2>("src", src, ld, dim)) return rc;
     LKG_REQUIRE(center && aligned16(center), "center must be a 16-byte aligned [dim] vector");
     LKG_REQUIRE(stats && out && m >= 0, "bad operand arguments (stats, out, m)");
     LKG_REQUIRE(ld_out >= dim + 4 && ld_out % 4 == 0 && aligned16(out),
@@ -1346,8 +1256,8 @@ extern "C" int lkg_rank_prepare_l2(const float* cand, int64_t ld_cand, const flo
                                    const float* query_aug, int64_t ld_aug, const int64_t* target_pos, int64_t n_queries,
                                    int32_t dim, const float* stats, const float* rec_query, const float* rec_cand,
                                    float* tau, float* thr, void* stream_) {
-    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    if (int rc = check_rows<kL2>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kL2>("query", query, ld_query, dim)) return rc;
     LKG_REQUIRE(query_aug && ld_aug >= dim + 4 && ld_aug % 4 == 0 && aligned16(query_aug),
                 "query_aug rows need dim + 4 columns and 16-byte alignment");
     LKG_REQUIRE(target_pos && stats && rec_query && rec_cand && tau && thr && n_queries >= 0 && n_queries < (1ll << 31),
@@ -1365,8 +1275,8 @@ extern "C" int lkg_rank_finalize_l2(const float* cand, int64_t ld_cand, const fl
                                     const int64_t* target_pos, const float* tau, const int32_t* above,
                                     const int32_t* band_cnt, const int32_t* band, int32_t band_cap, int64_t n_queries,
                                     int64_t n_cand, int32_t dim, int64_t* ranks, void* stream_) {
-    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    if (int rc = check_rows<kL2>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kL2>("query", query, ld_query, dim)) return rc;
     LKG_REQUIRE(target_pos && tau && above && band_cnt && band && ranks && band_cap > 0 && n_queries >= 0 &&
                     n_queries < (1ll << 31) && n_cand >= 0 && n_cand < (1ll << 31),
                 "bad rank arguments");
@@ -1383,8 +1293,8 @@ extern "C" int lkg_rank_filter_l2(const lkg_graph* known, const int64_t* anchors
                                   const float* cand, int64_t ld_cand, const float* query, int64_t ld_query, int32_t dim,
                                   const float* tau, int64_t* ranks, void* stream_) {
     if (int rc = check_filter_args(known, anchors, target_pos, n_queries, ranks)) return rc;
-    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
+    if (int rc = check_rows<kL2>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kL2>("query", query, ld_query, dim)) return rc;
     LKG_REQUIRE(tau, "bad filter arguments");
     if (n_queries == 0) return LKG_OK;
     rank_filter_kernel<kL2><<<(unsigned)n_queries, 256, 0, (cudaStream_t)stream_>>>(*known, anchors, rels, cand_map,
@@ -1473,7 +1383,7 @@ extern "C" int lkg_score_topk(const uint16_t* heads_hi, int64_t ld_heads_hi, con
             if (pass == 0) {
                 int p2 = 1;
                 while (p2 < n_st) p2 <<= 1;
-                score_sample_threshold_kernel<<<(unsigned)nh, 256, p2 * sizeof(float), stream>>>(
+                score_sample_threshold_kernel<<<(unsigned)nh, 256, p2 * sizeof(unsigned long long), stream>>>(
                     p.tilemax, n_st, k, head_norms + h0, tail_max_norm, dim, thr + h0);
                 LKG_LAUNCH_CHECK("score_sample_threshold_kernel");
             }
@@ -1519,17 +1429,15 @@ static int topk_exclude(const lkg_graph* known, const int64_t* anchors, const in
     return LKG_OK;
 }
 
-extern "C" int lkg_topk_threshold_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
-                                     int64_t ld_query, const float* query_aug, int64_t ld_aug, int64_t n_queries,
-                                     int32_t dim, const float* stats, const float* rec_query, const float* rec_cand,
-                                     int32_t k, int32_t n_sample, const lkg_graph* known, const int64_t* anchors,
-                                     const int64_t* rels, const int64_t* cand_ids, float* thr, float* theta,
-                                     void* stream_) {
-    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
-    LKG_REQUIRE(query_aug && ld_aug >= dim + 4 && ld_aug % 4 == 0 && aligned16(query_aug),
-                "query_aug rows need dim + 4 columns and 16-byte alignment");
-    LKG_REQUIRE(stats && rec_query && rec_cand && thr, "bad top-k arguments (stats, rec_query, rec_cand, thr)");
+// The checks and the launch the two kinds of the top-k threshold share (the rows and the kind's own operands are
+// checked by the caller).
+template <int Kind>
+static int launch_topk_threshold(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
+                                 int64_t ld_query, const float* aug, int64_t ld_aug, int64_t n_queries, int32_t dim,
+                                 const float* stats, const float* rec_query, const float* rec_cand, int32_t k,
+                                 int32_t n_sample, const lkg_graph* known, const int64_t* anchors, const int64_t* rels,
+                                 const int64_t* cand_ids, float* thr, float* theta, const TopkDot& dot,
+                                 cudaStream_t stream) {
     LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
                 "bad top-k shape (n_queries, n_cand)");
     LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
@@ -1537,21 +1445,20 @@ extern "C" int lkg_topk_threshold_l2(const float* cand, int64_t ld_cand, int64_t
     TopkExclude x;
     if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
     if (n_queries == 0) return LKG_OK;
-    topk_threshold_kernel<kL2><<<(unsigned)n_queries, kTopkThreads, 0, (cudaStream_t)stream_>>>(
-        cand, ld_cand, (int)n_cand, query, ld_query, query_aug, ld_aug, dim, k, n_sample, stats, rec_query, rec_cand, x,
-        thr, theta, TopkDot{});
-    LKG_LAUNCH_CHECK("topk_threshold_kernel<l2>");
+    topk_threshold_kernel<Kind><<<(unsigned)n_queries, kTopkThreads, 0, stream>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, aug, ld_aug, dim, k, n_sample, stats, rec_query, rec_cand, x, thr,
+        theta, dot);
+    LKG_LAUNCH_CHECK(Kind == kL2 ? "topk_threshold_kernel<l2>" : "topk_threshold_kernel<dot>");
     return LKG_OK;
 }
 
-extern "C" int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
-                                    int64_t ld_query, int64_t n_queries, int32_t dim, const int32_t* band_cnt,
-                                    const int32_t* band, int32_t cap, int32_t k, const lkg_graph* known,
-                                    const int64_t* anchors, const int64_t* rels, const int64_t* cand_ids, float* dist,
-                                    int64_t* pos, void* stream_) {
-    if (int rc = check_l2_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_l2_rows("query", query, ld_query, dim)) return rc;
-    LKG_REQUIRE(band_cnt && band && dist && pos, "bad top-k arguments (band_cnt, band, dist, pos)");
+// The same for the top-k finalize: shape, k, cap, the excluded set and the sort buffer (next_pow2(cap) keys).
+template <int Kind>
+static int launch_topk_finalize(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
+                                int64_t ld_query, int64_t n_queries, int32_t dim, const int32_t* band_cnt,
+                                const int32_t* band, int32_t cap, int32_t k, const lkg_graph* known,
+                                const int64_t* anchors, const int64_t* rels, const int64_t* cand_ids, float* val,
+                                int64_t* pos, const TopkDot& dot, cudaStream_t stream) {
     LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
                 "bad top-k shape (n_queries, n_cand)");
     LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
@@ -1562,46 +1469,56 @@ extern "C" int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t 
     int p2 = 1;
     while (p2 < cap) p2 <<= 1;
     const int smem = p2 * (int)sizeof(unsigned long long);
-    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_kernel<kL2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    topk_finalize_kernel<kL2><<<(unsigned)n_queries, kTopkThreads, smem, (cudaStream_t)stream_>>>(
-        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, dist, pos, TopkDot{});
-    LKG_LAUNCH_CHECK("topk_finalize_kernel<l2>");
+    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_kernel<Kind>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    topk_finalize_kernel<Kind><<<(unsigned)n_queries, kTopkThreads, smem, stream>>>(
+        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, val, pos, dot);
+    LKG_LAUNCH_CHECK(Kind == kL2 ? "topk_finalize_kernel<l2>" : "topk_finalize_kernel<dot>");
     return LKG_OK;
+}
+
+extern "C" int lkg_topk_threshold_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
+                                     int64_t ld_query, const float* query_aug, int64_t ld_aug, int64_t n_queries,
+                                     int32_t dim, const float* stats, const float* rec_query, const float* rec_cand,
+                                     int32_t k, int32_t n_sample, const lkg_graph* known, const int64_t* anchors,
+                                     const int64_t* rels, const int64_t* cand_ids, float* thr, float* theta,
+                                     void* stream_) {
+    if (int rc = check_rows<kL2>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kL2>("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(query_aug && ld_aug >= dim + 4 && ld_aug % 4 == 0 && aligned16(query_aug),
+                "query_aug rows need dim + 4 columns and 16-byte alignment");
+    LKG_REQUIRE(stats && rec_query && rec_cand && thr, "bad top-k arguments (stats, rec_query, rec_cand, thr)");
+    return launch_topk_threshold<kL2>(cand, ld_cand, n_cand, query, ld_query, query_aug, ld_aug, n_queries, dim, stats,
+                                      rec_query, rec_cand, k, n_sample, known, anchors, rels, cand_ids, thr, theta,
+                                      TopkDot{}, (cudaStream_t)stream_);
+}
+
+extern "C" int lkg_topk_finalize_l2(const float* cand, int64_t ld_cand, int64_t n_cand, const float* query,
+                                    int64_t ld_query, int64_t n_queries, int32_t dim, const int32_t* band_cnt,
+                                    const int32_t* band, int32_t cap, int32_t k, const lkg_graph* known,
+                                    const int64_t* anchors, const int64_t* rels, const int64_t* cand_ids, float* dist,
+                                    int64_t* pos, void* stream_) {
+    if (int rc = check_rows<kL2>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kL2>("query", query, ld_query, dim)) return rc;
+    LKG_REQUIRE(band_cnt && band && dist && pos, "bad top-k arguments (band_cnt, band, dist, pos)");
+    return launch_topk_finalize<kL2>(cand, ld_cand, n_cand, query, ld_query, n_queries, dim, band_cnt, band, cap, k,
+                                     known, anchors, rels, cand_ids, dist, pos, TopkDot{}, (cudaStream_t)stream_);
 }
 
 // ---- filtered top-k under the dot score -----------------------------------------------------------------------------
-static int check_dot_rows(const char* what, const float* p, int64_t ld, int32_t dim) {
-    LKG_REQUIRE(p, "%s is null", what);
-    LKG_REQUIRE(dim >= 4 && dim % 4 == 0 && dim <= kTopkRow,
-                "the dot top-k path supports dim %% 4 == 0, 4 <= dim <= %d, got %d", kTopkRow, dim);
-    LKG_REQUIRE(ld >= dim && ld % 4 == 0 && aligned16(p), "%s rows must be 16-byte aligned (ld %% 4 == 0, ld >= dim)",
-                what);
-    return LKG_OK;
-}
-
 extern "C" int lkg_topk_threshold_dot(const float* cand, int64_t ld_cand, const int64_t* cand_rows, int64_t n_cand,
                                       const float* query, int64_t ld_query, const int64_t* query_rows,
                                       int64_t n_queries, int32_t dim, const float* center, const float* cand_max_norm,
                                       const float* rec_query, const float* rec_cand, int32_t k, int32_t n_sample,
                                       const lkg_graph* known, const int64_t* anchors, const int64_t* rels,
                                       const int64_t* cand_ids, float* thr, float* theta, void* stream_) {
-    if (int rc = check_dot_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_dot_rows("query", query, ld_query, dim)) return rc;
+    if (int rc = check_rows<kDot>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kDot>("query", query, ld_query, dim)) return rc;
     LKG_REQUIRE(center && aligned16(center), "center must be a 16-byte aligned [dim] vector");
     LKG_REQUIRE(cand_max_norm && rec_query && rec_cand && thr,
                 "bad top-k arguments (cand_max_norm, rec_query, rec_cand, thr)");
-    LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
-                "bad top-k shape (n_queries, n_cand)");
-    LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
-    LKG_REQUIRE(n_sample >= 1 && n_sample <= n_cand, "n_sample must be in [1, n_cand], got %d", n_sample);
-    TopkExclude x;
-    if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
-    if (n_queries == 0) return LKG_OK;
-    topk_threshold_kernel<kDot><<<(unsigned)n_queries, kTopkThreads, 0, (cudaStream_t)stream_>>>(
-        cand, ld_cand, (int)n_cand, query, ld_query, nullptr, 0, dim, k, n_sample, cand_max_norm, rec_query, rec_cand,
-        x, thr, theta, TopkDot{cand_rows, query_rows, center});
-    LKG_LAUNCH_CHECK("topk_threshold_kernel<dot>");
-    return LKG_OK;
+    return launch_topk_threshold<kDot>(cand, ld_cand, n_cand, query, ld_query, nullptr, 0, n_queries, dim,
+                                       cand_max_norm, rec_query, rec_cand, k, n_sample, known, anchors, rels, cand_ids,
+                                       thr, theta, TopkDot{cand_rows, query_rows, center}, (cudaStream_t)stream_);
 }
 
 extern "C" int lkg_topk_finalize_dot(const float* cand, int64_t ld_cand, const int64_t* cand_rows, int64_t n_cand,
@@ -1610,23 +1527,10 @@ extern "C" int lkg_topk_finalize_dot(const float* cand, int64_t ld_cand, const i
                                      int32_t cap, int32_t k, const lkg_graph* known, const int64_t* anchors,
                                      const int64_t* rels, const int64_t* cand_ids, float* score, int64_t* pos,
                                      void* stream_) {
-    if (int rc = check_dot_rows("cand", cand, ld_cand, dim)) return rc;
-    if (int rc = check_dot_rows("query", query, ld_query, dim)) return rc;
+    if (int rc = check_rows<kDot>("cand", cand, ld_cand, dim)) return rc;
+    if (int rc = check_rows<kDot>("query", query, ld_query, dim)) return rc;
     LKG_REQUIRE(band_cnt && band && score && pos, "bad top-k arguments (band_cnt, band, score, pos)");
-    LKG_REQUIRE(n_queries >= 0 && n_queries < (1ll << 31) && n_cand >= 1 && n_cand < (1ll << 31),
-                "bad top-k shape (n_queries, n_cand)");
-    LKG_REQUIRE(k >= 1 && k <= kTopkMaxK, "k must be in [1, %d], got %d", kTopkMaxK, k);
-    LKG_REQUIRE(cap >= 2 * k && cap <= kTopkMaxCap, "cap must be in [2k, %d], got %d (k = %d)", kTopkMaxCap, cap, k);
-    TopkExclude x;
-    if (int rc = topk_exclude(known, anchors, rels, cand_ids, &x)) return rc;
-    if (n_queries == 0) return LKG_OK;
-    int p2 = 1;
-    while (p2 < cap) p2 <<= 1;
-    const int smem = p2 * (int)sizeof(unsigned long long);
-    LKG_CUDA(cudaFuncSetAttribute(topk_finalize_kernel<kDot>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    topk_finalize_kernel<kDot><<<(unsigned)n_queries, kTopkThreads, smem, (cudaStream_t)stream_>>>(
-        cand, ld_cand, (int)n_cand, query, ld_query, dim, band_cnt, band, cap, k, x, score, pos,
-        TopkDot{cand_rows, query_rows, nullptr});
-    LKG_LAUNCH_CHECK("topk_finalize_kernel<dot>");
-    return LKG_OK;
+    return launch_topk_finalize<kDot>(cand, ld_cand, n_cand, query, ld_query, n_queries, dim, band_cnt, band, cap, k,
+                                      known, anchors, rels, cand_ids, score, pos, TopkDot{cand_rows, query_rows, nullptr},
+                                      (cudaStream_t)stream_);
 }

@@ -16,6 +16,7 @@ Stage map (reference -> here)
 from __future__ import annotations
 
 import math
+from types import SimpleNamespace
 from typing import Dict, List, Optional, Tuple
 
 import torch
@@ -1280,70 +1281,26 @@ class LiteralKG(nn.Module):
         launch)."""
         if score not in ("dot", "triple"):
             raise ValueError('score must be "dot" or "triple"')
-        if predict not in ("tail", "head"):
-            raise ValueError('predict must be "tail" or "head"')
         triple = score == "triple"
-        if triple:
-            if relations is None:
-                raise ValueError("the triple score needs the relation of every query")
-            d_s = self.relation_embed.weight.shape[1]
-            if d_s > ops.L2_RANK_MAX_DIM:
-                raise ValueError(f"the triple score supports widths up to {ops.L2_RANK_MAX_DIM} (relation_dim {d_s})")
-        if predict == "head":
-            heads, tails = tails, heads
-            known = None if known is None else known.reversed()
-        dev = self._param_device()
+        if relations is not None and known is None and not triple:
+            raise ValueError("relations only select the filter set: pass the known triples as well")
         with torch.no_grad():
-            if all_embed is None:
-                all_embed = self.gat_embeddings()
-            all_embed = _lib.f32c(all_embed)
-            n, dim = all_embed.shape
-
-            heads, tails = _query_ids(heads, dev), _query_ids(tails, dev)
-            q = heads.numel()
-            rels = None if relations is None else _query_ids(relations, dev)
-            if tails.numel() != q or (rels is not None and rels.numel() != q):
-                raise ValueError("heads, tails and relations must have the same length")
-            if rels is not None and known is None and not triple:
-                raise ValueError("relations only select the filter set: pass the known triples as well")
-            if triple and self._triple_projection() is None and dim != self.relation_embed.weight.shape[1]:
-                raise ValueError(f"the TransE score adds relation embeddings ({self.relation_embed.weight.shape[1]} wide) "
-                                 f"to rows of the embeddings ({dim} wide)")
-            if known is not None and known.n_entities != n:
-                raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
-            if candidates is not None and q and len(candidates) == 0:
-                raise ValueError("no candidates")
-
-            bad = {"head or tail ids outside [0, n_entities)": _outside(heads, n) | _outside(tails, n)}
-            heads, tails = heads.clamp(0, n - 1), tails.clamp(0, n - 1)
-            cand, n_cand, cmap = _candidate_ids(candidates, n, dev, bad)
-            tpos = tails
-            if candidates is not None:
-                tpos = cmap[tails].long()
-                bad["a target tail is not a candidate"] = (tpos < 0).any()
-                tpos = tpos.clamp_min(0)
-            if triple:               # the relation selects M_r and e_r, not only a filter run
-                bad[f"relation ids outside [0, {self.n_relations}) of the model"] = _outside(rels, self.n_relations)
-                rels = rels.clamp(0, self.n_relations - 1)
-            if rels is not None and known is not None:
-                bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
-                rels = rels.clamp(0, known.n_relations - 1)
-
-            part, world, per, lo, hi = self._query_slice(q)
-            sl = slice(lo, hi)
+            qs = self._queries(predict, heads, relations, known, candidates, all_embed, targets=tails, triple=triple)
+            bad, sl = qs.bad, slice(qs.lo, qs.hi)
             if triple:
-                counts = torch.bincount(rels[sl], minlength=self.n_relations)
+                counts = torch.bincount(qs.rels[sl], minlength=self.n_relations)
                 host = torch.cat([torch.stack(list(bad.values())).long(), counts]).tolist()
                 _raise_flags(bad, host)
-                ranks = self._rank_triple(all_embed, heads[sl], tpos[sl], rels[sl], host[len(bad):], known, cmap, cand,
-                                          n_cand, batch_size, 1.0 if predict == "tail" else -1.0)
+                ranks = self._rank_triple(qs.emb, qs.anchors[sl], qs.tpos[sl], qs.rels[sl], host[len(bad):], qs.known,
+                                          qs.cmap, qs.cand, qs.n_cand, batch_size, 1.0 if predict == "tail" else -1.0)
             else:
-                ranks = self._rank_queries(all_embed, heads[sl], tpos[sl], None if rels is None else rels[sl], known,
-                                           cmap, cand, n_cand, batch_size)
-            if world > 1:
-                padded = torch.zeros(per, dtype=torch.int64, device=dev)
-                padded[:hi - lo] = ranks
-                ranks = part.all_gather_stack(padded).reshape(-1)[:q]
+                ranks = self._rank_queries(qs.emb, qs.anchors[sl], qs.tpos[sl], None if qs.rels is None else qs.rels[sl],
+                                           qs.known, qs.cmap, qs.cand, qs.n_cand, batch_size)
+            q = qs.q
+            if qs.world > 1:
+                padded = torch.zeros(qs.per, dtype=torch.int64, device=ranks.device)
+                padded[:qs.hi - qs.lo] = ranks
+                ranks = qs.part.all_gather_stack(padded).reshape(-1)[:q]
 
             r1 = ranks.double() + 1.0
             ks = [int(k) for k in ks]
@@ -1372,59 +1329,20 @@ class LiteralKG(nn.Module):
         relations are required, widths up to 508; the argument checks ride on one host read-back before the first
         launch.  Row partitioned (``set_partition``, world > 1) this is a collective: every rank completes a contiguous
         slice of the queries and every rank returns the whole result."""
-        if predict not in ("tail", "head"):
-            raise ValueError('predict must be "tail" or "head"')
-        if relations is None:
-            raise ValueError("the triple score needs the relation of every query")
-        if isinstance(k, bool) or int(k) != k or not 1 <= k <= ops.TOPK_L2_MAX_K:
-            raise ValueError(f"k must be an integer in [1, {ops.TOPK_L2_MAX_K}], got {k}")
-        k = int(k)
-        d_s = self.relation_embed.weight.shape[1]
-        if d_s > ops.L2_RANK_MAX_DIM:
-            raise ValueError(f"the triple score supports widths up to {ops.L2_RANK_MAX_DIM} (relation_dim {d_s})")
-        if predict == "head" and known is not None:
-            known = known.reversed()
-        dev = self._param_device()
         with torch.no_grad():
-            if all_embed is None:
-                all_embed = self.gat_embeddings()
-            all_embed = _lib.f32c(all_embed)
-            n, dim = all_embed.shape
-
-            anchors, rels = _query_ids(anchors, dev), _query_ids(relations, dev)
-            q = anchors.numel()
-            if rels.numel() != q:
-                raise ValueError("anchors and relations must have the same length")
-            if self._triple_projection() is None and dim != d_s:
-                raise ValueError(f"the TransE score adds relation embeddings ({d_s} wide) to rows of the embeddings "
-                                 f"({dim} wide)")
-            if known is not None and known.n_entities != n:
-                raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
-            if candidates is not None and len(candidates) == 0:
-                raise ValueError("no candidates")
-
-            bad = {"anchor ids outside [0, n_entities)": _outside(anchors, n)}
-            anchors = anchors.clamp(0, n - 1)
-            cand, n_cand, _ = _candidate_ids(candidates, n, dev, bad)
-            bad[f"relation ids outside [0, {self.n_relations}) of the model"] = _outside(rels, self.n_relations)
-            rels = rels.clamp(0, self.n_relations - 1)
-            if known is not None:
-                bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
-                rels = rels.clamp(0, known.n_relations - 1)
-
-            part, world, per, lo, hi = self._query_slice(q)
-            sl = slice(lo, hi)
-            counts = torch.bincount(rels[sl], minlength=self.n_relations)
-            host = torch.cat([torch.stack(list(bad.values())).long(), counts]).tolist()
-            _raise_flags(bad, host)
-            mine, a_sl, r_sl = hi - lo, anchors[sl], rels[sl]
-            dist = torch.empty((mine, k), dtype=torch.float32, device=dev)
-            pos = torch.empty((mine, k), dtype=torch.int64, device=dev)
-            for qs, index, qrows in self._triple_batches(all_embed, a_sl, r_sl, host[len(bad):], cand, n_cand,
-                                                         batch_size, 1.0 if predict == "tail" else -1.0):
-                exclude = None if known is None else (known, a_sl[qs], r_sl[qs], cand)
-                dist[qs], pos[qs] = ops.score_topk_l2(index, qrows, k, exclude=exclude)
-            return self._gather_topk(dist, pos, cand, q, per, float("inf"))
+            qs = self._queries(predict, anchors, relations, known, candidates, all_embed, k=k, triple=True)
+            k, sl = int(k), slice(qs.lo, qs.hi)
+            counts = torch.bincount(qs.rels[sl], minlength=self.n_relations)
+            host = torch.cat([torch.stack(list(qs.bad.values())).long(), counts]).tolist()
+            _raise_flags(qs.bad, host)
+            mine, a_sl, r_sl = qs.hi - qs.lo, qs.anchors[sl], qs.rels[sl]
+            dist = torch.empty((mine, k), dtype=torch.float32, device=a_sl.device)
+            pos = torch.empty((mine, k), dtype=torch.int64, device=a_sl.device)
+            for b, index, qrows in self._triple_batches(qs.emb, a_sl, r_sl, host[len(qs.bad):], qs.cand, qs.n_cand,
+                                                        batch_size, 1.0 if predict == "tail" else -1.0):
+                exclude = None if qs.known is None else (qs.known, a_sl[b], r_sl[b], qs.cand)
+                dist[b], pos[b] = ops.score_topk_l2(index, qrows, k, exclude=exclude)
+            return self._gather_topk(dist, pos, qs.cand, qs.q, qs.per, float("inf"))
 
     def topk_links(self, anchors, k, relations=None, known=None, candidates=None, predict="tail", batch_size=2048,
                    all_embed=None):
@@ -1445,11 +1363,6 @@ class LiteralKG(nn.Module):
         ``batch_size`` queries, no B x N score matrix at any width; the argument checks ride on one host read-back
         before the first launch.  Row partitioned (``set_partition``, world > 1) this is a collective: every rank
         completes a contiguous slice of the queries and every rank returns the whole result."""
-        if predict not in ("tail", "head"):
-            raise ValueError('predict must be "tail" or "head"')
-        if isinstance(k, bool) or int(k) != k or not 1 <= k <= ops.TOPK_L2_MAX_K:
-            raise ValueError(f"k must be an integer in [1, {ops.TOPK_L2_MAX_K}], got {k}")
-        k = int(k)
         if relations is not None and known is None:
             raise ValueError("relations only select the excluded set: pass the known triples as well")
 
@@ -1457,50 +1370,93 @@ class LiteralKG(nn.Module):
             if emb.shape[1] > ops.TOPK_DOT_MAX_DIM:
                 raise ValueError(f"the dot top-k supports widths up to {ops.TOPK_DOT_MAX_DIM} (got {emb.shape[1]})")
 
-        if all_embed is not None:
-            check_width(all_embed)
-        if predict == "head" and known is not None:
-            known = known.reversed()
-        dev = self._param_device()
         with torch.no_grad():
-            if all_embed is None:
-                all_embed = self.gat_embeddings()
-                check_width(all_embed)
-            all_embed = _lib.f32c(all_embed)
-            n, dim = all_embed.shape
-            anchors = _query_ids(anchors, dev)
-            q = anchors.numel()
-            rels = None if relations is None else _query_ids(relations, dev)
-            if rels is not None and rels.numel() != q:
-                raise ValueError("anchors and relations must have the same length")
-            if known is not None and known.n_entities != n:
-                raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
-            if candidates is not None and len(candidates) == 0:
-                raise ValueError("no candidates")
-
-            bad = {"anchor ids outside [0, n_entities)": _outside(anchors, n)}
-            anchors = anchors.clamp(0, n - 1)
-            cand, n_cand, _ = _candidate_ids(candidates, n, dev, bad)
-            if rels is not None:
-                bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
-                rels = rels.clamp(0, known.n_relations - 1)
-            part, world, per, lo, hi = self._query_slice(q)
-            _raise_flags(bad, torch.stack(list(bad.values())).tolist())
-
-            if dim % 4:                          # zero columns add nothing to a dot product
-                padded = torch.zeros((n, (dim + 3) // 4 * 4), dtype=torch.float32, device=dev)
-                padded[:, :dim] = all_embed
+            qs = self._queries(predict, anchors, relations, known, candidates, all_embed, k=k, check_width=check_width)
+            k, all_embed, n, dev = int(k), qs.emb, qs.emb.shape[0], qs.emb.device
+            _raise_flags(qs.bad, torch.stack(list(qs.bad.values())).tolist())
+            if all_embed.shape[1] % 4:           # zero columns add nothing to a dot product
+                padded = torch.zeros((n, (all_embed.shape[1] + 3) // 4 * 4), dtype=torch.float32, device=dev)
+                padded[:, :all_embed.shape[1]] = all_embed
                 all_embed = padded
-            index = ops.ScoreIndex(all_embed, cand)
-            mine, a_sl = hi - lo, anchors[lo:hi]
-            r_sl = None if rels is None else rels[lo:hi]
+            index = ops.ScoreIndex(all_embed, qs.cand)
+            mine, a_sl = qs.hi - qs.lo, qs.anchors[qs.lo:qs.hi]
+            r_sl = None if qs.rels is None else qs.rels[qs.lo:qs.hi]
             vals = torch.empty((mine, k), dtype=torch.float32, device=dev)
             pos = torch.empty((mine, k), dtype=torch.int64, device=dev)
             for b0 in range(0, mine, batch_size):
                 b = slice(b0, b0 + batch_size)
-                exclude = None if known is None else (known, a_sl[b], None if r_sl is None else r_sl[b], cand)
+                exclude = None if qs.known is None else (qs.known, a_sl[b], None if r_sl is None else r_sl[b], qs.cand)
                 vals[b], pos[b] = ops.score_topk_dot(all_embed, a_sl[b], k, index, exclude=exclude)
-            return self._gather_topk(vals, pos, cand, q, per, float("-inf"))
+            return self._gather_topk(vals, pos, qs.cand, qs.q, qs.per, float("-inf"))
+
+    def _queries(self, predict, anchors, relations, known, candidates, all_embed, targets=None, k=None, triple=False,
+                 check_width=None):
+        """The argument checks and query preparation of ``evaluate_ranking`` (``targets`` = its tails), ``topk_triple``
+        (``triple``) and ``topk_links`` (``check_width``, called on the embeddings), in the order that keeps every
+        refusal before the first launch.  Head prediction swaps anchors and targets and reverses ``known``.  The embedding
+        pass runs unless ``all_embed`` is given.  Ids outside their range are clamped and recorded in ``bad`` (message ->
+        device flag) for the caller's one host read-back.  -> a namespace of: emb (fp32 contiguous), anchors, tpos
+        (target positions among the candidates; None without targets), rels (None without relations), known, cand,
+        n_cand, cmap, bad, q and the row partition's slice part, world, per, lo, hi (``_query_slice``)."""
+        if predict not in ("tail", "head"):
+            raise ValueError('predict must be "tail" or "head"')
+        if k is not None and (isinstance(k, bool) or int(k) != k or not 1 <= k <= ops.TOPK_L2_MAX_K):
+            raise ValueError(f"k must be an integer in [1, {ops.TOPK_L2_MAX_K}], got {k}")
+        if triple:
+            if relations is None:
+                raise ValueError("the triple score needs the relation of every query")
+            d_s = self.relation_embed.weight.shape[1]
+            if d_s > ops.L2_RANK_MAX_DIM:
+                raise ValueError(f"the triple score supports widths up to {ops.L2_RANK_MAX_DIM} (relation_dim {d_s})")
+        if check_width is not None and all_embed is not None:
+            check_width(all_embed)
+        if predict == "head":
+            if targets is not None:
+                anchors, targets = targets, anchors
+            known = None if known is None else known.reversed()
+        dev = self._param_device()
+        if all_embed is None:
+            all_embed = self.gat_embeddings()
+            if check_width is not None:
+                check_width(all_embed)
+        all_embed = _lib.f32c(all_embed)
+        n, dim = all_embed.shape
+
+        anchors = _query_ids(anchors, dev)
+        q = anchors.numel()
+        tpos = None if targets is None else _query_ids(targets, dev)
+        rels = None if relations is None else _query_ids(relations, dev)
+        if (tpos is not None and tpos.numel() != q) or (rels is not None and rels.numel() != q):
+            raise ValueError("heads, tails and relations must have the same length" if targets is not None else
+                             "anchors and relations must have the same length")
+        if triple and self._triple_projection() is None and dim != self.relation_embed.weight.shape[1]:
+            raise ValueError(f"the TransE score adds relation embeddings ({self.relation_embed.weight.shape[1]} wide) "
+                             f"to rows of the embeddings ({dim} wide)")
+        if known is not None and known.n_entities != n:
+            raise ValueError(f"the known plan has {known.n_entities} entities, the embeddings {n}")
+        if candidates is not None and len(candidates) == 0 and (q or targets is None):
+            raise ValueError("no candidates")
+
+        if tpos is None:
+            bad = {"anchor ids outside [0, n_entities)": _outside(anchors, n)}
+        else:
+            bad = {"head or tail ids outside [0, n_entities)": _outside(anchors, n) | _outside(tpos, n)}
+            tpos = tpos.clamp(0, n - 1)
+        anchors = anchors.clamp(0, n - 1)
+        cand, n_cand, cmap = _candidate_ids(candidates, n, dev, bad)
+        if tpos is not None and candidates is not None:
+            tpos = cmap[tpos].long()
+            bad["a target tail is not a candidate"] = (tpos < 0).any()
+            tpos = tpos.clamp_min(0)
+        if triple:                   # the relation selects M_r and e_r, not only a filter run
+            bad[f"relation ids outside [0, {self.n_relations}) of the model"] = _outside(rels, self.n_relations)
+            rels = rels.clamp(0, self.n_relations - 1)
+        if rels is not None and known is not None:
+            bad[f"relation ids outside [0, {known.n_relations})"] = _outside(rels, known.n_relations)
+            rels = rels.clamp(0, known.n_relations - 1)
+        part, world, per, lo, hi = self._query_slice(q)
+        return SimpleNamespace(emb=all_embed, anchors=anchors, tpos=tpos, rels=rels, known=known, cand=cand,
+                               n_cand=n_cand, cmap=cmap, bad=bad, q=q, part=part, world=world, per=per, lo=lo, hi=hi)
 
     def _query_slice(self, q: int):
         """The queries a rank answers in a row-partitioned collective: -> (part, world, per, lo, hi), a contiguous

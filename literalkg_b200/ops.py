@@ -410,6 +410,44 @@ class ScoreIndex:
         return self._centered
 
 
+def _count_band(lib, query_planes, cand_planes, n_cand: int, thr: torch.Tensor, cap: int):
+    """lkg_score_rank of the query planes against ``n_cand`` candidate planes under the per-query thresholds ``thr``
+    (fp32 [B, 2]) -> (counters int32 [2, B], band int32 [B, cap]): counters[0] = columns above thr[:, 1], counters[1] =
+    columns at or above thr[:, 0] and not above thr[:, 1], listed in band (a count above ``cap``: the list overflowed)."""
+    nq = thr.shape[0]
+    counters = torch.zeros((2, nq), dtype=torch.int32, device=thr.device)
+    band = torch.empty((nq, max(cap, 1)), dtype=torch.int32, device=thr.device)
+    a, b = _lib.planes_operand([query_planes]), _lib.planes_operand([cand_planes])
+    _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), n_cand, thr.data_ptr(), counters[0].data_ptr(),
+                                  counters[1].data_ptr(), band.data_ptr(), cap, _lib.stream()))
+    return counters, band
+
+
+def _filter_ids(ranks: torch.Tensor, anchors, target_pos, relations, cand_map):
+    """The query ids of a rank filter on the device of ``ranks``, one per rank: -> (anchors, target_pos, relations)."""
+    assert ranks.dtype == torch.int64 and ranks.is_contiguous()
+    dev = ranks.device
+    anchors, tgt = _ids(anchors, dev), _ids(target_pos, dev)
+    rels = None if relations is None else _ids(relations, dev)
+    assert anchors.numel() == tgt.numel() == ranks.numel() and (rels is None or rels.numel() == ranks.numel())
+    assert cand_map is None or (cand_map.dtype == torch.int32 and cand_map.is_contiguous())
+    return anchors, tgt, rels
+
+
+def _exclude_args(exclude, nq: int, n_cand: int, dev):
+    """``exclude`` of the top-k calls, (known plan, anchors [nq], relations [nq] or None, candidate entity ids
+    [n_cand] or None), or None -> (plan reference or None, anchors, relations, ids) on ``dev``."""
+    if exclude is None:
+        return None, None, None, None
+    known, anchors, rels, cids = exclude
+    anchors = _ids(anchors, dev)
+    rels = None if rels is None else _ids(rels, dev)
+    cids = None if cids is None else _ids(cids, dev)
+    assert anchors.numel() == nq and (rels is None or rels.numel() == nq)
+    assert cids is None or cids.numel() == n_cand
+    return None if known is None else known.byref(), anchors, rels, cids
+
+
 def score_rank(emb: torch.Tensor, heads: Optional[torch.Tensor], target_pos: torch.Tensor, tail_index: ScoreIndex,
                head_emb: Optional[torch.Tensor] = None, band_cap: int = 8192,
                tau_out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -432,17 +470,13 @@ def score_rank(emb: torch.Tensor, heads: Optional[torch.Tensor], target_pos: tor
     tau = torch.empty(nh, dtype=torch.float32, device=emb.device) if tau_out is None else tau_out
     assert tau.dtype == torch.float32 and tau.is_contiguous() and tau.numel() == nh
     thr = torch.empty((nh, 2), dtype=torch.float32, device=emb.device)
-    counters = torch.zeros((2, nh), dtype=torch.int32, device=emb.device)
-    band = torch.empty((nh, band_cap), dtype=torch.int32, device=emb.device)
-    a, b = _lib.planes_operand([hp]), _lib.planes_operand([tp])
     with _dev_guard(emb, "score_rank", 3):
         lib = _lib.load()
         _lib.check(lib.lkg_rank_prepare(emb.data_ptr(), emb.stride(0), _lib.ptr(ti.rows), hsrc.data_ptr(), hsrc.stride(0),
                                         _lib.ptr(hrows), tgt.data_ptr(), nh, emb.shape[1], ci.max_norm.data_ptr(),
                                         ci.rec.data_ptr(), center.data_ptr(), tau.data_ptr(), thr.data_ptr(),
                                         _lib.stream()))
-        _lib.check(lib.lkg_score_rank(C.byref(a), nh, C.byref(b), ti.m, thr.data_ptr(), counters[0].data_ptr(),
-                                      counters[1].data_ptr(), band.data_ptr(), band_cap, _lib.stream()))
+        counters, band = _count_band(lib, hp, tp, ti.m, thr, band_cap)
         _lib.check(lib.lkg_rank_finalize(emb.data_ptr(), emb.stride(0), _lib.ptr(ti.rows), hsrc.data_ptr(), hsrc.stride(0),
                                          _lib.ptr(hrows), tgt.data_ptr(), tau.data_ptr(), counters[0].data_ptr(),
                                          counters[1].data_ptr(), band.data_ptr(), band_cap, nh, ti.m, emb.shape[1],
@@ -460,12 +494,7 @@ def filter_ranks(ranks: torch.Tensor, known: GraphPlan, heads: torch.Tensor, tar
     [N] or None = identity): candidate position of every entity, -1 = not a candidate.  The scores are either
     ``emb`` + ``tau`` (after ``score_rank`` on ``emb``: the same exact re-score and target scores) or ``scores`` (the
     [B, Nc] matrix ``topk_rows`` ranked)."""
-    assert ranks.dtype == torch.int64 and ranks.is_contiguous()
-    dev = ranks.device
-    heads, tgt = _ids(heads, dev), _ids(target_pos, dev)
-    rels = None if relations is None else _ids(relations, dev)
-    assert heads.numel() == tgt.numel() == ranks.numel() and (rels is None or rels.numel() == ranks.numel())
-    assert cand_map is None or (cand_map.dtype == torch.int32 and cand_map.is_contiguous())
+    heads, tgt, rels = _filter_ids(ranks, heads, target_pos, relations, cand_map)
     assert (scores is None) != (emb is None or tau is None), "give emb + tau (fused path) or scores (dense path)"
     with _dev_guard(ranks, "filter_ranks"):
         if scores is None:
@@ -546,17 +575,13 @@ def score_rank_l2(index: L2Index, query: torch.Tensor, target_pos: torch.Tensor,
     tau = torch.empty(nq, dtype=torch.float32, device=dev) if tau_out is None else tau_out
     assert tau.dtype == torch.float32 and tau.is_contiguous() and tau.numel() == nq
     thr = torch.empty((nq, 2), dtype=torch.float32, device=dev)
-    counters = torch.zeros((2, nq), dtype=torch.int32, device=dev)
-    band = torch.empty((nq, band_cap), dtype=torch.int32, device=dev)
-    a, b = _lib.planes_operand([qp]), _lib.planes_operand([index.planes])
     with _dev_guard(query, "score_rank_l2", 3):
         lib = _lib.load()
         _lib.check(lib.lkg_rank_prepare_l2(index.cand.data_ptr(), index.cand.stride(0), query.data_ptr(), query.stride(0),
                                            aug.data_ptr(), aug.stride(0), tgt.data_ptr(), nq, index.dim,
                                            index.stats.data_ptr(), qp.rec.data_ptr(), index.planes.rec.data_ptr(),
                                            tau.data_ptr(), thr.data_ptr(), _lib.stream()))
-        _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), index.m, thr.data_ptr(), counters[0].data_ptr(),
-                                      counters[1].data_ptr(), band.data_ptr(), band_cap, _lib.stream()))
+        counters, band = _count_band(lib, qp, index.planes, index.m, thr, band_cap)
         _lib.check(lib.lkg_rank_finalize_l2(index.cand.data_ptr(), index.cand.stride(0), query.data_ptr(),
                                             query.stride(0), tgt.data_ptr(), tau.data_ptr(), counters[0].data_ptr(),
                                             counters[1].data_ptr(), band.data_ptr(), band_cap, nq, index.m, index.dim,
@@ -572,12 +597,7 @@ def filter_ranks_l2(ranks: torch.Tensor, known: GraphPlan, anchors: torch.Tensor
     """``filter_ranks`` after ``score_rank_l2`` (lkg_rank_filter_l2): query i's filter set is the run of
     (anchors[i], relations[i]) in ``known``; a member f is re-scored with the same exact distance between ``query[i]``
     and its candidate row ``index.cand[cand_map[f]]`` and compared with the same ``tau``."""
-    assert ranks.dtype == torch.int64 and ranks.is_contiguous()
-    dev = ranks.device
-    anchors, tgt = _ids(anchors, dev), _ids(target_pos, dev)
-    rels = None if relations is None else _ids(relations, dev)
-    assert anchors.numel() == tgt.numel() == ranks.numel() and (rels is None or rels.numel() == ranks.numel())
-    assert cand_map is None or (cand_map.dtype == torch.int32 and cand_map.is_contiguous())
+    anchors, tgt, rels = _filter_ids(ranks, anchors, target_pos, relations, cand_map)
     _rowmajor(query)
     with _dev_guard(ranks, "filter_ranks_l2"):
         _lib.check(_lib.load().lkg_rank_filter_l2(known.byref(), anchors.data_ptr(), _lib.ptr(rels), _lib.ptr(cand_map),
@@ -618,22 +638,11 @@ def score_topk_l2(index: L2Index, query: torch.Tensor, k: int, exclude=None, cap
         return dist, pos
     if n_sample is None:
         n_sample = topk_l2_samples(index.m, k)
-    known = anchors = rels = cids = None
-    if exclude is not None:
-        known, anchors, rels, cids = exclude
-        anchors = _ids(anchors, dev)
-        rels = None if rels is None else _ids(rels, dev)
-        cids = None if cids is None else _ids(cids, dev)
-        assert anchors.numel() == nq and (rels is None or rels.numel() == nq)
-        assert cids is None or cids.numel() == index.m
-    kb = None if known is None else known.byref()
+    kb, anchors, rels, cids = _exclude_args(exclude, nq, index.m, dev)
     aug = l2_rank_rows(query, index.center, _lib.L2_QUERY, index.stats)
     qp = split_planes(aug)                               # own scale record: the two operands' factors multiply
     thr = torch.empty((nq, 2), dtype=torch.float32, device=dev)
     theta = torch.empty(nq, dtype=torch.float32, device=dev)
-    counters = torch.zeros((2, nq), dtype=torch.int32, device=dev)
-    band = torch.empty((nq, max(cap, 1)), dtype=torch.int32, device=dev)
-    a, b = _lib.planes_operand([qp]), _lib.planes_operand([index.planes])
     with _dev_guard(query, "score_topk_l2", 3):
         lib = _lib.load()
         _lib.check(lib.lkg_topk_threshold_l2(index.cand.data_ptr(), index.cand.stride(0), index.m, query.data_ptr(),
@@ -641,8 +650,7 @@ def score_topk_l2(index: L2Index, query: torch.Tensor, k: int, exclude=None, cap
                                              index.stats.data_ptr(), qp.rec.data_ptr(), index.planes.rec.data_ptr(),
                                              int(k), int(n_sample), kb, _lib.ptr(anchors), _lib.ptr(rels),
                                              _lib.ptr(cids), thr.data_ptr(), theta.data_ptr(), _lib.stream()))
-        _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), index.m, thr.data_ptr(), counters[0].data_ptr(),
-                                      counters[1].data_ptr(), band.data_ptr(), cap, _lib.stream()))
+        counters, band = _count_band(lib, qp, index.planes, index.m, thr, cap)
         _lib.check(lib.lkg_topk_finalize_l2(index.cand.data_ptr(), index.cand.stride(0), index.m, query.data_ptr(),
                                             query.stride(0), nq, index.dim, counters[1].data_ptr(), band.data_ptr(), cap,
                                             int(k), kb, _lib.ptr(anchors), _lib.ptr(rels), _lib.ptr(cids),
@@ -676,22 +684,11 @@ def score_topk_dot(emb: torch.Tensor, anchors: torch.Tensor, k: int, index: Scor
         return vals, pos
     if n_sample is None:
         n_sample = topk_l2_samples(index.m, k)
-    known = ex_anchors = rels = cids = None
-    if exclude is not None:
-        known, ex_anchors, rels, cids = exclude
-        ex_anchors = _ids(ex_anchors, dev)
-        rels = None if rels is None else _ids(rels, dev)
-        cids = None if cids is None else _ids(cids, dev)
-        assert ex_anchors.numel() == nq and (rels is None or rels.numel() == nq)
-        assert cids is None or cids.numel() == index.m
-    kb = None if known is None else known.byref()
+    kb, ex_anchors, rels, cids = _exclude_args(exclude, nq, index.m, dev)
     center, ci, cp = index.centered()
     qp = split_planes(emb, anchors)                      # own scale record: the two operands' factors multiply
     thr = torch.empty((nq, 2), dtype=torch.float32, device=dev)
     theta = torch.empty(nq, dtype=torch.float32, device=dev)
-    counters = torch.zeros((2, nq), dtype=torch.int32, device=dev)
-    band = torch.empty((nq, max(cap, 1)), dtype=torch.int32, device=dev)
-    a, b = _lib.planes_operand([qp]), _lib.planes_operand([cp])
     src = index.emb
     with _dev_guard(emb, "score_topk_dot", 3):
         lib = _lib.load()
@@ -701,8 +698,7 @@ def score_topk_dot(emb: torch.Tensor, anchors: torch.Tensor, k: int, index: Scor
                                               ci.rec.data_ptr(), int(k), int(n_sample), kb, _lib.ptr(ex_anchors),
                                               _lib.ptr(rels), _lib.ptr(cids), thr.data_ptr(), theta.data_ptr(),
                                               _lib.stream()))
-        _lib.check(lib.lkg_score_rank(C.byref(a), nq, C.byref(b), index.m, thr.data_ptr(), counters[0].data_ptr(),
-                                      counters[1].data_ptr(), band.data_ptr(), cap, _lib.stream()))
+        counters, band = _count_band(lib, qp, cp, index.m, thr, cap)
         _lib.check(lib.lkg_topk_finalize_dot(src.data_ptr(), src.stride(0), _lib.ptr(index.rows), index.m,
                                              emb.data_ptr(), emb.stride(0), anchors.data_ptr(), nq, dim,
                                              counters[1].data_ptr(), band.data_ptr(), cap, int(k), kb,
