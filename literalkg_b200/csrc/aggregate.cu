@@ -56,6 +56,7 @@ struct AggParams {
     float* side_out;   // training: saved side = A @ ego per local row (nullable), row stride ld_side
     int64_t ld_side;
     int n_solo;        // narrow kernel: leading rows of row_order that are scheduled one per warp
+    int ring;          // stream kernel, batched kBiZ: ring slots per warp (agg_route: the most that fit, <= 6)
 };
 
 template <int S, int NC, int MODE>
@@ -648,16 +649,64 @@ int dispatch_narrow(int mode, const AggParams& p, cudaStream_t stream) {
 // rowptr -> col -> gather chain of dependent round trips (ncu r01: 66 % of the HBM peak, long_scoreboard on top).
 // The folded combine reads the u-vectors (side | ego+side | ego*side) from a per-warp staging buffer and P from
 // shared memory in [d/4][channel][4] order: one 16-byte load per matrix feeds four FMAs.
+//
+// kBiZ with one channel chunk (layer 1 of the bi-interaction model) combines on tensor cores instead: the warp that
+// finishes a row writes u = ego * side as scaled fp16 hi/lo planes (plus the row's z sum) into one of 16 slots of a
+// CTA-wide row batch and goes straight on to its next gathers; the warp whose row completes the batch multiplies
+// [16 x K] by P2 [K x 32] with mma.sync m16n8k16 (hi*hi + lo*hi + hi*lo, the 3-product split of the GEMM engine) and
+// runs LeakyReLU / LayerNorm / normalise for the 16 rows from the accumulator fragments.  P2 is then read from shared
+// memory once per 16 rows instead of once per row (the per-row read was 300 M of the kernel's 760 M shared-memory
+// wavefronts, ncu r02), and a warp's ring sits idle behind one combine per 16 rows instead of one per row.
 constexpr int kStreamWarps = 16;
+constexpr int kBatchRows = 16;                 // rows per tensor-core batch (the M of m16n8k16)
 // neighbour rows in flight per warp: what fits next to the P tiles (kBiZ keeps one matrix instead of two)
-__host__ __device__ constexpr int stream_ring(int mode) { return mode == kBiZ ? 6 : 4; }  // 8 fits (228 KB) but measures slower: 5.95 vs 5.36 ms
+// kBiZ: 6 (8 fitted next to the fp32 P2 tile but measured slower, 5.95 vs 5.36 ms; next to the row batches 7 does not
+// fit at d = 300: 227.5 KB)
+__host__ __device__ constexpr int stream_ring(int mode) { return mode == kBiZ ? 6 : 4; }
+constexpr int kMinRing = 4;                    // batched kBiZ: the ring shrinks to this where 6 slots do not fit
+// batched kBiZ: K padded to the k-step; a batch plane row holds kp + 8 halves (kp / 2 + 4 words, = 4 mod 8: the A
+// fragment loads of the 8 row groups hit distinct banks); a batch = hi and lo planes, 16 int4 records, 16 z sums
+__host__ __device__ constexpr int batch_kp(int d_in) { return (d_in + 15) / 16 * 16; }
+__host__ __device__ constexpr int batch_rsw(int d_in) { return batch_kp(d_in) / 2 + 4; }
+__host__ __device__ constexpr size_t batch_bytes(int d_in) {
+    return (size_t)2 * kBatchRows * batch_rsw(d_in) * 4 + kBatchRows * 16 + kBatchRows * 32 * 4;
+}
+enum { kSyncClaim = 0, kSyncLeft, kSyncFilled, kSyncGen = kSyncFilled + 2, kSyncPMax = kSyncGen + 2, kSyncInts = 8 };
+
+// power-of-two scale 2^e that parks amax * 2^e in [2^11, 2^12) (the operand scale of the GEMM engine)
+__device__ __forceinline__ int plane_exp(float amax) {
+    int e = 0;
+    if (amax > 0.f && amax < 3.0e38f) {
+        int ex;
+        frexpf(amax, &ex);
+        e = 12 - ex;
+        e = e > 120 ? 120 : (e < -120 ? -120 : e);
+    }
+    return e;
+}
+__device__ __forceinline__ float pow2(int e) { return __int_as_float((127 + e) << 23); }
+// scaled fp32 pair -> {hi, lo} fp16 pairs (round to nearest, then the residual), packed for mma operands
+__device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
+    const __half2 h = __floats2half2_rn(a, b);
+    const float2 hf = __half22float2(h);
+    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
+    hi = *reinterpret_cast<const uint32_t*>(&h);
+    lo = *reinterpret_cast<const uint32_t*>(&l);
+}
+__device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+    asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
 
 template <int S, int NC, int MODE>
 __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(AggParams p) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     constexpr bool Z = MODE == kBiZ;                            // sum term pre-projected: only the product term is combined
+    constexpr bool TC = Z && NC == 1;                           // ... in 16-row batches on tensor cores
     constexpr int NT = (MODE == kOneTerm || Z) ? 1 : 2;
     constexpr int kRing = stream_ring(MODE);
+    const uint32_t nring = TC ? (uint32_t)p.ring : (uint32_t)kRing;   // slots in use (TC: <= kRing, what fits)
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int d_in = p.d_in, d_out = p.d_out, nvec = p.nvec;
@@ -665,15 +714,21 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
     const uint32_t row_bytes = (uint32_t)nvec * 16u;
     const uint32_t z_bytes = Z ? (uint32_t)d_out * 4u : 0u;      // a ring slot = neighbour row (+ its z row)
     const uint32_t slot_bytes = row_bytes + z_bytes;
-    // layout: P0 [nvec][cpad][4] | P1 | per warp { ring kRing x slot_bytes | stage NT x row_bytes } | barriers
+    // layout: P0 [nvec][cpad][4] | P1 | per warp { ring nring x slot_bytes | stage NT x row_bytes } | barriers
+    //     TC: P2 fragments [kp / 16][hi, lo][n 0-15, 16-31][lane] (uint4) | per warp ring | 2 batches | barriers | sync
+    const int kp = batch_kp(d_in), rsw = batch_rsw(d_in);
+    const size_t p_bytes = TC ? (size_t)kp * 128 : (size_t)NT * nvec * cpad * 16;
     float4* sp0 = reinterpret_cast<float4*>(smem_raw);
     float4* sp1 = sp0 + (size_t)nvec * cpad;
-    const size_t warp_bytes = (size_t)kRing * slot_bytes + (size_t)NT * row_bytes;
-    uint8_t* warp_base = smem_raw + (size_t)NT * nvec * cpad * 16 + (size_t)warp * warp_bytes;
+    const uint4* pfrag = reinterpret_cast<const uint4*>(smem_raw);
+    const size_t warp_bytes = (size_t)nring * slot_bytes + (TC ? 0 : (size_t)NT * row_bytes);
+    uint8_t* warp_base = smem_raw + p_bytes + (size_t)warp * warp_bytes;
     uint8_t* ring = warp_base;
-    float4* stage = reinterpret_cast<float4*>(warp_base + (size_t)kRing * slot_bytes);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + (size_t)NT * nvec * cpad * 16 +
-                                                 (size_t)kStreamWarps * warp_bytes) + warp * kRing;
+    float4* stage = reinterpret_cast<float4*>(warp_base + (size_t)nring * slot_bytes);
+    uint8_t* batches = smem_raw + p_bytes + (size_t)kStreamWarps * warp_bytes;
+    uint64_t* bars0 = reinterpret_cast<uint64_t*>(batches + (TC ? 2 * batch_bytes(d_in) : 0));
+    uint64_t* bars = bars0 + warp * kRing;
+    int* sync = reinterpret_cast<int*>(bars0 + kStreamWarps * kRing);
     // [ego row | z row] stored back to back in one table (model.py lays the gate output and its projection out like
     // that): ONE bulk copy per neighbour instead of two, and the 128-byte z row rides in the DRAM page of its ego row
     const bool zcontig = Z && p.z == p.ego + d_in && p.ld_z == p.ld_ego;
@@ -689,26 +744,56 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
             ring_issue(dst, p.ego + (int64_t)col * p.ld_ego, row_bytes, &bars[slot]);
         }
     };
-    for (int i = threadIdx.x; i < nvec * cpad; i += blockDim.x) {
-        const int d4 = i / cpad, c = i - d4 * cpad;
-        float w0[4] = {0, 0, 0, 0}, w1[4] = {0, 0, 0, 0};
-        if (c < d_out) {
+    if constexpr (TC) {
+        // P2 as the B fragments of m16n8k16, scaled by 2^ep from the matrix's max |P2|: entry (ks, plane, half, lane)
+        // holds {b0, b1} of the n-tiles 2 half and 2 half + 1 (n = 8 nt + lane / 4, k = 16 ks + 2 (lane % 4) (+ 8))
+        if (threadIdx.x < kSyncInts) sync[threadIdx.x] = 0;
+        __syncthreads();
+        float am = 0.f;
+        for (int i = threadIdx.x; i < d_in * d_out; i += blockDim.x) am = fmaxf(am, fabsf(p.p0[i]));
+        am = warp_max(am);
+        if (lane == 0 && am > 0.f) atomicMax(reinterpret_cast<unsigned*>(sync + kSyncPMax), __float_as_uint(am));
+        __syncthreads();
+        const float sp = pow2(plane_exp(__int_as_float(sync[kSyncPMax])));
+        uint4* pf = reinterpret_cast<uint4*>(smem_raw);
+        for (int i = threadIdx.x; i < kp * 8; i += blockDim.x) {
+            const int ks = i >> 7, plane = (i >> 6) & 1, half = (i >> 5) & 1, ln = i & 31;
+            uint32_t w[4];
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                w0[k] = p.p0[(4 * d4 + k) * d_out + c];
-                if (NT == 2) w1[k] = p.p1[(4 * d4 + k) * d_out + c];
+            for (int j = 0; j < 4; ++j) {
+                const int n = (2 * half + (j >> 1)) * 8 + (ln >> 2);
+                const int k = ks * 16 + 2 * (ln & 3) + 8 * (j & 1);
+                const float x0 = (n < d_out && k < d_in) ? p.p0[k * d_out + n] * sp : 0.f;
+                const float x1 = (n < d_out && k + 1 < d_in) ? p.p0[(k + 1) * d_out + n] * sp : 0.f;
+                uint32_t hi, lo;
+                split2(x0, x1, hi, lo);
+                w[j] = plane ? lo : hi;
             }
+            pf[i] = make_uint4(w[0], w[1], w[2], w[3]);
         }
-        sp0[i] = make_float4(w0[0], w0[1], w0[2], w0[3]);
-        if (NT == 2) sp1[i] = make_float4(w1[0], w1[1], w1[2], w1[3]);
+    } else {
+        for (int i = threadIdx.x; i < nvec * cpad; i += blockDim.x) {
+            const int d4 = i / cpad, c = i - d4 * cpad;
+            float w0[4] = {0, 0, 0, 0}, w1[4] = {0, 0, 0, 0};
+            if (c < d_out) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    w0[k] = p.p0[(4 * d4 + k) * d_out + c];
+                    if (NT == 2) w1[k] = p.p1[(4 * d4 + k) * d_out + c];
+                }
+            }
+            sp0[i] = make_float4(w0[0], w0[1], w0[2], w0[3]);
+            if (NT == 2) sp1[i] = make_float4(w1[0], w1[1], w1[2], w1[3]);
+        }
     }
-    if (lane < kRing) ring_bar_init(&bars[lane]);
+    if (lane < (int)nring) ring_bar_init(&bars[lane]);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
 
     const int n_rows = p.g.n_sched > 0 ? (int)p.g.n_sched : (int)(p.g.row_end - p.g.row_begin);   // schedule records
     const int4* sched = reinterpret_cast<const int4*>(p.g.row_sched);
-    uint32_t issued = 0, consumed = 0;
+    uint32_t issued = 0;                                         // copies issued
+    uint32_t cslot = 0, cphase = 0;                              // slot and barrier parity of the next copy consumed
     const bool need_ego = MODE != kOneTerm || p.sum_ego;
     const int zvec = d_out >> 2;                                 // float4 per z row
 
@@ -742,6 +827,116 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
             h.eg[s] = (live && need_ego && v < nvec) ? __ldg(erow + v) : make_float4(0, 0, 0, 0);
         }
         return h;
+    };
+
+    // TC: [16 x kp] u planes of batch buffer `buf` times P2 on tensor cores, then phase 3 of its first `cnt` rows.
+    // Lane (g = lane / 4, t = lane % 4) ends with rows g and g + 8, channels 8 nt + 2 t + {0, 1} of every n-tile nt.
+    auto combine = [&](int buf, int cnt) {
+        const uint8_t* bb = batches + (size_t)buf * batch_bytes(d_in);
+        const uint32_t* ahi = reinterpret_cast<const uint32_t*>(bb);
+        const uint32_t* alo = ahi + kBatchRows * rsw;
+        const int4* meta = reinterpret_cast<const int4*>(alo + kBatchRows * rsw);
+        const float* zs = reinterpret_cast<const float*>(meta + kBatchRows);
+        const int g = lane >> 2, t = lane & 3;
+        float acc[4][4];
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+        for (int ks = 0; ks < kp / 16; ++ks) {
+            const int w0 = g * rsw + ks * 8 + t, w1 = w0 + 8 * rsw;
+            const uint32_t ah[4] = {ahi[w0], ahi[w1], ahi[w0 + 4], ahi[w1 + 4]};
+            const uint32_t al[4] = {alo[w0], alo[w1], alo[w0 + 4], alo[w1 + 4]};
+            const uint4* bf = pfrag + ks * 128 + lane;
+            const uint4 bh[2] = {bf[0], bf[32]}, bl[2] = {bf[64], bf[96]};
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                mma16816(acc[2 * h], ah, bh[h].x, bh[h].y);
+                mma16816(acc[2 * h], al, bh[h].x, bh[h].y);
+                mma16816(acc[2 * h], ah, bl[h].x, bl[h].y);
+                mma16816(acc[2 * h + 1], ah, bh[h].z, bh[h].w);
+                mma16816(acc[2 * h + 1], al, bh[h].z, bh[h].w);
+                mma16816(acc[2 * h + 1], ah, bl[h].z, bl[h].w);
+            }
+        }
+        const float inv_p = pow2(-plane_exp(__int_as_float(sync[kSyncPMax])));
+        float lw[8], lb[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
+            lw[j] = ch < d_out ? __ldg(p.ln_w + ch) : 0.f;
+            lb[j] = ch < d_out ? __ldg(p.ln_b + ch) : 0.f;
+        }
+        const float pscale = p.xn_planes ? __ldg(p.xn_rec + 1) : 1.f;
+#pragma unroll
+        for (int hr = 0; hr < 2; ++hr) {
+            const int sl = g + 8 * hr;
+            const bool live = sl < cnt;
+            const int4 m = meta[sl];
+            const int row = live ? m.x : 0;
+            const int64_t lrow = live ? m.y : 0;
+            const float inv_u = pow2(live ? -m.z : 0);
+            float emb[8];
+            float s1 = 0.f;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
+                const bool ok = live && ch < d_out;
+                // o2: the product path r2 + (ego * side) @ P2, o1: the sum path r1 + A @ z
+                const float o2 = ((ok && p.r2) ? __ldg(p.r2 + lrow * p.ld_r + ch) : 0.f) +
+                                 acc[j >> 1][2 * hr + (j & 1)] * inv_p * inv_u;
+                const float o1 = ((ok && p.r1) ? __ldg(p.r1 + lrow * p.ld_r + ch) : 0.f) + zs[sl * 32 + ch];
+                if (p.o_out && ok) {
+                    p.o_out[lrow * p.ld_o + d_out + ch] = o2;
+                    p.o_out[lrow * p.ld_o + ch] = o1;
+                }
+                emb[j] = ch < d_out ? leaky(o2) + leaky(o1) : 0.f;
+                s1 += emb[j];
+            }
+            s1 += __shfl_xor_sync(kFull, s1, 1);
+            s1 += __shfl_xor_sync(kFull, s1, 2);
+            const float mean = s1 / (float)d_out;
+            float s2 = 0.f;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const float dlt = 8 * (j >> 1) + 2 * t + (j & 1) < d_out ? emb[j] - mean : 0.f;
+                s2 = fmaf(dlt, dlt, s2);
+            }
+            s2 += __shfl_xor_sync(kFull, s2, 1);
+            s2 += __shfl_xor_sync(kFull, s2, 2);
+            const float rstd = rsqrtf(s2 / (float)d_out + 1e-5f);
+            float sq = 0.f;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
+                float x = 0.f;
+                if (ch < d_out) {
+                    x = (emb[j] - mean) * rstd * lw[j] + lb[j];
+                    if (p.mask && live) x *= __ldg(p.mask + lrow * d_out + ch);
+                    if (live) p.x_out[(int64_t)row * p.ld_x + ch] = x;
+                }
+                emb[j] = x;
+                sq = fmaf(x, x, sq);
+            }
+            if (p.xn_out || p.xn_planes) {
+                sq += __shfl_xor_sync(kFull, sq, 1);
+                sq += __shfl_xor_sync(kFull, sq, 2);
+                const float inv = 1.f / fmaxf(sqrtf(sq), 1e-12f);
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
+                    if (live && ch < d_out) {
+                        const float xn = emb[j] * inv;
+                        if (p.xn_out) p.xn_out[lrow * p.ld_xn + ch] = xn;
+                        if (p.xn_planes) {
+                            const float xs = xn * pscale;
+                            const __half h = __float2half_rn(xs);
+                            const __half l = __float2half_rn(xs - __half2float(h));
+                            p.xn_planes[lrow * p.ld_planes + ch] = h;
+                            p.xn_planes[p.plane_stride + lrow * p.ld_planes + ch] = l;
+                        }
+                    }
+                }
+            }
+        }
     };
 
     int idx = __shfl_sync(kFull, fetch_idx(), 0);
@@ -780,17 +975,17 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
                 my_col = lane < cn ? __ldg(p.g.col + c0 + lane) : 0;
                 my_val = lane < cn ? __ldg(p.a_val + c0 + lane) : 0.f;
             }
-            const int first = min(cn, kRing);
+            const int first = min(cn, (int)nring);
             const int done = c0 == u0 ? pre_issued : 0;          // the first chunk's copies may already be in flight
             if (lane >= done && lane < first) {
-                issue((issued + lane - done) % kRing, my_col);
+                issue((issued + lane - done) % nring, my_col);
             }
             issued += first - done;
             if (!fetched) prefetch_rows();
             for (int e = 0; e < cn; ++e) {
                 const float a = __shfl_sync(kFull, my_val, e);
-                const uint32_t slot = consumed % kRing;
-                ring_wait(&bars[slot], (consumed / kRing) & 1);
+                const uint32_t slot = cslot;
+                ring_wait(&bars[slot], cphase);
                 const float4* nrow = reinterpret_cast<const float4*>(ring + slot * slot_bytes);
 #pragma unroll
                 for (int s = 0; s < S; ++s) {
@@ -810,9 +1005,12 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
                     zside.z = fmaf(a, x.z, zside.z);
                     zside.w = fmaf(a, x.w, zside.w);
                 }
-                ++consumed;
+                if (++cslot == nring) {
+                    cslot = 0;
+                    cphase ^= 1;
+                }
                 __syncwarp();                                    // every lane has read the slot before it is refilled
-                const int nxt = e + kRing;
+                const int nxt = e + (int)nring;
                 if (nxt < cn) {
                     if (lane == nxt) issue(slot, my_col);
                     ++issued;
@@ -823,8 +1021,8 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
         // the ring is empty: start the next row's first copies now, they land while this row is combined
         pre_issued = 0;
         if (idx1 < n_rows) {
-            pre_issued = min(kRing, min(32, rec1.u1 - rec1.u0));
-            if (lane < pre_issued) issue((issued + lane) % kRing, head1.col);
+            pre_issued = min((int)nring, min(32, rec1.u1 - rec1.u0));
+            if (lane < pre_issued) issue((issued + lane) % nring, head1.col);
             issued += pre_issued;
         }
 
@@ -873,8 +1071,71 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
             }
         }
 
+        // ---- TC: u = ego * side into a slot of the CTA's row batch; the warp that fills the batch combines it ---------
+        if constexpr (TC) {
+            if (finish) {
+                float4 u[S];
+                float am = 0.f;
+#pragma unroll
+                for (int s = 0; s < S; ++s) {
+                    const int v = lane + 32 * s;
+                    u[s] = make_float4(0, 0, 0, 0);
+                    if (v < nvec) {
+                        const float4 sd = side[s], eg = head.eg[s];
+                        if (p.side_out) reinterpret_cast<float4*>(p.side_out + lrow * p.ld_side)[v] = sd;
+                        u[s] = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
+                        am = fmaxf(fmaxf(fmaxf(am, fabsf(u[s].x)), fabsf(u[s].y)), fmaxf(fabsf(u[s].z), fabsf(u[s].w)));
+                    }
+                }
+                const int eu = plane_exp(warp_max(am));
+                const float su = pow2(eu);
+                // claim a slot; a buffer is reused for batch b only after batch b - 2 in it has been combined
+                int tk = 0;
+                if (lane == 0) {
+                    tk = atomicAdd(sync + kSyncClaim, 1);
+                    const int b = tk / kBatchRows;
+                    while (*reinterpret_cast<volatile int*>(sync + kSyncGen + (b & 1)) < b / 2) __nanosleep(32);
+                    __threadfence_block();
+                }
+                tk = __shfl_sync(kFull, tk, 0);
+                const int buf = (tk / kBatchRows) & 1, sl = tk % kBatchRows;
+                uint8_t* bb = batches + (size_t)buf * batch_bytes(d_in);
+                uint32_t* ahi = reinterpret_cast<uint32_t*>(bb) + sl * rsw;
+                uint32_t* alo = ahi + kBatchRows * rsw;
+                int4* meta = reinterpret_cast<int4*>(reinterpret_cast<uint32_t*>(bb) + 2 * kBatchRows * rsw);
+                float4* zs = reinterpret_cast<float4*>(meta + kBatchRows) + sl * 8;
+#pragma unroll
+                for (int s = 0; s < S; ++s) {
+                    const int v = lane + 32 * s;                 // K padding (v >= nvec) is written as zeros
+                    if (v < kp / 4) {
+                        uint2 h, l;
+                        split2(u[s].x * su, u[s].y * su, h.x, l.x);
+                        split2(u[s].z * su, u[s].w * su, h.y, l.y);
+                        reinterpret_cast<uint2*>(ahi)[v] = h;
+                        reinterpret_cast<uint2*>(alo)[v] = l;
+                    }
+                }
+                if (lane < zvec) zs[lane] = zside;
+                if (lane == 0) meta[sl] = make_int4(row, (int)lrow, eu, 0);
+                __syncwarp();
+                int last = 0;
+                if (lane == 0) {
+                    __threadfence_block();
+                    last = atomicAdd(sync + kSyncFilled + buf, 1) == kBatchRows - 1;
+                    if (last) sync[kSyncFilled + buf] = 0;
+                    __threadfence_block();
+                }
+                if (__shfl_sync(kFull, last, 0)) {
+                    combine(buf, kBatchRows);
+                    __syncwarp();
+                    if (lane == 0) {
+                        __threadfence_block();
+                        atomicAdd(sync + kSyncGen + buf, 1);
+                    }
+                }
+            }
+        } else if (finish) {
         // ---- phase 2: u-vectors to the staging buffer, folded combine with lane = output channel -------------
-        if (finish) {
 #pragma unroll
         for (int s = 0; s < S; ++s) {
             const int v = lane + 32 * s;
@@ -1010,6 +1271,19 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
         idx = idx1; rec = rec1; head = head1;
         idx1 = idx2; rec1 = rec2;
     }
+    if constexpr (TC) {      // the last warp out combines the partial batch (every claimed slot is written by then)
+        __syncwarp();
+        int last = 0;
+        if (lane == 0) {
+            __threadfence_block();
+            last = atomicAdd(sync + kSyncLeft, 1) == kStreamWarps - 1;
+            __threadfence_block();
+        }
+        if (__shfl_sync(kFull, last, 0)) {
+            const int claimed = *reinterpret_cast<volatile int*>(sync + kSyncClaim);
+            if (claimed % kBatchRows) combine((claimed / kBatchRows) & 1, claimed % kBatchRows);
+        }
+    }
 }
 
 template <int S, int NC, int MODE>
@@ -1062,13 +1336,14 @@ struct AggRoute {
     Route route;
     size_t smem;   // stream / generic kernel: dynamic shared memory
     int warps;     // generic kernel: warps per CTA
+    int ring;      // stream kernel: ring slots per warp
 };
 
 // narrow_ok: d_in in {16, 32, 64}, d_out % 4 == 0 and every operand the narrow kernel moves as float4 is aligned;
 // stream_ok: d_in >= 128 and the plan has a 16-byte aligned row schedule
 AggRoute agg_route(int mode, int d_in, int d_out, bool narrow_ok, bool stream_ok) {
     const int nvec = d_in / 4;
-    if (mode != kBiZ && narrow_ok) return {kRouteNarrow, 0, 0};
+    if (mode != kBiZ && narrow_ok) return {kRouteNarrow, 0, 0, 0};
     if (stream_ok) {
         const int slots_w = (nvec + 31) / 32, nc_w = (d_out + 31) / 32;
         // one 128-wide slot: only the z mode (layer 1 of a bi-interaction model at embed_dim 128); the other modes
@@ -1077,20 +1352,31 @@ AggRoute agg_route(int mode, int d_in, int d_out, bool narrow_ok, bool stream_ok
                               (slots_w == 3 && nc_w == 1) || (slots_w == 3 && nc_w == 2) || (slots_w == 4 && nc_w == 1);
         const int nt = (mode == kOneTerm || mode == kBiZ) ? 1 : 2;
         const size_t z_bytes = mode == kBiZ ? (size_t)d_out * 4 : 0;
-        const size_t smem = (size_t)nt * nvec * 32 * nc_w * 16 +
-                            (size_t)kStreamWarps * (stream_ring(mode) * (nvec * 16 + z_bytes) + (size_t)nt * nvec * 16) +
-                            kStreamWarps * stream_ring(mode) * 8;
-        if (instance && smem <= kMaxSmem) return {kRouteStream, smem, 0};
+        const size_t bars = (size_t)kStreamWarps * stream_ring(mode) * 8;
+        if (mode == kBiZ && nc_w == 1) {
+            // P2 fragments (hi + lo, kp x 32 halves each) | rings | two row batches | barriers | batch counters;
+            // the ring gives up slots down to kMinRing before the shape is refused
+            for (int ring = stream_ring(mode); instance && ring >= kMinRing; --ring) {
+                const size_t smem = (size_t)batch_kp(d_in) * 128 + (size_t)kStreamWarps * ring * (nvec * 16 + z_bytes) +
+                                    2 * batch_bytes(d_in) + bars + kSyncInts * 4;
+                if (smem <= kMaxSmem) return {kRouteStream, smem, 0, ring};
+            }
+        } else {
+            const size_t smem = (size_t)nt * nvec * 32 * nc_w * 16 +
+                                (size_t)kStreamWarps * (stream_ring(mode) * (nvec * 16 + z_bytes) + (size_t)nt * nvec * 16) +
+                                bars;
+            if (instance && smem <= kMaxSmem) return {kRouteStream, smem, 0, stream_ring(mode)};
+        }
     }
-    if (mode == kBiZ) return {kRouteNone, 0, 0};           // only the stream kernel gathers z
+    if (mode == kBiZ) return {kRouteNone, 0, 0, 0};           // only the stream kernel gathers z
     const int nt = mode == kOneTerm ? 1 : 2;
     const size_t p_bytes = (size_t)nt * d_in * ((d_out + 3) / 4 * 4) * sizeof(float);
     const size_t stage_per_warp = (size_t)kRows * nt * d_in * sizeof(float);
     int warps = 16;
     while (warps > 4 && p_bytes + warps * stage_per_warp > 200 * 1024) warps /= 2;
     const size_t smem = p_bytes + warps * stage_per_warp;
-    if (smem > kMaxSmem) return {kRouteNone, smem, warps};
-    return {kRouteGeneric, smem, warps};
+    if (smem > kMaxSmem) return {kRouteNone, smem, warps, 0};
+    return {kRouteGeneric, smem, warps, 0};
 }
 
 }  // namespace
@@ -1204,6 +1490,7 @@ extern "C" int lkg_aggregate_fwd(const lkg_graph* g, const float* a_values, cons
         LKG_FAIL(LKG_ERR_UNSUPPORTED, "aggregate shapes d_in %d d_out %d need %zu bytes of shared memory (%zu fit)",
                  d_in, d_out, rt.smem, kMaxSmem);
     }
+    p.ring = rt.ring;
     LKG_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(int), stream));
     if (rt.route == kRouteNarrow) {
         const int chunks = d_out / 4;
