@@ -3,14 +3,19 @@
 //
 // Replaces Aggregator.forward + residual_connection (model.py:90-164) and the F.normalize of
 // model.py:305.  The reference runs cuSPARSE SpMM, then 2-4 dense N x d x d GEMMs, ~10 elementwise
-// kernels and a LayerNorm, each a full pass over N x d.  Here one warp owns kRows head rows:
-//   phase 1  side = sum_j A[row, j] * ego[col_j]   128-bit streaming gathers, kUnroll neighbours in flight
-//   phase 2  u-vectors (side | ego+side | ego | ego*side) staged in shared memory, then the folded
-//            combine  o = u @ P + r[row]  with lane = output channel (P lives in shared memory)
-//   phase 3  leaky / add / LayerNorm / mask / L2 normalise, all in registers + warp shuffles
+// kernels and a LayerNorm, each a full pass over N x d.  Here one kernel takes a head row through three phases:
+//   phase 1  side = sum_j A[row, j] * ego[col_j]
+//   phase 2  the folded combine  o = u @ P + r[row]  over the u-vectors terms(ego, side) (side | ego+side | ego |
+//            ego*side)
+//   phase 3  row_epilogue: leaky / add / LayerNorm / mask / L2 normalise, in registers + shuffles
+// Three kernels differ in how phases 1 and 2 gather and combine; agg_route picks one per shape:
+//   aggregate_narrow_kernel  d_in 16 / 32 / 64: a group of d_in / 4 lanes per row, combine in registers
+//   aggregate_stream_kernel  d_in >= 128 and a row schedule: neighbour rows stream through a shared-memory ring;
+//                            layer 1 of the bi-interaction model combines 16 rows at a time on tensor cores
+//   aggregate_kernel         the other shapes: kRows rows per warp, gathers staged in registers
 // Folding (host side, DESIGN.md section 4): linear(res(hi)) = hi @ P + h0 @ Q + c, P = (1-a) M W^T.
 // HBM bound: algorithmic bytes = nnz*(4 col + 4 val + 4 d_in) + N*(4 d_in + 8 + r terms + 2*4*d_out).
-#include <cuda_fp16.h>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -59,6 +64,179 @@ struct AggParams {
     int ring;          // stream kernel, batched kBiZ: ring slots per warp (agg_route: the most that fit, <= 6)
 };
 
+// u-vectors of one row from 4 channels of its ego and side: t0 meets P0, t1 meets P1 (kBiZ: t0 = ego * side meets P2;
+// the sum term arrives pre-projected)
+struct Terms { float4 t0, t1; };
+template <int MODE>
+__device__ __forceinline__ Terms terms(float4 eg, float4 sd, int sum_ego) {
+    const float4 prod = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
+    if (MODE == kTwoTerms) return {eg, sd};
+    if (MODE == kBiZ) return {prod, prod};
+    return {sum_ego ? make_float4(eg.x + sd.x, eg.y + sd.y, eg.z + sd.z, eg.w + sd.w) : sd, prod};
+}
+
+// ---- phase 3, one function for every kernel path ----------------------------------------------------------------
+// A lane layout says which channels of a row a lane holds -- N slots, slot i = channels [ch(i), ch(i) + width of Slot)
+// -- and how the lanes of a row reduce.  Its Slot type says how a slot's values enter the lane's partial sums and how
+// they are loaded and stored.  The order of every sum is part of the output bits, so each path keeps its own.
+struct ScalarSlot {                         // one channel: sequential partial sums, squares by fma
+    using V = float;
+    static __device__ float& at(float& v, int) { return v; }
+    static __device__ float at(const float& v, int) { return v; }
+    static __device__ float add(float s, float v) { return s + v; }
+    static __device__ float add_dev2(float s, float d) { return fmaf(d, d, s); }
+    static __device__ float add_sq(float s, float v) { return fmaf(v, v, s); }
+    static __device__ float ld(const float* q) { return __ldg(q); }
+    static __device__ void st(float* q, float v) { *q = v; }
+    static __device__ void st_planes(__half* q, int64_t plane_stride, float v) {
+        __half h, l;
+        split_f16(v, h, l);
+        q[0] = h;
+        q[plane_stride] = l;
+    }
+};
+struct QuadSlot {                           // four channels: pairwise sums in the slot, 16-byte (planes: 8-byte) moves
+    using V = float4;
+    static __device__ float& at(float4& v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w)); }
+    static __device__ float at(const float4& v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w)); }
+    static __device__ float add(float s, float4 v) { return s + ((v.x + v.y) + (v.z + v.w)); }
+    // squares in pairs, one product fused into the other's add; the variance and the norm pair them the opposite way
+    // round, as this kernel always has (written out so that no contraction choice of the compiler can move the bits)
+    static __device__ float add_dev2(float s, float4 d) {
+        return s + (fmaf(d.x, d.x, d.y * d.y) + fmaf(d.z, d.z, d.w * d.w));
+    }
+    static __device__ float add_sq(float s, float4 v) {
+        return s + (fmaf(v.y, v.y, v.x * v.x) + fmaf(v.w, v.w, v.z * v.z));
+    }
+    static __device__ float4 ld(const float* q) { return __ldg(reinterpret_cast<const float4*>(q)); }
+    static __device__ void st(float* q, float4 v) { *reinterpret_cast<float4*>(q) = v; }
+    static __device__ void st_planes(__half* q, int64_t plane_stride, float4 v) {
+        __align__(8) __half h[4], l[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) split_f16(at(v, k), h[k], l[k]);
+        *reinterpret_cast<uint2*>(q) = *reinterpret_cast<const uint2*>(h);
+        *reinterpret_cast<uint2*>(q + plane_stride) = *reinterpret_cast<const uint2*>(l);
+    }
+};
+template <int NC>
+struct WarpChannels {                       // generic and stream per-row paths: channel lane + 32 i, the whole warp
+    using Slot = ScalarSlot;
+    static constexpr int N = NC;
+    int lane;
+    __device__ int ch(int i) const { return lane + 32 * i; }
+    static __device__ float reduce(float s) { return warp_sum(s); }
+};
+template <int LPR, int CPL>
+struct GroupQuads {                         // narrow kernel: channels 4 (gl + LPR i) + [0, 4), the LPR lanes of a group
+    using Slot = QuadSlot;
+    static constexpr int N = CPL;
+    int gl;
+    __device__ int ch(int i) const { return 4 * (gl + LPR * i); }
+    static __device__ float reduce(float s) {
+#pragma unroll
+        for (int o = LPR / 2; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+        return s;
+    }
+};
+struct MmaRowQuad {                         // tensor-core batch, m16n8k16 accumulator fragments: lane (g, t) holds
+    using Slot = ScalarSlot;                //   channels 8 (j >> 1) + 2 t + (j & 1) of rows g and g + 8, quad reduces
+    static constexpr int N = 8;
+    int t;
+    __device__ int ch(int j) const { return 8 * (j >> 1) + 2 * t + (j & 1); }
+    static __device__ float reduce(float s) {
+        s += __shfl_xor_sync(kFull, s, 1);
+        return s + __shfl_xor_sync(kFull, s, 2);
+    }
+};
+
+// One row from its pre-activations o1 (and o2, BI) as this lane holds them: saves [o1 | o2] for the backward,
+// emb = leaky(o1) (+ leaky(o2)), LayerNorm, dropout mask -> x_out, x / max(|x|, 1e-12) -> xn_out and its scaled hi/lo
+// fp16 planes.  The lanes of a row that is not live compute along and store nothing.
+template <bool BI, class L>
+__device__ __forceinline__ void row_epilogue(const AggParams& p, const L& ly, const typename L::Slot::V (&o1)[L::N],
+                                             const typename L::Slot::V (&o2)[L::N], bool live, int row, int64_t lrow) {
+    using S = typename L::Slot;
+    using V = typename S::V;
+    constexpr int W = sizeof(V) / sizeof(float);
+    const int d_out = p.d_out;
+    V v[L::N];
+    float s1 = 0.f;
+#pragma unroll
+    for (int i = 0; i < L::N; ++i) {
+        const int ch = ly.ch(i);
+        if (p.o_out && live && ch < d_out) {
+            S::st(p.o_out + lrow * p.ld_o + ch, o1[i]);
+            if (BI) S::st(p.o_out + lrow * p.ld_o + d_out + ch, o2[i]);
+        }
+#pragma unroll
+        for (int k = 0; k < W; ++k) {
+            float e = leaky(S::at(o1[i], k));
+            if (BI) e += leaky(S::at(o2[i], k));
+            S::at(v[i], k) = ch < d_out ? e : 0.f;
+        }
+        s1 = S::add(s1, v[i]);
+    }
+    const float mean = ly.reduce(s1) / (float)d_out;
+    float s2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < L::N; ++i) {
+        V dlt;
+#pragma unroll
+        for (int k = 0; k < W; ++k) S::at(dlt, k) = ly.ch(i) < d_out ? S::at(v[i], k) - mean : 0.f;
+        s2 = S::add_dev2(s2, dlt);
+    }
+    const float rstd = rsqrtf(ly.reduce(s2) / (float)d_out + 1e-5f);
+    float sq = 0.f;
+#pragma unroll
+    for (int i = 0; i < L::N; ++i) {
+        const int ch = ly.ch(i);
+        V x{};
+        if (ch < d_out) {
+            const V w = S::ld(p.ln_w + ch), b = S::ld(p.ln_b + ch);
+#pragma unroll
+            for (int k = 0; k < W; ++k) S::at(x, k) = (S::at(v[i], k) - mean) * rstd * S::at(w, k) + S::at(b, k);
+            if (p.mask && live) {
+                const V m = S::ld(p.mask + lrow * d_out + ch);
+#pragma unroll
+                for (int k = 0; k < W; ++k) S::at(x, k) *= S::at(m, k);
+            }
+            if (live) S::st(p.x_out + (int64_t)row * p.ld_x + ch, x);
+        }
+        v[i] = x;
+        sq = S::add_sq(sq, x);
+    }
+    if (!p.xn_out && !p.xn_planes) return;
+    const float inv = 1.f / fmaxf(sqrtf(ly.reduce(sq)), 1e-12f);
+    const float pscale = p.xn_planes ? __ldg(p.xn_rec + 1) : 1.f;
+#pragma unroll
+    for (int i = 0; i < L::N; ++i) {
+        const int ch = ly.ch(i);
+        if (!live || ch >= d_out) continue;
+        V xn, xs;
+#pragma unroll
+        for (int k = 0; k < W; ++k) {
+            S::at(xn, k) = S::at(v[i], k) * inv;
+            S::at(xs, k) = S::at(xn, k) * pscale;
+        }
+        if (p.xn_out) S::st(p.xn_out + lrow * p.ld_xn + ch, xn);
+        if (p.xn_planes) S::st_planes(p.xn_planes + lrow * p.ld_planes + ch, p.plane_stride, xs);
+    }
+}
+
+// f(std::integral_constant<int, MODE>) for the kernel mode `mode`; the kBiZ instance exists only where WITH_Z
+template <bool WITH_Z, class F>
+int with_mode(int mode, F&& f) {
+    if (mode == kOneTerm) return f(std::integral_constant<int, kOneTerm>{});
+    if (mode == kTwoTerms) return f(std::integral_constant<int, kTwoTerms>{});
+    if constexpr (WITH_Z) {
+        if (mode == kBiZ) return f(std::integral_constant<int, kBiZ>{});
+    }
+    return f(std::integral_constant<int, kBi>{});
+}
+
+// ---- generic kernel: one warp owns kRows head rows --------------------------------------------------------------
+//   phase 1  128-bit streaming gathers, UNROLL neighbours in flight; u-vectors staged in shared memory
+//   phase 2  lane = output channel, P lives in shared memory and is read once per kRows rows
 template <int S, int NC, int MODE>
 __global__ void __launch_bounds__(512, 1) aggregate_kernel(AggParams p) {
     extern __shared__ __align__(16) float smem[];
@@ -141,16 +319,9 @@ __global__ void __launch_bounds__(512, 1) aggregate_kernel(AggParams p) {
                         reinterpret_cast<float4*>(p.side_out + (row - p.local_row_base) * p.ld_side)[v] = sd;
                     float4 eg = make_float4(0, 0, 0, 0);
                     if (MODE != kOneTerm || p.sum_ego) eg = __ldg(reinterpret_cast<const float4*>(erow) + v);
-                    float4 t0, t1;
-                    if (MODE == kTwoTerms) {
-                        t0 = eg;
-                        t1 = sd;
-                    } else {
-                        t0 = p.sum_ego ? make_float4(eg.x + sd.x, eg.y + sd.y, eg.z + sd.z, eg.w + sd.w) : sd;
-                        t1 = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
-                    }
-                    reinterpret_cast<float4*>(st)[v] = t0;
-                    if (NT == 2) reinterpret_cast<float4*>(st + d_in)[v] = t1;
+                    const Terms u = terms<MODE>(eg, sd, p.sum_ego);
+                    reinterpret_cast<float4*>(st)[v] = u.t0;
+                    if (NT == 2) reinterpret_cast<float4*>(st + d_in)[v] = u.t1;
                 }
             }
         }
@@ -212,67 +383,12 @@ __global__ void __launch_bounds__(512, 1) aggregate_kernel(AggParams p) {
         }
         __syncwarp();   // staging buffer is reused by the next step
 
-        // ---- phase 3: activation, LayerNorm, mask, L2 normalise --------------------------------
+        // ---- phase 3 ---------------------------------------------------------------------------------
 #pragma unroll
         for (int rr = 0; rr < kRows; ++rr) {
             if (base + rr >= n) break;
             const int row = row_of(base + rr);
-            const int64_t lrow = row - p.local_row_base;
-            float emb[NC];
-            float s1 = 0.f;
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const int ch = lane + 32 * c;
-                if (p.o_out && ch < d_out) {
-                    p.o_out[lrow * p.ld_o + ch] = acc1[rr][c];
-                    if (MODE == kBi) p.o_out[lrow * p.ld_o + d_out + ch] = acc2[rr][c];
-                }
-                float e = leaky(acc1[rr][c]);
-                if (MODE == kBi) e += leaky(acc2[rr][c]);
-                emb[c] = ch < d_out ? e : 0.f;
-                s1 += emb[c];
-            }
-            const float mean = warp_sum(s1) / (float)d_out;
-            float s2 = 0.f;
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const int ch = lane + 32 * c;
-                const float dlt = ch < d_out ? emb[c] - mean : 0.f;
-                s2 = fmaf(dlt, dlt, s2);
-            }
-            const float rstd = rsqrtf(warp_sum(s2) / (float)d_out + 1e-5f);
-            float sq = 0.f;
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const int ch = lane + 32 * c;
-                float x = 0.f;
-                if (ch < d_out) {
-                    x = (emb[c] - mean) * rstd * __ldg(p.ln_w + ch) + __ldg(p.ln_b + ch);
-                    if (p.mask) x *= __ldg(p.mask + lrow * d_out + ch);
-                    p.x_out[(int64_t)row * p.ld_x + ch] = x;
-                }
-                emb[c] = x;
-                sq = fmaf(x, x, sq);
-            }
-            if (p.xn_out || p.xn_planes) {
-                const float inv = 1.f / fmaxf(sqrtf(warp_sum(sq)), 1e-12f);
-                const float pscale = p.xn_planes ? __ldg(p.xn_rec + 1) : 1.f;
-#pragma unroll
-                for (int c = 0; c < NC; ++c) {
-                    const int ch = lane + 32 * c;
-                    if (ch < d_out) {
-                        const float xn = emb[c] * inv;
-                        if (p.xn_out) p.xn_out[lrow * p.ld_xn + ch] = xn;
-                        if (p.xn_planes) {
-                            const float xs = xn * pscale;
-                            const __half h = __float2half_rn(xs);
-                            const __half l = __float2half_rn(xs - __half2float(h));
-                            p.xn_planes[lrow * p.ld_planes + ch] = h;
-                            p.xn_planes[p.plane_stride + lrow * p.ld_planes + ch] = l;
-                        }
-                    }
-                }
-            }
+            row_epilogue<MODE == kBi>(p, WarpChannels<NC>{lane}, acc1[rr], acc2[rr], true, row, row - p.local_row_base);
         }
     }
 }
@@ -451,13 +567,9 @@ __global__ void __launch_bounds__(256, MINB) aggregate_narrow_kernel(AggParams p
                 eg = __ldg(reinterpret_cast<const float4*>(p.ego + (int64_t)row[rr] * p.ld_ego) + gl);
             const float4 sd = side[rr];
             if (p.side_out && live[rr]) reinterpret_cast<float4*>(p.side_out + lrow[rr] * p.ld_side)[gl] = sd;
-            if (MODE == kTwoTerms) {
-                t0[rr] = eg;
-                t1[rr] = sd;
-            } else {
-                t0[rr] = p.sum_ego ? make_float4(eg.x + sd.x, eg.y + sd.y, eg.z + sd.z, eg.w + sd.w) : sd;
-                t1[rr] = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
-            }
+            const Terms u = terms<MODE>(eg, sd, p.sum_ego);
+            t0[rr] = u.t0;
+            t1[rr] = u.t1;
 #pragma unroll
             for (int i = 0; i < CPL; ++i) {
                 const int ch = 4 * (gl + LPR * i);
@@ -510,94 +622,10 @@ __global__ void __launch_bounds__(256, MINB) aggregate_narrow_kernel(AggParams p
             }
         }
 
-        // ---- phase 3: activation, LayerNorm, mask, L2 normalise (group-wide reductions), batch after batch ---
+        // ---- phase 3, batch after batch ------------------------------------------------------------------------
 #pragma unroll
-        for (int rr = 0; rr < RB; ++rr) {
-            const bool lv = live[rr];
-            const int64_t lr = lrow[rr];
-            float4 emb[CPL];
-            float s1 = 0.f;
-#pragma unroll
-            for (int i = 0; i < CPL; ++i) {
-                const int ch = 4 * (gl + LPR * i);
-                const float4 o1 = acc1[rr][i], o2 = acc2[rr][i];
-                if (p.o_out && lv && ch < d_out) {
-                    *reinterpret_cast<float4*>(p.o_out + lr * p.ld_o + ch) = o1;
-                    if (MODE == kBi) *reinterpret_cast<float4*>(p.o_out + lr * p.ld_o + d_out + ch) = o2;
-                }
-                float4 e = make_float4(leaky(o1.x), leaky(o1.y), leaky(o1.z), leaky(o1.w));
-                if (MODE == kBi) {
-                    e.x += leaky(o2.x);
-                    e.y += leaky(o2.y);
-                    e.z += leaky(o2.z);
-                    e.w += leaky(o2.w);
-                }
-                if (ch >= d_out) e = make_float4(0, 0, 0, 0);
-                emb[i] = e;
-                s1 += (e.x + e.y) + (e.z + e.w);
-            }
-#pragma unroll
-            for (int o = LPR / 2; o > 0; o >>= 1) s1 += __shfl_xor_sync(kFull, s1, o);
-            const float mean = s1 / (float)d_out;
-            float s2 = 0.f;
-#pragma unroll
-            for (int i = 0; i < CPL; ++i) {
-                if (4 * (gl + LPR * i) < d_out) {
-                    const float dx = emb[i].x - mean, dy = emb[i].y - mean, dz = emb[i].z - mean, dw = emb[i].w - mean;
-                    s2 += (dx * dx + dy * dy) + (dz * dz + dw * dw);
-                }
-            }
-#pragma unroll
-            for (int o = LPR / 2; o > 0; o >>= 1) s2 += __shfl_xor_sync(kFull, s2, o);
-            const float rstd = rsqrtf(s2 / (float)d_out + 1e-5f);
-            float sq = 0.f;
-#pragma unroll
-            for (int i = 0; i < CPL; ++i) {
-                const int ch = 4 * (gl + LPR * i);
-                float4 x = make_float4(0, 0, 0, 0);
-                if (ch < d_out) {
-                    const float4 lw = __ldg(reinterpret_cast<const float4*>(p.ln_w + ch));
-                    const float4 lb = __ldg(reinterpret_cast<const float4*>(p.ln_b + ch));
-                    x.x = (emb[i].x - mean) * rstd * lw.x + lb.x;
-                    x.y = (emb[i].y - mean) * rstd * lw.y + lb.y;
-                    x.z = (emb[i].z - mean) * rstd * lw.z + lb.z;
-                    x.w = (emb[i].w - mean) * rstd * lw.w + lb.w;
-                    if (p.mask && lv) {
-                        const float4 mk = __ldg(reinterpret_cast<const float4*>(p.mask + lr * d_out + ch));
-                        x.x *= mk.x; x.y *= mk.y; x.z *= mk.z; x.w *= mk.w;
-                    }
-                    if (lv) *reinterpret_cast<float4*>(p.x_out + (int64_t)row[rr] * p.ld_x + ch) = x;
-                }
-                emb[i] = x;
-                sq += (x.x * x.x + x.y * x.y) + (x.z * x.z + x.w * x.w);
-            }
-            if (p.xn_out || p.xn_planes) {
-#pragma unroll
-                for (int o = LPR / 2; o > 0; o >>= 1) sq += __shfl_xor_sync(kFull, sq, o);
-                const float inv = 1.f / fmaxf(sqrtf(sq), 1e-12f);
-                const float pscale = p.xn_planes ? __ldg(p.xn_rec + 1) : 1.f;
-#pragma unroll
-                for (int i = 0; i < CPL; ++i) {
-                    const int ch = 4 * (gl + LPR * i);
-                    if (ch < d_out && lv) {
-                        const float4 xn = make_float4(emb[i].x * inv, emb[i].y * inv, emb[i].z * inv, emb[i].w * inv);
-                        if (p.xn_out) *reinterpret_cast<float4*>(p.xn_out + lr * p.ld_xn + ch) = xn;
-                        if (p.xn_planes) {
-                            const float v[4] = {xn.x * pscale, xn.y * pscale, xn.z * pscale, xn.w * pscale};
-                            __align__(8) __half h[4], l[4];
-#pragma unroll
-                            for (int c = 0; c < 4; ++c) {
-                                h[c] = __float2half_rn(v[c]);
-                                l[c] = __float2half_rn(v[c] - __half2float(h[c]));
-                            }
-                            __half* hp = p.xn_planes + lr * p.ld_planes + ch;
-                            *reinterpret_cast<uint2*>(hp) = *reinterpret_cast<const uint2*>(h);
-                            *reinterpret_cast<uint2*>(hp + p.plane_stride) = *reinterpret_cast<const uint2*>(l);
-                        }
-                    }
-                }
-            }
-        }
+        for (int rr = 0; rr < RB; ++rr)
+            row_epilogue<MODE == kBi>(p, GroupQuads<LPR, CPL>{gl}, acc1[rr], acc2[rr], live[rr], row[rr], lrow[rr]);
         base = base_n;
         solo = solo_n;
 #pragma unroll
@@ -632,15 +660,6 @@ int launch_narrow(const AggParams& p, cudaStream_t stream) {
     else return launch_narrow_rb<LPR, MODE, CPL, 1>(p, stream);
 }
 
-template <int LPR, int CPL>
-int dispatch_narrow(int mode, const AggParams& p, cudaStream_t stream) {
-    switch (mode) {
-        case kOneTerm: return launch_narrow<LPR, kOneTerm, CPL>(p, stream);
-        case kTwoTerms: return launch_narrow<LPR, kTwoTerms, CPL>(p, stream);
-        default: return launch_narrow<LPR, kBi, CPL>(p, stream);
-    }
-}
-
 // ---- wide rows (layer 1, d_in = 300): gathered rows stream through a per-warp shared-memory ring --------------------
 // Same streaming structure as the attention update (attn.cu): the neighbour list is loaded 32 entries at a time in
 // one coalesced step, the 1 200-byte neighbour rows arrive by cp.async.bulk (one TMA-unit copy per row, kRing in
@@ -673,23 +692,11 @@ __host__ __device__ constexpr size_t batch_bytes(int d_in) {
 }
 enum { kSyncClaim = 0, kSyncLeft, kSyncFilled, kSyncGen = kSyncFilled + 2, kSyncPMax = kSyncGen + 2, kSyncInts = 8 };
 
-// power-of-two scale 2^e that parks amax * 2^e in [2^11, 2^12) (the operand scale of the GEMM engine)
-__device__ __forceinline__ int plane_exp(float amax) {
-    int e = 0;
-    if (amax > 0.f && amax < 3.0e38f) {
-        int ex;
-        frexpf(amax, &ex);
-        e = 12 - ex;
-        e = e > 120 ? 120 : (e < -120 ? -120 : e);
-    }
-    return e;
-}
-__device__ __forceinline__ float pow2(int e) { return __int_as_float((127 + e) << 23); }
-// scaled fp32 pair -> {hi, lo} fp16 pairs (round to nearest, then the residual), packed for mma operands
+// scaled fp32 pair -> {hi, lo} fp16 pairs, packed for mma operands
 __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
-    const __half2 h = __floats2half2_rn(a, b);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
+    __half2 h, l;
+    split_f16(a, h.x, l.x);
+    split_f16(b, h.y, l.y);
     hi = *reinterpret_cast<const uint32_t*>(&h);
     lo = *reinterpret_cast<const uint32_t*>(&l);
 }
@@ -858,84 +865,25 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
             }
         }
         const float inv_p = pow2(-plane_exp(__int_as_float(sync[kSyncPMax])));
-        float lw[8], lb[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
-            lw[j] = ch < d_out ? __ldg(p.ln_w + ch) : 0.f;
-            lb[j] = ch < d_out ? __ldg(p.ln_b + ch) : 0.f;
-        }
-        const float pscale = p.xn_planes ? __ldg(p.xn_rec + 1) : 1.f;
+        const MmaRowQuad ly{t};
 #pragma unroll
         for (int hr = 0; hr < 2; ++hr) {
             const int sl = g + 8 * hr;
             const bool live = sl < cnt;
             const int4 m = meta[sl];
-            const int row = live ? m.x : 0;
             const int64_t lrow = live ? m.y : 0;
             const float inv_u = pow2(live ? -m.z : 0);
-            float emb[8];
-            float s1 = 0.f;
+            float o1[8], o2[8];
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
-                const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
+                const int ch = ly.ch(j);
                 const bool ok = live && ch < d_out;
-                // o2: the product path r2 + (ego * side) @ P2, o1: the sum path r1 + A @ z
-                const float o2 = ((ok && p.r2) ? __ldg(p.r2 + lrow * p.ld_r + ch) : 0.f) +
-                                 acc[j >> 1][2 * hr + (j & 1)] * inv_p * inv_u;
-                const float o1 = ((ok && p.r1) ? __ldg(p.r1 + lrow * p.ld_r + ch) : 0.f) + zs[sl * 32 + ch];
-                if (p.o_out && ok) {
-                    p.o_out[lrow * p.ld_o + d_out + ch] = o2;
-                    p.o_out[lrow * p.ld_o + ch] = o1;
-                }
-                emb[j] = ch < d_out ? leaky(o2) + leaky(o1) : 0.f;
-                s1 += emb[j];
+                // o1: the sum path r1 + A @ z, o2: the product path r2 + (ego * side) @ P2
+                o1[j] = ((ok && p.r1) ? __ldg(p.r1 + lrow * p.ld_r + ch) : 0.f) + zs[sl * 32 + ch];
+                o2[j] = ((ok && p.r2) ? __ldg(p.r2 + lrow * p.ld_r + ch) : 0.f) +
+                        acc[j >> 1][2 * hr + (j & 1)] * inv_p * inv_u;
             }
-            s1 += __shfl_xor_sync(kFull, s1, 1);
-            s1 += __shfl_xor_sync(kFull, s1, 2);
-            const float mean = s1 / (float)d_out;
-            float s2 = 0.f;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const float dlt = 8 * (j >> 1) + 2 * t + (j & 1) < d_out ? emb[j] - mean : 0.f;
-                s2 = fmaf(dlt, dlt, s2);
-            }
-            s2 += __shfl_xor_sync(kFull, s2, 1);
-            s2 += __shfl_xor_sync(kFull, s2, 2);
-            const float rstd = rsqrtf(s2 / (float)d_out + 1e-5f);
-            float sq = 0.f;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
-                float x = 0.f;
-                if (ch < d_out) {
-                    x = (emb[j] - mean) * rstd * lw[j] + lb[j];
-                    if (p.mask && live) x *= __ldg(p.mask + lrow * d_out + ch);
-                    if (live) p.x_out[(int64_t)row * p.ld_x + ch] = x;
-                }
-                emb[j] = x;
-                sq = fmaf(x, x, sq);
-            }
-            if (p.xn_out || p.xn_planes) {
-                sq += __shfl_xor_sync(kFull, sq, 1);
-                sq += __shfl_xor_sync(kFull, sq, 2);
-                const float inv = 1.f / fmaxf(sqrtf(sq), 1e-12f);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const int ch = 8 * (j >> 1) + 2 * t + (j & 1);
-                    if (live && ch < d_out) {
-                        const float xn = emb[j] * inv;
-                        if (p.xn_out) p.xn_out[lrow * p.ld_xn + ch] = xn;
-                        if (p.xn_planes) {
-                            const float xs = xn * pscale;
-                            const __half h = __float2half_rn(xs);
-                            const __half l = __float2half_rn(xs - __half2float(h));
-                            p.xn_planes[lrow * p.ld_planes + ch] = h;
-                            p.xn_planes[p.plane_stride + lrow * p.ld_planes + ch] = l;
-                        }
-                    }
-                }
-            }
+            row_epilogue<true>(p, ly, o1, o2, live, live ? m.x : 0, lrow);
         }
     };
 
@@ -1081,9 +1029,9 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
                     const int v = lane + 32 * s;
                     u[s] = make_float4(0, 0, 0, 0);
                     if (v < nvec) {
-                        const float4 sd = side[s], eg = head.eg[s];
+                        const float4 sd = side[s];
                         if (p.side_out) reinterpret_cast<float4*>(p.side_out + lrow * p.ld_side)[v] = sd;
-                        u[s] = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
+                        u[s] = terms<kBiZ>(head.eg[s], sd, 0).t0;
                         am = fmaxf(fmaxf(fmaxf(am, fabsf(u[s].x)), fabsf(u[s].y)), fmaxf(fabsf(u[s].z), fabsf(u[s].w)));
                     }
                 }
@@ -1135,139 +1083,75 @@ __global__ void __launch_bounds__(kStreamWarps * 32, 1) aggregate_stream_kernel(
                 }
             }
         } else if (finish) {
-        // ---- phase 2: u-vectors to the staging buffer, folded combine with lane = output channel -------------
+            // ---- phase 2: u-vectors to the staging buffer, folded combine with lane = output channel ---------
 #pragma unroll
-        for (int s = 0; s < S; ++s) {
-            const int v = lane + 32 * s;
-            if (v < nvec) {
-                const float4 sd = side[s], eg = head.eg[s];
-                if (p.side_out) reinterpret_cast<float4*>(p.side_out + lrow * p.ld_side)[v] = sd;
-                float4 t0, t1;
+            for (int s = 0; s < S; ++s) {
+                const int v = lane + 32 * s;
+                if (v < nvec) {
+                    const float4 sd = side[s];
+                    if (p.side_out) reinterpret_cast<float4*>(p.side_out + lrow * p.ld_side)[v] = sd;
+                    const Terms u = terms<MODE>(head.eg[s], sd, p.sum_ego);
+                    stage[v] = u.t0;
+                    if (NT == 2) stage[nvec + v] = u.t1;
+                }
+            }
+            __syncwarp();
+            float acc1[NC], acc2[NC];
+#pragma unroll
+            for (int c = 0; c < NC; ++c) {
+                const int ch = lane + 32 * c;
+                // kBiZ: acc1 accumulates the product path (r2 + (ego * side) @ P2); the sum path is r1 + zside
+                const float* rp = Z ? p.r2 : p.r1;
+                acc1[c] = (ch < d_out && rp) ? __ldg(rp + lrow * p.ld_r + ch) : 0.f;
+                acc2[c] = (MODE == kBi && ch < d_out && p.r2) ? __ldg(p.r2 + lrow * p.ld_r + ch) : 0.f;
                 if (Z) {
-                    t0 = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
-                    t1 = t0;
-                } else if (MODE == kTwoTerms) {
-                    t0 = eg;
-                    t1 = sd;
-                } else {
-                    t0 = p.sum_ego ? make_float4(eg.x + sd.x, eg.y + sd.y, eg.z + sd.z, eg.w + sd.w) : sd;
-                    t1 = make_float4(eg.x * sd.x, eg.y * sd.y, eg.z * sd.z, eg.w * sd.w);
+                    const int src = (ch >> 2) & 31;
+                    const float zx = __shfl_sync(kFull, zside.x, src), zy = __shfl_sync(kFull, zside.y, src);
+                    const float zz = __shfl_sync(kFull, zside.z, src), zw = __shfl_sync(kFull, zside.w, src);
+                    const int comp = ch & 3;
+                    const float zv = comp == 0 ? zx : (comp == 1 ? zy : (comp == 2 ? zz : zw));
+                    acc2[c] = ((ch < d_out && p.r1) ? __ldg(p.r1 + lrow * p.ld_r + ch) : 0.f) + zv;
                 }
-                stage[v] = t0;
-                if (NT == 2) stage[nvec + v] = t1;
             }
-        }
-        __syncwarp();
-        float acc1[NC], acc2[NC];
-#pragma unroll
-        for (int c = 0; c < NC; ++c) {
-            const int ch = lane + 32 * c;
-            // kBiZ: acc1 accumulates the product path (r2 + (ego * side) @ P2); the sum path is r1 + zside
-            const float* rp = Z ? p.r2 : p.r1;
-            acc1[c] = (ch < d_out && rp) ? __ldg(rp + lrow * p.ld_r + ch) : 0.f;
-            acc2[c] = (MODE == kBi && ch < d_out && p.r2) ? __ldg(p.r2 + lrow * p.ld_r + ch) : 0.f;
-            if (Z) {
-                const int src = (ch >> 2) & 31;
-                const float zx = __shfl_sync(kFull, zside.x, src), zy = __shfl_sync(kFull, zside.y, src);
-                const float zz = __shfl_sync(kFull, zside.z, src), zw = __shfl_sync(kFull, zside.w, src);
-                const int comp = ch & 3;
-                const float zv = comp == 0 ? zx : (comp == 1 ? zy : (comp == 2 ? zz : zw));
-                acc2[c] = ((ch < d_out && p.r1) ? __ldg(p.r1 + lrow * p.ld_r + ch) : 0.f) + zv;
-            }
-        }
 #pragma unroll 5
-        for (int d4 = 0; d4 < nvec; ++d4) {
-            const float4 ua = stage[d4];
-            float4 ub = make_float4(0, 0, 0, 0);
-            if (NT == 2) ub = stage[nvec + d4];
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const float4 w0 = sp0[d4 * cpad + lane + 32 * c];
-                float x = acc1[c];
-                x = fmaf(ua.x, w0.x, x);
-                x = fmaf(ua.y, w0.y, x);
-                x = fmaf(ua.z, w0.z, x);
-                x = fmaf(ua.w, w0.w, x);
-                if (NT == 2) {
-                    const float4 w1 = sp1[d4 * cpad + lane + 32 * c];
-                    if (MODE == kTwoTerms) {
-                        x = fmaf(ub.x, w1.x, x);
-                        x = fmaf(ub.y, w1.y, x);
-                        x = fmaf(ub.z, w1.z, x);
-                        x = fmaf(ub.w, w1.w, x);
-                    } else {
-                        float y = acc2[c];
-                        y = fmaf(ub.x, w1.x, y);
-                        y = fmaf(ub.y, w1.y, y);
-                        y = fmaf(ub.z, w1.z, y);
-                        y = fmaf(ub.w, w1.w, y);
-                        acc2[c] = y;
-                    }
-                }
-                acc1[c] = x;
-            }
-        }
-        __syncwarp();   // the staging buffer is reused by the next row
-
-        // ---- phase 3: activation, LayerNorm, mask, L2 normalise ------------------------------------------------
-        {
-            float emb[NC];
-            float s1 = 0.f;
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const int ch = lane + 32 * c;
-                if (p.o_out && ch < d_out) {     // kBiZ: acc1 is the product path (o2), acc2 the sum path (o1)
-                    p.o_out[lrow * p.ld_o + (Z ? d_out : 0) + ch] = acc1[c];
-                    if (MODE == kBi || Z) p.o_out[lrow * p.ld_o + (Z ? 0 : d_out) + ch] = acc2[c];
-                }
-                float e = leaky(acc1[c]);
-                if (MODE == kBi || Z) e += leaky(acc2[c]);
-                emb[c] = ch < d_out ? e : 0.f;
-                s1 += emb[c];
-            }
-            const float mean = warp_sum(s1) / (float)d_out;
-            float s2 = 0.f;
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const int ch = lane + 32 * c;
-                const float dlt = ch < d_out ? emb[c] - mean : 0.f;
-                s2 = fmaf(dlt, dlt, s2);
-            }
-            const float rstd = rsqrtf(warp_sum(s2) / (float)d_out + 1e-5f);
-            float sq = 0.f;
-#pragma unroll
-            for (int c = 0; c < NC; ++c) {
-                const int ch = lane + 32 * c;
-                float x = 0.f;
-                if (ch < d_out) {
-                    x = (emb[c] - mean) * rstd * __ldg(p.ln_w + ch) + __ldg(p.ln_b + ch);
-                    if (p.mask) x *= __ldg(p.mask + lrow * d_out + ch);
-                    p.x_out[(int64_t)row * p.ld_x + ch] = x;
-                }
-                emb[c] = x;
-                sq = fmaf(x, x, sq);
-            }
-            if (p.xn_out || p.xn_planes) {
-                const float inv = 1.f / fmaxf(sqrtf(warp_sum(sq)), 1e-12f);
-                const float pscale = p.xn_planes ? __ldg(p.xn_rec + 1) : 1.f;
+            for (int d4 = 0; d4 < nvec; ++d4) {
+                const float4 ua = stage[d4];
+                float4 ub = make_float4(0, 0, 0, 0);
+                if (NT == 2) ub = stage[nvec + d4];
 #pragma unroll
                 for (int c = 0; c < NC; ++c) {
-                    const int ch = lane + 32 * c;
-                    if (ch < d_out) {
-                        const float xn = emb[c] * inv;
-                        if (p.xn_out) p.xn_out[lrow * p.ld_xn + ch] = xn;
-                        if (p.xn_planes) {
-                            const float xs = xn * pscale;
-                            const __half h = __float2half_rn(xs);
-                            const __half l = __float2half_rn(xs - __half2float(h));
-                            p.xn_planes[lrow * p.ld_planes + ch] = h;
-                            p.xn_planes[p.plane_stride + lrow * p.ld_planes + ch] = l;
+                    const float4 w0 = sp0[d4 * cpad + lane + 32 * c];
+                    float x = acc1[c];
+                    x = fmaf(ua.x, w0.x, x);
+                    x = fmaf(ua.y, w0.y, x);
+                    x = fmaf(ua.z, w0.z, x);
+                    x = fmaf(ua.w, w0.w, x);
+                    if (NT == 2) {
+                        const float4 w1 = sp1[d4 * cpad + lane + 32 * c];
+                        if (MODE == kTwoTerms) {
+                            x = fmaf(ub.x, w1.x, x);
+                            x = fmaf(ub.y, w1.y, x);
+                            x = fmaf(ub.z, w1.z, x);
+                            x = fmaf(ub.w, w1.w, x);
+                        } else {
+                            float y = acc2[c];
+                            y = fmaf(ub.x, w1.x, y);
+                            y = fmaf(ub.y, w1.y, y);
+                            y = fmaf(ub.z, w1.z, y);
+                            y = fmaf(ub.w, w1.w, y);
+                            acc2[c] = y;
                         }
                     }
+                    acc1[c] = x;
                 }
             }
+            __syncwarp();   // the staging buffer is reused by the next row
+
+            // ---- phase 3 ---------------------------------------------------------------------------------------
+            const float(&o1)[NC] = Z ? acc2 : acc1;
+            const float(&o2)[NC] = Z ? acc1 : acc2;
+            row_epilogue<MODE == kBi || Z>(p, WarpChannels<NC>{lane}, o1, o2, true, row, lrow);
         }
-        }   // finish
         idx = idx1; rec = rec1; head = head1;
         idx1 = idx2; rec1 = rec2;
     }
@@ -1295,16 +1179,6 @@ int launch_stream(const AggParams& p, size_t smem, cudaStream_t stream) {
     return LKG_OK;
 }
 
-template <int S, int NC>
-int dispatch_stream(int mode, const AggParams& p, size_t smem, cudaStream_t stream) {
-    switch (mode) {
-        case kOneTerm: return launch_stream<S, NC, kOneTerm>(p, smem, stream);
-        case kTwoTerms: return launch_stream<S, NC, kTwoTerms>(p, smem, stream);
-        case kBiZ: return launch_stream<S, NC, kBiZ>(p, smem, stream);
-        default: return launch_stream<S, NC, kBi>(p, smem, stream);
-    }
-}
-
 template <int S, int NC, int MODE>
 int launch(const AggParams& p, int threads, size_t smem, cudaStream_t stream) {
     auto kern = aggregate_kernel<S, NC, MODE>;
@@ -1316,15 +1190,6 @@ int launch(const AggParams& p, int threads, size_t smem, cudaStream_t stream) {
     kern<<<grid, threads, smem, stream>>>(p);
     LKG_LAUNCH_CHECK("aggregate_kernel");
     return LKG_OK;
-}
-
-template <int S, int NC>
-int dispatch_mode(int mode, const AggParams& p, int threads, size_t smem, cudaStream_t stream) {
-    switch (mode) {
-        case kOneTerm: return launch<S, NC, kOneTerm>(p, threads, smem, stream);
-        case kTwoTerms: return launch<S, NC, kTwoTerms>(p, threads, smem, stream);
-        default: return launch<S, NC, kBi>(p, threads, smem, stream);
-    }
 }
 
 // ---- which kernel runs a shape ---------------------------------------------------------------------------------
@@ -1494,8 +1359,11 @@ extern "C" int lkg_aggregate_fwd(const lkg_graph* g, const float* a_values, cons
     LKG_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(int), stream));
     if (rt.route == kRouteNarrow) {
         const int chunks = d_out / 4;
-#define LKG_NARROW_CASE(LL, CC) \
-    if (d_in == 4 * LL && (chunks + LL - 1) / LL == CC) return dispatch_narrow<LL, CC>(mode, p, stream);
+#define LKG_NARROW_CASE(LL, CC)                                          \
+    if (d_in == 4 * LL && (chunks + LL - 1) / LL == CC)                  \
+        return with_mode<false>(mode, [&](auto m) {                      \
+            return launch_narrow<LL, decltype(m)::value, CC>(p, stream); \
+        });
         LKG_NARROW_CASE(4, 1) LKG_NARROW_CASE(4, 2) LKG_NARROW_CASE(4, 3) LKG_NARROW_CASE(4, 4)
         LKG_NARROW_CASE(8, 1) LKG_NARROW_CASE(8, 2)
         LKG_NARROW_CASE(16, 1)
@@ -1504,17 +1372,23 @@ extern "C" int lkg_aggregate_fwd(const lkg_graph* g, const float* a_values, cons
     if (rt.route == kRouteStream) {
         const int slots_w = (p.nvec + 31) / 32, nc_w = (d_out + 31) / 32;
         if (slots_w == 1 && nc_w == 1) return launch_stream<1, 1, kBiZ>(p, rt.smem, stream);
-        if (slots_w == 2 && nc_w == 1) return dispatch_stream<2, 1>(mode, p, rt.smem, stream);
-        if (slots_w == 3 && nc_w == 1) return dispatch_stream<3, 1>(mode, p, rt.smem, stream);
-        if (slots_w == 3 && nc_w == 2) return dispatch_stream<3, 2>(mode, p, rt.smem, stream);
-        if (slots_w == 4 && nc_w == 1) return dispatch_stream<4, 1>(mode, p, rt.smem, stream);
+#define LKG_STREAM_CASE(SS, CC)                                                   \
+    if (slots_w == SS && nc_w == CC)                                              \
+        return with_mode<true>(mode, [&](auto m) {                                \
+            return launch_stream<SS, CC, decltype(m)::value>(p, rt.smem, stream); \
+        });
+        LKG_STREAM_CASE(2, 1) LKG_STREAM_CASE(3, 1) LKG_STREAM_CASE(3, 2) LKG_STREAM_CASE(4, 1)
+#undef LKG_STREAM_CASE
     }
     if (rt.route == kRouteGeneric) {
         const int threads = rt.warps * 32;
         const int slots = (p.nvec + 31) / 32;
         const int nc = (d_out + 31) / 32;
-#define LKG_AGG_CASE(SS, CC) \
-    if (slots == SS && nc == CC) return dispatch_mode<SS, CC>(mode, p, threads, rt.smem, stream);
+#define LKG_AGG_CASE(SS, CC)                                                        \
+    if (slots == SS && nc == CC)                                                    \
+        return with_mode<false>(mode, [&](auto m) {                                 \
+            return launch<SS, CC, decltype(m)::value>(p, threads, rt.smem, stream); \
+        });
         LKG_AGG_CASE(1, 1) LKG_AGG_CASE(2, 1) LKG_AGG_CASE(3, 1) LKG_AGG_CASE(4, 1)
         LKG_AGG_CASE(1, 2) LKG_AGG_CASE(2, 2) LKG_AGG_CASE(3, 2) LKG_AGG_CASE(4, 2)
 #undef LKG_AGG_CASE

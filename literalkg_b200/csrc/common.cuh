@@ -1,5 +1,6 @@
 // Shared helpers for liblkg (sm_100a only).
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -106,6 +107,25 @@ __device__ __forceinline__ void ring_wait(uint64_t* bar, uint32_t parity) {
 }
 
 __device__ __forceinline__ float leaky(float x) { return x > 0.f ? x : 0.01f * x; }
+
+// ---- fp16 hi/lo operands of the tensor-core paths: s x = hi + lo, hi = fp16(s x), lo = fp16(s x - hi), s = 2^e ----
+// e that parks amax * 2^e in [2^11, 2^12), clamped to [-lim, lim] (0 for a zero or non-finite amax)
+__device__ __forceinline__ int plane_exp(float amax, int lim = 120) {
+    int e = 0;
+    if (amax > 0.f && amax < 3.0e38f) {
+        int ex;
+        frexpf(amax, &ex);                 // amax = f * 2^ex, f in [0.5, 1)
+        e = 12 - ex;
+        e = e > lim ? lim : (e < -lim ? -lim : e);
+    }
+    return e;
+}
+__device__ __forceinline__ float pow2(int e) { return __int_as_float((127 + e) << 23); }   // 2^e, |e| <= 126
+// x is already multiplied by the operand's power-of-two scale
+__device__ __forceinline__ void split_f16(float x, __half& hi, __half& lo) {
+    hi = __float2half_rn(x);
+    lo = __float2half_rn(x - __half2float(hi));
+}
 
 // tanh with ~2e-7 absolute error: odd polynomial near zero, (1-e)/(1+e) with e = exp(-2|x|) elsewhere
 __device__ __forceinline__ float tanh_acc(float x) {

@@ -96,11 +96,6 @@ __device__ __forceinline__ uint32_t order_enc(float f) {
     const uint32_t u = __float_as_uint(f);
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
-// x is already multiplied by the operand's power-of-two scale
-__device__ __forceinline__ void split_f16(float x, __half& hi, __half& lo) {
-    hi = __float2half_rn(x);
-    lo = __float2half_rn(x - __half2float(hi));
-}
 
 // ---- epilogue of one 32-row x 32-column accumulator block, staged in shared memory as st[row * kStagePitch + col] ----
 __device__ __forceinline__ float4 ld4_guard(const float* ptr, int valid, bool vec) {
@@ -649,13 +644,7 @@ int launch_tc(TcParams& p, const lkg_planes* a, int64_t m, const lkg_planes* b, 
 // ---- operand preparation -------------------------------------------------------------------------------
 // Scale record {absmax, scale, 1/scale, counter, seg absmax x4}: scale = 2^e parks absmax * scale in [2^11, 2^12).
 __device__ __forceinline__ void write_record(float* rec, float amax) {
-    int e = 0;
-    if (amax > 0.f && amax < 3.0e38f) {
-        int ex;
-        frexpf(amax, &ex);                 // amax = f * 2^ex, f in [0.5, 1)
-        e = 12 - ex;
-        e = e > 60 ? 60 : (e < -60 ? -60 : e);
-    }
+    const int e = plane_exp(amax, 60);
     rec[0] = amax;
     rec[1] = ldexpf(1.f, e);
     rec[2] = ldexpf(1.f, -e);
@@ -849,14 +838,7 @@ __global__ void seg_absmax_kernel(const float* __restrict__ w, int64_t ldw, int 
 __device__ __forceinline__ float pack_total_scale(const PackSegs& segs, const float* w_rec) {
     float cmax = 0.f;
     for (int s = 0; s < segs.n_segments; ++s) cmax = fmaxf(cmax, w_rec[4 + s] * __ldg(segs.a_rec[s] + 2));
-    int e = 0;
-    if (cmax > 0.f && cmax < 3.0e38f) {
-        int ex;
-        frexpf(cmax, &ex);
-        e = 12 - ex;
-        e = e > 120 ? 120 : (e < -120 ? -120 : e);
-    }
-    return ldexpf(1.f, e);
+    return ldexpf(1.f, plane_exp(cmax));
 }
 __global__ void pack_weight_kernel(const float* __restrict__ w, int64_t ldw, int n, PackSegs segs,
                                    __half* __restrict__ dst, int kb, int64_t plane_stride, float* __restrict__ w_rec) {
