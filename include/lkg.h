@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define LKG_ABI_VERSION 8
+#define LKG_ABI_VERSION 9
 
 typedef enum {
     LKG_OK = 0,
@@ -310,11 +310,7 @@ int lkg_bi_bwd_rows(int64_t n, int32_t d, int32_t c, const float* d_o2, int64_t 
                     const float* x, int64_t ld_x, const float* side, int64_t ld_side, float* w_out, int64_t ld_w,
                     float* dx, int64_t ld_dx, int32_t accumulate, float* xs_out, int64_t ld_xs, float* xs_amax,
                     void* stream);
-/* Parameter gradients: out[i, j] += sum_rows x[row, i] * (x2 ? x2[row, i] : 1) * y[row, j]; x == NULL with dx == 1
- * gives the column sums of y (bias gradients).  out [dx, cy] is accumulated into (zero it first). */
-int lkg_xt_y(const float* x /*nullable*/, int64_t ld_x, const float* x2 /*nullable*/, int64_t ld_x2, int32_t dx,
-             const float* y, int64_t ld_y, int32_t cy, int64_t n, float* out, int64_t ld_out, void* stream);
-/* The same reduction on the tensor cores: out[dx, cy] += x^T y with both operands given as fp16 hi/lo planes
+/* Parameter gradients on the tensor cores: out[dx, cy] += x^T y with both operands given as fp16 hi/lo planes
  * ([n_rows, k] row-major, single segment; the planes the forward GEMMs already use).  MN-major tcgen05 operands,
  * split over row ranges, fp32 atomics into out. */
 int lkg_xt_y_planes(const lkg_planes* x, const lkg_planes* y, int64_t n_rows, float* out, int64_t ld_out, void* stream);

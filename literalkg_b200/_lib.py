@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_PKG, "liblkg.so")
 
 LKG_MAX_SEGMENTS = 4
 LKG_SCALE_FLOATS = 8
-ABI_VERSION = 8
+ABI_VERSION = 9
 SOLO_DEGREE, SEG_DEGREE, MAX_SEGS, SEG_STRIDE = 256, 512, 8, 576
 ACT_NONE, ACT_LEAKY_RELU, ACT_TANH, ACT_ACCUMULATE = 0, 1, 2, 256
 AGG_ONE_TERM, AGG_TWO_TERMS, AGG_BI, AGG_BI_Z = 0, 1, 2, 3     # lkg_agg_mode
@@ -74,7 +74,6 @@ SIGNATURES = {
     "lkg_spmm_coo": (C.c_int, [vp, vp, vp, vp, i64, vp, i64, i32, vp, i64, vp]),
     "lkg_layer_bwd_rows": (C.c_int, [i64, i32, i32, vp, i64, vp, i64, vp, vp, i64, vp, i64, vp, vp, i64, vp, vp, vp, vp]),
     "lkg_bi_bwd_rows": (C.c_int, [i64, i32, i32, vp, i64, vp, vp, i64, vp, i64, vp, i64, vp, i64, i32, vp, i64, vp, vp]),
-    "lkg_xt_y": (C.c_int, [vp, i64, vp, i64, i32, vp, i64, i32, i64, vp, i64, vp]),
     "lkg_xt_y_planes": (C.c_int, [C.POINTER(LkgPlanes), C.POINTER(LkgPlanes), i64, vp, i64, vp]),
     "lkg_colsum": (C.c_int, [vp, i64, i64, i32, vp, vp]),
     "lkg_gate_bwd": (C.c_int, [vp, i64, vp, i64, vp, i64, i64, i32, vp, i64, vp, i64, vp, vp]),

@@ -7,8 +7,8 @@
 //   spmm_coo         out += A^T X as a segmented reduction over the transposed COO list (equal nnz per
 //                    worker: a tail with 10^5 in-edges costs what 10^5 separate entries cost)
 //   bi_bwd_rows      the product path of the bi-interaction aggregator (d_out -> d_in expansion in the kernel)
-//   xt_y             parameter gradients  X^T Y  reduced over the N entity rows
-// plus the tensor-core GEMM engine (gemm_tc.cu) for the N x k x d products.  All HBM bound except xt_y.
+// plus the tensor-core GEMM engine (gemm_tc.cu) for the N x k x d products and the tensor-core X^T Y reduction
+// (xty_tc.cu) for the parameter gradients.  All HBM bound.
 #include <cub/device/device_radix_sort.cuh>
 
 #include <algorithm>
@@ -183,202 +183,119 @@ struct LayerBwdParams {
     float* amax2;                            // nullable: a second record that covers d_o (the buffer it is a part of)
 };
 
-template <int NC>
+// Lanes per row of a layout: the whole warp for WarpChannels, a group of LPR lanes for GroupQuads
+template <class L> constexpr int kLanesPerRow = 32;
+template <int LPR, int CPL> constexpr int kLanesPerRow<GroupQuads<LPR, CPL>> = LPR;
+
+// a slot's values at q, or fill in each of its channels where !ok
+template <class S>
+__device__ __forceinline__ typename S::V ld_or(const float* q, bool ok, float fill) {
+    typename S::V v;
+#pragma unroll
+    for (int k = 0; k < (int)(sizeof(v) / sizeof(float)); ++k) S::at(v, k) = fill;
+    return ok ? S::ld(q) : v;
+}
+
+// One row per LPR lanes over a lane layout of the forward: WarpChannels<1 | 2> (a warp per row, any rows) or
+// GroupQuads<8 | 16, 1> (one 16-byte vector of channels per lane, 32 / LPR rows per warp: a warp moves 512 bytes per
+// array, not 128; needs c % 4 == 0 and 16-byte aligned rows).  A lane sums its values in sequence, slot after slot and
+// channel after channel (not pairwise like the forward's QuadSlot::add).  An absent dy_in adds +0, an absent mask
+// multiplies by 1.
+template <class L>
 __global__ void __launch_bounds__(256) layer_bwd_rows_kernel(LayerBwdParams p) {
-    __shared__ float red[8][2 * 32 * NC];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int C = p.c;
-    const float inv_c = 1.f / (float)C;
-    float dgam[NC], dbet[NC], lw[NC];
-#pragma unroll
-    for (int c = 0; c < NC; ++c) {
-        dgam[c] = dbet[c] = 0.f;
-        const int ch = lane + 32 * c;
-        lw[c] = ch < C ? __ldg(p.ln_w + ch) : 0.f;
-    }
-    float amax = 0.f;
-    const int64_t stride = (int64_t)gridDim.x * 8;
-    for (int64_t row = (int64_t)blockIdx.x * 8 + warp; row < p.n; row += stride) {
-        float o1[NC], o2[NC], e[NC], y[NC], g[NC];
-        float s1 = 0.f, sq = 0.f, dot = 0.f;
-#pragma unroll
-        for (int c = 0; c < NC; ++c) {
-            const int ch = lane + 32 * c;
-            const bool ok = ch < C;
-            o1[c] = ok ? __ldg(p.o + row * p.ld_o + ch) : 0.f;
-            o2[c] = (ok && p.has_o2) ? __ldg(p.o + row * p.ld_o + C + ch) : 0.f;
-            e[c] = ok ? leaky(o1[c]) + (p.has_o2 ? leaky(o2[c]) : 0.f) : 0.f;
-            y[c] = ok ? __ldg(p.y + row * p.ld_y + ch) : 0.f;
-            g[c] = (ok && p.dyn) ? __ldg(p.dyn + row * p.ld_dyn + ch) : 0.f;
-            s1 += e[c];
-            sq = fmaf(y[c], y[c], sq);
-            dot = fmaf(g[c], y[c], dot);
-        }
-        const float mean = warp_sum(s1) * inv_c;
-        float s2 = 0.f;
-#pragma unroll
-        for (int c = 0; c < NC; ++c) {
-            const float dlt = (lane + 32 * c) < C ? e[c] - mean : 0.f;
-            s2 = fmaf(dlt, dlt, s2);
-        }
-        const float rstd = rsqrtf(warp_sum(s2) * inv_c + 1e-5f);
-        sq = warp_sum(sq);
-        dot = warp_sum(dot);
-        const float nrm = sqrtf(sq);
-        const float den = fmaxf(nrm, 1e-12f);
-        const float k1 = 1.f / den;
-        const float k2 = nrm > 1e-12f ? dot / (den * den * den) : 0.f;    // clamp_min passes no gradient below eps
-        float dhat[NC], ehat[NC];
-        float m1 = 0.f, m2 = 0.f;
-#pragma unroll
-        for (int c = 0; c < NC; ++c) {
-            const int ch = lane + 32 * c;
-            const bool ok = ch < C;
-            float dy = g[c] * k1 - y[c] * k2;
-            if (ok && p.dy_in) dy += __ldg(p.dy_in + row * p.ld_dy + ch);
-            if (ok && p.mask) dy *= __ldg(p.mask + row * C + ch);
-            if (!ok) dy = 0.f;
-            ehat[c] = ok ? (e[c] - mean) * rstd : 0.f;
-            dgam[c] = fmaf(dy, ehat[c], dgam[c]);
-            dbet[c] += dy;
-            dhat[c] = dy * lw[c];
-            m1 += dhat[c];
-            m2 = fmaf(dhat[c], ehat[c], m2);
-        }
-        m1 = warp_sum(m1) * inv_c;
-        m2 = warp_sum(m2) * inv_c;
-#pragma unroll
-        for (int c = 0; c < NC; ++c) {
-            const int ch = lane + 32 * c;
-            if (ch < C) {
-                const float de = (dhat[c] - m1 - ehat[c] * m2) * rstd;
-                const float d1 = de * (o1[c] > 0.f ? 1.f : 0.01f);
-                p.d_o[row * p.ld_do + ch] = d1;
-                amax = fmaxf(amax, fabsf(d1));
-                if (p.has_o2) {
-                    const float d2 = de * (o2[c] > 0.f ? 1.f : 0.01f);
-                    p.d_o[row * p.ld_do + C + ch] = d2;
-                    amax = fmaxf(amax, fabsf(d2));
-                }
-            }
-        }
-    }
-    if (p.amax || p.amax2) {
-        amax = warp_max(amax);
-        if (lane == 0 && amax > 0.f) {
-            if (p.amax) atomicMax(reinterpret_cast<uint32_t*>(p.amax), __float_as_uint(amax));
-            if (p.amax2) atomicMax(reinterpret_cast<uint32_t*>(p.amax2), __float_as_uint(amax));
-        }
-    }
-#pragma unroll
-    for (int c = 0; c < NC; ++c) {
-        red[warp][lane + 32 * c] = dgam[c];
-        red[warp][32 * NC + lane + 32 * c] = dbet[c];
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < 2 * 32 * NC; i += blockDim.x) {
-        float s = 0.f;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += red[w][i];
-        const int half = i / (32 * NC), ch = i % (32 * NC);
-        if (ch < C) atomicAdd(p.dgb + half * C + ch, s);
-    }
-}
-
-// Narrow rows as 16-byte vectors: LPR lanes per row (one float4 of channels each), 32 / LPR rows per warp -- the
-// warp-per-row kernel above moves 128 bytes per warp and array, this one a full 512.  Needs c % 4 == 0, c <= 4 LPR
-// and 16-byte aligned rows everywhere.
-__device__ __forceinline__ float4 ld4_or(const float* p, bool ok, float fill) {
-    return ok ? __ldg(reinterpret_cast<const float4*>(p)) : make_float4(fill, fill, fill, fill);
-}
-template <int LPR>
-__device__ __forceinline__ float group_sum(float v) {
-#pragma unroll
-    for (int o = LPR / 2; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
-    return v;
-}
-
-template <int LPR>
-__global__ void __launch_bounds__(256) layer_bwd_rows_vec_kernel(LayerBwdParams p) {
-    constexpr int RPW = 32 / LPR, CW = 4 * LPR;
+    using S = typename L::Slot;
+    using V = typename S::V;
+    constexpr int N = L::N, W = sizeof(V) / sizeof(float), LPR = kLanesPerRow<L>, RPW = 32 / LPR, CW = LPR * N * W;
     __shared__ float red[8][2][CW];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int grp = lane / LPR, gl = lane % LPR;
-    const int C = p.c, ch = 4 * gl;
-    const bool okc = ch < C;
+    const L ly{lane % LPR};
+    const int C = p.c;
     const float inv_c = 1.f / (float)C;
-    float lw[4], dgam[4], dbet[4];
+    V lw[N], dgam[N], dbet[N];
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        lw[q] = okc ? __ldg(p.ln_w + ch + q) : 0.f;
-        dgam[q] = dbet[q] = 0.f;
-    }
+    for (int i = 0; i < N; ++i)
+#pragma unroll
+        for (int k = 0; k < W; ++k) {
+            S::at(lw[i], k) = ly.ch(i) < C ? __ldg(p.ln_w + ly.ch(i) + k) : 0.f;
+            S::at(dgam[i], k) = S::at(dbet[i], k) = 0.f;
+        }
     float amax = 0.f;
     const int64_t units = (p.n + RPW - 1) / RPW;
     for (int64_t unit = (int64_t)blockIdx.x * 8 + warp; unit < units; unit += (int64_t)gridDim.x * 8) {
-        const int64_t row = unit * RPW + grp;
-        const bool live = okc && row < p.n;
-        const float4 o1v = ld4_or(p.o + row * p.ld_o + ch, live, 0.f);
-        const float4 o2v = ld4_or(p.o + row * p.ld_o + C + ch, live && p.has_o2, 0.f);
-        const float4 yv = ld4_or(p.y + row * p.ld_y + ch, live, 0.f);
-        const float4 gv = ld4_or(p.dyn + row * p.ld_dyn + ch, live && p.dyn, 0.f);
-        const float4 dyv = ld4_or(p.dy_in + row * p.ld_dy + ch, live && p.dy_in, 0.f);
-        const float4 mkv = ld4_or(p.mask + row * C + ch, live && p.mask, 1.f);
-        const float o1[4] = {o1v.x, o1v.y, o1v.z, o1v.w}, o2[4] = {o2v.x, o2v.y, o2v.z, o2v.w};
-        const float y[4] = {yv.x, yv.y, yv.z, yv.w}, g[4] = {gv.x, gv.y, gv.z, gv.w};
-        const float dyi[4] = {dyv.x, dyv.y, dyv.z, dyv.w}, mk[4] = {mkv.x, mkv.y, mkv.z, mkv.w};
-        float e[4];
+        const int64_t row = unit * RPW + lane / LPR;
+        const bool live = RPW == 1 || row < p.n;         // a unit of one row is in range by the loop bound
+        bool ok[N];
+        V o1[N], o2[N], y[N], g[N], dyi[N], mk[N], e[N];
         float s1 = 0.f, sq = 0.f, dot = 0.f;
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            e[q] = live ? leaky(o1[q]) + (p.has_o2 ? leaky(o2[q]) : 0.f) : 0.f;
-            s1 += e[q];
-            sq = fmaf(y[q], y[q], sq);
-            dot = fmaf(g[q], y[q], dot);
+        for (int i = 0; i < N; ++i) {
+            const int ch = ly.ch(i);
+            ok[i] = live && ch < C;
+            o1[i] = ld_or<S>(p.o + row * p.ld_o + ch, ok[i], 0.f);
+            o2[i] = ld_or<S>(p.o + row * p.ld_o + C + ch, ok[i] && p.has_o2, 0.f);
+            y[i] = ld_or<S>(p.y + row * p.ld_y + ch, ok[i], 0.f);
+            g[i] = ld_or<S>(p.dyn + row * p.ld_dyn + ch, ok[i] && p.dyn, 0.f);
+            dyi[i] = ld_or<S>(p.dy_in + row * p.ld_dy + ch, ok[i] && p.dy_in, 0.f);
+            mk[i] = ld_or<S>(p.mask + row * C + ch, ok[i] && p.mask, 1.f);
+#pragma unroll
+            for (int k = 0; k < W; ++k) {
+                const float ek = ok[i] ? leaky(S::at(o1[i], k)) + (p.has_o2 ? leaky(S::at(o2[i], k)) : 0.f) : 0.f;
+                S::at(e[i], k) = ek;
+                s1 += ek;
+                sq = fmaf(S::at(y[i], k), S::at(y[i], k), sq);
+                dot = fmaf(S::at(g[i], k), S::at(y[i], k), dot);
+            }
         }
-        const float mean = group_sum<LPR>(s1) * inv_c;
+        const float mean = ly.reduce(s1) * inv_c;
         float s2 = 0.f;
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const float dlt = live ? e[q] - mean : 0.f;
-            s2 = fmaf(dlt, dlt, s2);
-        }
-        const float rstd = rsqrtf(group_sum<LPR>(s2) * inv_c + 1e-5f);
-        sq = group_sum<LPR>(sq);
-        dot = group_sum<LPR>(dot);
+        for (int i = 0; i < N; ++i)
+#pragma unroll
+            for (int k = 0; k < W; ++k) {
+                const float dlt = ok[i] ? S::at(e[i], k) - mean : 0.f;
+                s2 = fmaf(dlt, dlt, s2);
+            }
+        const float rstd = rsqrtf(ly.reduce(s2) * inv_c + 1e-5f);
+        sq = ly.reduce(sq);
+        dot = ly.reduce(dot);
         const float nrm = sqrtf(sq);
         const float den = fmaxf(nrm, 1e-12f);
         const float k1 = 1.f / den;
         const float k2 = nrm > 1e-12f ? dot / (den * den * den) : 0.f;    // clamp_min passes no gradient below eps
-        float dhat[4], ehat[4];
+        V dhat[N], ehat[N];
         float m1 = 0.f, m2 = 0.f;
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            float dy = g[q] * k1 - y[q] * k2 + dyi[q];
-            dy *= mk[q];
-            if (!live) dy = 0.f;
-            ehat[q] = live ? (e[q] - mean) * rstd : 0.f;
-            dgam[q] = fmaf(dy, ehat[q], dgam[q]);
-            dbet[q] += dy;
-            dhat[q] = dy * lw[q];
-            m1 += dhat[q];
-            m2 = fmaf(dhat[q], ehat[q], m2);
-        }
-        m1 = group_sum<LPR>(m1) * inv_c;
-        m2 = group_sum<LPR>(m2) * inv_c;
-        if (live) {
-            float d1[4], d2[4];
+        for (int i = 0; i < N; ++i)
 #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float de = (dhat[q] - m1 - ehat[q] * m2) * rstd;
-                d1[q] = de * (o1[q] > 0.f ? 1.f : 0.01f);
-                d2[q] = de * (o2[q] > 0.f ? 1.f : 0.01f);
-                amax = fmaxf(amax, fabsf(d1[q]));
-                if (p.has_o2) amax = fmaxf(amax, fabsf(d2[q]));
+            for (int k = 0; k < W; ++k) {
+                float dy = S::at(g[i], k) * k1 - S::at(y[i], k) * k2 + S::at(dyi[i], k);
+                dy *= S::at(mk[i], k);
+                if (!ok[i]) dy = 0.f;
+                const float eh = ok[i] ? (S::at(e[i], k) - mean) * rstd : 0.f;
+                S::at(dgam[i], k) = fmaf(dy, eh, S::at(dgam[i], k));
+                S::at(dbet[i], k) += dy;
+                const float dh = dy * S::at(lw[i], k);
+                S::at(ehat[i], k) = eh;
+                S::at(dhat[i], k) = dh;
+                m1 += dh;
+                m2 = fmaf(dh, eh, m2);
             }
-            *reinterpret_cast<float4*>(p.d_o + row * p.ld_do + ch) = make_float4(d1[0], d1[1], d1[2], d1[3]);
-            if (p.has_o2)
-                *reinterpret_cast<float4*>(p.d_o + row * p.ld_do + C + ch) = make_float4(d2[0], d2[1], d2[2], d2[3]);
+        m1 = ly.reduce(m1) * inv_c;
+        m2 = ly.reduce(m2) * inv_c;
+#pragma unroll
+        for (int i = 0; i < N; ++i) {
+            if (!ok[i]) continue;
+            V d1, d2;
+#pragma unroll
+            for (int k = 0; k < W; ++k) {
+                const float de = (S::at(dhat[i], k) - m1 - S::at(ehat[i], k) * m2) * rstd;
+                S::at(d1, k) = de * (S::at(o1[i], k) > 0.f ? 1.f : 0.01f);
+                S::at(d2, k) = de * (S::at(o2[i], k) > 0.f ? 1.f : 0.01f);
+                amax = fmaxf(amax, fabsf(S::at(d1, k)));
+                if (p.has_o2) amax = fmaxf(amax, fabsf(S::at(d2, k)));
+            }
+            S::st(p.d_o + row * p.ld_do + ly.ch(i), d1);
+            if (p.has_o2) S::st(p.d_o + row * p.ld_do + C + ly.ch(i), d2);
         }
     }
     if (p.amax || p.amax2) {
@@ -388,19 +305,23 @@ __global__ void __launch_bounds__(256) layer_bwd_rows_vec_kernel(LayerBwdParams 
             if (p.amax2) atomicMax(reinterpret_cast<uint32_t*>(p.amax2), __float_as_uint(amax));
         }
     }
-    // LayerNorm weight / bias gradients: groups of the warp, then the 8 warps, then one atomic per channel and CTA
+    // LayerNorm weight / bias gradients: the rows of the warp, then the 8 warps, then one atomic per channel and CTA
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {
+    for (int i = 0; i < N; ++i)
 #pragma unroll
-        for (int o = LPR; o < 32; o <<= 1) {
-            dgam[q] += __shfl_xor_sync(kFull, dgam[q], o);
-            dbet[q] += __shfl_xor_sync(kFull, dbet[q], o);
+        for (int k = 0; k < W; ++k) {
+            float& dg = S::at(dgam[i], k);
+            float& db = S::at(dbet[i], k);
+#pragma unroll
+            for (int o = LPR; o < 32; o <<= 1) {
+                dg += __shfl_xor_sync(kFull, dg, o);
+                db += __shfl_xor_sync(kFull, db, o);
+            }
+            if (lane < LPR) {
+                red[warp][0][ly.ch(i) + k] = dg;
+                red[warp][1][ly.ch(i) + k] = db;
+            }
         }
-        if (grp == 0) {
-            red[warp][0][ch + q] = dgam[q];
-            red[warp][1][ch + q] = dbet[q];
-        }
-    }
     __syncthreads();
     for (int i = threadIdx.x; i < 2 * CW; i += blockDim.x) {
         const int half = i / CW, c = i % CW;
@@ -515,9 +436,9 @@ __global__ void __launch_bounds__(256) bi_bwd_rows_vec_kernel(BiBwdParams p) {
     for (int64_t unit = (int64_t)blockIdx.x * 8 + warp; unit < units; unit += (int64_t)gridDim.x * 8) {
         const int64_t row = unit * RPW + grp;
         const bool live = row < p.n;
-        const float4 dq = ld4_or(p.d_o2 + row * p.ld_do + 4 * gl, live && gl < chunks, 0.f);
-        const float4 xv = ld4_or(p.x + row * p.ld_x + i0, live && oki, 0.f);
-        const float4 sv = ld4_or(p.side + row * p.ld_side + i0, live && oki, 0.f);
+        const float4 dq = ld_or<QuadSlot>(p.d_o2 + row * p.ld_do + 4 * gl, live && gl < chunks, 0.f);
+        const float4 xv = ld_or<QuadSlot>(p.x + row * p.ld_x + i0, live && oki, 0.f);
+        const float4 sv = ld_or<QuadSlot>(p.side + row * p.ld_side + i0, live && oki, 0.f);
         float4 dv = make_float4(0.f, 0.f, 0.f, 0.f);
         if (live && oki && p.accumulate) dv = *reinterpret_cast<const float4*>(p.dx + row * p.ld_dx + i0);
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -547,163 +468,69 @@ __global__ void __launch_bounds__(256) bi_bwd_rows_vec_kernel(BiBwdParams p) {
     if (p.xs_amax) raise_absmax(p.xs_amax, amax);
 }
 
-// ---- parameter gradients: out[i, j] += sum_rows x[row, i] (* x2[row, i]) * y[row, j] ------------------------------
-struct XtyParams {
-    const float* x;   int64_t ld_x;    // nullable: a column of ones (dx == 1): column sums of y
-    const float* x2;  int64_t ld_x2;   // nullable
-    int dx;
-    const float* y;   int64_t ld_y;
-    int cy;
-    int64_t n;
-    int64_t rows_per_cta;
-    float* out;       int64_t ld_out;
-};
-
-constexpr int kXtyTI = 128, kXtyTJ = 64, kXtyKR = 32;
-
-__global__ void __launch_bounds__(256) xt_y_kernel(XtyParams p) {
-    __shared__ __align__(16) float xs[kXtyKR][kXtyTI];
-    __shared__ __align__(16) float ys[kXtyKR][kXtyTJ];
-    const int tid = threadIdx.x;
-    const int ti = tid >> 4, tj = tid & 15;                 // 16 x 16 threads, 8 x 4 outputs each
-    const int i0 = blockIdx.x * kXtyTI, j0 = blockIdx.y * kXtyTJ;
-    const int64_t r_begin = (int64_t)blockIdx.z * p.rows_per_cta;
-    const int64_t r_end = min(p.n, r_begin + p.rows_per_cta);
-    float acc[8][4];
-#pragma unroll
-    for (int a = 0; a < 8; ++a)
-#pragma unroll
-        for (int b = 0; b < 4; ++b) acc[a][b] = 0.f;
-    for (int64_t r0 = r_begin; r0 < r_end; r0 += kXtyKR) {
-#pragma unroll
-        for (int q = 0; q < kXtyKR * kXtyTI / 256; ++q) {
-            const int idx = tid + 256 * q;
-            const int rr = idx / kXtyTI, cc = idx % kXtyTI;
-            const int64_t row = r0 + rr;
-            float v = 0.f;
-            if (row < r_end && i0 + cc < p.dx) {
-                v = p.x ? __ldg(p.x + row * p.ld_x + i0 + cc) : 1.f;
-                if (p.x2) v *= __ldg(p.x2 + row * p.ld_x2 + i0 + cc);
-            }
-            xs[rr][cc] = v;
-        }
-#pragma unroll
-        for (int q = 0; q < kXtyKR * kXtyTJ / 256; ++q) {
-            const int idx = tid + 256 * q;
-            const int rr = idx / kXtyTJ, cc = idx % kXtyTJ;
-            const int64_t row = r0 + rr;
-            ys[rr][cc] = (row < r_end && j0 + cc < p.cy) ? __ldg(p.y + row * p.ld_y + j0 + cc) : 0.f;
-        }
-        __syncthreads();
-#pragma unroll 8
-        for (int k = 0; k < kXtyKR; ++k) {
-            const float4 xa = *reinterpret_cast<const float4*>(&xs[k][ti * 8]);
-            const float4 xb = *reinterpret_cast<const float4*>(&xs[k][ti * 8 + 4]);
-            const float4 yv = *reinterpret_cast<const float4*>(&ys[k][tj * 4]);
-            const float xv[8] = {xa.x, xa.y, xa.z, xa.w, xb.x, xb.y, xb.z, xb.w};
-            const float yy[4] = {yv.x, yv.y, yv.z, yv.w};
-#pragma unroll
-            for (int a = 0; a < 8; ++a)
-#pragma unroll
-                for (int b = 0; b < 4; ++b) acc[a][b] = fmaf(xv[a], yy[b], acc[a][b]);
-        }
-        __syncthreads();
-    }
-#pragma unroll
-    for (int a = 0; a < 8; ++a) {
-        const int i = i0 + ti * 8 + a;
-        if (i >= p.dx) continue;
-#pragma unroll
-        for (int b = 0; b < 4; ++b) {
-            const int j = j0 + tj * 4 + b;
-            if (j < p.cy) atomicAdd(p.out + (int64_t)i * p.ld_out + j, acc[a][b]);
-        }
-    }
-}
-
 // ---- gate backward, elementwise part (gate.py:22-28): out = (1 - z) e + z g ----------------------------------------
 //   d_pre[2j] = dh z (1 - g^2)   d_pre[2j+1] = dh (g - e) z (1 - z)   d_ent = dh (1 - z)
-__global__ void gate_bwd_kernel(const float* __restrict__ dh, int64_t ld_dh, const float* __restrict__ gz, int64_t ld_gz,
-                                const float* __restrict__ ent, int64_t ld_ent, int64_t n, int dim,
-                                float* __restrict__ d_pre, int64_t ld_pre, float* __restrict__ d_ent, int64_t ld_de,
-                                float* __restrict__ pre_amax) {
-    const int64_t total = n * dim;
-    float amax = 0.f;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t row = i / dim;
-        const int j = (int)(i - row * dim);
-        const float2 a = __ldg(reinterpret_cast<const float2*>(gz + row * ld_gz) + j);
-        const float g = a.x, z = a.y;
-        const float d = __ldg(dh + row * ld_dh + j);
-        const float e = __ldg(ent + row * ld_ent + j);
-        const float2 dp = make_float2(d * z * (1.f - g * g), d * (g - e) * z * (1.f - z));
-        reinterpret_cast<float2*>(d_pre + row * ld_pre)[j] = dp;
-        amax = fmaxf(amax, fmaxf(fabsf(dp.x), fabsf(dp.y)));
-        d_ent[row * ld_de + j] = d * (1.f - z);
-    }
-    if (pre_amax) raise_absmax(pre_amax, amax);
+// The interleaved (g, z) pairs and d_pre move as one float2 per channel, or as two float4 per quad of channels.
+__device__ __forceinline__ void ld_pairs(const float* q, float& g, float& z) {
+    const float2 a = __ldg(reinterpret_cast<const float2*>(q));
+    g = a.x;
+    z = a.y;
+}
+__device__ __forceinline__ void ld_pairs(const float* q, float4& g, float4& z) {
+    const float4 a0 = __ldg(reinterpret_cast<const float4*>(q)), a1 = __ldg(reinterpret_cast<const float4*>(q) + 1);
+    g = make_float4(a0.x, a0.z, a1.x, a1.z);
+    z = make_float4(a0.y, a0.w, a1.y, a1.w);
+}
+__device__ __forceinline__ void st_pairs(float* q, float g, float z) { *reinterpret_cast<float2*>(q) = make_float2(g, z); }
+__device__ __forceinline__ void st_pairs(float* q, float4 g, float4 z) {
+    reinterpret_cast<float4*>(q)[0] = make_float4(g.x, z.x, g.y, z.y);
+    reinterpret_cast<float4*>(q)[1] = make_float4(g.z, z.z, g.w, z.w);
 }
 
-// dpre = g * leaky'(out)   (sign(out) == sign of the pre-activation)
-__global__ void leaky_bwd_kernel(const float* __restrict__ g, int64_t ld_g, const float* __restrict__ out, int64_t ld_out,
-                                 int64_t n, int c, float* __restrict__ d, int64_t ld_d, float* __restrict__ d_amax) {
-    const int64_t total = n * c;
-    float amax = 0.f;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t row = i / c;
-        const int j = (int)(i - row * c);
-        const float v = __ldg(g + row * ld_g + j) * (__ldg(out + row * ld_out + j) > 0.f ? 1.f : 0.01f);
-        d[row * ld_d + j] = v;
-        amax = fmaxf(amax, fabsf(v));
-    }
-    if (d_amax) raise_absmax(d_amax, amax);
-}
-
-// The same two kernels over 16-byte units ([n, dim / 4] walked flat, 32-bit index arithmetic while it fits, two units
-// in flight per thread); the scalar kernels above stay for unaligned operands.
-template <typename I>
-__global__ void __launch_bounds__(256) gate_bwd_vec_kernel(const float* __restrict__ dh, int64_t ld_dh,
-                                                           const float* __restrict__ gz, int64_t ld_gz,
-                                                           const float* __restrict__ ent, int64_t ld_ent, int64_t n, int dim,
-                                                           float* __restrict__ d_pre, int64_t ld_pre,
-                                                           float* __restrict__ d_ent, int64_t ld_de,
-                                                           float* __restrict__ pre_amax) {
-    const I qv = (I)(dim >> 2), total = (I)n * qv, stride = (I)gridDim.x * blockDim.x;
+// Both elementwise backwards walk [n, c / width of the slot] flat: ScalarSlot for any operands, QuadSlot (16-byte units)
+// when every row is 16-byte aligned; 32-bit index arithmetic while it fits.
+template <class S, typename I>
+__global__ void __launch_bounds__(256) gate_bwd_kernel(const float* __restrict__ dh, int64_t ld_dh,
+                                                       const float* __restrict__ gz, int64_t ld_gz,
+                                                       const float* __restrict__ ent, int64_t ld_ent, int64_t n, int dim,
+                                                       float* __restrict__ d_pre, int64_t ld_pre,
+                                                       float* __restrict__ d_ent, int64_t ld_de,
+                                                       float* __restrict__ pre_amax) {
+    using V = typename S::V;
+    constexpr int W = sizeof(V) / sizeof(float);
+    const I qv = (I)(dim / W), total = (I)n * qv, stride = (I)gridDim.x * blockDim.x;
     float amax = 0.f;
     for (I i = (I)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const I row = i / qv;
-        const int j = 4 * (int)(i - row * qv);
-        const float4 a0 = __ldg(reinterpret_cast<const float4*>(gz + (int64_t)row * ld_gz + 2 * j));
-        const float4 a1 = __ldg(reinterpret_cast<const float4*>(gz + (int64_t)row * ld_gz + 2 * j) + 1);
-        const float4 dv = __ldg(reinterpret_cast<const float4*>(dh + (int64_t)row * ld_dh + j));
-        const float4 ev = __ldg(reinterpret_cast<const float4*>(ent + (int64_t)row * ld_ent + j));
-        const float g[4] = {a0.x, a0.z, a1.x, a1.z}, z[4] = {a0.y, a0.w, a1.y, a1.w};
-        const float d[4] = {dv.x, dv.y, dv.z, dv.w}, e[4] = {ev.x, ev.y, ev.z, ev.w};
-        float pg[4], pz[4], de[4];
+        const int j = W * (int)(i - row * qv);
+        V g, z, pg, pz, de;
+        ld_pairs(gz + (int64_t)row * ld_gz + 2 * j, g, z);
+        const V d = S::ld(dh + (int64_t)row * ld_dh + j), e = S::ld(ent + (int64_t)row * ld_ent + j);
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            pg[q] = d[q] * z[q] * (1.f - g[q] * g[q]);
-            pz[q] = d[q] * (g[q] - e[q]) * z[q] * (1.f - z[q]);
-            de[q] = d[q] * (1.f - z[q]);
-            amax = fmaxf(amax, fmaxf(fabsf(pg[q]), fabsf(pz[q])));
+        for (int k = 0; k < W; ++k) {
+            const float dk = S::at(d, k), gk = S::at(g, k), zk = S::at(z, k);
+            S::at(pg, k) = dk * zk * (1.f - gk * gk);
+            S::at(pz, k) = dk * (gk - S::at(e, k)) * zk * (1.f - zk);
+            S::at(de, k) = dk * (1.f - zk);
+            amax = fmaxf(amax, fmaxf(fabsf(S::at(pg, k)), fabsf(S::at(pz, k))));
         }
-        float4* dst = reinterpret_cast<float4*>(d_pre + (int64_t)row * ld_pre + 2 * j);
-        dst[0] = make_float4(pg[0], pz[0], pg[1], pz[1]);
-        dst[1] = make_float4(pg[2], pz[2], pg[3], pz[3]);
-        *reinterpret_cast<float4*>(d_ent + (int64_t)row * ld_de + j) = make_float4(de[0], de[1], de[2], de[3]);
+        st_pairs(d_pre + (int64_t)row * ld_pre + 2 * j, pg, pz);
+        S::st(d_ent + (int64_t)row * ld_de + j, de);
     }
     if (pre_amax) raise_absmax(pre_amax, amax);
 }
 
-template <typename I>
-__global__ void __launch_bounds__(256) leaky_bwd_vec_kernel(const float* __restrict__ g, int64_t ld_g,
-                                                            const float* __restrict__ out, int64_t ld_out, int64_t n, int c,
-                                                            float* __restrict__ d, int64_t ld_d, float* __restrict__ d_amax) {
-    constexpr int U = 2;
-    const I cv = (I)(c >> 2), total = (I)n * cv, stride = (I)gridDim.x * blockDim.x;
+// dpre = g * leaky'(out)   (sign(out) == sign of the pre-activation); two units in flight per thread
+template <class S, typename I>
+__global__ void __launch_bounds__(256) leaky_bwd_kernel(const float* __restrict__ g, int64_t ld_g,
+                                                        const float* __restrict__ out, int64_t ld_out, int64_t n, int c,
+                                                        float* __restrict__ d, int64_t ld_d, float* __restrict__ d_amax) {
+    using V = typename S::V;
+    constexpr int W = sizeof(V) / sizeof(float), U = 2;
+    const I cv = (I)(c / W), total = (I)n * cv, stride = (I)gridDim.x * blockDim.x;
     float amax = 0.f;
     for (I i = (I)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += U * stride) {
-        float4 gv[U], ov[U];
+        V gv[U], ov[U];
         I row[U];
         int col[U];
 #pragma unroll
@@ -711,19 +538,22 @@ __global__ void __launch_bounds__(256) leaky_bwd_vec_kernel(const float* __restr
             const I j = i + (I)u * stride;
             const bool ok = j < total;
             row[u] = ok ? j / cv : 0;
-            col[u] = ok ? 4 * (int)(j - row[u] * cv) : -1;
+            col[u] = ok ? W * (int)(j - row[u] * cv) : -1;
             if (ok) {
-                gv[u] = __ldg(reinterpret_cast<const float4*>(g + (int64_t)row[u] * ld_g + col[u]));
-                ov[u] = __ldg(reinterpret_cast<const float4*>(out + (int64_t)row[u] * ld_out + col[u]));
+                gv[u] = S::ld(g + (int64_t)row[u] * ld_g + col[u]);
+                ov[u] = S::ld(out + (int64_t)row[u] * ld_out + col[u]);
             }
         }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             if (col[u] < 0) continue;
-            const float4 v = make_float4(gv[u].x * (ov[u].x > 0.f ? 1.f : 0.01f), gv[u].y * (ov[u].y > 0.f ? 1.f : 0.01f),
-                                         gv[u].z * (ov[u].z > 0.f ? 1.f : 0.01f), gv[u].w * (ov[u].w > 0.f ? 1.f : 0.01f));
-            *reinterpret_cast<float4*>(d + (int64_t)row[u] * ld_d + col[u]) = v;
-            amax = fmaxf(fmaxf(amax, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
+            V v;
+#pragma unroll
+            for (int k = 0; k < W; ++k) {
+                S::at(v, k) = S::at(gv[u], k) * (S::at(ov[u], k) > 0.f ? 1.f : 0.01f);
+                amax = fmaxf(amax, fabsf(S::at(v, k)));
+            }
+            S::st(d + (int64_t)row[u] * ld_d + col[u], v);
         }
     }
     if (d_amax) raise_absmax(d_amax, amax);
@@ -800,19 +630,14 @@ extern "C" int lkg_layer_bwd_rows(int64_t n, int32_t c, int32_t has_o2, const fl
     if (c > 64) LKG_FAIL(LKG_ERR_UNSUPPORTED, "layer backward: d_out %d > 64", c);
     LayerBwdParams p{n, c, has_o2, y, ld_y, o, ld_o, mask, dy_in, ld_dy, dyn, ld_dyn, ln_weight, d_o, ld_do, dgamma_dbeta,
                      amax, amax2};
-    if (c % 4 == 0 && rows16(y, ld_y) && rows16(o, ld_o) && rows16(mask, c) && rows16(dy_in, ld_dy) && rows16(dyn, ld_dyn) &&
-        rows16(d_o, ld_do)) {
-        const int lpr = c <= 32 ? 8 : 16;
-        const int64_t units = (n + 32 / lpr - 1) / (32 / lpr);
-        const int grid = (int)std::min<int64_t>((units + 7) / 8, (int64_t)sm_count() * 8);
-        if (lpr == 8) layer_bwd_rows_vec_kernel<8><<<grid, 256, 0, stream>>>(p);
-        else layer_bwd_rows_vec_kernel<16><<<grid, 256, 0, stream>>>(p);
-        LKG_LAUNCH_CHECK("layer_bwd_rows_vec_kernel");
-        return LKG_OK;
-    }
-    const int grid = (int)std::min<int64_t>((n + 7) / 8, (int64_t)sm_count() * 8);
-    if (c <= 32) layer_bwd_rows_kernel<1><<<grid, 256, 0, stream>>>(p);
-    else layer_bwd_rows_kernel<2><<<grid, 256, 0, stream>>>(p);
+    const bool vec = c % 4 == 0 && rows16(y, ld_y) && rows16(o, ld_o) && rows16(mask, c) && rows16(dy_in, ld_dy) &&
+                     rows16(dyn, ld_dyn) && rows16(d_o, ld_do);
+    const int lpr = vec ? (c <= 32 ? 8 : 16) : 32;
+    const int64_t units = (n + 32 / lpr - 1) / (32 / lpr);
+    const int grid = (int)std::min<int64_t>((units + 7) / 8, (int64_t)sm_count() * 8);
+    auto* kernel = vec ? (c <= 32 ? layer_bwd_rows_kernel<GroupQuads<8, 1>> : layer_bwd_rows_kernel<GroupQuads<16, 1>>)
+                       : (c <= 32 ? layer_bwd_rows_kernel<WarpChannels<1>> : layer_bwd_rows_kernel<WarpChannels<2>>);
+    kernel<<<grid, 256, 0, stream>>>(p);
     LKG_LAUNCH_CHECK("layer_bwd_rows_kernel");
     return LKG_OK;
 }
@@ -859,25 +684,6 @@ extern "C" int lkg_bi_bwd_rows(int64_t n, int32_t d, int32_t c, const float* d_o
     LKG_FAIL(LKG_ERR_UNSUPPORTED, "bi backward: d_out %d", c);
 }
 
-extern "C" int lkg_xt_y(const float* x, int64_t ld_x, const float* x2, int64_t ld_x2, int32_t dx, const float* y,
-                        int64_t ld_y, int32_t cy, int64_t n, float* out, int64_t ld_out, void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
-    if (n == 0 || dx == 0 || cy == 0) return LKG_OK;
-    LKG_REQUIRE(y && out && dx > 0 && cy > 0 && (x || dx == 1), "bad arguments");
-    XtyParams p{x, ld_x, x2, ld_x2, dx, y, ld_y, cy, n, 0, out, ld_out};
-    const int ti = (dx + kXtyTI - 1) / kXtyTI, tj = (cy + kXtyTJ - 1) / kXtyTJ;
-    int64_t chunks = ((int64_t)sm_count() * 4 + ti * tj - 1) / (ti * tj);
-    const int64_t max_chunks = (n + 4 * kXtyKR - 1) / (4 * kXtyKR);
-    if (chunks > max_chunks) chunks = max_chunks;
-    if (chunks < 1) chunks = 1;
-    if (chunks > 65535) chunks = 65535;
-    p.rows_per_cta = ((n + chunks - 1) / chunks + kXtyKR - 1) / kXtyKR * kXtyKR;
-    chunks = (n + p.rows_per_cta - 1) / p.rows_per_cta;
-    xt_y_kernel<<<dim3(ti, tj, (unsigned)chunks), 256, 0, stream>>>(p);
-    LKG_LAUNCH_CHECK("xt_y_kernel");
-    return LKG_OK;
-}
-
 extern "C" int lkg_gate_bwd(const float* dh, int64_t ld_dh, const float* gz, int64_t ld_gz, const float* ent,
                             int64_t ld_ent, int64_t n, int32_t dim, float* d_pre, int64_t ld_pre, float* d_ent,
                             int64_t ld_de, float* pre_amax, void* stream_) {
@@ -886,21 +692,14 @@ extern "C" int lkg_gate_bwd(const float* dh, int64_t ld_dh, const float* gz, int
     LKG_REQUIRE(dh && gz && ent && d_pre && d_ent && dim > 0, "null argument");
     LKG_REQUIRE(ld_gz % 2 == 0 && ld_pre % 2 == 0 && (reinterpret_cast<uintptr_t>(gz) & 7u) == 0 &&
                     (reinterpret_cast<uintptr_t>(d_pre) & 7u) == 0, "gate backward: (g, z) pairs must be 8-byte aligned");
-    if (dim % 4 == 0 && rows16(dh, ld_dh) && rows16(gz, ld_gz) && rows16(ent, ld_ent) && rows16(d_pre, ld_pre) &&
-        rows16(d_ent, ld_de)) {
-        const int64_t units = n * (dim / 4);
-        const int grid = (int)std::min<int64_t>((units + 255) / 256, (int64_t)sm_count() * 8);
-        if (units < ((int64_t)1 << 30))
-            gate_bwd_vec_kernel<uint32_t><<<grid, 256, 0, stream>>>(dh, ld_dh, gz, ld_gz, ent, ld_ent, n, dim, d_pre, ld_pre,
-                                                                    d_ent, ld_de, pre_amax);
-        else
-            gate_bwd_vec_kernel<uint64_t><<<grid, 256, 0, stream>>>(dh, ld_dh, gz, ld_gz, ent, ld_ent, n, dim, d_pre, ld_pre,
-                                                                    d_ent, ld_de, pre_amax);
-        LKG_LAUNCH_CHECK("gate_bwd_vec_kernel");
-        return LKG_OK;
-    }
-    gate_bwd_kernel<<<sm_count() * 8, 256, 0, stream>>>(dh, ld_dh, gz, ld_gz, ent, ld_ent, n, dim, d_pre, ld_pre, d_ent, ld_de,
-                                                            pre_amax);
+    const bool vec = dim % 4 == 0 && rows16(dh, ld_dh) && rows16(gz, ld_gz) && rows16(ent, ld_ent) &&
+                     rows16(d_pre, ld_pre) && rows16(d_ent, ld_de);
+    const int64_t units = n * (vec ? dim / 4 : dim);
+    const int grid = (int)std::min<int64_t>((units + 255) / 256, (int64_t)sm_count() * 8);
+    const bool wide = units >= ((int64_t)1 << 30);
+    auto* kernel = vec ? (wide ? gate_bwd_kernel<QuadSlot, uint64_t> : gate_bwd_kernel<QuadSlot, uint32_t>)
+                       : (wide ? gate_bwd_kernel<ScalarSlot, uint64_t> : gate_bwd_kernel<ScalarSlot, uint32_t>);
+    kernel<<<grid, 256, 0, stream>>>(dh, ld_dh, gz, ld_gz, ent, ld_ent, n, dim, d_pre, ld_pre, d_ent, ld_de, pre_amax);
     LKG_LAUNCH_CHECK("gate_bwd_kernel");
     return LKG_OK;
 }
@@ -910,17 +709,13 @@ extern "C" int lkg_leaky_bwd(const float* grad, int64_t ld_g, const float* out, 
     cudaStream_t stream = (cudaStream_t)stream_;
     if (n == 0) return LKG_OK;
     LKG_REQUIRE(grad && out && d_pre && c > 0, "null argument");
-    if (c % 4 == 0 && rows16(grad, ld_g) && rows16(out, ld_out) && rows16(d_pre, ld_d)) {
-        const int64_t units = n * (c / 4);
-        const int grid = (int)std::min<int64_t>((units + 511) / 512, (int64_t)sm_count() * 8);
-        if (units < ((int64_t)1 << 30))
-            leaky_bwd_vec_kernel<uint32_t><<<std::max(grid, 1), 256, 0, stream>>>(grad, ld_g, out, ld_out, n, c, d_pre, ld_d, amax);
-        else
-            leaky_bwd_vec_kernel<uint64_t><<<std::max(grid, 1), 256, 0, stream>>>(grad, ld_g, out, ld_out, n, c, d_pre, ld_d, amax);
-        LKG_LAUNCH_CHECK("leaky_bwd_vec_kernel");
-        return LKG_OK;
-    }
-    leaky_bwd_kernel<<<sm_count() * 8, 256, 0, stream>>>(grad, ld_g, out, ld_out, n, c, d_pre, ld_d, amax);
+    const bool vec = c % 4 == 0 && rows16(grad, ld_g) && rows16(out, ld_out) && rows16(d_pre, ld_d);
+    const int64_t units = n * (vec ? c / 4 : c);
+    const int grid = (int)std::min<int64_t>((units + 511) / 512, (int64_t)sm_count() * 8);
+    const bool wide = units >= ((int64_t)1 << 30);
+    auto* kernel = vec ? (wide ? leaky_bwd_kernel<QuadSlot, uint64_t> : leaky_bwd_kernel<QuadSlot, uint32_t>)
+                       : (wide ? leaky_bwd_kernel<ScalarSlot, uint64_t> : leaky_bwd_kernel<ScalarSlot, uint32_t>);
+    kernel<<<std::max(grid, 1), 256, 0, stream>>>(grad, ld_g, out, ld_out, n, c, d_pre, ld_d, amax);
     LKG_LAUNCH_CHECK("leaky_bwd_kernel");
     return LKG_OK;
 }

@@ -142,4 +142,68 @@ __device__ __forceinline__ float tanh_acc(float x) {
 
 __device__ __forceinline__ float sigmoid_acc(float x) { return 1.f / (1.f + __expf(-x)); }
 
+// ---- lane layouts of a row, shared by the aggregation layer's forward and backward ----------------------------------
+// A lane layout says which channels of a row a lane holds -- N slots, slot i = channels [ch(i), ch(i) + width of Slot)
+// -- and how the lanes of a row reduce.  Its Slot type says how a slot's values enter the lane's partial sums and how
+// they are loaded and stored.  The order of every sum is part of the output bits, so each path keeps its own.
+struct ScalarSlot {                         // one channel: sequential partial sums, squares by fma
+    using V = float;
+    static __device__ float& at(float& v, int) { return v; }
+    static __device__ float at(const float& v, int) { return v; }
+    static __device__ float add(float s, float v) { return s + v; }
+    static __device__ float add_dev2(float s, float d) { return fmaf(d, d, s); }
+    static __device__ float add_sq(float s, float v) { return fmaf(v, v, s); }
+    static __device__ float ld(const float* q) { return __ldg(q); }
+    static __device__ void st(float* q, float v) { *q = v; }
+    static __device__ void st_planes(__half* q, int64_t plane_stride, float v) {
+        __half h, l;
+        split_f16(v, h, l);
+        q[0] = h;
+        q[plane_stride] = l;
+    }
+};
+struct QuadSlot {                           // four channels: pairwise sums in the slot, 16-byte (planes: 8-byte) moves
+    using V = float4;
+    static __device__ float& at(float4& v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w)); }
+    static __device__ float at(const float4& v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : (k == 2 ? v.z : v.w)); }
+    static __device__ float add(float s, float4 v) { return s + ((v.x + v.y) + (v.z + v.w)); }
+    // squares in pairs, one product fused into the other's add; the variance and the norm pair them the opposite way
+    // round, as this kernel always has (written out so that no contraction choice of the compiler can move the bits)
+    static __device__ float add_dev2(float s, float4 d) {
+        return s + (fmaf(d.x, d.x, d.y * d.y) + fmaf(d.z, d.z, d.w * d.w));
+    }
+    static __device__ float add_sq(float s, float4 v) {
+        return s + (fmaf(v.y, v.y, v.x * v.x) + fmaf(v.w, v.w, v.z * v.z));
+    }
+    static __device__ float4 ld(const float* q) { return __ldg(reinterpret_cast<const float4*>(q)); }
+    static __device__ void st(float* q, float4 v) { *reinterpret_cast<float4*>(q) = v; }
+    static __device__ void st_planes(__half* q, int64_t plane_stride, float4 v) {
+        __align__(8) __half h[4], l[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) split_f16(at(v, k), h[k], l[k]);
+        *reinterpret_cast<uint2*>(q) = *reinterpret_cast<const uint2*>(h);
+        *reinterpret_cast<uint2*>(q + plane_stride) = *reinterpret_cast<const uint2*>(l);
+    }
+};
+template <int NC>
+struct WarpChannels {                       // generic and stream per-row paths: channel lane + 32 i, the whole warp
+    using Slot = ScalarSlot;
+    static constexpr int N = NC;
+    int lane;
+    __device__ int ch(int i) const { return lane + 32 * i; }
+    static __device__ float reduce(float s) { return warp_sum(s); }
+};
+template <int LPR, int CPL>
+struct GroupQuads {                         // narrow kernel: channels 4 (gl + LPR i) + [0, 4), the LPR lanes of a group
+    using Slot = QuadSlot;
+    static constexpr int N = CPL;
+    int gl;
+    __device__ int ch(int i) const { return 4 * (gl + LPR * i); }
+    static __device__ float reduce(float s) {
+#pragma unroll
+        for (int o = LPR / 2; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+        return s;
+    }
+};
+
 }  // namespace lkg

@@ -822,21 +822,6 @@ def bi_bwd_rows(d_o2: torch.Tensor, p2: torch.Tensor, x: torch.Tensor, side: tor
                                                _lib.ptr(xs_amax), _lib.stream()))
 
 
-def xt_y(x: Optional[torch.Tensor], y: torch.Tensor, x2: Optional[torch.Tensor] = None,
-         out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """x^T @ y reduced over the rows (x None: column sums of y, shape [1, cy]); optional elementwise factor x2."""
-    _rowmajor(y)
-    n, cy = y.shape
-    dx = 1 if x is None else _rowmajor(x).shape[1]
-    if out is None:
-        out = torch.zeros((dx, cy), dtype=torch.float32, device=y.device)
-    with _dev_guard(y, f"xt_y_{dx}x{cy}"):
-        _lib.check(_lib.load().lkg_xt_y(_lib.ptr(x), 0 if x is None else x.stride(0), _lib.ptr(x2),
-                                        0 if x2 is None else _rowmajor(x2).stride(0), dx, y.data_ptr(), y.stride(0), cy, n,
-                                        out.data_ptr(), out.stride(0), _lib.stream()))
-    return out
-
-
 def xt_y_planes(xp, yp, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """x^T @ y over the rows on the tensor cores; xp / yp: Planes or PlanesView of [n, dx] and [n, cy]."""
     assert xp.rows == yp.rows

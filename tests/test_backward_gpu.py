@@ -86,22 +86,6 @@ def test_spmm_strided_views():
     assert outb[:, :2 * d].abs().max().item() == 0.0
 
 
-@pytest.mark.parametrize("dx,cy,n", [(300, 192, 5000), (32, 64, 999), (600, 300, 2100), (2, 600, 1500), (1, 256, 777)])
-def test_xt_y(dx, cy, n):
-    from literalkg_b200 import ops
-    g = torch.Generator(device="cuda").manual_seed(dx + cy)
-    x = torch.randn(n, dx, generator=g, device="cuda")
-    x2 = torch.randn(n, dx, generator=g, device="cuda")
-    ybig = torch.randn(n, cy + 8, generator=g, device="cuda")
-    y = ybig[:, 4:4 + cy]
-    assert rel_err(ops.xt_y(x, y), x.double().t() @ y.double()) < 1e-5
-    assert rel_err(ops.xt_y(x, y, x2=x2), (x.double() * x2.double()).t() @ y.double()) < 1e-5
-    assert rel_err(ops.xt_y(None, y).view(-1), y.double().sum(0)) < 1e-5
-    out = torch.zeros(dx, cy + 3, device="cuda")
-    ops.xt_y(x, y, out=out[:, 3:])
-    assert rel_err(out[:, 3:], x.double().t() @ y.double()) < 1e-5 and out[:, :3].abs().max().item() == 0.0
-
-
 @pytest.mark.parametrize("dx,cy,n", [(600, 302, 5000), (32, 32, 70001), (224, 300, 4097), (256, 96, 999), (64, 2, 300),
                                      (128, 256, 64), (300, 600, 12345)])
 def test_xt_y_tensor_core(dx, cy, n):
@@ -122,11 +106,17 @@ def test_xt_y_tensor_core(dx, cy, n):
     assert rel_err(ops.colsum(y), y.double().sum(0)) < 1e-5
 
 
-@pytest.mark.parametrize("c,has_o2,use_mask,use_dy,use_dyn", [(32, True, True, True, True), (32, False, False, False, True),
-                                                             (64, True, False, True, True), (16, False, True, True, False),
-                                                             (48, True, True, True, True), (10, True, True, True, True),
-                                                             (4, False, False, True, True)])
-def test_layer_bwd_rows(c, has_o2, use_mask, use_dy, use_dyn):
+# off = 1 places y, o and d_o one float into wider buffers: rows that are not 16-byte aligned take the warp-per-row
+# kernel at any c
+LAYER_BWD = [(32, True, True, True, True, 0), (32, False, False, False, True, 0), (64, True, False, True, True, 0),
+             (16, False, True, True, False, 0), (48, True, True, True, True, 0), (10, True, True, True, True, 0),
+             (4, False, False, True, True, 0), (50, True, True, True, True, 0), (32, True, True, True, True, 1),
+             (48, False, True, False, True, 1)]
+
+
+@pytest.mark.parametrize("c,has_o2,use_mask,use_dy,use_dyn,off", LAYER_BWD,
+                         ids=["-".join(map(str, t[:5])) + ("-off" if t[5] else "") for t in LAYER_BWD])
+def test_layer_bwd_rows(c, has_o2, use_mask, use_dy, use_dyn, off):
     from literalkg_b200 import ops
     n = 1234
     g = torch.Generator().manual_seed(c)
@@ -151,9 +141,16 @@ def test_layer_bwd_rows(c, has_o2, use_mask, use_dy, use_dyn):
         loss = loss + (torch.nn.functional.normalize(y, p=2, dim=1) * dyn).sum()
     loss.backward()
     f = lambda t: None if t is None else t.float().cuda()
-    d_o = torch.empty(n, nt * c, device="cuda")
+
+    def placed(t):
+        buf = torch.zeros(t.shape[0], t.shape[1] + off, device="cuda")
+        buf[:, off:] = t
+        return buf[:, off:]
+
+    d_o = placed(torch.empty(n, nt * c))
     dgb = torch.zeros(2 * c, device="cuda")
-    ops.layer_bwd_rows(f(y.detach()), f(o.detach()), has_o2, f(mask), f(dy), f(dyn), f(lw.detach()), d_o, dgb)
+    ops.layer_bwd_rows(placed(f(y.detach())), placed(f(o.detach())), has_o2, f(mask), f(dy), f(dyn), f(lw.detach()), d_o,
+                       dgb)
     assert rel_err(d_o, o.grad) < 1e-4
     assert rel_err(dgb[:c], lw.grad) < 1e-4
     assert rel_err(dgb[c:], lb.grad) < 1e-4

@@ -98,7 +98,7 @@ def _refused(lib, rc, words):
 
 def test_abi_version(lib):
     from literalkg_b200 import _lib
-    assert lib.lkg_abi_version() == 8 == _lib.ABI_VERSION
+    assert lib.lkg_abi_version() == 9 == _lib.ABI_VERSION
     for name in ("lkg_l2_rank_rows", "lkg_rank_prepare_l2", "lkg_rank_finalize_l2", "lkg_rank_filter_l2"):
         assert name in _lib.SIGNATURES and hasattr(lib, name)
 

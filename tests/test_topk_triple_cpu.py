@@ -102,7 +102,7 @@ def _graph(att=FAKE):
 
 def test_abi_entry_points(lib):
     from literalkg_b200 import _lib
-    assert lib.lkg_abi_version() == 8 == _lib.ABI_VERSION
+    assert lib.lkg_abi_version() == 9 == _lib.ABI_VERSION
     for name in ("lkg_topk_threshold_l2", "lkg_topk_finalize_l2"):
         assert name in _lib.SIGNATURES and hasattr(lib, name)
 
